@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (our CUDA path)
     python bench.py --impl reference --gpus N --steps K ...  (the reference's CPU path, host cores)
+    python bench.py --steps K --dump-outputs DIR              (also writes what step K returned, for comparing builds)
 
 A "step" is one pass of the hot path over one batch (loci_per_step loci x 30 reads, BASELINE config 2
 distributions: "synthetic genome-wide catalog 1M loci x 30x HiFi reads, loci sharded across GPUs").  The
@@ -59,7 +60,34 @@ def parse_args():
                     help="--scaling strong: stream a partition in blocks of about 1/N of it (0 = the catalog's own blocks)")
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = the same number of blocks as --steps")
     ap.add_argument("--loci3", type=int, default=100_000, help="--config 3: loci in the config")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0: per-read counts, reference-window counts) "
+                         "to DIR/<name>.npy as float64; default workload only")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2 or args.scaling != "weak"):
+        ap.error("--dump-outputs: the default workload only (--impl ours --config 2 --scaling weak)")
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes every array of `arrays` (name -> 2-D array of int32 results) as out_dir/<name>.npy in float64, which
+    holds each int32 exactly.  Above `limit` bytes in all, each array keeps the same share of its rows: a sample drawn
+    by np.random.default_rng(0), sorted, so that it depends on the array shapes only and two builds run with the same
+    arguments write the same rows."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.shape[0] * a.shape[1] * 8 for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            keep = int(a.shape[0] * limit // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def workload_name(args):
@@ -665,6 +693,7 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     agg = {k: 0.0 for k in STAT_KEYS}
     agg_ref = {k: 0.0 for k in STAT_KEYS}
+    ref_out = None
     ev0.record()
     for k in range(args.steps):
         fut = ref_step_async(k) if ref_sets else None
@@ -673,13 +702,19 @@ def main():
         for key in agg:
             agg[key] += st[key]
         if fut:
-            st = fut.result()[1]
+            ref_out, st = fut.result()
             for key in agg_ref:
                 agg_ref[key] += st[key]
     ev1.record()
     barrier()
     elapsed_ms = reduce_max(ev0.elapsed_time(ev1))
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # the last step's batch still holds its results on the device: download them outside the timed region
+        outputs = {"read_counts": eng.download(dev_batches[(args.steps - 1) % args.pool])}
+        if ref_out is not None:
+            outputs["ref_counts"] = ref_out
+        dump_outputs(args.dump_outputs, outputs)
     total_reads = reduce_sum(float(reads_per_step) * args.steps)
     value = total_reads / (elapsed_ms * 1e-3)
     exec_cells = reduce_sum(agg["executed_cells"] + agg_ref["executed_cells"])

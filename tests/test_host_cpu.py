@@ -216,6 +216,33 @@ def test_bench_strong_scaling_line_is_json(monkeypatch):
     assert "workload" in d["config"]
 
 
+def test_bench_dump_outputs_exact_and_capped(monkeypatch, tmp_path):
+    """bench.py --dump-outputs: int32 results land as float64 without loss; above the size cap every array keeps the
+    same seeded sample of its rows, identical from call to call; the flag is refused outside the default workload."""
+    import importlib
+    import sys
+
+    bench = importlib.import_module("bench")
+    rng = np.random.default_rng(3)
+    reads = rng.integers(-2**31, 2**31 - 1, size=(3000, 4), dtype=np.int64).astype(np.int32)
+    ref = rng.integers(-2**31, 2**31 - 1, size=(100, 8), dtype=np.int64).astype(np.int32)
+    bench.dump_outputs(str(tmp_path / "full"), {"read_counts": reads, "ref_counts": ref})
+    for name, a in (("read_counts", reads), ("ref_counts", ref)):
+        got = np.load(tmp_path / "full" / f"{name}.npy")
+        assert got.dtype == np.float64 and np.array_equal(got.astype(np.int32), a)
+    limit = (3000 * 4 + 100 * 8) * 8 // 4
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"read_counts": reads, "ref_counts": ref}, limit=limit)
+    a, b = (np.load(tmp_path / d / "read_counts.npy") for d in ("a", "b"))
+    assert a.shape == (750, 4) and np.array_equal(a, b)
+    rows = {tuple(r) for r in reads.tolist()}
+    assert all(tuple(int(v) for v in row) in rows for row in a)
+    assert sum((tmp_path / "a" / f).stat().st_size - 128 for f in ("read_counts.npy", "ref_counts.npy")) <= limit
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--config", "3", "--dump-outputs", str(tmp_path / "x")])
+    with pytest.raises(SystemExit):
+        bench.parse_args()
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # host batcher: nibble arenas, compact slices, the C packing helper
 # ---------------------------------------------------------------------------------------------------------------

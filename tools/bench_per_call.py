@@ -1,4 +1,4 @@
-import sys, time; sys.path.insert(0, '/root/repo')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, strkit_b200
 rng = np.random.default_rng(1)
 def rs(n): return "".join(rng.choice(list("ACGT"), size=n))
