@@ -77,13 +77,65 @@ struct DevBuf {
     }
 };
 
+// Work items of a DP pass binned by rows-per-lane class (0 = general kernel only), with the per-class maxima the packed
+// launches size their tables by.
+struct ClassLists {
+    std::vector<int> items[STRK_PK_NBIN];
+    std::vector<int> flat;  // every list, class after class: the host source of one H2D copy
+    int mmax[STRK_PK_NBIN] = {0}, flank[STRK_PK_NBIN] = {0}, w_max[STRK_PK_NBIN] = {0};
+    void clear() {
+        for (int k = 0; k < STRK_PK_NBIN; ++k) items[k].clear(), mmax[k] = flank[k] = w_max[k] = 0;
+    }
+    void add(int k, int item) { items[k].push_back(item); }
+    void add(int k, int item, int m, int fl, int fr, int w = 0) {
+        items[k].push_back(item);
+        mmax[k] = std::max(mmax[k], m);
+        flank[k] = std::max(flank[k], std::max(fl, fr));
+        w_max[k] = std::max(w_max[k], w);
+    }
+    // Queues the copy of the lists into `buf` on `st` and points seg_list / seg_cnt (launch_pass) at the device
+    // segments.  `flat` is read by the copy until `st` has passed it.
+    int upload(DevBuf<int> &buf, cudaStream_t st, const int **seg_list, long long *seg_cnt) {
+        size_t at[STRK_PK_NBIN];
+        flat.clear();
+        for (int k = 0; k < STRK_PK_NBIN; ++k) {
+            at[k] = flat.size();
+            flat.insert(flat.end(), items[k].begin(), items[k].end());
+        }
+        if (buf.reserve(flat.size()) != cudaSuccess) {
+            cudaGetLastError();
+            return set_err(STRK_ERR_NOMEM, "cannot allocate the class lists of a pass");
+        }
+        CU(cudaMemcpyAsync(buf.p, flat.data(), flat.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_list[k] = buf.p + at[k], seg_cnt[k] = (long long)items[k].size();
+        return STRK_OK;
+    }
+};
+
+// The reference path's per-locus state (strk_ref_counts), recycled across calls
+struct RefBufs {
+    DevBuf<unsigned char> arena;
+    DevBuf<unsigned long long> seq_off, motif_off;
+    DevBuf<int> lens, start, ref_size, rc, motif_len;  // the caller's arrays
+    DevBuf<int> wd;                                    // half-width of each locus' first boundary window
+    DevBuf<int> l_off, r_off, n_off;                   // phase 1 results
+    DevBuf<int> ids_a, ids_b;                          // locus lists: pending loci of phase 1, the loci of a tier
+    DevBuf<int> lists;                                 // class lists of a packed pass
+    DevBuf<unsigned int> cnt;                          // counters of ref_replay1_kernel: [0, 4) a pass, [4, 8) a second look
+    DevBuf<int> out;                                   // fast path: the results, assembled on the device
+    // host sources of asynchronous copies: alive until the stream has passed them (the fast path synchronises once)
+    std::vector<int> h_wd;
+    ClassLists classes;
+    void release() {
+        arena.release(), seq_off.release(), motif_off.release(), lens.release(), start.release(), ref_size.release();
+        rc.release(), motif_len.release(), wd.release(), l_off.release(), r_off.release(), n_off.release();
+        ids_a.release(), ids_b.release(), lists.release(), cnt.release(), out.release();
+    }
+};
+
 struct strk_ctx {
     int device = 0;
     int n_sm = 0;
-    size_t l2_persist_max = 0, l2_window_max = 0;  // L2 set-aside for the capture scratch (see launch_packed_r)
-    const void *l2_window_ptr = nullptr;
-    size_t l2_window_bytes = 0;
-    cudaStream_t l2_window_stream = nullptr;
     // small passes: one side stream per rows-per-lane class, so the class launches (each under one wave) overlap
     cudaStream_t side[STRK_PK_NBIN] = {nullptr};
     cudaEvent_t side_ev[STRK_PK_NBIN] = {nullptr};
@@ -108,13 +160,9 @@ struct strk_ctx {
     DevBuf<uint4> pk_scratch;        // captured DP columns of the packed kernel (per resident warp)
     DevBuf<double> al_rep[3];        // allele calling: replicate means / weights / stdevs of one chunk of loci
     DevBuf<unsigned char> al_peaks;  //                 replicate peak counts
-    // reference path (strk_ref_counts): per-locus arrays, pending lists, and the one-read-per-locus batch of phase 2
-    DevBuf<unsigned char> ref_arena;
-    DevBuf<unsigned long long> ref_u64[2];
-    DevBuf<int> ref_i[13];
+    // reference path (strk_ref_counts): per-locus state, and the one-read-per-locus batch of phase 2
+    RefBufs ref;
     struct strk_batch *ref_batch = nullptr;
-    std::vector<int> ref_flat, ref_hwd;  // host sources of asynchronous copies of the reference path's fast path
-    DevBuf<int> ref_out;                 // its results, assembled on the device
     DevBuf<int> al_i[8];             //                 per-read / per-locus integer arrays (recycled across calls)
     DevBuf<double> al_d[3];
     DevBuf<long long> al_rb;
@@ -201,11 +249,6 @@ extern "C" int strk_init(int device, const int8_t matrix[STRK_NSYM * STRK_NSYM],
     }
     if (device < 0 || device >= n_dev) return set_err(STRK_ERR_ARG, "device %d out of range (%d devices)", device, n_dev);
     CU(cudaSetDevice(device));
-    // STRK_BLOCKING_SYNC=1: host threads sleep in stream synchronisation instead of spinning (for boxes with fewer
-    // host cores than ranks x host threads; the streamed path keeps three host threads per GPU busy otherwise)
-    if (getenv("STRK_BLOCKING_SYNC")) {
-        if (cudaSetDeviceFlags(cudaDeviceScheduleBlockingSync) != cudaSuccess) cudaGetLastError();
-    }
     strk_ctx *ctx = new (std::nothrow) strk_ctx();
     if (!ctx) return set_err(STRK_ERR_NOMEM, "out of host memory");
     // any failure below releases what has been created so far (strk_destroy copes with a half-built context)
@@ -219,15 +262,6 @@ extern "C" int strk_init(int device, const int8_t matrix[STRK_NSYM * STRK_NSYM],
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
     ctx->n_sm = prop.multiProcessorCount;
-    ctx->l2_persist_max = (size_t)prop.persistingL2CacheMaxSize;
-    ctx->l2_window_max = (size_t)prop.accessPolicyMaxWindowSize;
-    // L2 set-aside for persisting lines (the packed kernel's capture scratch): a device-wide limit, set once here
-    if (ctx->l2_persist_max && getenv("STRK_L2_WINDOW")) {
-        if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, ctx->l2_persist_max) != cudaSuccess) {
-            cudaGetLastError();
-            ctx->l2_persist_max = 0;
-        }
-    }
     ctx->gap = gap_open;
     ctx->end_flags = end_flags;
     ctx->tie_flags = tie_flags;
@@ -290,7 +324,6 @@ extern "C" int strk_init(int device, const int8_t matrix[STRK_NSYM * STRK_NSYM],
     {
         int lo = 0, hi = 0;
         CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));  // lo = least, hi = greatest (numerically smaller)
-        if (getenv("STRK_NO_PRIORITY")) hi = lo;          // (measurement only: every stream at the default priority)
         ctx->prio_hi = hi;
         CU(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, hi));
         CU(cudaStreamCreateWithPriority(&ctx->fill_stream, cudaStreamNonBlocking, lo));
@@ -327,10 +360,7 @@ extern "C" int strk_destroy(strk_ctx *ctx) {
     ctx->reuse = nullptr;
     if (ctx->ref_batch) strk_batch_free(ctx, ctx->ref_batch);
     ctx->ref_batch = nullptr;
-    ctx->ref_arena.release();
-    ctx->ref_out.release();
-    for (int k = 0; k < 2; ++k) ctx->ref_u64[k].release();
-    for (int k = 0; k < 13; ++k) ctx->ref_i[k].release();
+    ctx->ref.release();
     ctx->scratch.release();
     ctx->fams.release();
     ctx->table.release();
@@ -497,8 +527,7 @@ static int launch_packed_r(strk_ctx *ctx, const FamDesc *fams, const int *list, 
     // plan_scratch != nullptr: only report the capture scratch (uint4 units) this launch needs.
     // scratch_off >= 0: the launch uses pk_scratch + scratch_off, reserved by the caller (concurrent class launches).
     constexpr int HALVES = 32 / L;
-    size_t smem = pk_smem_bytes(R, dims, L);
-    if (const char *env = getenv("STRK_PK_EXTRA_SMEM")) smem += (size_t)atoi(env);  // occupancy experiments only
+    const size_t smem = pk_smem_bytes(R, dims, L);
     // the opt-in shared-memory size is a per-device attribute of the function, shared by every context of the
     // process on that device (the streamed path keeps two): only ever raised, under a lock
     {
@@ -526,31 +555,11 @@ static int launch_packed_r(strk_ctx *ctx, const FamDesc *fams, const int *list, 
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "cannot allocate %zu bytes of capture scratch", words * 4);
     }
-    // The capture scratch is written and read back within one read's lifetime and then overwritten by the next
-    // read of the same warp.  STRK_L2_WINDOW=1 keeps it resident in L2 (persisting access window) so that it is not
-    // written back to HBM on eviction: measured 1176 -> 89 MB of DRAM traffic per launch of the R = 10 class, no
-    // change in kernel time (the kernel is integer-issue bound, the write-backs use ~10 % of HBM bandwidth), -2 % on
-    // the streamed path where two contexts' windows compete for the set-aside.  Off by default for that reason.
-    {
-        const size_t bytes = ctx->pk_scratch.cap * sizeof(uint4);  // the whole buffer: set again only when it moves
-        static const bool off = getenv("STRK_L2_WINDOW") == nullptr;
-        if (!off && scratch_off < 0 && ctx->l2_persist_max && ctx->l2_window_max &&
-            (ctx->l2_window_ptr != ctx->pk_scratch.p || ctx->l2_window_bytes != bytes || ctx->l2_window_stream != st)) {
-            const size_t win = bytes < ctx->l2_window_max ? bytes : ctx->l2_window_max;
-            const size_t carve = win < ctx->l2_persist_max ? win : ctx->l2_persist_max;
-            cudaStreamAttrValue attr;
-            memset(&attr, 0, sizeof(attr));
-            attr.accessPolicyWindow.base_ptr = (void *)ctx->pk_scratch.p;
-            attr.accessPolicyWindow.num_bytes = win;
-            attr.accessPolicyWindow.hitRatio = win ? (float)((double)carve / (double)win) : 0.f;
-            attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-            if (cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &attr) != cudaSuccess) cudaGetLastError();
-            ctx->l2_window_ptr = ctx->pk_scratch.p;
-            ctx->l2_window_bytes = bytes;
-            ctx->l2_window_stream = st;
-        }
-    }
+    // The capture scratch is written and read back within one read's lifetime and then overwritten by the next read of
+    // the same warp.  Keeping it resident in L2 (persisting access window) was measured: 1176 -> 89 MB of DRAM traffic
+    // per launch of the R = 10 class, no change in kernel time (the kernel is integer-issue bound, the write-backs use
+    // ~10 % of HBM bandwidth), -2 % on the streamed path where two contexts' windows compete for the set-aside: it is
+    // not pinned (DESIGN.md 5.1).
     unsigned int *work_counter = ctx->d_queue + 8 + (L == 16 ? R / 2 : R);  // one queue per rows-per-lane class
     CU(cudaMemsetAsync(work_counter, 0, sizeof(unsigned int), st));
     dp_packed_kernel<R, L><<<(unsigned)grid, pk_warps(L) * 32, smem, st>>>(fams, list, n, arena, ctx->d_consts, table, dims,
@@ -689,7 +698,7 @@ static int launch_packed_classes(strk_ctx *ctx, const int *const *list, const lo
 static int launch_pass(strk_ctx *ctx, const int *const *list, const long long *cnt, const int *flank, const int *mmax,
                        const int *w_max, long long n_slots, const FamDesc *fams, const unsigned char *arena, void *table,
                        int b_len, int rowlen, cudaStream_t st, int ref_mode, long long *n_packed) {
-    bool overlap = cnt[0] > 0 && getenv("STRK_GENERAL_SERIAL") == nullptr;  // (the switch: measurement only)
+    bool overlap = cnt[0] > 0;
     long long packed_total = 0;
     for (int k = 1; k < STRK_PK_NBIN; ++k) {
         if (!cnt[k]) continue;
@@ -738,12 +747,29 @@ static int launch_pass(strk_ctx *ctx, const int *const *list, const long long *c
 // ------------------------------------------------------------------------------------------------
 // batches
 // ------------------------------------------------------------------------------------------------
-template <typename T>
-static cudaError_t upload(DevBuf<T> &buf, T **dst, const T *src, size_t n, cudaStream_t st) {
-    cudaError_t e = buf.reserve(n ? n : 1);
-    if (e != cudaSuccess) return e;
-    *dst = buf.p;
-    if (n) e = cudaMemcpyAsync(buf.p, src, n * sizeof(T), cudaMemcpyHostToDevice, st);
+// Reserves the per-read and per-locus buffers of `b` for n_reads reads of n_loci loci, points the d_* aliases at them
+// and clears the work plan (batch_plan / batch_plan_host fill it in).  The arena is the caller's to set.
+static cudaError_t batch_bind(strk_batch *b, long long n_reads, long long n_loci) {
+    const size_t nr = (size_t)(n_reads ? n_reads : 1), nl = (size_t)(n_loci ? n_loci : 1);
+    cudaError_t e = b->seq_off.reserve(nr);
+    if (e == cudaSuccess) e = b->lens.reserve(3 * nr);
+    if (e == cudaSuccess) e = b->est.reserve(nr);
+    if (e == cudaSuccess) e = b->read_locus.reserve(nr);
+    if (e == cudaSuccess) e = b->order.reserve(nr);
+    if (e == cudaSuccess) e = b->bin.reserve(nr);
+    if (e == cudaSuccess) e = b->out.reserve(4 * nr);
+    if (e == cudaSuccess) e = b->read_begin.reserve((size_t)n_loci + 1);
+    if (e == cudaSuccess) e = b->motif_off.reserve(nl);
+    if (e == cudaSuccess) e = b->motif_len.reserve(nl);
+    if (e == cudaSuccess) e = b->status.reserve(nl);
+    b->n_reads = n_reads;
+    b->n_loci = n_loci;
+    b->d_seq_off = b->seq_off.p, b->d_lens = b->lens.p, b->d_est = b->est.p, b->d_read_locus = b->read_locus.p;
+    b->d_order = b->order.p, b->d_out = b->out.p, b->d_read_begin = b->read_begin.p;
+    b->d_motif_off = b->motif_off.p, b->d_motif_len = b->motif_len.p, b->d_status = b->status.p;
+    b->n_general = 0;
+    for (int k = 0; k < STRK_PK_NBIN; ++k) b->bin_off[k] = b->bin_cnt[k] = 0, b->bin_mmax[k] = b->bin_flank[k] = 0;
+    b->max_n1 = b->mb_cols_base = b->mb_m = 0;
     return e;
 }
 
@@ -753,6 +779,17 @@ extern "C" int strk_batch_free(strk_ctx *ctx, strk_batch *b) {
     b->release();
     delete b;
     return STRK_OK;
+}
+
+// The error of a batch whose planning found one: first_error = (index << 8) | kind of the first (PlanError)
+static int plan_error(unsigned long long first_error) {
+    static const char *what[] = {"", "has a negative length", "is empty (fl + tr + fr has no bases)", "is too long",
+                                 "runs past the end of the arena", "has an out-of-range est_cn", "has an empty motif",
+                                 "has a motif that runs past the end of the arena", "has a non-monotone read_begin"};
+    const long long idx = (long long)(first_error >> 8);
+    const int kind = (int)(first_error & 0xff);
+    return set_err(STRK_ERR_ARG, "batch: %s %lld %s", kind >= PLAN_ERR_MOTIF_EMPTY ? "locus" : "read", idx,
+                   what[kind <= 8 ? kind : 0]);
 }
 
 // Validation + work planning of a batch whose arrays are already on the device (b->d_*, n_reads, n_loci set).
@@ -801,15 +838,7 @@ static int batch_plan(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes) {
         CU(cudaMemcpyAsync(&hp, ctx->d_plan, sizeof(PlanStats), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
     }
-    if (hp.first_error != ~0ull) {
-        const long long idx = (long long)(hp.first_error >> 8);
-        static const char *what[] = {"", "has a negative length", "is empty (fl + tr + fr has no bases)", "is too long",
-                                     "runs past the end of the arena", "has an out-of-range est_cn", "has an empty motif",
-                                     "has a motif that runs past the end of the arena", "has a non-monotone read_begin"};
-        const int kind = (int)(hp.first_error & 0xff);
-        return set_err(STRK_ERR_ARG, "batch: %s %lld %s", kind >= PLAN_ERR_MOTIF_EMPTY ? "locus" : "read", idx,
-                       what[kind <= 8 ? kind : 0]);
-    }
+    if (hp.first_error != ~0ull) return plan_error(hp.first_error);
     // segment offsets: general first, then packed classes from R = 16 down to 2 (class 1 stays empty)
     unsigned off[STRK_PK_NBIN];
     unsigned acc = hp.bin_cnt[0];
@@ -849,9 +878,6 @@ static int batch_plan_host(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes, c
         CU(cudaStreamSynchronize(st));
         return STRK_OK;
     }
-    static const char *what[] = {"", "has a negative length", "is empty (fl + tr + fr has no bases)", "is too long",
-                                 "runs past the end of the arena", "has an out-of-range est_cn", "has an empty motif",
-                                 "has a motif that runs past the end of the arena", "has a non-monotone read_begin"};
     std::vector<int> read_locus((size_t)n_reads, 0), order((size_t)n_reads);
     std::vector<unsigned char> bin((size_t)n_reads, 0);
     unsigned long long first_error = ~0ull;
@@ -891,9 +917,7 @@ static int batch_plan_host(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes, c
                 report(r, PLAN_ERR_EST);
             else {
                 const int m = motif_len[read_locus[(size_t)r]];
-                int R = ctx->h_consts.packed_ok ? strk_pick_rows_packed((int)n1 + 1) : 0;
-                if (fl < 1 || fr < 1 || fl > PK_FLANK_MAX || fr > PK_FLANK_MAX || m * R > 128 || m <= 0) R = 0;
-                bb = R;
+                bb = ctx->h_consts.packed_ok ? strk_pk_class(fl, tr, fr, m) : 0;
                 b->max_n1 = std::max(b->max_n1, (int)n1);
                 if (bb) {
                     b->bin_mmax[bb] = std::max(b->bin_mmax[bb], m);
@@ -908,12 +932,7 @@ static int batch_plan_host(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes, c
             ++cnt[bb];
         }
     }
-    if (first_error != ~0ull) {
-        const long long idx = (long long)(first_error >> 8);
-        const int kind = (int)(first_error & 0xff);
-        return set_err(STRK_ERR_ARG, "batch: %s %lld %s", kind >= PLAN_ERR_MOTIF_EMPTY ? "locus" : "read", idx,
-                       what[kind <= 8 ? kind : 0]);
-    }
+    if (first_error != ~0ull) return plan_error(first_error);
     // segment offsets: general first, then packed classes from R = 16 down to 2 (as batch_plan)
     long long off[STRK_PK_NBIN], acc = cnt[0];
     off[0] = 0;
@@ -949,21 +968,16 @@ static int batch_fill(strk_ctx *ctx, strk_batch *b, const uint8_t *arena, uint64
     if (read_begin[0] != 0 || read_begin[n_loci] != n_reads)
         return set_err(STRK_ERR_ARG, "batch: read_begin must run from 0 to n_reads");
     CU(cudaSetDevice(ctx->device));
-    b->n_reads = n_reads;
-    b->n_loci = n_loci;
     b->h_read_begin.assign(read_begin, read_begin + n_loci + 1);
-    b->n_general = 0;
-    for (int k = 0; k < STRK_PK_NBIN; ++k) b->bin_off[k] = b->bin_cnt[k] = 0, b->bin_mmax[k] = b->bin_flank[k] = 0;
-    b->max_n1 = b->mb_cols_base = b->mb_m = 0;
 
     cudaStream_t st = ctx->fill_stream;
-    cudaError_t e = cudaSuccess;
-#define UP(buf, dst, src, n) \
-    if (e == cudaSuccess) e = upload(b->buf, &b->dst, src, (size_t)(n), st)
+    cudaError_t e = batch_bind(b, n_reads, n_loci);
+#define UP(dst, src, n) \
+    if (e == cudaSuccess && (n)) e = cudaMemcpyAsync(b->dst, src, (size_t)(n) * sizeof(*b->dst), cudaMemcpyHostToDevice, st)
     if (arena_format == STRK_ARENA_NIBBLE) {
         // packed bytes in, byte-per-symbol arena out (offsets and lengths are in symbols either way)
         const size_t quads = (size_t)((arena_bytes + 15) / 16);
-        e = b->arena4.reserve(quads ? quads : 1);
+        if (e == cudaSuccess) e = b->arena4.reserve(quads ? quads : 1);
         if (e == cudaSuccess) e = b->arena.reserve((size_t)(arena_bytes ? 2 * arena_bytes : 1));
         b->d_arena = b->arena.p;
         if (e == cudaSuccess && arena_bytes) {
@@ -976,25 +990,17 @@ static int batch_fill(strk_ctx *ctx, strk_batch *b, const uint8_t *arena, uint64
         }
         arena_bytes *= 2;  // symbols
     } else {
-        UP(arena, d_arena, (const unsigned char *)arena, arena_bytes);
+        if (e == cudaSuccess) e = b->arena.reserve((size_t)(arena_bytes ? arena_bytes : 1));
+        b->d_arena = b->arena.p;
+        UP(d_arena, arena, arena_bytes);
     }
-    UP(seq_off, d_seq_off, (const unsigned long long *)seq_off, n_reads);
-    UP(lens, d_lens, (const int *)lens, 3 * n_reads);
-    UP(est, d_est, (const int *)est_cn, n_reads);
-    UP(read_begin, d_read_begin, (const long long *)read_begin, n_loci + 1);
-    UP(motif_off, d_motif_off, (const unsigned long long *)motif_off, n_loci);
-    UP(motif_len, d_motif_len, (const int *)motif_len, n_loci);
+    UP(d_seq_off, seq_off, n_reads);
+    UP(d_lens, lens, 3 * n_reads);
+    UP(d_est, est_cn, n_reads);
+    UP(d_read_begin, read_begin, n_loci + 1);
+    UP(d_motif_off, motif_off, n_loci);
+    UP(d_motif_len, motif_len, n_loci);
 #undef UP
-    const size_t nr = (size_t)(n_reads ? n_reads : 1);
-    if (e == cudaSuccess) e = b->read_locus.reserve(nr);
-    if (e == cudaSuccess) e = b->order.reserve(nr);
-    if (e == cudaSuccess) e = b->bin.reserve(nr);
-    if (e == cudaSuccess) e = b->out.reserve(nr * 4);
-    if (e == cudaSuccess) e = b->status.reserve((size_t)(n_loci ? n_loci : 1));
-    b->d_read_locus = b->read_locus.p;
-    b->d_order = b->order.p;
-    b->d_out = b->out.p;
-    b->d_status = b->status.p;
     if (e != cudaSuccess) {
         cudaGetLastError();
         return set_err(e == cudaErrorMemoryAllocation ? STRK_ERR_NOMEM : STRK_ERR_CUDA, "batch upload: %s",
@@ -1053,6 +1059,25 @@ static void scratch_dims(const strk_batch *b, int wd, int *b_len, int *rowlen) {
     *rowlen = b->max_n1 > 32 * 16 ? b->mb_cols_base + b->mb_m * wd + 2 : 2;
 }
 
+// Replay of a pass over ctx->table (W sizes per slot), one thread per locus of `b` or of d_locus_ids; narrow windows
+// take the kernel that keeps each read's row in shared memory.  The caller counts the launch.
+static int launch_replay(strk_ctx *ctx, const strk_batch *b, int W, int wd, int ws, const int *d_locus_ids,
+                         const long long *d_slot_begin, long long n_list, int max_iters, int range, int step,
+                         const int *d_rep, double *d_hint, cudaStream_t st) {
+    if (W <= REPLAY_WMAX)
+        replay_reads_small_kernel<<<(unsigned)((n_list + REPLAY_THREADS - 1) / REPLAY_THREADS), REPLAY_THREADS, 0, st>>>(
+            ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
+            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->d_queue + 1, ctx->d_acc,
+            d_rep, d_hint);
+    else
+        replay_reads_kernel<<<(unsigned)((n_list + 127) / 128), 128, 0, st>>>(
+            ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
+            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->d_queue + 1, ctx->d_acc,
+            d_rep, d_hint);
+    CU(cudaGetLastError());
+    return STRK_OK;
+}
+
 extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int local_search_range, int step_size,
                               int kernel, void *stream) {
     if (!ctx || !b) return set_err(STRK_ERR_ARG, "strk_batch_run: null argument");
@@ -1085,7 +1110,6 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
     std::vector<int> h_read_ids, h_locus_ids;
     std::vector<long long> h_slot_begin;
     std::vector<unsigned char> h_status, h_bin;
-    std::vector<int> h_class_lists;
     float ms_dp = 0.f, ms_replay = 0.f;
     double acc[2] = {0, 0};  // [0] reference-equivalent cells, [1] executed cells
 
@@ -1158,7 +1182,6 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
                     CU(cudaMemcpyAsync(h_bin.data(), b->bin.p, (size_t)b->n_reads, cudaMemcpyDeviceToHost, st));
                     CU(cudaStreamSynchronize(st));
                 }
-                std::vector<int> by_class[STRK_PK_NBIN];
                 // A small pass is launch-latency bound (one read's sweep is ~100 us whatever the grid): its reads run
                 // in the largest class of their lane group (pad rows cost nothing there), two launches instead of 15.
                 int merged[STRK_PK_NBIN];
@@ -1178,22 +1201,11 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
                             }
                     }
                 }
-                for (size_t sl = 0; sl < h_read_ids.size(); ++sl)
-                    by_class[merged[h_bin[(size_t)h_read_ids[sl]]]].push_back((int)sl);
-                h_class_lists.clear();
-                size_t at[STRK_PK_NBIN];
-                for (int k = 0; k < STRK_PK_NBIN; ++k) {
-                    at[k] = h_class_lists.size();
-                    h_class_lists.insert(h_class_lists.end(), by_class[k].begin(), by_class[k].end());
-                }
-                if (ctx->list_d.reserve(h_class_lists.size()) != cudaSuccess) {
-                    cudaGetLastError();
-                    return set_err(STRK_ERR_NOMEM, "cannot allocate widening lists");
-                }
-                CU(cudaMemcpyAsync(ctx->list_d.p, h_class_lists.data(), h_class_lists.size() * sizeof(int),
-                                   cudaMemcpyHostToDevice, st));
-                CU(cudaStreamSynchronize(st));  // h_class_lists is reused by the next pass
-                for (int k = 0; k < STRK_PK_NBIN; ++k) seg_list[k] = ctx->list_d.p + at[k], seg_cnt[k] = (long long)by_class[k].size();
+                ClassLists lists;
+                for (size_t sl = 0; sl < h_read_ids.size(); ++sl) lists.add(merged[h_bin[(size_t)h_read_ids[sl]]], (int)sl);
+                rc = lists.upload(ctx->list_d, st, seg_list, seg_cnt);
+                if (rc) return rc;
+                CU(cudaStreamSynchronize(st));  // `lists` is read by the copy
             }
             CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
             int seg_w[STRK_PK_NBIN];
@@ -1205,17 +1217,9 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
         CU(cudaEventRecord(ctx->ev[1], st));
         CU(cudaMemsetAsync(ctx->d_queue + 1, 0, sizeof(unsigned int), st));
         CU(cudaMemsetAsync(ctx->d_queue + 3, 0, sizeof(unsigned int), st));
-        if (W <= REPLAY_WMAX)
-            replay_reads_small_kernel<<<(unsigned)((n_list + REPLAY_THREADS - 1) / REPLAY_THREADS), REPLAY_THREADS, 0, st>>>(
-                ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
-                b->d_motif_len, max_iters, local_search_range, step_size, ctx->tie_flags, b->d_out, b->d_status,
-                ctx->d_queue + 1, ctx->d_acc, pass == 0 ? b->d_rep : nullptr, b->hint.p);
-        else
-            replay_reads_kernel<<<(unsigned)((n_list + 127) / 128), 128, 0, st>>>(
-                ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
-                b->d_motif_len, max_iters, local_search_range, step_size, ctx->tie_flags, b->d_out, b->d_status,
-                ctx->d_queue + 1, ctx->d_acc, pass == 0 ? b->d_rep : nullptr, b->hint.p);
-        CU(cudaGetLastError());
+        rc = launch_replay(ctx, b, W, wd, ws, d_locus_ids, d_slot_begin, n_list, max_iters, local_search_range, step_size,
+                           pass == 0 ? b->d_rep : nullptr, b->hint.p, st);
+        if (rc) return rc;
         ctx->stats[2] += 1;
         CU(cudaEventRecord(ctx->ev[2], st));
         // [0] loci whose search left the window, [1] packed-kernel fallbacks, [2] loci saved by the wide_short margin
@@ -1440,53 +1444,28 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
         if (rc) return rc;
     } else {
         // same routing as strk_batch_run: packed kernel per R, the rest (and its fallbacks) to the general kernel
-        std::vector<int> lists[STRK_PK_NBIN];
-        int mmax[STRK_PK_NBIN] = {0}, flank[STRK_PK_NBIN] = {0}, wmax[STRK_PK_NBIN] = {0};
+        ClassLists lists;
         for (int64_t r = 0; r < n_reads; ++r) {
             const FamDesc &f = fams[(size_t)r];
-            int R = strk_pick_rows_packed(f.n_fl + f.n_tr + f.n_fr + 1);
-            if (f.n_fl < 1 || f.n_fr < 1 || f.n_fl > PK_FLANK_MAX || f.n_fr > PK_FLANK_MAX || f.m * R > 128 ||
-                f.n_hi - f.n_lo + 1 > 64)
-                R = 0;
-            lists[R].push_back((int)r);
-            mmax[R] = std::max(mmax[R], f.m);
-            flank[R] = std::max(flank[R], std::max(f.n_fl, f.n_fr));
-            wmax[R] = std::max(wmax[R], f.n_hi - f.n_lo + 1);
+            const int w = f.n_hi - f.n_lo + 1;
+            lists.add(w > 64 ? 0 : strk_pk_class(f.n_fl, f.n_tr, f.n_fr, f.m), (int)r, f.m, f.n_fl, f.n_fr, w);
         }
-        std::vector<int> flat;
-        size_t offs[STRK_PK_NBIN];
-        for (int k = 0; k < STRK_PK_NBIN; ++k) {
-            offs[k] = flat.size();
-            flat.insert(flat.end(), lists[k].begin(), lists[k].end());
+        if (ctx->fallback.reserve((size_t)n_reads) != cudaSuccess) {
+            cudaGetLastError();
+            return set_err(STRK_ERR_NOMEM, "%s: cannot allocate the fallback list", who);
         }
-        int *d_lists = nullptr;
-        e = tmp.up(&d_lists, flat.data(), flat.size());
-        if (e == cudaSuccess) e = ctx->fallback.reserve((size_t)n_reads);
-        int *d_fb = ctx->fallback.p;
-        if (e != cudaSuccess) return set_err(STRK_ERR_NOMEM, "%s: %s", who, cudaGetErrorString(e));
+        const int *seg_list[STRK_PK_NBIN];
+        long long seg_cnt[STRK_PK_NBIN];
+        int seg_w[STRK_PK_NBIN];
+        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w[k] = (lists.w_max[k] + 3) / 4 * 4;
+        rc = lists.upload(ctx->list_d, ctx->stream, seg_list, seg_cnt);
+        if (rc) return rc;
         CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), ctx->stream));
         long long n_packed = 0;
-        for (int k = STRK_PK_RMAX; k >= 1; --k) {
-            if (lists[k].empty()) continue;
-            const PackedDims dims = pk_dims_for_class(k, flank[k], mmax[k], (wmax[k] + 3) / 4 * 4);
-            if (pk_smem_for_class(k, dims) > 200 * 1024) {
-                rc = launch_general(ctx, false, d_fams, d_lists + offs[k], (long long)lists[k].size(), d_arena, d_table,
-                                    b_len, rowlen, ctx->stream);
-                if (rc) return rc;
-                continue;
-            }
-            rc = launch_packed(ctx, k, d_fams, d_lists + offs[k], (int)lists[k].size(), d_arena, (int *)d_table, dims,
-                               ctx->stream);
-            if (rc) return rc;
-            n_packed += (long long)lists[k].size();
-        }
-        rc = launch_general(ctx, false, d_fams, d_lists + offs[0], (long long)lists[0].size(), d_arena, d_table, b_len,
-                            rowlen, ctx->stream);
+        rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w, n_reads, d_fams, d_arena, d_table, b_len,
+                         rowlen, ctx->stream, 0, &n_packed);
         if (rc) return rc;
         if (n_packed) {
-            rc = launch_general(ctx, false, d_fams, d_fb, n_packed, d_arena, d_table, b_len, rowlen, ctx->stream,
-                                ctx->d_queue + 2);
-            if (rc) return rc;
             unsigned int fb = 0;
             CU(cudaMemcpyAsync(&fb, ctx->d_queue + 2, sizeof(unsigned int), cudaMemcpyDeviceToHost, ctx->stream));
             CU(cudaStreamSynchronize(ctx->stream));
@@ -1532,44 +1511,6 @@ extern "C" int strk_ref_boundary_tables(strk_ctx *ctx, const uint8_t *arena, uin
                                         const int32_t *motif_len, const uint64_t *out_off, int32_t *out) {
     return tables_common(ctx, true, arena, arena_bytes, seq_off, lens, nullptr, n_lo, n_hi, n_loci, motif_off, motif_len,
                          n_loci, out_off, STRK_KERNEL_GENERAL, out);
-}
-
-// One DP pass over `fams` (general kernel) and download of the raw table (int scores, or packed argmax keys).
-template <typename T>
-static int dp_tables_to_host(strk_ctx *ctx, bool ref, const std::vector<FamDesc> &fams, const unsigned char *d_arena,
-                             size_t total_elems, std::vector<T> &host_table) {
-    int b_len = 2, rowlen = 2;
-    for (const FamDesc &f : fams) {
-        const int n1 = f.n_fl + f.n_tr + f.n_fr;
-        b_len = std::max(b_len, n1 + 2);
-        if (n1 > 32 * 16) rowlen = std::max(rowlen, std::max(f.n_fl, f.n_fr) + f.m * f.n_hi + 2);
-    }
-    if (ctx->fams.reserve(fams.size()) != cudaSuccess) {
-        cudaGetLastError();
-        return set_err(STRK_ERR_NOMEM, "cannot allocate family descriptors");
-    }
-    void *d_table = nullptr;
-    if (ref) {
-        if (ctx->table64.reserve(total_elems) != cudaSuccess) {
-            cudaGetLastError();
-            return set_err(STRK_ERR_NOMEM, "cannot allocate the boundary table");
-        }
-        d_table = ctx->table64.p;
-    } else {
-        if (ctx->table.reserve(total_elems) != cudaSuccess) {
-            cudaGetLastError();
-            return set_err(STRK_ERR_NOMEM, "cannot allocate the score table");
-        }
-        d_table = ctx->table.p;
-    }
-    CU(cudaMemcpyAsync(ctx->fams.p, fams.data(), fams.size() * sizeof(FamDesc), cudaMemcpyHostToDevice, ctx->stream));
-    int rc = launch_general(ctx, ref, ctx->fams.p, nullptr, (long long)fams.size(), d_arena, d_table, b_len, rowlen,
-                            ctx->stream);
-    if (rc) return rc;
-    host_table.resize(total_elems);
-    CU(cudaMemcpyAsync(host_table.data(), d_table, total_elems * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return STRK_OK;
 }
 
 // get_ref_repeat_count (repeats.py:73-192) for a batch of loci, device-resident from upload to results.
@@ -1634,29 +1575,81 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     return STRK_OK;
 }
 
+// First window of the boundary search: start +- max(6, range + step + 2) sizes, like the read path's (a search that
+// starts where it ends touches start +- (range + step)); one that leaves it is redone 4x wider.  Measured on 32 768
+// HiFi-sized windows: +- 9 sizes 3.89 ms, +- 7 3.79 ms, +- 6 3.33 ms per block.  STRK_REF_WD=<n> raises the floor of 6
+// (tuning only).
+static int ref_first_wd(int range, int step) {
+    static const int wd_env = getenv("STRK_REF_WD") ? atoi(getenv("STRK_REF_WD")) : 6;
+    return std::max(wd_env > 0 ? wd_env : 6, range + step + 2);
+}
+
+// The steps both drivers of strk_ref_counts start with: argument checks, the first boundary window of every locus
+// (ctx->ref.h_wd), the context's reference buffers, and the upload of the inputs with phase 1's results cleared, queued
+// on `st`.
+static int ref_setup(strk_ctx *ctx, cudaStream_t st, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
+                     const int32_t *lens, const int32_t *start_count, const int32_t *ref_size, const int32_t *rc_params,
+                     int64_t n_loci, const uint64_t *motif_off, const int32_t *motif_len) {
+    int rc = validate_reads("strk_ref_counts", arena_bytes, seq_off, lens, n_loci);
+    if (rc) return rc;
+    rc = validate_motifs("strk_ref_counts", arena_bytes, motif_off, motif_len, n_loci);
+    if (rc) return rc;
+    RefBufs &d = ctx->ref;
+    const size_t n = (size_t)n_loci;
+    d.h_wd.resize(n);
+    for (size_t l = 0; l < n; ++l) {
+        if (start_count[l] < 0 || start_count[l] > (1 << 22) ||
+            (long long)motif_len[l] * (long long)start_count[l] > (1ll << 24) || rc_params[3 * l] < 0 || rc_params[3 * l + 1] < 0 ||
+            rc_params[3 * l + 2] < 0 || rc_params[3 * l + 1] > 1000 || rc_params[3 * l + 2] > 1000)
+            return set_err(STRK_ERR_ARG, "strk_ref_counts: bad start count / search parameters for locus %lld", (long long)l);
+        d.h_wd[l] = ref_first_wd(rc_params[3 * l + 1], rc_params[3 * l + 2]);
+    }
+    CU(cudaSetDevice(ctx->device));
+    for (int k = 0; k < 8; ++k) ctx->stats[k] = 0;
+    cudaError_t e = d.arena.reserve((size_t)arena_bytes);
+    if (e == cudaSuccess) e = d.seq_off.reserve(n);
+    if (e == cudaSuccess) e = d.motif_off.reserve(n);
+    for (DevBuf<int> *p : {&d.lens, &d.rc})
+        if (e == cudaSuccess) e = p->reserve(3 * n);
+    for (DevBuf<int> *p : {&d.start, &d.ref_size, &d.motif_len, &d.wd, &d.l_off, &d.r_off, &d.n_off, &d.ids_a, &d.ids_b})
+        if (e == cudaSuccess) e = p->reserve(n);
+    if (e == cudaSuccess) e = d.cnt.reserve(8);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
+    }
+    CU(cudaMemcpyAsync(d.arena.p, arena, (size_t)arena_bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.seq_off.p, seq_off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.motif_off.p, motif_off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.lens.p, lens, 3 * n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.start.p, start_count, n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.ref_size.p, ref_size, n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.rc.p, rc_params, 3 * n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.motif_len.p, motif_len, n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.wd.p, d.h_wd.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(d.l_off.p, 0, n * sizeof(int), st));
+    CU(cudaMemsetAsync(d.r_off.p, 0, n * sizeof(int), st));
+    CU(cudaMemsetAsync(d.n_off.p, 0, n * sizeof(int), st));
+    return STRK_OK;
+}
+
 static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
                            const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
                            const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off,
                            const int32_t *motif_len, int vcf_anchor_size, int respect_coords, int32_t *out) {
     if (n_loci <= 0 || n_loci > 0x7ffffff0LL) return set_err(STRK_ERR_ARG, "strk_ref_counts: bad locus count");
-    int rc = validate_reads("strk_ref_counts", arena_bytes, seq_off, lens, n_loci);
+    const bool timing = getenv("STRK_REF_TIMING") != nullptr;  // coarse phase timers on stderr (tuning only)
+    auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+    const double t_begin = now();
+    cudaStream_t st = ctx->stream;
+    int rc = ref_setup(ctx, st, arena, arena_bytes, seq_off, lens, start_count, ref_size, rc_params, n_loci, motif_off,
+                       motif_len);
     if (rc) return rc;
-    rc = validate_motifs("strk_ref_counts", arena_bytes, motif_off, motif_len, n_loci);
-    if (rc) return rc;
+    RefBufs &d = ctx->ref;
+    const std::vector<int> &h_wd = d.h_wd;
     const int WD_MAX = (STRK_MAX_WINDOW - 1) / 2;
-    std::vector<int> h_wd((size_t)n_loci);
     int max_wd = 6, max_n1 = 0, mb_cols = 0, mb_m = 0;
     for (int64_t l = 0; l < n_loci; ++l) {
-        if (start_count[l] < 0 || start_count[l] > (1 << 22) ||
-            (long long)motif_len[l] * (long long)start_count[l] > (1ll << 24) || rc_params[3 * l] < 0 || rc_params[3 * l + 1] < 0 ||
-            rc_params[3 * l + 2] < 0 || rc_params[3 * l + 1] > 1000 || rc_params[3 * l + 2] > 1000)
-            return set_err(STRK_ERR_ARG, "strk_ref_counts: bad start count / search parameters for locus %lld", (long long)l);
-        // first window of the boundary search: start +- max(6, range + step + 2) sizes, like the read path's (a search
-        // that starts where it ends touches start +- (range + step)); one that leaves it is redone 4x wider.  Measured
-        // on 32 768 HiFi-sized windows: +- 9 sizes 3.89 ms, +- 7 3.79 ms, +- 6 3.33 ms per block.  STRK_REF_WD=<n>
-        // raises the floor of 6 (tuning only).
-        static const int wd_env = getenv("STRK_REF_WD") ? atoi(getenv("STRK_REF_WD")) : 6;
-        h_wd[(size_t)l] = std::max(wd_env > 0 ? wd_env : 6, rc_params[3 * l + 1] + rc_params[3 * l + 2] + 2);
         max_wd = std::max(max_wd, h_wd[(size_t)l]);
         const int n1 = lens[3 * l] + lens[3 * l + 1] + lens[3 * l + 2];
         max_n1 = std::max(max_n1, n1);
@@ -1665,49 +1658,16 @@ static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
             mb_m = std::max(mb_m, motif_len[l]);
         }
     }
-    CU(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
-    for (int k = 0; k < 8; ++k) ctx->stats[k] = 0;
     // counters of this call (strk_get_stats afterwards): the boundary sweeps of phase 1 + the batch runs of phase 2
     double acc_stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     const size_t n = (size_t)n_loci;
-    const bool timing = getenv("STRK_REF_TIMING") != nullptr;  // coarse phase timers on stderr (tuning only)
-    auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double t_begin = now();
-    // ---- device-resident inputs and per-locus state (context-owned, recycled across calls)
-    cudaError_t e = ctx->ref_arena.reserve((size_t)arena_bytes);
-    for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = ctx->ref_u64[k].reserve(n);
-    const size_t isz[13] = {3 * n, n, n, 3 * n, n, n, n, n, n, n, n, 4, n};
-    for (int k = 0; k < 13 && e == cudaSuccess; ++k) e = ctx->ref_i[k].reserve(isz[k]);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
-    }
-    unsigned char *d_arena = ctx->ref_arena.p;
-    unsigned long long *d_seq_off = ctx->ref_u64[0].p, *d_motif_off = ctx->ref_u64[1].p;
-    int *d_lens = ctx->ref_i[0].p, *d_start = ctx->ref_i[1].p, *d_ref_size = ctx->ref_i[2].p, *d_rc = ctx->ref_i[3].p;
-    int *d_motif_len = ctx->ref_i[4].p, *d_wd = ctx->ref_i[5].p, *d_l_off = ctx->ref_i[6].p, *d_r_off = ctx->ref_i[7].p;
-    int *d_n_off = ctx->ref_i[8].p, *d_ids_a = ctx->ref_i[9].p, *d_ids_b = ctx->ref_i[10].p;
-    unsigned int *d_cnt = (unsigned int *)ctx->ref_i[11].p;
-    CU(cudaMemcpyAsync(d_arena, arena, (size_t)arena_bytes, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_seq_off, seq_off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_motif_off, motif_off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_lens, lens, 3 * n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_start, start_count, n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_ref_size, ref_size, n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_rc, rc_params, 3 * n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_motif_len, motif_len, n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_wd, h_wd.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemsetAsync(d_l_off, 0, n * sizeof(int), st));
-    CU(cudaMemsetAsync(d_r_off, 0, n * sizeof(int), st));
-    CU(cudaMemsetAsync(d_n_off, 0, n * sizeof(int), st));
     const int T = 128;
 
     // ---- phase 1: boundary extension (skipped with respect_coords, repeats.py:99)
     if (!respect_coords) {
         long long n_pending = n_loci;
         const int *d_ids = nullptr;
-        int *d_again = d_ids_a;
+        int *d_again = d.ids_a.p;
         int cur_wd = max_wd;
         while (n_pending > 0) {
             const int stride_w = 2 * cur_wd + 1;
@@ -1716,8 +1676,8 @@ static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
                 cudaGetLastError();
                 return set_err(STRK_ERR_NOMEM, "strk_ref_counts: cannot allocate the boundary tables");
             }
-            ref_plan1_kernel<<<(unsigned)((n_pending + T - 1) / T), T, 0, st>>>(d_ids, (int)n_pending, d_seq_off, d_lens,
-                                                                                d_start, d_wd, d_motif_off, d_motif_len,
+            ref_plan1_kernel<<<(unsigned)((n_pending + T - 1) / T), T, 0, st>>>(d_ids, (int)n_pending, d.seq_off.p, d.lens.p,
+                                                                                d.start.p, d.wd.p, d.motif_off.p, d.motif_len.p,
                                                                                 stride_w, ctx->fams.p);
             CU(cudaGetLastError());
             const int b_len = max_n1 + 2;
@@ -1733,56 +1693,41 @@ static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
             if (d_ids == nullptr && ctx->h_consts.packed_ok && 2 * stride_w <= PK_WINDOW_MAX) {
                 // first pass (locus q = q): packed kernel in reference mode per rows-per-lane class, the forward and
                 // the reverse sg_qe alignment of a locus in the two halves of its lane words; the rest -> general
-                std::vector<int> lists[STRK_PK_NBIN];
-                int mmax[STRK_PK_NBIN] = {0}, flank[STRK_PK_NBIN] = {0};
+                ClassLists lists;
                 for (int64_t l = 0; l < n_loci; ++l) {
-                    const int fl = lens[3 * l], tr = lens[3 * l + 1], fr = lens[3 * l + 2], m = motif_len[l];
-                    int R = strk_pick_rows_packed(fl + tr + fr + 1);
-                    if (fl < 1 || fr < 1 || fl > PK_FLANK_MAX || fr > PK_FLANK_MAX || m * R > 128) R = 0;
-                    lists[R].push_back((int)l);
-                    mmax[R] = std::max(mmax[R], m);
-                    flank[R] = std::max(flank[R], std::max(fl, fr));
+                    const int fl = lens[3 * l], fr = lens[3 * l + 2], m = motif_len[l];
+                    lists.add(strk_pk_class(fl, lens[3 * l + 1], fr, m), (int)l, m, fl, fr);
                 }
-                std::vector<int> flat;
-                size_t at[STRK_PK_NBIN];
-                for (int k = 0; k < STRK_PK_NBIN; ++k) {
-                    at[k] = flat.size();
-                    flat.insert(flat.end(), lists[k].begin(), lists[k].end());
-                }
-                int *d_lists = ctx->ref_i[12].p;
                 if (ctx->fallback.reserve(n) != cudaSuccess) {
                     cudaGetLastError();
                     return set_err(STRK_ERR_NOMEM, "strk_ref_counts: cannot allocate the fallback list");
                 }
-                CU(cudaMemcpyAsync(d_lists, flat.data(), flat.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-                CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
-                long long n_packed = 0;
                 const int *seg_list[STRK_PK_NBIN];
                 long long seg_cnt[STRK_PK_NBIN];
                 int seg_w[STRK_PK_NBIN];
-                for (int k = 0; k < STRK_PK_NBIN; ++k) {
-                    seg_list[k] = d_lists + at[k];
-                    seg_cnt[k] = (long long)lists[k].size();
-                    seg_w[k] = 2 * stride_w - 1;  // forward + reverse columns of every size of the window
-                }
-                rc = launch_pass(ctx, seg_list, seg_cnt, flank, mmax, seg_w, n_loci, ctx->fams.p, d_arena, ctx->table64.p, b_len,
-                                 rowlen, st, 1, &n_packed);
+                for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w[k] = 2 * stride_w - 1;  // forward + reverse columns of every size
+                rc = lists.upload(d.lists, st, seg_list, seg_cnt);
                 if (rc) return rc;
-                CU(cudaStreamSynchronize(st));  // `flat` is read by the copy above
+                CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
+                long long n_packed = 0;
+                rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w, n_loci, ctx->fams.p, d.arena.p,
+                                 ctx->table64.p, b_len, rowlen, st, 1, &n_packed);
+                if (rc) return rc;
+                CU(cudaStreamSynchronize(st));  // `lists` is read by the copy
             } else {
-                rc = launch_general(ctx, true, ctx->fams.p, nullptr, n_pending, d_arena, ctx->table64.p, b_len, rowlen, st);
+                rc = launch_general(ctx, true, ctx->fams.p, nullptr, n_pending, d.arena.p, ctx->table64.p, b_len, rowlen, st);
                 if (rc) return rc;
             }
             CU(cudaEventRecord(ctx->ev[1], st));
-            CU(cudaMemsetAsync(d_cnt, 0, 4 * sizeof(unsigned int), st));
+            CU(cudaMemsetAsync(d.cnt.p, 0, 4 * sizeof(unsigned int), st));
             ref_replay1_kernel<<<(unsigned)((n_pending + T - 1) / T), T, 0, st>>>(
-                d_ids, (int)n_pending, ctx->table64.p, ctx->fams.p, d_start, d_rc, d_ref_size, vcf_anchor_size, WD_MAX, d_wd,
-                d_l_off, d_r_off, d_n_off, d_again, d_cnt);
+                d_ids, (int)n_pending, ctx->table64.p, ctx->fams.p, d.start.p, d.rc.p, d.ref_size.p, vcf_anchor_size, WD_MAX,
+                d.wd.p, d.l_off.p, d.r_off.p, d.n_off.p, d_again, d.cnt.p);
             CU(cudaGetLastError());
             CU(cudaEventRecord(ctx->ev[2], st));
             ctx->stats[2] += 2;
             unsigned int h_cnt[4] = {0, 0, 0, 0};
-            CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(h_cnt, d.cnt.p, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
             CU(cudaStreamSynchronize(st));
             {
                 float t0 = 0.f, t1 = 0.f;
@@ -1802,16 +1747,16 @@ static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
             n_pending = h_cnt[0];
             acc_stats[5] += (double)n_pending;
             d_ids = d_again;
-            d_again = d_again == d_ids_a ? d_ids_b : d_ids_a;
+            d_again = d_again == d.ids_a.p ? d.ids_b.p : d.ids_a.p;
             cur_wd = std::min(WD_MAX, cur_wd * 4);
         }
     }
     const double t_phase1 = now();
     acc_stats[2] = ctx->stats[2];
     std::vector<int> l_off(n), r_off(n), n_off(n);
-    CU(cudaMemcpyAsync(l_off.data(), d_l_off, n * sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(r_off.data(), d_r_off, n * sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(n_off.data(), d_n_off, n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(l_off.data(), d.l_off.p, n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(r_off.data(), d.r_off.p, n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(n_off.data(), d.n_off.p, n * sizeof(int), cudaMemcpyDeviceToHost, st));
 
     // ---- phase 2: final count on the adjusted flanks (repeats.py:171-188), one batch run per parameter tier
     std::vector<std::vector<int>> tiers;
@@ -1835,36 +1780,19 @@ static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
     for (size_t t = 0; t < tiers.size(); ++t) {
         const std::vector<int> &ids = tiers[t];
         const size_t nt = ids.size();
-        e = b->seq_off.reserve(nt);
-        if (e == cudaSuccess) e = b->lens.reserve(3 * nt);
-        if (e == cudaSuccess) e = b->est.reserve(nt);
-        if (e == cudaSuccess) e = b->motif_off.reserve(nt);
-        if (e == cudaSuccess) e = b->motif_len.reserve(nt);
-        if (e == cudaSuccess) e = b->read_begin.reserve(nt + 1);
-        if (e == cudaSuccess) e = b->read_locus.reserve(nt);
-        if (e == cudaSuccess) e = b->order.reserve(nt);
-        if (e == cudaSuccess) e = b->bin.reserve(nt);
-        if (e == cudaSuccess) e = b->out.reserve(nt * 4);
-        if (e == cudaSuccess) e = b->status.reserve(nt);
+        const cudaError_t e = batch_bind(b, (long long)nt, (long long)nt);
         if (e != cudaSuccess) {
             cudaGetLastError();
             return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
         }
-        b->n_reads = b->n_loci = (long long)nt;
-        b->d_arena = d_arena;
-        b->d_seq_off = b->seq_off.p, b->d_lens = b->lens.p, b->d_est = b->est.p, b->d_motif_off = b->motif_off.p;
-        b->d_motif_len = b->motif_len.p, b->d_read_begin = b->read_begin.p, b->d_read_locus = b->read_locus.p;
-        b->d_order = b->order.p, b->d_out = b->out.p, b->d_status = b->status.p;
+        b->d_arena = d.arena.p;
         b->h_read_begin.resize(nt + 1);
         for (size_t q = 0; q <= nt; ++q) b->h_read_begin[q] = (long long)q;
-        b->n_general = 0;
-        for (int k = 0; k < STRK_PK_NBIN; ++k) b->bin_off[k] = b->bin_cnt[k] = 0, b->bin_mmax[k] = b->bin_flank[k] = 0;
-        b->max_n1 = b->mb_cols_base = b->mb_m = 0;
-        CU(cudaMemcpyAsync(d_ids_a, ids.data(), nt * sizeof(int), cudaMemcpyHostToDevice, st));
-        ref_plan2_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(d_ids_a, (int)nt, d_seq_off, d_lens, d_start, d_motif_off,
-                                                                     d_motif_len, d_l_off, d_r_off, b->d_seq_off, b->d_lens,
-                                                                     b->d_est, b->d_motif_off, b->d_motif_len,
-                                                                     b->d_read_begin);
+        CU(cudaMemcpyAsync(d.ids_a.p, ids.data(), nt * sizeof(int), cudaMemcpyHostToDevice, st));
+        ref_plan2_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(d.ids_a.p, (int)nt, d.seq_off.p, d.lens.p, d.start.p,
+                                                                     d.motif_off.p, d.motif_len.p, d.l_off.p, d.r_off.p,
+                                                                     b->d_seq_off, b->d_lens, b->d_est, b->d_motif_off,
+                                                                     b->d_motif_len, b->d_read_begin);
         CU(cudaGetLastError());
         CU(cudaStreamSynchronize(st));  // `ids` is read by the copy above
         rc = batch_plan(ctx, b, arena_bytes);
@@ -1910,27 +1838,26 @@ static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
         if (rc_params[3 * l] != rc_params[0] || rc_params[3 * l + 1] != rc_params[1] || rc_params[3 * l + 2] != rc_params[2])
             return STRK_OK;  // several tiers: the general path groups them
     const int max_iters = rc_params[0], range = rc_params[1], step = rc_params[2];
-    int rc = validate_reads("strk_ref_counts", arena_bytes, seq_off, lens, n_loci);
-    if (rc) return rc;
-    rc = validate_motifs("strk_ref_counts", arena_bytes, motif_off, motif_len, n_loci);
-    if (rc) return rc;
     if (max_iters < 0 || range < 0 || step < 0 || range > 1000 || step > 1000)
         return set_err(STRK_ERR_ARG, "strk_ref_counts: bad search parameters");
-    static const int wd_env = getenv("STRK_REF_WD") ? atoi(getenv("STRK_REF_WD")) : 6;
-    const int wd1 = std::max(wd_env > 0 ? wd_env : 6, range + step + 2);
+    const int wd1 = ref_first_wd(range, step);
     const int stride_w = 2 * wd1 + 1;
     int wd2 = range + step + 2;  // phase 2: the read path's first window
     if (wd2 < 6) wd2 = 6;
     const int W2 = 2 * wd2 + 1;
     if (2 * stride_w > PK_WINDOW_MAX || W2 > PK_WINDOW_MAX) return STRK_OK;
+    *taken = true;
+    cudaStream_t st = ctx->stream;
+    int rc = ref_setup(ctx, st, arena, arena_bytes, seq_off, lens, start_count, ref_size, rc_params, n_loci, motif_off,
+                       motif_len);
+    if (rc) return rc;
+    RefBufs &d = ctx->ref;
     const size_t n = (size_t)n_loci;
     int max_n1 = 0, mb_cols = 0, mb_m = 0;
-    std::vector<int> lists[STRK_PK_NBIN];
-    int mmax[STRK_PK_NBIN] = {0}, flank[STRK_PK_NBIN] = {0};
+    ClassLists &lists = d.classes;  // (on the context: read by an asynchronous copy until the one synchronisation)
+    lists.clear();
     double cells1 = 0.0;
     for (int64_t l = 0; l < n_loci; ++l) {
-        if (start_count[l] < 0 || start_count[l] > (1 << 22) || (long long)motif_len[l] * (long long)start_count[l] > (1ll << 24))
-            return set_err(STRK_ERR_ARG, "strk_ref_counts: bad start count / search parameters for locus %lld", (long long)l);
         const int fl = lens[3 * l], tr = lens[3 * l + 1], fr = lens[3 * l + 2], m = motif_len[l];
         const int n1 = fl + tr + fr;
         max_n1 = std::max(max_n1, n1);
@@ -1940,39 +1867,19 @@ static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
             mb_cols = std::max(mb_cols, std::max(fl, fr) + m * (start_count[l] + (fl + fr) / m + 1));
             mb_m = std::max(mb_m, m);
         }
-        int R = strk_pick_rows_packed(n1 + 1);
-        if (fl < 1 || fr < 1 || fl > PK_FLANK_MAX || fr > PK_FLANK_MAX || m * R > 128) R = 0;
-        lists[R].push_back((int)l);
-        mmax[R] = std::max(mmax[R], m);
-        flank[R] = std::max(flank[R], std::max(fl, fr));
+        lists.add(strk_pk_class(fl, tr, fr, m), (int)l, m, fl, fr);
         cells1 += (double)n1 * ((double)fl + fr + 2.0 * m * ((double)start_count[l] + wd1));
     }
-    *taken = true;
-    CU(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
-    for (int k = 0; k < 8; ++k) ctx->stats[k] = 0;
     // ---- device buffers (context-owned, recycled)
-    cudaError_t e = ctx->ref_arena.reserve((size_t)arena_bytes);
-    for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = ctx->ref_u64[k].reserve(n);
-    const size_t isz[13] = {3 * n, n, n, 3 * n, n, n, n, n, n, n, n, 8, n};
-    for (int k = 0; k < 13 && e == cudaSuccess; ++k) e = ctx->ref_i[k].reserve(isz[k]);
-    if (e == cudaSuccess) e = ctx->ref_out.reserve(8 * n + 8);
     if (!ctx->ref_batch) ctx->ref_batch = new (std::nothrow) strk_batch();
     if (!ctx->ref_batch) return set_err(STRK_ERR_NOMEM, "out of host memory");
     strk_batch *b = ctx->ref_batch;
-    if (e == cudaSuccess) e = b->seq_off.reserve(n);
-    if (e == cudaSuccess) e = b->lens.reserve(3 * n);
-    if (e == cudaSuccess) e = b->est.reserve(n);
-    if (e == cudaSuccess) e = b->motif_off.reserve(n);
-    if (e == cudaSuccess) e = b->motif_len.reserve(n);
-    if (e == cudaSuccess) e = b->read_begin.reserve(n + 1);
-    if (e == cudaSuccess) e = b->read_locus.reserve(n);
-    if (e == cudaSuccess) e = b->out.reserve(4 * n);
-    if (e == cudaSuccess) e = b->status.reserve(n);
     // second look at phase 1, still on the device: up to CAP2 loci whose search left the first window, 4x wider
     const int CAP2 = 4096;
     const int WD_MAX = (STRK_MAX_WINDOW - 1) / 2;
     const int wd1b = std::min(WD_MAX, 4 * wd1), stride_w2 = 2 * wd1b + 1;
+    cudaError_t e = d.out.reserve(8 * n + 8);
+    if (e == cudaSuccess) e = batch_bind(b, (long long)n, (long long)n);
     if (e == cudaSuccess) e = ctx->fams.reserve(std::max(n, (size_t)CAP2));
     if (e == cudaSuccess) e = ctx->table64.reserve(std::max(n * (size_t)stride_w * 2, (size_t)CAP2 * (size_t)stride_w2 * 2));
     if (e == cudaSuccess) e = ctx->table.reserve(n * (size_t)W2);
@@ -1981,85 +1888,56 @@ static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
     }
-    unsigned char *d_arena = ctx->ref_arena.p;
-    unsigned long long *d_seq_off = ctx->ref_u64[0].p, *d_motif_off = ctx->ref_u64[1].p;
-    int *d_lens = ctx->ref_i[0].p, *d_start = ctx->ref_i[1].p, *d_ref_size = ctx->ref_i[2].p, *d_rc = ctx->ref_i[3].p;
-    int *d_motif_len = ctx->ref_i[4].p, *d_wd = ctx->ref_i[5].p, *d_l_off = ctx->ref_i[6].p, *d_r_off = ctx->ref_i[7].p;
-    int *d_n_off = ctx->ref_i[8].p, *d_again = ctx->ref_i[9].p, *d_lists = ctx->ref_i[12].p;
-    unsigned int *d_cnt = (unsigned int *)ctx->ref_i[11].p;
-    ctx->ref_hwd.assign(n, wd1);
-    ctx->ref_flat.clear();
-    size_t at[STRK_PK_NBIN];
-    for (int k = 0; k < STRK_PK_NBIN; ++k) {
-        at[k] = ctx->ref_flat.size();
-        ctx->ref_flat.insert(ctx->ref_flat.end(), lists[k].begin(), lists[k].end());
-    }
-    CU(cudaMemcpyAsync(d_arena, arena, (size_t)arena_bytes, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_seq_off, seq_off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_motif_off, motif_off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_lens, lens, 3 * n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_start, start_count, n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_ref_size, ref_size, n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_rc, rc_params, 3 * n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_motif_len, motif_len, n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_wd, ctx->ref_hwd.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_lists, ctx->ref_flat.data(), ctx->ref_flat.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemsetAsync(d_l_off, 0, n * sizeof(int), st));
-    CU(cudaMemsetAsync(d_r_off, 0, n * sizeof(int), st));
-    CU(cudaMemsetAsync(d_n_off, 0, n * sizeof(int), st));
-    CU(cudaMemsetAsync(d_cnt, 0, 8 * sizeof(unsigned int), st));
+    b->d_arena = d.arena.p;
+    const int *seg_list[STRK_PK_NBIN];
+    long long seg_cnt[STRK_PK_NBIN];
+    rc = lists.upload(d.lists, st, seg_list, seg_cnt);
+    if (rc) return rc;
+    CU(cudaMemsetAsync(d.cnt.p, 0, 8 * sizeof(unsigned int), st));
     CU(cudaMemsetAsync(ctx->d_acc, 0, 4 * sizeof(double), st));
     CU(cudaMemsetAsync(ctx->d_queue + 1, 0, 3 * sizeof(unsigned int), st));
     const int T = 128;
     const int b_len = max_n1 + 2;
     const int rowlen = max_n1 > 32 * 16 ? mb_cols + mb_m * std::max(std::max(wd1, wd2), wd1b) + 2 : 2;
-    const int *seg_list[STRK_PK_NBIN];
-    long long seg_cnt[STRK_PK_NBIN];
     int seg_w1[STRK_PK_NBIN], seg_w2[STRK_PK_NBIN];
     for (int k = 0; k < STRK_PK_NBIN; ++k) {
-        seg_list[k] = d_lists + at[k];
-        seg_cnt[k] = (long long)lists[k].size();
         seg_w1[k] = 2 * stride_w - 1;
         seg_w2[k] = (W2 + 3) / 4 * 4;
     }
     // ---- phase 1
-    ref_plan1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d_seq_off, d_lens, d_start, d_wd, d_motif_off,
-                                                               d_motif_len, stride_w, ctx->fams.p);
+    ref_plan1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d.seq_off.p, d.lens.p, d.start.p, d.wd.p,
+                                                               d.motif_off.p, d.motif_len.p, stride_w, ctx->fams.p);
     CU(cudaGetLastError());
     CU(cudaEventRecord(ctx->ev[0], st));
     long long n_packed = 0;
-    rc = launch_pass(ctx, seg_list, seg_cnt, flank, mmax, seg_w1, n_loci, ctx->fams.p, d_arena, ctx->table64.p, b_len, rowlen, st,
-                     1, &n_packed);
+    rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w1, n_loci, ctx->fams.p, d.arena.p, ctx->table64.p,
+                     b_len, rowlen, st, 1, &n_packed);
     if (rc) return rc;
     CU(cudaEventRecord(ctx->ev[1], st));
-    ref_replay1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, ctx->table64.p, ctx->fams.p, d_start, d_rc,
-                                                                 d_ref_size, vcf_anchor_size, WD_MAX, d_wd, d_l_off, d_r_off,
-                                                                 d_n_off, d_again, d_cnt);
+    ref_replay1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, ctx->table64.p, ctx->fams.p, d.start.p, d.rc.p,
+                                                                 d.ref_size.p, vcf_anchor_size, WD_MAX, d.wd.p, d.l_off.p,
+                                                                 d.r_off.p, d.n_off.p, d.ids_a.p, d.cnt.p);
     CU(cudaGetLastError());
     {
         // the loci whose search left the first window (a percent of a block at +-6 sizes): 4x wider through the general
-        // kernel, list and count on the device (d_again, d_cnt[0]); what still does not settle is left to the host
-        int *d_again2 = ctx->ref_i[10].p;
-        ref_clamp_count_kernel<<<1, 32, 0, st>>>(d_cnt, (unsigned)CAP2);  // (loci beyond the cap keep their flag: host redo)
-        ref_plan1_kernel<<<(unsigned)((CAP2 + T - 1) / T), T, 0, st>>>(d_again, CAP2, d_seq_off, d_lens, d_start, d_wd, d_motif_off,
-                                                                      d_motif_len, stride_w2, ctx->fams.p, d_cnt);
+        // kernel, list and count on the device (ids_a, cnt[0]); what still does not settle is left to the host
+        ref_clamp_count_kernel<<<1, 32, 0, st>>>(d.cnt.p, (unsigned)CAP2);  // (loci beyond the cap keep their flag: host redo)
+        ref_plan1_kernel<<<(unsigned)((CAP2 + T - 1) / T), T, 0, st>>>(d.ids_a.p, CAP2, d.seq_off.p, d.lens.p, d.start.p, d.wd.p,
+                                                                      d.motif_off.p, d.motif_len.p, stride_w2, ctx->fams.p, d.cnt.p);
         CU(cudaGetLastError());
-        rc = launch_general(ctx, true, ctx->fams.p, nullptr, CAP2, d_arena, ctx->table64.p, b_len, rowlen, st, d_cnt);
+        rc = launch_general(ctx, true, ctx->fams.p, nullptr, CAP2, d.arena.p, ctx->table64.p, b_len, rowlen, st, d.cnt.p);
         if (rc) return rc;
-        ref_replay1_kernel<<<(unsigned)((CAP2 + T - 1) / T), T, 0, st>>>(d_again, CAP2, ctx->table64.p, ctx->fams.p, d_start, d_rc,
-                                                                        d_ref_size, vcf_anchor_size, WD_MAX, d_wd, d_l_off,
-                                                                        d_r_off, d_n_off, d_again2, d_cnt + 4, d_cnt);
+        ref_replay1_kernel<<<(unsigned)((CAP2 + T - 1) / T), T, 0, st>>>(d.ids_a.p, CAP2, ctx->table64.p, ctx->fams.p, d.start.p,
+                                                                        d.rc.p, d.ref_size.p, vcf_anchor_size, WD_MAX, d.wd.p,
+                                                                        d.l_off.p, d.r_off.p, d.n_off.p, d.ids_b.p, d.cnt.p + 4,
+                                                                        d.cnt.p);
         CU(cudaGetLastError());
     }
     // ---- phase 2 (loci whose phase 1 is not final yet run with their unadjusted flanks; their rows are redone)
-    b->n_reads = b->n_loci = (long long)n;
-    b->d_arena = d_arena;
-    b->d_seq_off = b->seq_off.p, b->d_lens = b->lens.p, b->d_est = b->est.p, b->d_motif_off = b->motif_off.p;
-    b->d_motif_len = b->motif_len.p, b->d_read_begin = b->read_begin.p, b->d_read_locus = b->read_locus.p;
-    b->d_out = b->out.p, b->d_status = b->status.p;
-    ref_plan2_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d_seq_off, d_lens, d_start, d_motif_off,
-                                                               d_motif_len, d_l_off, d_r_off, b->d_seq_off, b->d_lens, b->d_est,
-                                                               b->d_motif_off, b->d_motif_len, b->d_read_begin, b->d_read_locus);
+    ref_plan2_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d.seq_off.p, d.lens.p, d.start.p, d.motif_off.p,
+                                                               d.motif_len.p, d.l_off.p, d.r_off.p, b->d_seq_off, b->d_lens,
+                                                               b->d_est, b->d_motif_off, b->d_motif_len, b->d_read_begin,
+                                                               b->d_read_locus);
     CU(cudaGetLastError());
     plan_reads_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(nullptr, (long long)n, b->d_seq_off, b->d_lens, b->d_est,
                                                                   b->d_read_locus, b->d_motif_off, b->d_motif_len, wd2, 0, W2,
@@ -2068,30 +1946,23 @@ static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
     CU(cudaEventRecord(ctx->ev[2], st));
     CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
     long long n_packed2 = 0;
-    rc = launch_pass(ctx, seg_list, seg_cnt, flank, mmax, seg_w2, n_loci, ctx->fams.p, d_arena, ctx->table.p, b_len, rowlen, st, 0,
-                     &n_packed2);
+    rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w2, n_loci, ctx->fams.p, d.arena.p, ctx->table.p, b_len,
+                     rowlen, st, 0, &n_packed2);
     if (rc) return rc;
     CU(cudaEventRecord(ctx->ev[3], st));
-    if (W2 <= REPLAY_WMAX)
-        replay_reads_small_kernel<<<(unsigned)((n + REPLAY_THREADS - 1) / REPLAY_THREADS), REPLAY_THREADS, 0, st>>>(
-            ctx->table.p, W2, wd2, 0, nullptr, nullptr, (int)n, b->d_read_begin, b->d_est, b->d_lens, b->d_motif_len, max_iters,
-            range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->d_queue + 1, ctx->d_acc, nullptr);
-    else
-        replay_reads_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(
-            ctx->table.p, W2, wd2, 0, nullptr, nullptr, (int)n, b->d_read_begin, b->d_est, b->d_lens, b->d_motif_len, max_iters,
-            range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->d_queue + 1, ctx->d_acc, nullptr);
-    CU(cudaGetLastError());
-    ref_assemble_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>((int)n, b->d_out, b->d_status, d_lens, d_l_off, d_r_off, d_n_off,
-                                                                  ctx->ref_out.p);
+    rc = launch_replay(ctx, b, W2, wd2, 0, nullptr, nullptr, (long long)n, max_iters, range, step, nullptr, nullptr, st);
+    if (rc) return rc;
+    ref_assemble_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>((int)n, b->d_out, b->d_status, d.lens.p, d.l_off.p, d.r_off.p,
+                                                                  d.n_off.p, d.out.p);
     CU(cudaGetLastError());
     CU(cudaEventRecord(ctx->ev[4], st));
     // ---- the one synchronisation: results, flags, counters
     std::vector<unsigned char> status(n);
     unsigned int h_cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     double acc[2] = {0, 0};
-    CU(cudaMemcpyAsync(out, ctx->ref_out.p, 8 * n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(out, d.out.p, 8 * n * sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(status.data(), b->d_status, n, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_cnt, d.cnt.p, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(acc, ctx->d_acc, sizeof(acc), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (h_cnt[1] || h_cnt[5]) {

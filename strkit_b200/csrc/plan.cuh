@@ -24,6 +24,15 @@ enum PlanError {
     PLAN_ERR_MOTIF_EMPTY = 6, PLAN_ERR_MOTIF_PAST_ARENA = 7, PLAN_ERR_READ_BEGIN = 8
 };
 
+// Rows-per-lane class of the packed kernel for a window of flanks fl / fr around a tract of tr bases and a motif of m
+// bases; 0 = the general kernel only (too long, a flank it cannot stage, or a motif profile wider than 128 rows).
+// Callers add their own gates: the matrix (packed_ok) and the window of candidate sizes.
+__host__ __device__ inline int strk_pk_class(int fl, int tr, int fr, int m) {
+    const int R = strk_pick_rows_packed(fl + tr + fr + 1);
+    if (fl < 1 || fr < 1 || fl > PK_FLANK_MAX || fr > PK_FLANK_MAX || m * R > 128 || m <= 0) return 0;
+    return R;
+}
+
 __device__ __forceinline__ void plan_report(PlanStats *st, long long index, int kind) {
     atomicMin(&st->first_error, ((unsigned long long)index << 8) | (unsigned long long)kind);
 }
@@ -75,9 +84,7 @@ __global__ void plan_reads_scan_kernel(const unsigned long long *__restrict__ se
             plan_report(st, r, PLAN_ERR_EST);  // candidate columns (64-bit): a garbage estimate must not size scratch
         else {
             const int m = motif_len[read_locus[r]];
-            int R = packed_ok ? strk_pick_rows_packed((int)n1 + 1) : 0;
-            if (fl < 1 || fr < 1 || fl > PK_FLANK_MAX || fr > PK_FLANK_MAX || m * R > 128 || m <= 0) R = 0;
-            b = R;
+            b = packed_ok ? strk_pk_class(fl, tr, fr, m) : 0;
             atomicMax(&s_max_n1, (int)n1);
             if (b) {
                 atomicMax(&s_mmax[b], m);

@@ -452,7 +452,9 @@ def test_get_ref_repeat_count_golden(sb, golden):
 
 def test_ref_counts_batch_with_reference_tiers(sb, oracle):
     """One C-ABI call for many loci, search parameters tiered like repeat_count_params.py:17-42
-    (steps of 3 / 5 / 15 for large reference tracts)."""
+    (steps of 3 / 5 / 15 for large reference tracts), then the same loci one call per tier: a single tier takes the
+    fast path, and start counts off by tens of copies send searches out of their first window (the device-side second
+    look and the loci redone on the host)."""
     rng = np.random.default_rng(21)
     fams, starts, ref_sizes, rcs = [], [], [], []
     for i in range(40):
@@ -477,6 +479,21 @@ def test_ref_counts_batch_with_reference_tiers(sb, oracle):
         (cn, score), lo, ro, (n_off, n_fin), (fl2, tr2, fr2) = oracle.get_ref_repeat_count(
             starts[i], tr, fl, fr, motif, ref_sizes[i], 5, rcs[i][0], rcs[i][1], rcs[i][2])
         assert got[i].tolist() == [cn, score, lo, ro, n_off, n_fin, len(fl2), len(fr2)], (i, fams[i][0], rcs[i])
+    starts = np.array(starts)
+    bad = rng.random(starts.shape[0]) < 0.2
+    starts[bad] = np.maximum(0, starts[bad] + rng.integers(-30, 60, int(bad.sum())))
+    redone = 0
+    for tier in sorted({tuple(r) for r in rcs}):
+        idx = [i for i, r in enumerate(rcs) if tuple(r) == tier]
+        got = eng.ref_counts(families_to_batch([fams[i] for i in idx]), starts[idx], [ref_sizes[i] for i in idx],
+                             np.array([rcs[i] for i in idx]), vcf_anchor_size=5)
+        redone += int(eng.stats()["widening_passes"])
+        for row, i in zip(got, idx):
+            motif, tr, fl, fr = fams[i]
+            (cn, score), lo, ro, (n_off, n_fin), (fl2, tr2, fr2) = oracle.get_ref_repeat_count(
+                int(starts[i]), tr, fl, fr, motif, ref_sizes[i], 5, *tier)
+            assert row.tolist() == [cn, score, lo, ro, n_off, n_fin, len(fl2), len(fr2)], (i, motif, tier, starts[i])
+    assert redone > 0   # some searches did leave their first window
 
 
 def test_ragged_loci_zero_one_and_max_reads(sb, oracle):
