@@ -2024,3 +2024,19 @@ extern "C" int strk_measure_int_peak(strk_ctx *ctx, double out_tiops[3]) {
 // ------------------------------------------------------------------------------------------------
 #include "alleles_api.cuh"
 #include "realign_api.cuh"
+
+#if PK_PHASE_TIMERS
+// Measurement build only (not in include/strkit_b200.h): copies the packed kernel's phase timers of `device` to
+// out[2 * 2 * 17 * 4] (the layout of pk_phase_clk in dp_packed.cuh) and, with reset != 0, clears them.
+extern "C" int strk_pk_phase_timers(int device, unsigned long long *out, int reset) {
+    if (!out) return set_err(STRK_ERR_ARG, "strk_pk_phase_timers: null argument");
+    CU(cudaSetDevice(device));
+    CU(cudaDeviceSynchronize());
+    CU(cudaMemcpyFromSymbol(out, pk_phase_clk, sizeof(pk_phase_clk)));
+    if (reset) {
+        static const unsigned long long zero[2 * 2 * 17 * 4] = {0ull};
+        CU(cudaMemcpyToSymbol(pk_phase_clk, zero, sizeof(pk_phase_clk)));
+    }
+    return STRK_OK;
+}
+#endif

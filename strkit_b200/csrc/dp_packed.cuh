@@ -64,6 +64,18 @@ __host__ __device__ constexpr int pk_warps(int L) { return L == 16 ? PK_WARPS_PA
 #define PK_MIN_CTAS(R) ((R) <= 10 ? 5 : ((R) <= 18 ? 4 : 3))
 #endif
 
+// Measurement build only (-DPK_PHASE_TIMERS=1, off by default): clock64() phase timers of the per-read code.
+// pk_phase_clk[ref_mode][L == 16][R][phase] sums SM cycles over the warps of every launch since the last reset:
+// phase 0 = prologue (queue pop, eligibility, staging, tables, profile, borders, step ranges), 1 = step loops,
+// 2 = epilogue (combine or reference-mode reduction), 3 = warp iterations that ran the step loops.  Each warp
+// accumulates in registers and adds its totals once, when it leaves the work queue.  tools/pk_phase_timers.py reads it.
+#ifndef PK_PHASE_TIMERS
+#define PK_PHASE_TIMERS 0
+#endif
+#if PK_PHASE_TIMERS
+__device__ unsigned long long pk_phase_clk[2][2][17][4];
+#endif
+
 struct PackedDims {
     int colt_entries;  // uint4 entries of the per-column table  (>= max flank + 64)
     int prof_words;    // u32 words of the packed profile        (>= m_max * R * 32)
@@ -284,6 +296,20 @@ __device__ __forceinline__ void pk_run(PkState<R> &st, int &s, const int s_end, 
     }
 }
 
+// max over my rows of forward + paired backward value for one captured candidate column (low halves only)
+template <int R, int QN>
+__device__ __forceinline__ unsigned pk_cand_max(const uint4 (&c)[QN], const unsigned (&Bv)[R]) {
+    unsigned acc = 0u;
+#pragma unroll
+    for (int q = 0; q < QN; ++q) {
+        if (4 * q + 0 < R) acc = __viaddmax_u16x2(c[q].x, Bv[(4 * q + 0) % R], acc);
+        if (4 * q + 1 < R) acc = __viaddmax_u16x2(c[q].y, Bv[(4 * q + 1) % R], acc);
+        if (4 * q + 2 < R) acc = __viaddmax_u16x2(c[q].z, Bv[(4 * q + 2) % R], acc);
+        if (4 * q + 3 < R) acc = __viaddmax_u16x2(c[q].w, Bv[(4 * q + 3) % R], acc);
+    }
+    return acc & 0xffffu;
+}
+
 template <int R, int L>
 __global__ void __launch_bounds__(pk_warps(L) * 32, PK_MIN_CTAS(R) * PK_WARPS / pk_warps(L))
 dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list, int n_list,
@@ -297,6 +323,8 @@ dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list,
     constexpr int N = L * R;
     constexpr int QN = (R + 1 + 3) / 4;
     constexpr int RH = (R + 1) / 2;  // row pairs of the packed profile
+    constexpr int WB = 4;   // combine: candidate columns per batch of loads (hides the L2 round trip)
+    constexpr int WBR = 2;  // reference mode: columns per batch (with 4, ptxas laid out some classes' step loops worse)
     extern __shared__ uint4 smem_raw[];
     __shared__ SmemConsts sc;
     __shared__ unsigned long long t8f[STRK_NSYM_], t8b[STRK_NSYM_];
@@ -348,12 +376,32 @@ dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list,
     // Work items come from a queue (one atomic per warp and read, nothing next to a 100-microsecond sweep): a launch
     // that shares the SMs with another context's kernels (the streamed path), or whose CTAs do not all start together,
     // no longer ends on the slowest statically assigned slice.  Both units of a warp take consecutive items.
-    (void)total_units;
-    for (;;) {
-        unsigned int base = 0u;
-        if (wlane == 0) base = atomicAdd(work_counter, (unsigned int)HALVES);
-        base = __shfl_sync(0xffffffffu, base, 0);
+#if PK_PHASE_TIMERS
+    unsigned long long clk_acc[4] = {0ull, 0ull, 0ull, 0ull}, clk_t = clock64();
+#define PK_CLK(P)                                      \
+    do {                                               \
+        const unsigned long long t_ = clock64();       \
+        clk_acc[P] += t_ - clk_t;                      \
+        clk_t = t_;                                    \
+    } while (0)
+#else
+#define PK_CLK(P) \
+    do {          \
+    } while (0)
+#endif
+    // The next item is popped one read ahead while the queue is far from empty (the atomic's latency then hides behind
+    // a read); near the end it is popped after the read, so that no warp holds an item while others run out of work.
+    unsigned int next = 0u;
+    auto pop = [&] {
+        if (wlane == 0) next = atomicAdd(work_counter, (unsigned int)HALVES);
+    };
+    pop();
+    bool ahead = false;
+    for (;; ahead ? (void)0 : pop()) {
+        const unsigned int base = __shfl_sync(0xffffffffu, next, 0);
         if (base >= (unsigned int)n_list) break;
+        ahead = base + 2u * (unsigned int)total_units < (unsigned int)n_list;
+        if (ahead) pop();
         // a unit without a read of its own in the last round re-runs the last read of the list and stores nothing
         const int fam_idx_raw = (int)base + half;
         const bool have = fam_idx_raw < n_list;
@@ -457,23 +505,29 @@ dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list,
         const bool plain_unit = all_unit(rows_plain);  // evaluated by every lane (it votes across the warp)
         const bool one_table = __all_sync(0xffffffffu, (one_table_ok && cols_acgt) || plain_unit);
         // ---- packed profile for the motif phase (row pairs, see pk_prof_rows), column j = Lmax + 1 + k (mod m)
-        if (one_table_ok && motif_acgt) {
-            for (int k = 0; k < m; ++k) {
-                const unsigned tf = (unsigned)t8f[mcodes[mod_m(k + Lmax - f.n_fl)]];
-                const unsigned tb = (unsigned)t8b[mcodes[m - 1 - mod_m(k + Lmax - f.n_fr)]];
+        // motif positions of column k stepped instead of reduced mod m per column; one base pointer per lane
+        {
+            int jf = mod_m(Lmax - f.n_fl), jb = m - 1 - mod_m(Lmax - f.n_fr);
+            unsigned *pc = prof + 2 * lane;
+            if (one_table_ok && motif_acgt) {
+                for (int k = 0; k < m; ++k, pc += 2 * RH * L) {
+                    const unsigned tf = (unsigned)t8f[mcodes[jf]], tb = (unsigned)t8b[mcodes[jb]];
 #pragma unroll
-                for (int r = 0; r < R; ++r)
-                    prof[((k * RH + (r >> 1)) * L + lane) * 2 + (r & 1)] = pk_prmt(tf, tb, st.selA[r]) + st.selB[r];
-            }
-        } else {
-            for (int k = 0; k < m; ++k) {
-                const int sf = mcodes[mod_m(k + Lmax - f.n_fl)];
-                const int sb = mcodes[m - 1 - mod_m(k + Lmax - f.n_fr)];
+                    for (int r = 0; r < R; ++r) pc[(r >> 1) * 2 * L + (r & 1)] = pk_prmt(tf, tb, st.selA[r]) + st.selB[r];
+                    jf = jf + 1 == m ? 0 : jf + 1;
+                    jb = jb == 0 ? m - 1 : jb - 1;
+                }
+            } else {
+                for (int k = 0; k < m; ++k, pc += 2 * RH * L) {
+                    const int sf = mcodes[jf], sb = mcodes[jb];
 #pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    const int vf = sc.smat[myF[r] * STRK_NSYM_ + sf] + g2;
-                    const int vb = sc.smat[myB[r] * STRK_NSYM_ + sb] + g2;
-                    prof[((k * RH + (r >> 1)) * L + lane) * 2 + (r & 1)] = (unsigned)vf | ((unsigned)vb << 16);
+                    for (int r = 0; r < R; ++r) {
+                        const int vf = sc.smat[myF[r] * STRK_NSYM_ + sf] + g2;
+                        const int vb = sc.smat[myB[r] * STRK_NSYM_ + sb] + g2;
+                        pc[(r >> 1) * 2 * L + (r & 1)] = (unsigned)vf | ((unsigned)vb << 16);
+                    }
+                    jf = jf + 1 == m ? 0 : jf + 1;
+                    jb = jb == 0 ? m - 1 : jb - 1;
                 }
             }
         }
@@ -537,6 +591,7 @@ dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list,
     pk_run<R, L, CORE, FC, BC>(st, s, END, lane0, lane, one, tinc, ginc, ctp, prof_lane, pstride, pwrap, m,     \
                                last_cand_step, last_cand_stepB, scr)
 
+        PK_CLK(0);
         int s = 0;
         // ---- flank phase (PRMT look-ups).  Steps 0..SK-1 are the ramp-up of the unit's last lane, after which
         // the prefix maximum of the last row starts from scratch.
@@ -611,41 +666,79 @@ dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list,
 #undef PK_RUN
 
         __syncwarp();
+        PK_CLK(1);
+#if PK_PHASE_TIMERS
+        clk_acc[3] += 1ull;
+#endif
         // From here on the two units of a warp may run different trip counts (window sizes): every warp-level
         // primitive below names only the lanes of the unit (hmask).
         if (ref_mode) {
             // ---- reference mode: per size, the best cell of the captured column and the smallest row attaining it
             // (parasail end_query), for the forward (low halves, slots 0..nW) and the reverse alignment (high halves,
             // slots nW..2nW).  Key = (score + 32768) << 16 | (0xffff - row): one REDUX per column and direction.
+            // score + 32768 = h + (32768 - g * I) - g * p: the row term is a per-read constant, the column term is
+            // uniform, and PRMT puts the low 16 bits of the sum above the row code.  Pad rows take selector 0 on a
+            // zero byte: key 0, the value the maximum starts from, so they never win.
             long long *out64 = (long long *)table + 2 * f.out_off;
-            for (int w2 = 0; w2 < 2 * nW; ++w2) {
-                const int dir = w2 >= nW, w = dir ? w2 - nW : w2;
-                const int p = (dir ? f.n_fr : f.n_fl) + m * (f.n_lo + w);
-                unsigned key = 0u;
+            unsigned rc[R], rk[R], rsel[R];
 #pragma unroll
-                for (int q = 0; q < QN; ++q) {
-                    const uint4 v = scr[(unsigned)((w2 * QN + q) * L + lane)];
-                    const unsigned wv[4] = {v.x, v.y, v.z, v.w};
+            for (int r = 0; r < R; ++r) {
+                const int I = lane * R + r + 1, i = I - off;
+                rc[r] = (unsigned)(32768 - g * I);
+                rk[r] = i >= 1 ? (unsigned)(0xffff - i) : 0u;
+                rsel[r] = i >= 1 ? 0x5410u : 0u;  // bytes {rk.0, rk.1, x.0, x.1}
+            }
+            const uint4 *col = scr + lane;  // this lane's quads of captured column 0
+            for (int dir = 0; dir < 2; ++dir) {
+                if (dir) {  // high halves: the same sum, 16 bits up (no carry comes out of the low half: its addend is 0)
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const int r = 4 * q + j;
-                        if (r < R) {
-                            const int I = lane * R + r + 1, i = I - off;
-                            const int h = (int)(dir ? wv[j] >> 16 : wv[j] & 0xffffu);
-                            const unsigned k = ((unsigned)(h - g * (I + p) + 32768) << 16) | (unsigned)(0xffff - i);
-                            if (i >= 1) key = max(key, k);
-                        }
+                    for (int r = 0; r < R; ++r) {
+                        rc[r] <<= 16;
+                        rsel[r] = rsel[r] ? 0x7610u : 0u;  // bytes {rk.0, rk.1, x.2, x.3}
                     }
                 }
-                key = __reduce_max_sync(hmask, key);
-                if (lane0 && have) {
-                    const int score = (int)(key >> 16) - 32768, row = 0xffff - (int)(key & 0xffffu);
-                    out64[w2] = ((long long)score << 32) | (long long)(unsigned)(0x7fffffff - row);
+                const int p0 = (dir ? f.n_fr : f.n_fl) + m * f.n_lo;
+                auto column = [&](const uint4(&c)[QN], int w) {
+                    const unsigned gp = (unsigned)(-g * (p0 + m * w)), np = dir ? gp << 16 : gp;
+                    unsigned key = 0u;
+#pragma unroll
+                    for (int q = 0; q < QN; ++q) {
+                        const unsigned wv[4] = {c[q].x, c[q].y, c[q].z, c[q].w};
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) {
+                            const int r = 4 * q + j;
+                            if (r < R) key = max(key, pk_prmt(rk[r], wv[j] + rc[r] + np, rsel[r]));
+                        }
+                    }
+                    key = __reduce_max_sync(hmask, key);
+                    if (lane0 && have) {
+                        const int score = (int)(key >> 16) - 32768, row = 0xffff - (int)(key & 0xffffu);
+                        out64[dir * nW + w] = ((long long)score << 32) | (long long)(unsigned)(0x7fffffff - row);
+                    }
+                };
+                // WBR columns per batch of loads, so that their L2 round trips overlap
+                int w = 0;
+                for (; w + WBR <= nW; w += WBR, col += WBR * QN * L) {
+                    uint4 q4[WBR][QN];
+#pragma unroll
+                    for (int b = 0; b < WBR; ++b)
+#pragma unroll
+                        for (int q = 0; q < QN; ++q) q4[b][q] = col[(b * QN + q) * L];
+#pragma unroll
+                    for (int b = 0; b < WBR; ++b) column(q4[b], w + b);
+                }
+#pragma unroll 1
+                for (; w < nW; ++w, col += QN * L) {
+                    uint4 q1[QN];
+#pragma unroll
+                    for (int q = 0; q < QN; ++q) q1[q] = col[q * L];
+                    column(q1, w);
                 }
             }
             __syncwarp();
             for (int ln = lane; ln < 2 * nW * QN * L / 8; ln += L) pk_discard_line(scr + ln * 8);  // 128-byte lines
             __syncwarp();
+            PK_CLK(2);
             continue;
         }
         // ---- combine: score(n) for every candidate of the window
@@ -666,52 +759,60 @@ dp_packed_kernel(const FamDesc *__restrict__ fams, const int *__restrict__ list,
             }
         }
         const int bextra = (int)(scw[bbase + (unsigned)(((R >> 2) * L + (L - 1)) * 4 + (R & 3))] >> 16);
-        constexpr int WB = 4;  // candidates per batch of loads (hides the L2 round trip)
-        for (int g0 = 0; g0 < nW; g0 += L) {  // L candidates at a time: lane w keeps the reduced values of g0 + w
-            const int gend = g0 + L < nW ? g0 + L : nW;
-            unsigned my_v = 0u, my_flast = 0u;
-            for (int w0 = g0; w0 < gend; w0 += WB) {
+        constexpr int CW = QN * L;  // uint4 per captured column
+        for (int g0 = 0; g0 < nW; g0 += L) {  // L candidates at a time: lane w keeps the reduced value of g0 + w
+            const int gn = nW - g0 < L ? nW - g0 : L;
+            const uint4 *col = scr + (size_t)g0 * CW + lane;  // loads at compile-time offsets from one pointer
+            unsigned my_v = 0u;
+            int k = 0;
+            // whole batches without a per-candidate exit, then the remainder one candidate at a time
+            for (; k + WB <= gn; k += WB, col += WB * CW) {
                 uint4 q4[WB][QN];
 #pragma unroll
+                for (int b = 0; b < WB; ++b)
+#pragma unroll
+                    for (int q = 0; q < QN; ++q) q4[b][q] = col[b * CW + q * L];
+                const int lk = lane - k;
+#pragma unroll
                 for (int b = 0; b < WB; ++b) {
-                    const int ww = w0 + b < gend ? w0 + b : gend - 1;
-#pragma unroll
-                    for (int q = 0; q < QN; ++q) q4[b][q] = scr[(unsigned)((ww * QN + q) * L + lane)];
-                }
-#pragma unroll
-                for (int b = 0; b < WB; ++b) {
-                    const int ww = w0 + b;
-                    if (ww >= gend) break;  // uniform within the unit
-                    unsigned acc = 0u;
-#pragma unroll
-                    for (int q = 0; q < QN; ++q) {
-                        const uint4 v = q4[b][q];
-                        if (4 * q + 0 < R) acc = __viaddmax_u16x2(v.x, Bv[(4 * q + 0) % R], acc);
-                        if (4 * q + 1 < R) acc = __viaddmax_u16x2(v.y, Bv[(4 * q + 1) % R], acc);
-                        if (4 * q + 2 < R) acc = __viaddmax_u16x2(v.z, Bv[(4 * q + 2) % R], acc);
-                        if (4 * q + 3 < R) acc = __viaddmax_u16x2(v.w, Bv[(4 * q + 3) % R], acc);
-                    }
-                    const unsigned v = __reduce_max_sync(hmask, acc & 0xffffu);
-                    // the unit's last lane holds the prefix-max word of this candidate column (forward half)
-                    const unsigned pmw = (&q4[b][R >> 2].x)[R & 3];
-                    const unsigned flast = __shfl_sync(hmask, pmw, L - 1, L) & 0xffffu;
-                    if (lane == ww - g0) my_v = v, my_flast = flast;
+                    const unsigned v = __reduce_max_sync(hmask, pk_cand_max<R, QN>(q4[b], Bv));
+                    my_v = lk == b ? v : my_v;
                 }
             }
-            if (g0 + lane < gend && have) {  // un-bias and close the free-end cases: one candidate per lane
-                const int p = f.n_fl + m * (a_lo + g0 + lane);
+#pragma unroll 1
+            for (; k < gn; ++k, col += CW) {
+                uint4 q1[QN];
+#pragma unroll
+                for (int q = 0; q < QN; ++q) q1[q] = col[q * L];
+                const unsigned v = __reduce_max_sync(hmask, pk_cand_max<R, QN>(q1, Bv));
+                my_v = lane == k ? v : my_v;
+            }
+            if (lane < gn && have) {  // un-bias and close the free-end cases: one candidate per lane
+                const int w = g0 + lane;
+                const int p = f.n_fl + m * (a_lo + w);
                 int best = (int)my_v - g * (N + off + p + colsB);
-                if (s2_end) best = max(best, (int)my_flast - g * (N + p));
+                if (s2_end) {  // prefix maximum of the last row (forward half), word R of the unit's last lane
+                    const unsigned flast = scw[(unsigned)(((w * QN + (R >> 2)) * L + (L - 1)) * 4 + (R & 3))] & 0xffffu;
+                    best = max(best, (int)flast - g * (N + p));
+                }
                 if (s2_beg) {
                     const int border = s1_end ? -g : -g * n1;  // backward cell (n1, 0)
                     best = max(best, max(bextra - g * (N + colsB), border));
                 }
-                table[f.out_off + g0 + lane] = best;
+                table[f.out_off + w] = best;
             }
         }
         __syncwarp();
         // the captured columns of this read are dead: drop their lines from L2 instead of writing them back
         for (int ln = lane; ln < (nW + 1) * QN * L / 8; ln += L) pk_discard_line(scr + ln * 8);
         __syncwarp();
+        PK_CLK(2);
     }
+#if PK_PHASE_TIMERS
+    if (wlane == 0) {
+        unsigned long long *acc = pk_phase_clk[ref_mode ? 1 : 0][L == 16 ? 1 : 0][R];
+        for (int k = 0; k < 4; ++k) atomicAdd(acc + k, clk_acc[k]);
+    }
+#endif
+#undef PK_CLK
 }
