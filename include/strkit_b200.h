@@ -68,7 +68,8 @@ typedef struct strk_batch strk_batch;
 
 #define STRK_NSYM 17
 
-/* kernel selection for strk_batch_run / strk_count_reads */
+/* kernel selection for strk_batch_run / strk_count_reads and the raw tables (strk_score_tables,
+ * strk_ref_boundary_tables) */
 #define STRK_KERNEL_AUTO 0    /* packed u16x2 kernel where its preconditions hold, else general */
 #define STRK_KERNEL_GENERAL 1 /* int32 general kernel for everything (any length / alphabet)    */
 
@@ -172,7 +173,7 @@ int strk_score_tables(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes,
 int strk_ref_boundary_tables(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
                              const int32_t *lens, const int32_t *n_lo, const int32_t *n_hi, int64_t n_loci,
                              const uint64_t *motif_off, const int32_t *motif_len, const uint64_t *out_off,
-                             int32_t *out);
+                             int kernel, int32_t *out);
 
 /* get_ref_repeat_count for n_loci loci.  start_count / ref_size / rc params per locus
  * (rc_params[3l..] = {max_iters, local_search_range, step_size}, repeat_count_params.py:17-42).

@@ -56,7 +56,8 @@ def _load() -> C.CDLL:
                                             C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp]),
         "strk_score_tables": (C.c_int, [_vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp, C.c_int,
                                         _vp]),
-        "strk_ref_boundary_tables": (C.c_int, [_vp, _vp, _u64, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
+        "strk_ref_boundary_tables": (C.c_int, [_vp, _vp, _u64, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, C.c_int,
+                                               _vp]),
         "strk_ref_counts": (C.c_int, [_vp, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, C.c_int, C.c_int, _vp]),
         "strk_call_alleles": (C.c_int, [_vp, _vp, _vp, _vp, _i64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double,
                                         C.c_int, C.c_int, _u64, _vp, _vp, _vp, _vp]),

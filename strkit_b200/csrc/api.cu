@@ -1439,16 +1439,19 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
         return set_err(STRK_ERR_NOMEM, "%s: %s", who, cudaGetErrorString(e));
     }
     for (int k = 0; k < 8; ++k) ctx->stats[k] = 0;
-    if (ref || kernel == STRK_KERNEL_GENERAL || !ctx->h_consts.packed_ok) {
+    if (kernel == STRK_KERNEL_GENERAL || !ctx->h_consts.packed_ok) {
         rc = launch_general(ctx, ref, d_fams, nullptr, n_reads, d_arena, d_table, b_len, rowlen, ctx->stream);
         if (rc) return rc;
     } else {
-        // same routing as strk_batch_run: packed kernel per R, the rest (and its fallbacks) to the general kernel
+        // same routing as the batch paths (strk_batch_run, the first pass of strk_ref_counts): packed kernel per R,
+        // the rest (and its fallbacks) to the general kernel.  A reference window holds a forward and a reverse
+        // column per size, so it counts twice against PK_WINDOW_MAX.
         ClassLists lists;
         for (int64_t r = 0; r < n_reads; ++r) {
             const FamDesc &f = fams[(size_t)r];
             const int w = f.n_hi - f.n_lo + 1;
-            lists.add(w > 64 ? 0 : strk_pk_class(f.n_fl, f.n_tr, f.n_fr, f.m), (int)r, f.m, f.n_fl, f.n_fr, w);
+            const int cls = (ref ? 2 * w : w) > PK_WINDOW_MAX ? 0 : strk_pk_class(f.n_fl, f.n_tr, f.n_fr, f.m);
+            lists.add(cls, (int)r, f.m, f.n_fl, f.n_fr, w);
         }
         if (ctx->fallback.reserve((size_t)n_reads) != cudaSuccess) {
             cudaGetLastError();
@@ -1457,13 +1460,14 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
         const int *seg_list[STRK_PK_NBIN];
         long long seg_cnt[STRK_PK_NBIN];
         int seg_w[STRK_PK_NBIN];
-        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w[k] = (lists.w_max[k] + 3) / 4 * 4;
+        for (int k = 0; k < STRK_PK_NBIN; ++k)  // reference mode: forward + reverse columns of every size
+            seg_w[k] = ref ? 2 * lists.w_max[k] - 1 : (lists.w_max[k] + 3) / 4 * 4;
         rc = lists.upload(ctx->list_d, ctx->stream, seg_list, seg_cnt);
         if (rc) return rc;
         CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), ctx->stream));
         long long n_packed = 0;
         rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w, n_reads, d_fams, d_arena, d_table, b_len,
-                         rowlen, ctx->stream, 0, &n_packed);
+                         rowlen, ctx->stream, ref ? 1 : 0, &n_packed);
         if (rc) return rc;
         if (n_packed) {
             unsigned int fb = 0;
@@ -1471,8 +1475,8 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
             CU(cudaStreamSynchronize(ctx->stream));
             ctx->stats[6] = (double)(n_packed - (long long)fb);
         }
-        ctx->stats[7] = (double)n_reads - ctx->stats[6];
     }
+    ctx->stats[7] = (double)n_reads - ctx->stats[6];
     CU(cudaStreamSynchronize(ctx->stream));
     if (!ref) {
         CU(cudaMemcpy(out_host, d_table, (size_t)total * sizeof(int), cudaMemcpyDeviceToHost));
@@ -1508,9 +1512,9 @@ extern "C" int strk_score_tables(strk_ctx *ctx, const uint8_t *arena, uint64_t a
 extern "C" int strk_ref_boundary_tables(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes,
                                         const uint64_t *seq_off, const int32_t *lens, const int32_t *n_lo,
                                         const int32_t *n_hi, int64_t n_loci, const uint64_t *motif_off,
-                                        const int32_t *motif_len, const uint64_t *out_off, int32_t *out) {
+                                        const int32_t *motif_len, const uint64_t *out_off, int kernel, int32_t *out) {
     return tables_common(ctx, true, arena, arena_bytes, seq_off, lens, nullptr, n_lo, n_hi, n_loci, motif_off, motif_len,
-                         n_loci, out_off, STRK_KERNEL_GENERAL, out);
+                         n_loci, out_off, kernel, out);
 }
 
 // get_ref_repeat_count (repeats.py:73-192) for a batch of loci, device-resident from upload to results.

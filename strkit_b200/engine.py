@@ -221,7 +221,7 @@ class Engine:
                                     _p(batch.motif_len), batch.n_loci, _p(out_off), kernel, _p(scores)))
         return scores, out_off
 
-    def ref_boundary_tables(self, batch: ReadBatch, n_lo: np.ndarray, n_hi: np.ndarray):
+    def ref_boundary_tables(self, batch: ReadBatch, n_lo: np.ndarray, n_hi: np.ndarray, kernel: int = KERNEL_AUTO):
         """score_ref_boundaries for a window of sizes; one 'read' (the reference window) per locus.
         Returns (table[k] = (fwd_score, fwd_end_query, rev_score, rev_end_query), out_off)."""
         batch.validate()
@@ -236,7 +236,7 @@ class Engine:
         out = np.empty((int(width.sum()), 4), dtype=np.int32)
         check(lib.strk_ref_boundary_tables(self._ctx, _p(batch.arena), batch.arena.nbytes, _p(batch.seq_off),
                                            _p(batch.lens), _p(n_lo), _p(n_hi), batch.n_loci, _p(batch.motif_off),
-                                           _p(batch.motif_len), _p(out_off), _p(out)))
+                                           _p(batch.motif_len), _p(out_off), kernel, _p(out)))
         return out, out_off
 
     def ref_counts(self, batch: ReadBatch, start_count, ref_size, rc_params, vcf_anchor_size: int,

@@ -392,23 +392,29 @@ def test_ref_boundary_tables_many_strips(sb, oracle):
 
 
 def test_ref_boundary_tables_golden(sb, oracle, golden):
+    """Both kernels pinned to the golden vectors: the packed kernel in reference mode (KERNEL_AUTO) and the general
+    kernel's ARGMAX sweeps."""
     eng = sb.Engine()
     fams = [(c["motif"], c["tr_seq"], c["flank_left_seq"], c["flank_right_seq"]) for c in golden["boundaries"]]
     ns = np.array([c["n"] for c in golden["boundaries"]])
     lo = np.maximum(ns - 2, np.array([0 if (f[2] and f[3]) else 1 for f in fams]))
     hi = ns + 2
-    tab, off = eng.ref_boundary_tables(families_to_batch(fams), lo, hi)
-    for i, c in enumerate(golden["boundaries"]):
-        fs, fe, rs, re = (int(v) for v in tab[int(off[i]) + c["n"] - int(lo[i])])
-        r_adj = fe + 1 - len(c["flank_left_seq"]) - c["ref_size"]
-        l_adj = re + 1 - len(c["flank_right_seq"]) - c["ref_size"]
-        assert [fs, r_adj, rs, l_adj] == c["expect"], c
-        for n in range(int(lo[i]), int(hi[i]) + 1):  # the rest of the window against the oracle
-            (ofs, ora), (ors, ola) = oracle.score_ref_boundaries(c["tr_seq"], c["flank_left_seq"],
-                                                                 c["flank_right_seq"], c["motif"], n, c["ref_size"])
-            fs, fe, rs, re = (int(v) for v in tab[int(off[i]) + n - int(lo[i])])
-            assert (fs, fe + 1 - len(c["flank_left_seq"]) - c["ref_size"]) == (ofs, ora)
-            assert (rs, re + 1 - len(c["flank_right_seq"]) - c["ref_size"]) == (ors, ola)
+    for kernel in (sb.KERNEL_AUTO, sb.KERNEL_GENERAL):
+        tab, off = eng.ref_boundary_tables(families_to_batch(fams), lo, hi, kernel=kernel)
+        st = eng.stats()
+        assert st["reads_packed_kernel"] + st["reads_general_kernel"] == len(fams)
+        assert (st["reads_packed_kernel"] > 0) == (kernel == sb.KERNEL_AUTO)
+        for i, c in enumerate(golden["boundaries"]):
+            fs, fe, rs, re = (int(v) for v in tab[int(off[i]) + c["n"] - int(lo[i])])
+            r_adj = fe + 1 - len(c["flank_left_seq"]) - c["ref_size"]
+            l_adj = re + 1 - len(c["flank_right_seq"]) - c["ref_size"]
+            assert [fs, r_adj, rs, l_adj] == c["expect"], (kernel, c)
+            for n in range(int(lo[i]), int(hi[i]) + 1):  # the rest of the window against the oracle
+                (ofs, ora), (ors, ola) = oracle.score_ref_boundaries(c["tr_seq"], c["flank_left_seq"],
+                                                                     c["flank_right_seq"], c["motif"], n, c["ref_size"])
+                fs, fe, rs, re = (int(v) for v in tab[int(off[i]) + n - int(lo[i])])
+                assert (fs, fe + 1 - len(c["flank_left_seq"]) - c["ref_size"]) == (ofs, ora), (kernel, c, n)
+                assert (rs, re + 1 - len(c["flank_right_seq"]) - c["ref_size"]) == (ors, ola), (kernel, c, n)
 
 
 def test_invalid_inputs_raise(sb):
