@@ -177,7 +177,9 @@ int strk_ref_boundary_tables(strk_ctx *ctx, const uint8_t *arena, uint64_t arena
 
 /* get_ref_repeat_count for n_loci loci.  start_count / ref_size / rc params per locus
  * (rc_params[3l..] = {max_iters, local_search_range, step_size}, repeat_count_params.py:17-42).
- * out[8l..] = {cn, score, l_offset, r_offset, n_offset_scores, n_iters_final, new_len_fl, new_len_fr}. */
+ * out[8l..] = {cn, score, l_offset, r_offset, n_offset_scores, n_iters_final, new_len_fl, new_len_fr}.
+ * Afterwards stats[5] (strk_get_stats) counts the loci whose search left the windows the device tried first and that
+ * the host finished. */
 int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
                     const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
                     const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off, const int32_t *motif_len,

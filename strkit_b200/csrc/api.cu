@@ -112,24 +112,35 @@ struct ClassLists {
     }
 };
 
+// One search-parameter tier of a strk_ref_counts call (repeat_count_params.py:17-42): phase 2 runs once per tier
+struct RefTier {
+    int rc[3];             // max_iters, local search range, step size
+    int wd2, W2;           // phase 2's first window: half-width, sizes
+    std::vector<int> ids;  // its loci, ascending
+    ClassLists classes;    // phase 2's classes over the tier's slots (unused when phase 1's lists serve)
+};
+
 // The reference path's per-locus state (strk_ref_counts), recycled across calls
 struct RefBufs {
     DevBuf<unsigned char> arena;
     DevBuf<unsigned long long> seq_off, motif_off;
     DevBuf<int> lens, start, ref_size, rc, motif_len;  // the caller's arrays
-    DevBuf<int> wd;                                    // half-width of each locus' first boundary window
+    DevBuf<int> wd;                                    // half-width of each locus' next boundary window
     DevBuf<int> l_off, r_off, n_off;                   // phase 1 results
-    DevBuf<int> ids_a, ids_b;                          // locus lists: pending loci of phase 1, the loci of a tier
+    DevBuf<int> ids_a, ids_b;                          // locus lists: pending loci of phase 1, the flagged loci of a tier
+    DevBuf<int> tier_ids;                              // the loci of every tier, tier after tier
     DevBuf<int> lists;                                 // class lists of a packed pass
     DevBuf<unsigned int> cnt;                          // counters of ref_replay1_kernel: [0, 4) a pass, [4, 8) a second look
-    DevBuf<int> out;                                   // fast path: the results, assembled on the device
-    // host sources of asynchronous copies: alive until the stream has passed them (the fast path synchronises once)
+    DevBuf<int> out;                                   // the results, assembled on the device
+    DevBuf<unsigned char> redo;                        // per locus: left to the host (a search left its window)
+    // host sources of asynchronous copies: alive until the stream has passed them (one synchronisation per call)
     std::vector<int> h_wd;
     ClassLists classes;
+    std::vector<RefTier> tiers;
     void release() {
         arena.release(), seq_off.release(), motif_off.release(), lens.release(), start.release(), ref_size.release();
         rc.release(), motif_len.release(), wd.release(), l_off.release(), r_off.release(), n_off.release();
-        ids_a.release(), ids_b.release(), lists.release(), cnt.release(), out.release();
+        ids_a.release(), ids_b.release(), tier_ids.release(), lists.release(), cnt.release(), out.release(), redo.release();
     }
 };
 
@@ -1517,68 +1528,6 @@ extern "C" int strk_ref_boundary_tables(strk_ctx *ctx, const uint8_t *arena, uin
                          n_loci, out_off, kernel, out);
 }
 
-// get_ref_repeat_count (repeats.py:73-192) for a batch of loci, device-resident from upload to results.
-// Phase 1: boundary tables (two sg_qe sweeps per locus, every candidate size of a window at once, general kernel)
-// + the dual-score search replayed one thread per locus -> l_offset / r_offset; loci whose search leaves the
-// window are redone 4x wider.  Phase 2: the final get_repeat_count on the adjusted flanks = the read-path batch
-// machinery (packed kernel, device replay, widening) with one "read" per locus, one run per search-parameter tier.
-static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
-                           const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
-                           const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off, const int32_t *motif_len,
-                           int vcf_anchor_size, int32_t *out, std::vector<int> &redo, bool *taken);
-static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
-                           const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
-                           const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off,
-                           const int32_t *motif_len, int vcf_anchor_size, int respect_coords, int32_t *out);
-
-// Fast path first (one host synchronisation for the whole call: every decision between the kernels is taken on the
-// device); the loci it could not finish -- a search that left its first window -- and the calls it does not take
-// (several search-parameter tiers, respect_coords) go through the general path below, pass by pass.
-extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
-                               const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
-                               const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off,
-                               const int32_t *motif_len, int vcf_anchor_size, int respect_coords, int32_t *out) {
-    if (!ctx || !arena || !seq_off || !lens || !start_count || !ref_size || !rc_params || !motif_off || !motif_len || !out)
-        return set_err(STRK_ERR_ARG, "strk_ref_counts: null argument");
-    if (n_loci <= 0 || n_loci > 0x7ffffff0LL) return set_err(STRK_ERR_ARG, "strk_ref_counts: bad locus count");
-    static const bool no_fast = getenv("STRK_REF_SLOW") != nullptr;  // (measurement only)
-    bool taken = false;
-    std::vector<int> redo;
-    if (!respect_coords && !no_fast) {
-        int rc = ref_counts_fast(ctx, arena, arena_bytes, seq_off, lens, start_count, ref_size, rc_params, n_loci, motif_off,
-                                 motif_len, vcf_anchor_size, out, redo, &taken);
-        if (rc) return rc;
-    }
-    if (!taken)
-        return ref_counts_slow(ctx, arena, arena_bytes, seq_off, lens, start_count, ref_size, rc_params, n_loci, motif_off,
-                               motif_len, vcf_anchor_size, respect_coords, out);
-    if (redo.empty()) return STRK_OK;
-    // the few loci left over: their own little call through the general path (compact copies of their sequences)
-    double keep[8];
-    memcpy(keep, ctx->stats, sizeof(keep));
-    const size_t nr = redo.size();
-    std::vector<unsigned char> sub_arena;
-    std::vector<uint64_t> so(nr), mo(nr);
-    std::vector<int32_t> ln(3 * nr), sc(nr), rs(nr), rcp(3 * nr), ml(nr), sub_out(8 * nr);
-    for (size_t q = 0; q < nr; ++q) {
-        const int l = redo[q];
-        const int n1 = lens[3 * l] + lens[3 * l + 1] + lens[3 * l + 2];
-        so[q] = sub_arena.size();
-        sub_arena.insert(sub_arena.end(), arena + seq_off[l], arena + seq_off[l] + n1);
-        mo[q] = sub_arena.size();
-        sub_arena.insert(sub_arena.end(), arena + motif_off[l], arena + motif_off[l] + motif_len[l]);
-        for (int k = 0; k < 3; ++k) ln[3 * q + k] = lens[3 * l + k], rcp[3 * q + k] = rc_params[3 * l + k];
-        sc[q] = start_count[l], rs[q] = ref_size[l], ml[q] = motif_len[l];
-    }
-    int rc = ref_counts_slow(ctx, sub_arena.data(), sub_arena.size(), so.data(), ln.data(), sc.data(), rs.data(), rcp.data(),
-                             (int64_t)nr, mo.data(), ml.data(), vcf_anchor_size, 0, sub_out.data());
-    if (rc) return rc;
-    for (size_t q = 0; q < nr; ++q) memcpy(out + 8 * (size_t)redo[q], sub_out.data() + 8 * q, 8 * sizeof(int32_t));
-    for (int k = 0; k < 8; ++k) ctx->stats[k] += keep[k];
-    ctx->stats[5] = keep[5] + (double)nr;  // loci redone
-    return STRK_OK;
-}
-
 // First window of the boundary search: start +- max(6, range + step + 2) sizes, like the read path's (a search that
 // starts where it ends touches start +- (range + step)); one that leaves it is redone 4x wider.  Measured on 32 768
 // HiFi-sized windows: +- 9 sizes 3.89 ms, +- 7 3.79 ms, +- 6 3.33 ms per block.  STRK_REF_WD=<n> raises the floor of 6
@@ -1588,9 +1537,8 @@ static int ref_first_wd(int range, int step) {
     return std::max(wd_env > 0 ? wd_env : 6, range + step + 2);
 }
 
-// The steps both drivers of strk_ref_counts start with: argument checks, the first boundary window of every locus
-// (ctx->ref.h_wd), the context's reference buffers, and the upload of the inputs with phase 1's results cleared, queued
-// on `st`.
+// The first steps of strk_ref_counts: argument checks, the first boundary window of every locus (ctx->ref.h_wd), the
+// context's reference buffers, and the upload of the inputs with phase 1's results cleared, queued on `st`.
 static int ref_setup(strk_ctx *ctx, cudaStream_t st, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
                      const int32_t *lens, const int32_t *start_count, const int32_t *ref_size, const int32_t *rc_params,
                      int64_t n_loci, const uint64_t *motif_off, const int32_t *motif_len) {
@@ -1615,9 +1563,13 @@ static int ref_setup(strk_ctx *ctx, cudaStream_t st, const uint8_t *arena, uint6
     if (e == cudaSuccess) e = d.motif_off.reserve(n);
     for (DevBuf<int> *p : {&d.lens, &d.rc})
         if (e == cudaSuccess) e = p->reserve(3 * n);
-    for (DevBuf<int> *p : {&d.start, &d.ref_size, &d.motif_len, &d.wd, &d.l_off, &d.r_off, &d.n_off, &d.ids_a, &d.ids_b})
+    // (lists: every class-list upload of the call then fits, and none reallocates a buffer a queued pass still reads)
+    for (DevBuf<int> *p : {&d.start, &d.ref_size, &d.motif_len, &d.wd, &d.l_off, &d.r_off, &d.n_off, &d.ids_a, &d.ids_b,
+                           &d.tier_ids, &d.lists})
         if (e == cudaSuccess) e = p->reserve(n);
     if (e == cudaSuccess) e = d.cnt.reserve(8);
+    if (e == cudaSuccess) e = d.out.reserve(8 * n + 8);
+    if (e == cudaSuccess) e = d.redo.reserve(n);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
@@ -1637,12 +1589,55 @@ static int ref_setup(strk_ctx *ctx, cudaStream_t st, const uint8_t *arena, uint6
     return STRK_OK;
 }
 
-static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
-                           const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
-                           const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off,
-                           const int32_t *motif_len, int vcf_anchor_size, int respect_coords, int32_t *out) {
+// One widening round of phase 1: the loci of `ids` (n of them; with d_n, the first min(n, *d_n)) at the windows
+// ref_replay1_kernel raised for them (d.wd, at most wd sizes either side) through the general kernel, then replayed.
+// Those that leave their window again are appended to `again`; `cnt` gets the counters of ref_replay1_kernel.
+static int ref_widen(strk_ctx *ctx, const int *ids, int n, const unsigned int *d_n, int wd, int *again, unsigned int *cnt,
+                     int b_len, int rowlen, int vcf_anchor_size) {
+    RefBufs &d = ctx->ref;
+    cudaStream_t st = ctx->stream;
+    const int T = 128, WD_MAX = (STRK_MAX_WINDOW - 1) / 2;
+    ref_plan1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(ids, n, d.seq_off.p, d.lens.p, d.start.p, d.wd.p, d.motif_off.p,
+                                                               d.motif_len.p, 2 * wd + 1, ctx->fams.p, d_n);
+    CU(cudaGetLastError());
+    int rc = launch_general(ctx, true, ctx->fams.p, nullptr, n, d.arena.p, ctx->table64.p, b_len, rowlen, st, d_n);
+    if (rc) return rc;
+    ref_replay1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(ids, n, ctx->table64.p, ctx->fams.p, d.start.p, d.rc.p,
+                                                                 d.ref_size.p, vcf_anchor_size, WD_MAX, d.wd.p, d.l_off.p,
+                                                                 d.r_off.p, d.n_off.p, again, cnt, d_n);
+    CU(cudaGetLastError());
+    return STRK_OK;
+}
+
+// The errors of a phase 1 pass, from the counters of ref_replay1_kernel
+static int ref_search_error(const unsigned int *cnt, const int32_t *rc_params) {
+    if (cnt[2])
+        return set_err(STRK_ERR_SEARCH, "strk_ref_counts: locus %lld left the widest window", (long long)(0x7fffffffu - cnt[2]));
+    if (cnt[1]) {
+        const long long l = (long long)(0x7fffffffu - cnt[1]);
+        return set_err(STRK_ERR_SEARCH, "strk_ref_counts: locus %lld scored no size (max_iters = %d)", l, rc_params[3 * l]);
+    }
+    return STRK_OK;
+}
+
+// get_ref_repeat_count (repeats.py:73-192) for a batch of loci, device-resident from upload to results.
+// Phase 1 (skipped with respect_coords, repeats.py:99): boundary tables (two sg_qe sweeps per locus, every candidate
+// size of a window at once: the packed kernel in reference mode) + the dual-score search replayed one thread per locus
+// -> l_offset / r_offset; a second look redoes up to CAP2 loci whose search left the first window 4x wider.  Phase 2:
+// the final count on the adjusted flanks = the read-path kernels (packed kernel, device replay) with one "read" per
+// locus, one pass per search-parameter tier, and a kernel that assembles the 8 result ints per locus.  Everything is
+// queued on the context's stream; ONE synchronisation brings back the results and the flags of the loci the device did
+// not settle (a search that left the window of the second look, or of phase 2).  The host finishes those, on the
+// buffers already resident: phase 1 4x wider per round, then phase 2 through strk_batch_run, which widens as far as a
+// search needs.  (Every host synchronisation of a call under another context's read kernels waits for SM slots that
+// the persistent read CTAs free only at the end of a class launch.)
+extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
+                               const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
+                               const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off,
+                               const int32_t *motif_len, int vcf_anchor_size, int respect_coords, int32_t *out) {
+    if (!ctx || !arena || !seq_off || !lens || !start_count || !ref_size || !rc_params || !motif_off || !motif_len || !out)
+        return set_err(STRK_ERR_ARG, "strk_ref_counts: null argument");
     if (n_loci <= 0 || n_loci > 0x7ffffff0LL) return set_err(STRK_ERR_ARG, "strk_ref_counts: bad locus count");
-    const bool timing = getenv("STRK_REF_TIMING") != nullptr;  // coarse phase timers on stderr (tuning only)
     auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     const double t_begin = now();
     cudaStream_t st = ctx->stream;
@@ -1650,217 +1645,21 @@ static int ref_counts_slow(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
                        motif_len);
     if (rc) return rc;
     RefBufs &d = ctx->ref;
-    const std::vector<int> &h_wd = d.h_wd;
-    const int WD_MAX = (STRK_MAX_WINDOW - 1) / 2;
-    int max_wd = 6, max_n1 = 0, mb_cols = 0, mb_m = 0;
-    for (int64_t l = 0; l < n_loci; ++l) {
-        max_wd = std::max(max_wd, h_wd[(size_t)l]);
-        const int n1 = lens[3 * l] + lens[3 * l + 1] + lens[3 * l + 2];
-        max_n1 = std::max(max_n1, n1);
-        if (n1 > 32 * 16) {  // multi-pass reads of the general kernel keep a boundary row per candidate column
-            mb_cols = std::max(mb_cols, std::max(lens[3 * l], lens[3 * l + 2]) + motif_len[l] * start_count[l]);
-            mb_m = std::max(mb_m, motif_len[l]);
-        }
-    }
-    // counters of this call (strk_get_stats afterwards): the boundary sweeps of phase 1 + the batch runs of phase 2
-    double acc_stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     const size_t n = (size_t)n_loci;
-    const int T = 128;
+    const bool phase1 = !respect_coords;
+    const bool packed_ok = ctx->h_consts.packed_ok;
+    const int CAP2 = 4096, WD_MAX = (STRK_MAX_WINDOW - 1) / 2, T = 128;
+    // phase 1's table stride: the widest first window; the second look's: 4x that
+    const int wd1 = *std::max_element(d.h_wd.begin(), d.h_wd.end()), stride_w = 2 * wd1 + 1;
+    const int wd1b = std::min(WD_MAX, 4 * wd1), stride_w2 = 2 * wd1b + 1;
+    const bool packed1 = packed_ok && 2 * stride_w <= PK_WINDOW_MAX;  // a forward and a reverse column per size
 
-    // ---- phase 1: boundary extension (skipped with respect_coords, repeats.py:99)
-    if (!respect_coords) {
-        long long n_pending = n_loci;
-        const int *d_ids = nullptr;
-        int *d_again = d.ids_a.p;
-        int cur_wd = max_wd;
-        while (n_pending > 0) {
-            const int stride_w = 2 * cur_wd + 1;
-            if (ctx->fams.reserve((size_t)n_pending) != cudaSuccess ||
-                ctx->table64.reserve((size_t)n_pending * (size_t)stride_w * 2) != cudaSuccess) {
-                cudaGetLastError();
-                return set_err(STRK_ERR_NOMEM, "strk_ref_counts: cannot allocate the boundary tables");
-            }
-            ref_plan1_kernel<<<(unsigned)((n_pending + T - 1) / T), T, 0, st>>>(d_ids, (int)n_pending, d.seq_off.p, d.lens.p,
-                                                                                d.start.p, d.wd.p, d.motif_off.p, d.motif_len.p,
-                                                                                stride_w, ctx->fams.p);
-            CU(cudaGetLastError());
-            const int b_len = max_n1 + 2;
-            const int rowlen = max_n1 > 32 * 16 ? mb_cols + mb_m * cur_wd + 2 : 2;
-            CU(cudaEventRecord(ctx->ev[0], st));
-            if (d_ids == nullptr) {  // executed cells of the first pass: two sweeps of db x (flank + motif * n_hi)
-                for (int64_t l = 0; l < n_loci; ++l) {
-                    const double n1 = (double)lens[3 * l] + lens[3 * l + 1] + lens[3 * l + 2];
-                    const double hi = (double)start_count[l] + h_wd[(size_t)l];
-                    acc_stats[0] += n1 * ((double)lens[3 * l] + lens[3 * l + 2] + 2.0 * motif_len[l] * hi);
-                }
-            }
-            if (d_ids == nullptr && ctx->h_consts.packed_ok && 2 * stride_w <= PK_WINDOW_MAX) {
-                // first pass (locus q = q): packed kernel in reference mode per rows-per-lane class, the forward and
-                // the reverse sg_qe alignment of a locus in the two halves of its lane words; the rest -> general
-                ClassLists lists;
-                for (int64_t l = 0; l < n_loci; ++l) {
-                    const int fl = lens[3 * l], fr = lens[3 * l + 2], m = motif_len[l];
-                    lists.add(strk_pk_class(fl, lens[3 * l + 1], fr, m), (int)l, m, fl, fr);
-                }
-                if (ctx->fallback.reserve(n) != cudaSuccess) {
-                    cudaGetLastError();
-                    return set_err(STRK_ERR_NOMEM, "strk_ref_counts: cannot allocate the fallback list");
-                }
-                const int *seg_list[STRK_PK_NBIN];
-                long long seg_cnt[STRK_PK_NBIN];
-                int seg_w[STRK_PK_NBIN];
-                for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w[k] = 2 * stride_w - 1;  // forward + reverse columns of every size
-                rc = lists.upload(d.lists, st, seg_list, seg_cnt);
-                if (rc) return rc;
-                CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
-                long long n_packed = 0;
-                rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w, n_loci, ctx->fams.p, d.arena.p,
-                                 ctx->table64.p, b_len, rowlen, st, 1, &n_packed);
-                if (rc) return rc;
-                CU(cudaStreamSynchronize(st));  // `lists` is read by the copy
-            } else {
-                rc = launch_general(ctx, true, ctx->fams.p, nullptr, n_pending, d.arena.p, ctx->table64.p, b_len, rowlen, st);
-                if (rc) return rc;
-            }
-            CU(cudaEventRecord(ctx->ev[1], st));
-            CU(cudaMemsetAsync(d.cnt.p, 0, 4 * sizeof(unsigned int), st));
-            ref_replay1_kernel<<<(unsigned)((n_pending + T - 1) / T), T, 0, st>>>(
-                d_ids, (int)n_pending, ctx->table64.p, ctx->fams.p, d.start.p, d.rc.p, d.ref_size.p, vcf_anchor_size, WD_MAX,
-                d.wd.p, d.l_off.p, d.r_off.p, d.n_off.p, d_again, d.cnt.p);
-            CU(cudaGetLastError());
-            CU(cudaEventRecord(ctx->ev[2], st));
-            ctx->stats[2] += 2;
-            unsigned int h_cnt[4] = {0, 0, 0, 0};
-            CU(cudaMemcpyAsync(h_cnt, d.cnt.p, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            {
-                float t0 = 0.f, t1 = 0.f;
-                CU(cudaEventElapsedTime(&t0, ctx->ev[0], ctx->ev[1]));
-                CU(cudaEventElapsedTime(&t1, ctx->ev[1], ctx->ev[2]));
-                acc_stats[3] += t0;
-                acc_stats[4] += t1;
-            }
-            if (h_cnt[2])
-                return set_err(STRK_ERR_SEARCH, "strk_ref_counts: locus %lld left the widest window",
-                               (long long)(0x7fffffffu - h_cnt[2]));
-            if (h_cnt[1]) {
-                const long long l = (long long)(0x7fffffffu - h_cnt[1]);
-                return set_err(STRK_ERR_SEARCH, "strk_ref_counts: locus %lld scored no size (max_iters = %d)", l,
-                               rc_params[3 * l]);
-            }
-            n_pending = h_cnt[0];
-            acc_stats[5] += (double)n_pending;
-            d_ids = d_again;
-            d_again = d_again == d.ids_a.p ? d.ids_b.p : d.ids_a.p;
-            cur_wd = std::min(WD_MAX, cur_wd * 4);
-        }
-    }
-    const double t_phase1 = now();
-    acc_stats[2] = ctx->stats[2];
-    std::vector<int> l_off(n), r_off(n), n_off(n);
-    CU(cudaMemcpyAsync(l_off.data(), d.l_off.p, n * sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(r_off.data(), d.r_off.p, n * sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(n_off.data(), d.n_off.p, n * sizeof(int), cudaMemcpyDeviceToHost, st));
-
-    // ---- phase 2: final count on the adjusted flanks (repeats.py:171-188), one batch run per parameter tier
-    std::vector<std::vector<int>> tiers;
-    std::vector<int> tier_key;  // 3 ints per tier
-    for (int64_t l = 0; l < n_loci; ++l) {
-        size_t t = 0;
-        for (; t < tiers.size(); ++t)
-            if (tier_key[3 * t] == rc_params[3 * l] && tier_key[3 * t + 1] == rc_params[3 * l + 1] &&
-                tier_key[3 * t + 2] == rc_params[3 * l + 2])
-                break;
-        if (t == tiers.size()) {
-            tiers.emplace_back();
-            tier_key.insert(tier_key.end(), rc_params + 3 * l, rc_params + 3 * l + 3);
-        }
-        tiers[t].push_back((int)l);
-    }
-    if (!ctx->ref_batch) ctx->ref_batch = new (std::nothrow) strk_batch();
-    if (!ctx->ref_batch) return set_err(STRK_ERR_NOMEM, "out of host memory");
-    strk_batch *b = ctx->ref_batch;
-    std::vector<int> res;
-    for (size_t t = 0; t < tiers.size(); ++t) {
-        const std::vector<int> &ids = tiers[t];
-        const size_t nt = ids.size();
-        const cudaError_t e = batch_bind(b, (long long)nt, (long long)nt);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
-        }
-        b->d_arena = d.arena.p;
-        b->h_read_begin.resize(nt + 1);
-        for (size_t q = 0; q <= nt; ++q) b->h_read_begin[q] = (long long)q;
-        CU(cudaMemcpyAsync(d.ids_a.p, ids.data(), nt * sizeof(int), cudaMemcpyHostToDevice, st));
-        ref_plan2_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(d.ids_a.p, (int)nt, d.seq_off.p, d.lens.p, d.start.p,
-                                                                     d.motif_off.p, d.motif_len.p, d.l_off.p, d.r_off.p,
-                                                                     b->d_seq_off, b->d_lens, b->d_est, b->d_motif_off,
-                                                                     b->d_motif_len, b->d_read_begin);
-        CU(cudaGetLastError());
-        CU(cudaStreamSynchronize(st));  // `ids` is read by the copy above
-        rc = batch_plan(ctx, b, arena_bytes);
-        if (rc) return rc;
-        rc = strk_batch_run(ctx, b, tier_key[3 * t], tier_key[3 * t + 1], tier_key[3 * t + 2], STRK_KERNEL_AUTO, nullptr);
-        if (rc) return rc;
-        for (int k = 0; k < 8; ++k) acc_stats[k] += ctx->stats[k];  // strk_batch_run reports its own run only
-        res.resize(nt * 4);
-        CU(cudaMemcpy(res.data(), b->d_out, nt * 4 * sizeof(int), cudaMemcpyDeviceToHost));
-        for (size_t q = 0; q < nt; ++q) {
-            const int l = ids[q];
-            int32_t *o = out + 8 * (size_t)l;
-            o[0] = res[4 * q], o[1] = res[4 * q + 1], o[2] = l_off[(size_t)l], o[3] = r_off[(size_t)l];
-            o[4] = n_off[(size_t)l], o[5] = res[4 * q + 2];
-            o[6] = lens[3 * l] - std::max(0, l_off[(size_t)l]);
-            o[7] = lens[3 * l + 2] - std::max(0, r_off[(size_t)l]);
-        }
-    }
-    for (int k = 0; k < 8; ++k) ctx->stats[k] = acc_stats[k];
-    if (timing)
-        fprintf(stderr, "[strk_ref_counts] %lld loci: upload + phase 1 %.2f ms, phase 2 %.2f ms (host clock); DP kernels %.2f ms, "
-                "replay kernels %.2f ms (device clock), %d kernels\n", (long long)n_loci, t_phase1 - t_begin, now() - t_phase1,
-                acc_stats[3], acc_stats[4], (int)acc_stats[2]);
-    return STRK_OK;
-}
-
-// The fast path of strk_ref_counts: one search-parameter tier, first windows that fit the packed kernel.  Everything
-// from the upload to the assembled results is queued on the context's stream without a host round trip in between:
-// phase 1 (boundary tables + dual-score replay), phase 2 (the final count: the same loci as one "read" each through
-// the read-path kernels -- their rows-per-lane class depends on the window's length only, which moving bases between
-// flank and tract does not change, so the class lists built on the host for phase 1 serve both phases and no device-side
-// planning pass is needed), and a kernel that assembles the 8 result ints per locus.  ONE synchronisation at the end
-// brings back the results and the flags of the loci whose search left a window; those are returned in `redo`.
-// (The general path takes 8 host synchronisations per call: harmless alone, but under another context's read kernels
-// every one of them waits for SM slots that the persistent read CTAs free only at the end of a class launch.)
-static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_bytes, const uint64_t *seq_off,
-                           const int32_t *lens, const int32_t *start_count, const int32_t *ref_size,
-                           const int32_t *rc_params, int64_t n_loci, const uint64_t *motif_off, const int32_t *motif_len,
-                           int vcf_anchor_size, int32_t *out, std::vector<int> &redo, bool *taken) {
-    *taken = false;
-    if (!ctx->h_consts.packed_ok) return STRK_OK;
-    for (int64_t l = 1; l < n_loci; ++l)
-        if (rc_params[3 * l] != rc_params[0] || rc_params[3 * l + 1] != rc_params[1] || rc_params[3 * l + 2] != rc_params[2])
-            return STRK_OK;  // several tiers: the general path groups them
-    const int max_iters = rc_params[0], range = rc_params[1], step = rc_params[2];
-    if (max_iters < 0 || range < 0 || step < 0 || range > 1000 || step > 1000)
-        return set_err(STRK_ERR_ARG, "strk_ref_counts: bad search parameters");
-    const int wd1 = ref_first_wd(range, step);
-    const int stride_w = 2 * wd1 + 1;
-    int wd2 = range + step + 2;  // phase 2: the read path's first window
-    if (wd2 < 6) wd2 = 6;
-    const int W2 = 2 * wd2 + 1;
-    if (2 * stride_w > PK_WINDOW_MAX || W2 > PK_WINDOW_MAX) return STRK_OK;
-    *taken = true;
-    cudaStream_t st = ctx->stream;
-    int rc = ref_setup(ctx, st, arena, arena_bytes, seq_off, lens, start_count, ref_size, rc_params, n_loci, motif_off,
-                       motif_len);
-    if (rc) return rc;
-    RefBufs &d = ctx->ref;
-    const size_t n = (size_t)n_loci;
-    int max_n1 = 0, mb_cols = 0, mb_m = 0;
-    ClassLists &lists = d.classes;  // (on the context: read by an asynchronous copy until the one synchronisation)
-    lists.clear();
+    // ---- host plan: phase 1's classes, scratch maxima, the tiers in first-appearance order
+    int max_n1 = 0, mb_cols = 0, mb_m = 0, wd2_max = 0;
     double cells1 = 0.0;
+    ClassLists &lists = d.classes;
+    lists.clear();
+    size_t n_tiers = 0;
     for (int64_t l = 0; l < n_loci; ++l) {
         const int fl = lens[3 * l], tr = lens[3 * l + 1], fr = lens[3 * l + 2], m = motif_len[l];
         const int n1 = fl + tr + fr;
@@ -1871,22 +1670,50 @@ static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
             mb_cols = std::max(mb_cols, std::max(fl, fr) + m * (start_count[l] + (fl + fr) / m + 1));
             mb_m = std::max(mb_m, m);
         }
-        lists.add(strk_pk_class(fl, tr, fr, m), (int)l, m, fl, fr);
-        cells1 += (double)n1 * ((double)fl + fr + 2.0 * m * ((double)start_count[l] + wd1));
+        if (phase1) {  // executed cells of the first pass: two sweeps of db x (flank + motif * n_hi)
+            lists.add(packed1 ? strk_pk_class(fl, tr, fr, m) : 0, (int)l, m, fl, fr);
+            cells1 += (double)n1 * ((double)fl + fr + 2.0 * m * ((double)start_count[l] + d.h_wd[(size_t)l]));
+        }
+        const int32_t *p = rc_params + 3 * l;
+        size_t t = 0;
+        while (t < n_tiers && !std::equal(p, p + 3, d.tiers[t].rc)) ++t;
+        if (t == n_tiers) {
+            if (n_tiers == d.tiers.size()) d.tiers.emplace_back();
+            RefTier &nt = d.tiers[n_tiers++];
+            std::copy(p, p + 3, nt.rc);
+            nt.wd2 = std::max(6, p[1] + p[2] + 2);  // the read path's first window
+            nt.W2 = 2 * nt.wd2 + 1;
+            nt.ids.clear();
+            nt.classes.clear();
+            wd2_max = std::max(wd2_max, nt.wd2);
+        }
+        d.tiers[t].ids.push_back((int)l);
     }
+    d.tiers.resize(n_tiers);  // (the vectors of the tiers kept keep their capacity for the next call)
+    // one tier classed like phase 1: phase 2 takes phase 1's lists (moving bases between flank and tract does not change
+    // a window's class), slot q = locus q
+    const bool reuse = phase1 && d.tiers.size() == 1 && packed1 == (packed_ok && d.tiers[0].W2 <= PK_WINDOW_MAX);
+    size_t table2 = 0;
+    for (RefTier &t : d.tiers) {
+        table2 = std::max(table2, t.ids.size() * (size_t)t.W2);
+        const bool packed2 = packed_ok && t.W2 <= PK_WINDOW_MAX;
+        for (size_t q = 0; q < t.ids.size() && !reuse; ++q) {
+            const int l = t.ids[q];
+            const int fl = lens[3 * l], tr = lens[3 * l + 1], fr = lens[3 * l + 2], m = motif_len[l];
+            t.classes.add(packed2 ? strk_pk_class(fl, tr, fr, m) : 0, (int)q, m, fl, fr);
+        }
+    }
+    auto rowlen_for = [&](int wd) { return max_n1 > 32 * 16 ? mb_cols + mb_m * wd + 2 : 2; };
+    const int b_len = max_n1 + 2, rowlen = rowlen_for(std::max(std::max(wd1, wd2_max), wd1b));
+
     // ---- device buffers (context-owned, recycled)
     if (!ctx->ref_batch) ctx->ref_batch = new (std::nothrow) strk_batch();
     if (!ctx->ref_batch) return set_err(STRK_ERR_NOMEM, "out of host memory");
     strk_batch *b = ctx->ref_batch;
-    // second look at phase 1, still on the device: up to CAP2 loci whose search left the first window, 4x wider
-    const int CAP2 = 4096;
-    const int WD_MAX = (STRK_MAX_WINDOW - 1) / 2;
-    const int wd1b = std::min(WD_MAX, 4 * wd1), stride_w2 = 2 * wd1b + 1;
-    cudaError_t e = d.out.reserve(8 * n + 8);
-    if (e == cudaSuccess) e = batch_bind(b, (long long)n, (long long)n);
+    cudaError_t e = batch_bind(b, (long long)n, (long long)n);
     if (e == cudaSuccess) e = ctx->fams.reserve(std::max(n, (size_t)CAP2));
     if (e == cudaSuccess) e = ctx->table64.reserve(std::max(n * (size_t)stride_w * 2, (size_t)CAP2 * (size_t)stride_w2 * 2));
-    if (e == cudaSuccess) e = ctx->table.reserve(n * (size_t)W2);
+    if (e == cudaSuccess) e = ctx->table.reserve(table2);
     if (e == cudaSuccess) e = ctx->fallback.reserve(n);
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -1895,102 +1722,181 @@ static int ref_counts_fast(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_b
     b->d_arena = d.arena.p;
     const int *seg_list[STRK_PK_NBIN];
     long long seg_cnt[STRK_PK_NBIN];
-    rc = lists.upload(d.lists, st, seg_list, seg_cnt);
-    if (rc) return rc;
+    if (phase1) {
+        rc = lists.upload(d.lists, st, seg_list, seg_cnt);
+        if (rc) return rc;
+    }
     CU(cudaMemsetAsync(d.cnt.p, 0, 8 * sizeof(unsigned int), st));
     CU(cudaMemsetAsync(ctx->d_acc, 0, 4 * sizeof(double), st));
     CU(cudaMemsetAsync(ctx->d_queue + 1, 0, 3 * sizeof(unsigned int), st));
-    const int T = 128;
-    const int b_len = max_n1 + 2;
-    const int rowlen = max_n1 > 32 * 16 ? mb_cols + mb_m * std::max(std::max(wd1, wd2), wd1b) + 2 : 2;
-    int seg_w1[STRK_PK_NBIN], seg_w2[STRK_PK_NBIN];
-    for (int k = 0; k < STRK_PK_NBIN; ++k) {
-        seg_w1[k] = 2 * stride_w - 1;
-        seg_w2[k] = (W2 + 3) / 4 * 4;
-    }
-    // ---- phase 1
-    ref_plan1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d.seq_off.p, d.lens.p, d.start.p, d.wd.p,
-                                                               d.motif_off.p, d.motif_len.p, stride_w, ctx->fams.p);
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(ctx->ev[0], st));
-    long long n_packed = 0;
-    rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w1, n_loci, ctx->fams.p, d.arena.p, ctx->table64.p,
-                     b_len, rowlen, st, 1, &n_packed);
-    if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[1], st));
-    ref_replay1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, ctx->table64.p, ctx->fams.p, d.start.p, d.rc.p,
-                                                                 d.ref_size.p, vcf_anchor_size, WD_MAX, d.wd.p, d.l_off.p,
-                                                                 d.r_off.p, d.n_off.p, d.ids_a.p, d.cnt.p);
-    CU(cudaGetLastError());
-    {
-        // the loci whose search left the first window (a percent of a block at +-6 sizes): 4x wider through the general
-        // kernel, list and count on the device (ids_a, cnt[0]); what still does not settle is left to the host
-        ref_clamp_count_kernel<<<1, 32, 0, st>>>(d.cnt.p, (unsigned)CAP2);  // (loci beyond the cap keep their flag: host redo)
-        ref_plan1_kernel<<<(unsigned)((CAP2 + T - 1) / T), T, 0, st>>>(d.ids_a.p, CAP2, d.seq_off.p, d.lens.p, d.start.p, d.wd.p,
-                                                                      d.motif_off.p, d.motif_len.p, stride_w2, ctx->fams.p, d.cnt.p);
+
+    // ---- phase 1, then the second look: the loci whose search left the first window (a percent of a block at +-6
+    // sizes), listed and counted on the device (ids_a, cnt[0]), up to CAP2 of them 4x wider; the rest keep their flag
+    if (phase1) {
+        ref_plan1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d.seq_off.p, d.lens.p, d.start.p, d.wd.p,
+                                                                   d.motif_off.p, d.motif_len.p, stride_w, ctx->fams.p);
         CU(cudaGetLastError());
-        rc = launch_general(ctx, true, ctx->fams.p, nullptr, CAP2, d.arena.p, ctx->table64.p, b_len, rowlen, st, d.cnt.p);
+        CU(cudaEventRecord(ctx->ev[0], st));
+        int seg_w1[STRK_PK_NBIN];
+        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w1[k] = 2 * stride_w - 1;  // forward + reverse columns of every size
+        long long n_packed = 0;
+        rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w1, n_loci, ctx->fams.p, d.arena.p,
+                         ctx->table64.p, b_len, rowlen, st, 1, &n_packed);
         if (rc) return rc;
-        ref_replay1_kernel<<<(unsigned)((CAP2 + T - 1) / T), T, 0, st>>>(d.ids_a.p, CAP2, ctx->table64.p, ctx->fams.p, d.start.p,
-                                                                        d.rc.p, d.ref_size.p, vcf_anchor_size, WD_MAX, d.wd.p,
-                                                                        d.l_off.p, d.r_off.p, d.n_off.p, d.ids_b.p, d.cnt.p + 4,
-                                                                        d.cnt.p);
+        CU(cudaEventRecord(ctx->ev[1], st));
+        ref_replay1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, ctx->table64.p, ctx->fams.p, d.start.p,
+                                                                     d.rc.p, d.ref_size.p, vcf_anchor_size, WD_MAX, d.wd.p,
+                                                                     d.l_off.p, d.r_off.p, d.n_off.p, d.ids_a.p, d.cnt.p);
+        CU(cudaGetLastError());
+        ref_clamp_count_kernel<<<1, 32, 0, st>>>(d.cnt.p, (unsigned)CAP2);
+        rc = ref_widen(ctx, d.ids_a.p, CAP2, d.cnt.p, wd1b, d.ids_b.p, d.cnt.p + 4, b_len, rowlen, vcf_anchor_size);
+        if (rc) return rc;
+    }
+
+    // ---- phase 2, one pass per tier in stream order (each overwrites ctx->table and the slots of the batch); loci whose
+    // phase 1 is not final yet run with their unadjusted flanks and are flagged
+    size_t at = 0;
+    for (size_t t = 0; t < d.tiers.size(); ++t) {
+        RefTier &tier = d.tiers[t];
+        const int nt = (int)tier.ids.size();
+        const ClassLists &cl = reuse ? lists : tier.classes;
+        int *ids = nullptr;
+        if (!reuse) {
+            ids = d.tier_ids.p + at;
+            CU(cudaMemcpyAsync(ids, tier.ids.data(), nt * sizeof(int), cudaMemcpyHostToDevice, st));
+            rc = tier.classes.upload(d.lists, st, seg_list, seg_cnt);
+            if (rc) return rc;
+        }
+        at += (size_t)nt;
+        ref_plan2_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(ids, nt, d.seq_off.p, d.lens.p, d.start.p, d.motif_off.p,
+                                                                    d.motif_len.p, d.l_off.p, d.r_off.p, b->d_seq_off,
+                                                                    b->d_lens, b->d_est, b->d_motif_off, b->d_motif_len,
+                                                                    b->d_read_begin, b->d_read_locus);
+        CU(cudaGetLastError());
+        plan_reads_kernel<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(nullptr, (long long)nt, b->d_seq_off, b->d_lens,
+                                                                       b->d_est, b->d_read_locus, b->d_motif_off,
+                                                                       b->d_motif_len, tier.wd2, 0, tier.W2, ctx->fams.p,
+                                                                       ctx->d_acc + 1, nullptr);
+        CU(cudaGetLastError());
+        if (t == 0) CU(cudaEventRecord(ctx->ev[2], st));
+        CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
+        int seg_w2[STRK_PK_NBIN];
+        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w2[k] = (tier.W2 + 3) / 4 * 4;
+        long long n_packed = 0;
+        rc = launch_pass(ctx, seg_list, seg_cnt, cl.flank, cl.mmax, seg_w2, nt, ctx->fams.p, d.arena.p, ctx->table.p, b_len,
+                         rowlen, st, 0, &n_packed);
+        if (rc) return rc;
+        if (t + 1 == d.tiers.size()) CU(cudaEventRecord(ctx->ev[3], st));
+        rc = launch_replay(ctx, b, tier.W2, tier.wd2, 0, nullptr, nullptr, nt, tier.rc[0], tier.rc[1], tier.rc[2], nullptr,
+                           nullptr, st);
+        if (rc) return rc;
+        ref_assemble_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(ids, nt, b->d_out, b->d_status, d.lens.p, d.l_off.p,
+                                                                       d.r_off.p, d.n_off.p, d.out.p, d.redo.p);
         CU(cudaGetLastError());
     }
-    // ---- phase 2 (loci whose phase 1 is not final yet run with their unadjusted flanks; their rows are redone)
-    ref_plan2_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, d.seq_off.p, d.lens.p, d.start.p, d.motif_off.p,
-                                                               d.motif_len.p, d.l_off.p, d.r_off.p, b->d_seq_off, b->d_lens,
-                                                               b->d_est, b->d_motif_off, b->d_motif_len, b->d_read_begin,
-                                                               b->d_read_locus);
-    CU(cudaGetLastError());
-    plan_reads_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(nullptr, (long long)n, b->d_seq_off, b->d_lens, b->d_est,
-                                                                  b->d_read_locus, b->d_motif_off, b->d_motif_len, wd2, 0, W2,
-                                                                  ctx->fams.p, ctx->d_acc + 1, nullptr);
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(ctx->ev[2], st));
-    CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
-    long long n_packed2 = 0;
-    rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w2, n_loci, ctx->fams.p, d.arena.p, ctx->table.p, b_len,
-                     rowlen, st, 0, &n_packed2);
-    if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[3], st));
-    rc = launch_replay(ctx, b, W2, wd2, 0, nullptr, nullptr, (long long)n, max_iters, range, step, nullptr, nullptr, st);
-    if (rc) return rc;
-    ref_assemble_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>((int)n, b->d_out, b->d_status, d.lens.p, d.l_off.p, d.r_off.p,
-                                                                  d.n_off.p, d.out.p);
-    CU(cudaGetLastError());
     CU(cudaEventRecord(ctx->ev[4], st));
+
     // ---- the one synchronisation: results, flags, counters
-    std::vector<unsigned char> status(n);
+    std::vector<unsigned char> flags(n);
     unsigned int h_cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     double acc[2] = {0, 0};
     CU(cudaMemcpyAsync(out, d.out.p, 8 * n * sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(status.data(), b->d_status, n, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(flags.data(), d.redo.p, n, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(h_cnt, d.cnt.p, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(acc, ctx->d_acc, sizeof(acc), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    if (h_cnt[1] || h_cnt[5]) {
-        const long long l = (long long)(0x7fffffffu - (h_cnt[1] ? h_cnt[1] : h_cnt[5]));
-        return set_err(STRK_ERR_SEARCH, "strk_ref_counts: locus %lld scored no size (max_iters = %d)", l, max_iters);
-    }
-    // loci to redo through the general path: phase 1 left its window (flagged in the assembled row), or phase 2 did
-    for (size_t l = 0; l < n; ++l)
-        if (status[l] || out[8 * l + 4] < 0) redo.push_back((int)l);
-    float t1 = 0.f, t2 = 0.f, t3 = 0.f, t4 = 0.f;
-    CU(cudaEventElapsedTime(&t1, ctx->ev[0], ctx->ev[1]));
-    CU(cudaEventElapsedTime(&t2, ctx->ev[1], ctx->ev[2]));
-    CU(cudaEventElapsedTime(&t3, ctx->ev[2], ctx->ev[3]));
-    CU(cudaEventElapsedTime(&t4, ctx->ev[3], ctx->ev[4]));
+    rc = ref_search_error(h_cnt, rc_params);
+    if (!rc) rc = ref_search_error(h_cnt + 4, rc_params);
+    if (rc) return rc;
+    // DP kernels: ev 0-1 (phase 1), 2-3 (phase 2; with several tiers, the replays between them too); replay, second look
+    // and planning kernels: ev 1-2, 3-4
+    float ms[4] = {0.f, 0.f, 0.f, 0.f};
+    for (int k = phase1 ? 0 : 2; k < 4; ++k) CU(cudaEventElapsedTime(&ms[k], ctx->ev[k], ctx->ev[k + 1]));
     ctx->stats[0] = cells1 + acc[1];
     ctx->stats[1] = acc[0];
-    ctx->stats[2] += 7;  // (launch_* count their own)
-    ctx->stats[3] = t1 + t3;
-    ctx->stats[4] = t2 + t4;
-    ctx->stats[5] = 0;
+    ctx->stats[2] += (phase1 ? 3 : 0) + 4 * (double)d.tiers.size();  // (launch_* count their own)
+    ctx->stats[3] = ms[0] + ms[2];
+    ctx->stats[4] = ms[1] + ms[3];
+
+    // ---- host finish of the flagged loci
+    std::vector<int> redo, ids;
+    for (size_t l = 0; l < n; ++l)
+        if (flags[l]) redo.push_back((int)l);
+    const double t_finish = now();
+    if (!redo.empty()) {
+        // phase 1 not final (n_off < 0): 4x wider per round; no window is wider than 16x the first one yet
+        for (int l : redo)
+            if (out[8 * (size_t)l + 4] < 0) ids.push_back(l);
+        int *d_ids = d.ids_a.p, *d_again = d.ids_b.p;
+        unsigned int n_pending = (unsigned int)ids.size();
+        if (n_pending) CU(cudaMemcpyAsync(d_ids, ids.data(), ids.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        for (int wd = std::min(WD_MAX, 16 * wd1); n_pending > 0; wd = std::min(WD_MAX, 4 * wd)) {
+            if (ctx->fams.reserve(n_pending) != cudaSuccess ||
+                ctx->table64.reserve((size_t)n_pending * (size_t)(2 * wd + 1) * 2) != cudaSuccess) {
+                cudaGetLastError();
+                return set_err(STRK_ERR_NOMEM, "strk_ref_counts: cannot allocate the boundary tables");
+            }
+            CU(cudaMemsetAsync(d.cnt.p, 0, 4 * sizeof(unsigned int), st));
+            CU(cudaEventRecord(ctx->ev[0], st));
+            rc = ref_widen(ctx, d_ids, (int)n_pending, nullptr, wd, d_again, d.cnt.p, b_len, rowlen_for(wd), vcf_anchor_size);
+            if (rc) return rc;
+            CU(cudaEventRecord(ctx->ev[1], st));
+            unsigned int c[4] = {0, 0, 0, 0};
+            CU(cudaMemcpyAsync(c, d.cnt.p, sizeof(c), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            rc = ref_search_error(c, rc_params);
+            if (rc) return rc;
+            float t_round = 0.f;
+            CU(cudaEventElapsedTime(&t_round, ctx->ev[0], ctx->ev[1]));
+            ctx->stats[2] += 2;
+            ctx->stats[4] += t_round;
+            n_pending = c[0];
+            std::swap(d_ids, d_again);
+        }
+        // phase 2 of every flagged locus, per tier (strk_batch_run counts its own run only)
+        double keep[8];
+        memcpy(keep, ctx->stats, sizeof(keep));
+        for (const RefTier &tier : d.tiers) {
+            ids.clear();
+            for (int l : tier.ids)
+                if (flags[(size_t)l]) ids.push_back(l);
+            if (ids.empty()) continue;
+            const int nt = (int)ids.size();
+            e = batch_bind(b, nt, nt);
+            if (e != cudaSuccess) {
+                cudaGetLastError();
+                return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
+            }
+            b->d_arena = d.arena.p;
+            b->h_read_begin.resize((size_t)nt + 1);
+            for (int q = 0; q <= nt; ++q) b->h_read_begin[(size_t)q] = q;
+            CU(cudaMemcpyAsync(d.ids_a.p, ids.data(), nt * sizeof(int), cudaMemcpyHostToDevice, st));
+            ref_plan2_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(d.ids_a.p, nt, d.seq_off.p, d.lens.p, d.start.p,
+                                                                        d.motif_off.p, d.motif_len.p, d.l_off.p, d.r_off.p,
+                                                                        b->d_seq_off, b->d_lens, b->d_est, b->d_motif_off,
+                                                                        b->d_motif_len, b->d_read_begin);
+            CU(cudaGetLastError());
+            CU(cudaStreamSynchronize(st));  // batch_plan reads the batch on the fill stream
+            rc = batch_plan(ctx, b, arena_bytes);
+            if (rc) return rc;
+            rc = strk_batch_run(ctx, b, tier.rc[0], tier.rc[1], tier.rc[2], STRK_KERNEL_AUTO, nullptr);
+            if (rc) return rc;
+            for (int k = 0; k < 8; ++k) keep[k] += ctx->stats[k];
+            ref_assemble_kernel<<<(unsigned)((nt + T - 1) / T), T, 0, st>>>(d.ids_a.p, nt, b->d_out, b->d_status, d.lens.p,
+                                                                           d.l_off.p, d.r_off.p, d.n_off.p, d.out.p, d.redo.p);
+            CU(cudaGetLastError());
+            keep[2] += 2;
+        }
+        CU(cudaMemcpyAsync(out, d.out.p, 8 * n * sizeof(int), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        memcpy(ctx->stats, keep, sizeof(keep));
+    }
+    ctx->stats[5] = (double)redo.size();  // loci finished on the host
     if (getenv("STRK_REF_TIMING"))
-        fprintf(stderr, "[strk_ref_counts] fast path, %lld loci: DP kernels %.2f + %.2f ms, replay / second look / planning kernels "
-                "%.2f + %.2f ms (device clock), %u loci took the second look, %zu left to redo\n", (long long)n_loci, t1, t3, t2, t4,
-                h_cnt[0], redo.size());
+        fprintf(stderr, "[strk_ref_counts] %lld loci, %zu tiers: DP kernels %.2f + %.2f ms, replay / second look / planning "
+                "kernels %.2f + %.2f ms (device clock), %u loci took the second look; %zu finished on the host in %.2f ms, "
+                "%.2f ms in all (host clock)\n", (long long)n_loci, d.tiers.size(), ms[0], ms[2], ms[1], ms[3], h_cnt[0],
+                redo.size(), now() - t_finish, now() - t_begin);
     return STRK_OK;
 }
 

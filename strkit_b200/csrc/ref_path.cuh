@@ -1,7 +1,8 @@
 // ref_path.cuh -- device-side planning and replay of get_ref_repeat_count (strkit/call/repeats.py:73-192),
 // one thread per locus.  Phase 1: the boundary search over the two sg_qe tables (score_ref_boundaries, :23-43;
 // climb_ref in replay.cuh restates :100-169) -> l_offset / r_offset.  Phase 2 re-uses the read-path batch machinery
-// on the adjusted flanks (:171-188).  The host only sees counters (how many loci left their window) and the results.
+// on the adjusted flanks (:171-188).  The host only sees counters, the results and the flags of the loci whose search
+// left its window (those it finishes itself).
 #pragma once
 #include "replay.cuh"
 #include "strk_common.cuh"
@@ -47,7 +48,7 @@ __global__ void ref_replay1_kernel(const int *__restrict__ ids, int n, const lon
     const RefClimbResult cr = climb_ref(tab + 2 * f.out_off, f.n_lo, f.n_hi, start[l], rc[3 * l], rc[3 * l + 1],
                                         rc[3 * l + 2], f.n_fl, f.n_fr, ref_size[l], vcf_anchor_size, seen);
     if (cr.status == 1) {
-        n_off[l] = -1;  // not final yet (the fast path of strk_ref_counts reads this flag; a redo overwrites it)
+        n_off[l] = -1;  // not final yet (ref_assemble_kernel flags the locus for the host; a wider pass overwrites it)
         if (wd[l] >= wd_max) {
             atomicMax(&counters[2], 0x7fffffffu - (unsigned)l);
             return;
@@ -95,24 +96,28 @@ __global__ void ref_plan2_kernel(const int *__restrict__ ids, int n, const unsig
     read_begin2[q] = q;
 }
 
-// Fast path of strk_ref_counts: the 8 result ints of every locus, assembled on the device.
+// The 8 result ints of the loci of a phase 2 pass (slot q = locus ids[q]; ids == nullptr: locus q), assembled on the
+// device, and their redo flags: the host finishes the loci whose phase 1 is not final or whose phase 2 search failed.
 //   out[8l..] = {cn, score, l_offset, r_offset, n_offset_scores (-1: phase 1 not final), n_iters_final, new fl, new fr}
-__global__ void ref_assemble_kernel(int n, const int *__restrict__ res4, const unsigned char *__restrict__ status,
-                                    const int *__restrict__ lens, const int *__restrict__ l_off,
-                                    const int *__restrict__ r_off, const int *__restrict__ n_off, int *__restrict__ out) {
-    const int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l >= n) return;
+__global__ void ref_assemble_kernel(const int *__restrict__ ids, int n, const int *__restrict__ res4,
+                                    const unsigned char *__restrict__ status, const int *__restrict__ lens,
+                                    const int *__restrict__ l_off, const int *__restrict__ r_off,
+                                    const int *__restrict__ n_off, int *__restrict__ out, unsigned char *__restrict__ redo) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n) return;
+    const int l = ids ? ids[q] : q;
     const int lo = l_off[l], ro = r_off[l];
     int *o = out + 8 * (size_t)l;
-    const bool ok = status[l] == 0;
-    o[0] = ok ? res4[4 * l] : 0;
-    o[1] = ok ? res4[4 * l + 1] : 0;
+    const bool ok = status[q] == 0;
+    o[0] = ok ? res4[4 * q] : 0;
+    o[1] = ok ? res4[4 * q + 1] : 0;
     o[2] = lo;
     o[3] = ro;
     o[4] = n_off[l];
-    o[5] = ok ? res4[4 * l + 2] : 0;
+    o[5] = ok ? res4[4 * q + 2] : 0;
     o[6] = lens[3 * l] - (lo > 0 ? lo : 0);
     o[7] = lens[3 * l + 2] - (ro > 0 ? ro : 0);
+    redo[l] = !ok || n_off[l] < 0;
 }
 
 __global__ void ref_clamp_count_kernel(unsigned int *count, unsigned int cap) {

@@ -458,9 +458,9 @@ def test_get_ref_repeat_count_golden(sb, golden):
 
 def test_ref_counts_batch_with_reference_tiers(sb, oracle):
     """One C-ABI call for many loci, search parameters tiered like repeat_count_params.py:17-42
-    (steps of 3 / 5 / 15 for large reference tracts), then the same loci one call per tier: a single tier takes the
-    fast path, and start counts off by tens of copies send searches out of their first window (the device-side second
-    look and the loci redone on the host)."""
+    (steps of 3 / 5 / 15 for large reference tracts), then the same loci one call per tier, with start counts off by
+    tens of copies that send searches out of their first window (the device-side second look and the loci finished on
+    the host)."""
     rng = np.random.default_rng(21)
     fams, starts, ref_sizes, rcs = [], [], [], []
     for i in range(40):

@@ -3,10 +3,15 @@
 next to the read path it precedes in call_locus: loci/s of strk_ref_counts on a block of synthetic loci whose
 reference window is an error-free copy of the locus (one sequence per locus), checked against the CPU oracle.
 
-    python tools/bench_ref_path.py [n_loci]
+    python tools/bench_ref_path.py [n_loci] [--mixed-tiers] [--reps N]
+
+--mixed-tiers: the rows of search parameters cycle over the four tiers of repeat_count_params.py:17-42 (a block
+whose loci span them, as BlockSession sends it) instead of all using the first one.  The call is timed N times
+(default 10) after a warm-up; the median is reported.
 """
 from __future__ import annotations
 
+import argparse
 import json
 import os
 import sys
@@ -17,6 +22,9 @@ sys.path.insert(0, ROOT)
 
 import numpy as np  # noqa: E402
 
+# (max_iters, local search range, step size) below 200, from 200, 1000 and 2000 reference copies
+TIERS = np.array([[250, 3, 1], [200, 3, 3], [150, 3, 5], [50, 1, 15]], dtype=np.int32)
+
 
 def main():
     import torch
@@ -26,7 +34,12 @@ def main():
     from strkit_b200.batcher import ReadBatch
     from tests import oracle_lib
 
-    n_loci = int(sys.argv[1]) if len(sys.argv) > 1 else 32768
+    ap = argparse.ArgumentParser()
+    ap.add_argument("n_loci", nargs="?", type=int, default=32768)
+    ap.add_argument("--mixed-tiers", action="store_true")
+    ap.add_argument("--reps", type=int, default=10)
+    args = ap.parse_args()
+    n_loci = args.n_loci
     dev = "cuda" if torch.cuda.is_available() else "cpu"
     rb = synth.generate(synth.CONFIGS[2], n_loci, seed=77, device=dev).to_host()
     first = rb.read_begin[:-1]  # the first read of every locus plays the reference window
@@ -43,12 +56,17 @@ def main():
                     read_begin=np.arange(n_loci + 1, dtype=np.int64), motif_off=motif_off, motif_len=rb.motif_len)
     start = ref.est_cn.copy()
     ref_size = ref.lens[:, 1].copy()
-    rc = np.tile(np.array([250, 3, 1], dtype=np.int32), (n_loci, 1))  # repeat_count_params.py:25-27 (< 200 copies)
+    rc = TIERS[np.arange(n_loci) % len(TIERS)] if args.mixed_tiers else np.tile(TIERS[0], (n_loci, 1))
+    rc = np.ascontiguousarray(rc)
     eng = strkit_b200.Engine()
     eng.ref_counts(ref, start, ref_size, rc, 5)  # grows the recycled device buffers to block size
-    t0 = time.perf_counter()
-    out = eng.ref_counts(ref, start, ref_size, rc, 5)
-    dt = time.perf_counter() - t0
+    times = []
+    for _ in range(max(1, args.reps)):
+        t0 = time.perf_counter()
+        out = eng.ref_counts(ref, start, ref_size, rc, 5)
+        times.append(time.perf_counter() - t0)
+    dt = float(np.median(times))
+    st = eng.stats()
     params = strkit_b200.RepeatCountParams("repalign", 50, 3, 1)
     rbp = synth.generate(synth.CONFIGS[2], n_loci, seed=77, device=dev).to_host(pin=True)
     eng.count_reads(rbp, params)
@@ -65,10 +83,12 @@ def main():
         s = arena[o:o + fl + tr + fr].decode()
         mo, ml = int(ref.motif_off[l]), int(ref.motif_len[l])
         (cn, score), lo, ro, (n_off, n_fin), (fl2, tr2, fr2) = orc.get_ref_repeat_count(
-            int(start[l]), s[fl:fl + tr], s[:fl], s[fl + tr:], arena[mo:mo + ml].decode(), int(ref_size[l]), 5, 250, 3, 1)
+            int(start[l]), s[fl:fl + tr], s[:fl], s[fl + tr:], arena[mo:mo + ml].decode(), int(ref_size[l]), 5, *rc[l].tolist())
         ok = ok and out[l].tolist() == [cn, score, lo, ro, n_off, n_fin, len(fl2), len(fr2)]
     dt_cpu = time.perf_counter() - tc
-    print(json.dumps({"n_loci": n_loci, "ref_path_s": dt, "ref_loci_per_s": n_loci / dt,
+    print(json.dumps({"n_loci": n_loci, "tiers": 4 if args.mixed_tiers else 1, "ref_path_s": dt,
+                      "ref_ms_per_call": [round(t * 1e3, 3) for t in times], "ref_loci_per_s": n_loci / dt,
+                      "widening_passes": int(st["widening_passes"]),
                       "read_path_same_loci_s": dt_reads, "ref_share_of_locus_block": dt / (dt + dt_reads),
                       "parity_sample_bit_exact": bool(ok), "cpu_oracle_loci_per_s_1core": n_chk / dt_cpu}))
 
