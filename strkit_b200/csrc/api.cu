@@ -208,7 +208,7 @@ struct strk_batch {
     DevBuf<double> hint;  // per locus {smallest, largest} carried-offset fraction seen at a window miss (strk_slot_window)
     int *d_rep = nullptr;
     long long n_dup = 0;
-    int max_n1 = 0, mb_cols_base = 0, mb_m = 0;
+    GenExtent ext = {};  // the general kernel's scratch for these reads
     // first-window policy, carried from one block of loci to the next one filled into this object: 1 = short motifs
     // get the wider first window of strk_read_wd (set when a block sent > 2.5 % of its loci to a second pass,
     // cleared when < 1 % of a block's loci used the margin).  Speed only: results never depend on the window.
@@ -428,13 +428,16 @@ extern "C" int strk_get_stats(strk_ctx *ctx, double stats[8]) {
 static int validate_reads(const char *who, uint64_t arena_bytes, const uint64_t *seq_off, const int32_t *lens,
                           int64_t n_reads) {
     for (int64_t r = 0; r < n_reads; ++r) {
-        const int a = lens[3 * r], b = lens[3 * r + 1], c = lens[3 * r + 2];
-        if (a < 0 || b < 0 || c < 0) return set_err(STRK_ERR_ARG, "%s: read %lld has a negative length", who, (long long)r);
-        const int64_t n1 = (int64_t)a + b + c;
-        if (n1 <= 0) return set_err(STRK_ERR_ARG, "%s: read %lld is empty (fl + tr + fr has no bases)", who, (long long)r);
-        if (n1 > (1 << 24)) return set_err(STRK_ERR_ARG, "%s: read %lld is too long (%lld)", who, (long long)r, (long long)n1);
-        if (seq_off[r] > arena_bytes || (uint64_t)n1 > arena_bytes - seq_off[r])
+        const int32_t *L = lens + 3 * r;
+        switch (strk_check_read(L[0], L[1], L[2], seq_off[r], arena_bytes)) {
+        case PLAN_ERR_NEG_LEN: return set_err(STRK_ERR_ARG, "%s: read %lld has a negative length", who, (long long)r);
+        case PLAN_ERR_EMPTY:
+            return set_err(STRK_ERR_ARG, "%s: read %lld is empty (fl + tr + fr has no bases)", who, (long long)r);
+        case PLAN_ERR_TOO_LONG:
+            return set_err(STRK_ERR_ARG, "%s: read %lld is too long (%lld)", who, (long long)r, (long long)L[0] + L[1] + L[2]);
+        case PLAN_ERR_PAST_ARENA:
             return set_err(STRK_ERR_ARG, "%s: read %lld runs past the end of the arena", who, (long long)r);
+        }
     }
     return STRK_OK;
 }
@@ -442,9 +445,11 @@ static int validate_reads(const char *who, uint64_t arena_bytes, const uint64_t 
 static int validate_motifs(const char *who, uint64_t arena_bytes, const uint64_t *motif_off, const int32_t *motif_len,
                            int64_t n) {
     for (int64_t l = 0; l < n; ++l) {
-        if (motif_len[l] <= 0) return set_err(STRK_ERR_ARG, "%s: motif %lld is empty", who, (long long)l);
-        if (motif_off[l] > arena_bytes || (uint64_t)motif_len[l] > arena_bytes - motif_off[l])
+        switch (strk_check_locus(0, 0, 0, motif_off[l], motif_len[l], arena_bytes)) {  // (motifs only: no reads)
+        case PLAN_ERR_MOTIF_EMPTY: return set_err(STRK_ERR_ARG, "%s: motif %lld is empty", who, (long long)l);
+        case PLAN_ERR_MOTIF_PAST_ARENA:
             return set_err(STRK_ERR_ARG, "%s: motif %lld runs past the end of the arena", who, (long long)l);
+        }
     }
     return STRK_OK;
 }
@@ -780,7 +785,7 @@ static cudaError_t batch_bind(strk_batch *b, long long n_reads, long long n_loci
     b->d_motif_off = b->motif_off.p, b->d_motif_len = b->motif_len.p, b->d_status = b->status.p;
     b->n_general = 0;
     for (int k = 0; k < STRK_PK_NBIN; ++k) b->bin_off[k] = b->bin_cnt[k] = 0, b->bin_mmax[k] = b->bin_flank[k] = 0;
-    b->max_n1 = b->mb_cols_base = b->mb_m = 0;
+    b->ext = GenExtent{};
     return e;
 }
 
@@ -792,15 +797,28 @@ extern "C" int strk_batch_free(strk_ctx *ctx, strk_batch *b) {
     return STRK_OK;
 }
 
-// The error of a batch whose planning found one: first_error = (index << 8) | kind of the first (PlanError)
-static int plan_error(unsigned long long first_error) {
+// The error of a batch whose planning found one: the first faulty read or locus and its PlanError
+static int plan_error(long long index, int kind) {
     static const char *what[] = {"", "has a negative length", "is empty (fl + tr + fr has no bases)", "is too long",
                                  "runs past the end of the arena", "has an out-of-range est_cn", "has an empty motif",
                                  "has a motif that runs past the end of the arena", "has a non-monotone read_begin"};
-    const long long idx = (long long)(first_error >> 8);
-    const int kind = (int)(first_error & 0xff);
-    return set_err(STRK_ERR_ARG, "batch: %s %lld %s", kind >= PLAN_ERR_MOTIF_EMPTY ? "locus" : "read", idx,
+    return set_err(STRK_ERR_ARG, "batch: %s %lld %s", kind >= PLAN_ERR_MOTIF_EMPTY ? "locus" : "read", index,
                    what[kind <= 8 ? kind : 0]);
+}
+
+// The work plan of a batch from its per-class read counts, per-class maxima and general-kernel extents: segment
+// offsets with the general kernel's reads first, then packed classes from R = 16 down to 2 (class 1 stays empty).
+static void batch_layout(strk_batch *b, const unsigned *cnt, const int *mmax, const int *flank, const GenExtent &ext) {
+    long long acc = cnt[0];
+    b->n_general = cnt[0];
+    for (int k = STRK_PK_RMAX; k >= 1; --k) {
+        b->bin_off[k] = acc;
+        b->bin_cnt[k] = cnt[k];
+        b->bin_mmax[k] = mmax[k];
+        b->bin_flank[k] = flank[k];
+        acc += cnt[k];
+    }
+    b->ext = ext;
 }
 
 // Validation + work planning of a batch whose arrays are already on the device (b->d_*, n_reads, n_loci set).
@@ -849,24 +867,11 @@ static int batch_plan(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes) {
         CU(cudaMemcpyAsync(&hp, ctx->d_plan, sizeof(PlanStats), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
     }
-    if (hp.first_error != ~0ull) return plan_error(hp.first_error);
-    // segment offsets: general first, then packed classes from R = 16 down to 2 (class 1 stays empty)
-    unsigned off[STRK_PK_NBIN];
-    unsigned acc = hp.bin_cnt[0];
-    off[0] = 0;
-    b->n_general = hp.bin_cnt[0];
-    for (int k = STRK_PK_RMAX; k >= 1; --k) {
-        off[k] = acc;
-        b->bin_off[k] = acc;
-        b->bin_cnt[k] = hp.bin_cnt[k];
-        b->bin_mmax[k] = hp.bin_mmax[k];
-        b->bin_flank[k] = hp.bin_flank[k];
-        acc += hp.bin_cnt[k];
-    }
-    b->max_n1 = hp.max_n1;
-    b->mb_cols_base = hp.mb_cols_base;
-    b->mb_m = hp.mb_m;
+    if (hp.first_error != ~0ull) return plan_error((long long)(hp.first_error >> 8), (int)(hp.first_error & 0xff));
+    batch_layout(b, hp.bin_cnt, hp.bin_mmax, hp.bin_flank, hp.ext);
     b->n_dup = b->d_rep ? (long long)hp.n_dup : 0;
+    unsigned off[STRK_PK_NBIN];
+    for (int k = 0; k < STRK_PK_NBIN; ++k) off[k] = (unsigned)b->bin_off[k];
     CU(cudaMemcpyAsync(ctx->d_bin_off, off, sizeof(off), cudaMemcpyHostToDevice, st));
     plan_reads_scatter_kernel<<<(unsigned)((n_reads + T - 1) / T), T, 0, st>>>(b->bin.p, n_reads, ctx->d_bin_off,
                                                                               ctx->d_plan, b->d_order, b->d_rep);
@@ -876,7 +881,8 @@ static int batch_plan(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes) {
 }
 
 // The same validation + planning on the host, for small batches (the per-call wrappers of the drop-in API send one
-// read at a time): no planning kernels, no read-backs, no stream synchronisation.  Mirrors plan.cuh rule for rule.
+// read at a time): no planning kernels, no read-backs, one stream synchronisation.  Loci are checked before reads,
+// and the first fault is reported, as on the device.
 #define STRK_SMALL_BATCH 512
 static int batch_plan_host(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes, const uint64_t *seq_off, const int32_t *lens,
                            const int32_t *est_cn, const int64_t *read_begin, const uint64_t *motif_off,
@@ -891,69 +897,33 @@ static int batch_plan_host(strk_ctx *ctx, strk_batch *b, uint64_t arena_bytes, c
     }
     std::vector<int> read_locus((size_t)n_reads, 0), order((size_t)n_reads);
     std::vector<unsigned char> bin((size_t)n_reads, 0);
-    unsigned long long first_error = ~0ull;
-    auto report = [&](long long index, int kind) {
-        const unsigned long long key = ((unsigned long long)index << 8) | (unsigned long long)kind;
-        if (key < first_error) first_error = key;
-    };
     for (long long l = 0; l < n_loci; ++l) {
         const long long r0 = read_begin[l], r1 = read_begin[l + 1];
-        if (r1 < r0 || r0 < 0 || r1 > n_reads) {
-            report(l, PLAN_ERR_READ_BEGIN);
-            continue;
-        }
-        if (motif_len[l] <= 0)
-            report(l, PLAN_ERR_MOTIF_EMPTY);
-        else if (motif_off[l] > arena_bytes || (unsigned long long)motif_len[l] > arena_bytes - motif_off[l])
-            report(l, PLAN_ERR_MOTIF_PAST_ARENA);
+        const int kind = strk_check_locus(r0, r1, n_reads, motif_off[l], motif_len[l], arena_bytes);
+        if (kind) return plan_error(l, kind);
         for (long long r = r0; r < r1; ++r) read_locus[(size_t)r] = (int)l;
     }
-    long long cnt[STRK_PK_NBIN] = {0};
-    if (first_error == ~0ull) {
-        for (long long r = 0; r < n_reads; ++r) {
-            const int fl = lens[3 * r], tr = lens[3 * r + 1], fr = lens[3 * r + 2];
-            const long long n1 = (long long)fl + tr + fr;
-            const int est = est_cn[r];
-            int bb = 0;
-            if (fl < 0 || tr < 0 || fr < 0)
-                report(r, PLAN_ERR_NEG_LEN);
-            else if (n1 <= 0)
-                report(r, PLAN_ERR_EMPTY);
-            else if (n1 > (1 << 24))
-                report(r, PLAN_ERR_TOO_LONG);
-            else if (seq_off[r] > arena_bytes || (unsigned long long)n1 > arena_bytes - seq_off[r])
-                report(r, PLAN_ERR_PAST_ARENA);
-            else if (est < 0 || est > (1 << 22) ||
-                     (long long)motif_len[read_locus[(size_t)r]] * (long long)est > (1ll << 24))
-                report(r, PLAN_ERR_EST);
-            else {
-                const int m = motif_len[read_locus[(size_t)r]];
-                bb = ctx->h_consts.packed_ok ? strk_pk_class(fl, tr, fr, m) : 0;
-                b->max_n1 = std::max(b->max_n1, (int)n1);
-                if (bb) {
-                    b->bin_mmax[bb] = std::max(b->bin_mmax[bb], m);
-                    b->bin_flank[bb] = std::max(b->bin_flank[bb], std::max(fl, fr));
-                }
-                if (n1 > 32 * 16 && m > 0) {
-                    b->mb_cols_base = std::max(b->mb_cols_base, std::max(fl, fr) + m * est);
-                    b->mb_m = std::max(b->mb_m, m);
-                }
-            }
-            bin[(size_t)r] = (unsigned char)bb;
-            ++cnt[bb];
+    unsigned cnt[STRK_PK_NBIN] = {0};
+    int mmax[STRK_PK_NBIN] = {0}, flank[STRK_PK_NBIN] = {0};
+    GenExtent ext = {};
+    for (long long r = 0; r < n_reads; ++r) {
+        const int fl = lens[3 * r], tr = lens[3 * r + 1], fr = lens[3 * r + 2];
+        const int m = motif_len[read_locus[(size_t)r]], est = est_cn[r];
+        int kind = strk_check_read(fl, tr, fr, seq_off[r], arena_bytes);
+        if (!kind) kind = strk_check_est(est, m);
+        if (kind) return plan_error(r, kind);
+        const int bb = ctx->h_consts.packed_ok ? strk_pk_class(fl, tr, fr, m) : 0;
+        if (bb) {
+            mmax[bb] = std::max(mmax[bb], m);
+            flank[bb] = std::max(flank[bb], std::max(fl, fr));
         }
+        ext.add(fl, fr, fl + tr + fr, m, est);
+        bin[(size_t)r] = (unsigned char)bb;
+        ++cnt[bb];
     }
-    if (first_error != ~0ull) return plan_error(first_error);
-    // segment offsets: general first, then packed classes from R = 16 down to 2 (as batch_plan)
-    long long off[STRK_PK_NBIN], acc = cnt[0];
-    off[0] = 0;
-    b->n_general = cnt[0];
-    for (int k = STRK_PK_RMAX; k >= 1; --k) {
-        off[k] = acc;
-        b->bin_off[k] = acc;
-        b->bin_cnt[k] = cnt[k];
-        acc += cnt[k];
-    }
+    batch_layout(b, cnt, mmax, flank, ext);
+    long long off[STRK_PK_NBIN];
+    std::copy(b->bin_off, b->bin_off + STRK_PK_NBIN, off);
     for (long long r = 0; r < n_reads; ++r) order[(size_t)off[bin[(size_t)r]]++] = (int)r;
     CU(cudaMemcpyAsync(b->d_read_locus, read_locus.data(), (size_t)n_reads * sizeof(int), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(b->d_order, order.data(), (size_t)n_reads * sizeof(int), cudaMemcpyHostToDevice, st));
@@ -1063,13 +1033,6 @@ extern "C" int strk_batch_upload(strk_ctx *ctx, const uint8_t *arena, uint64_t a
     return STRK_OK;
 }
 
-// scratch sizes of the general kernel: backward column (longest db + 2) and, for multi-pass reads (db > 512),
-// the boundary row (longest candidate prefix + 2)
-static void scratch_dims(const strk_batch *b, int wd, int *b_len, int *rowlen) {
-    *b_len = b->max_n1 + 2;
-    *rowlen = b->max_n1 > 32 * 16 ? b->mb_cols_base + b->mb_m * wd + 2 : 2;
-}
-
 // Replay of a pass over ctx->table (W sizes per slot), one thread per locus of `b` or of d_locus_ids; narrow windows
 // take the kernel that keeps each read's row in shared memory.  The caller counts the launch.
 static int launch_replay(strk_ctx *ctx, const strk_batch *b, int W, int wd, int ws, const int *d_locus_ids,
@@ -1154,8 +1117,8 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
             cudaGetLastError();
             return set_err(STRK_ERR_NOMEM, "cannot allocate score tables for %lld reads x %d sizes", n_slots, W);
         }
-        int b_len, rowlen;
-        scratch_dims(b, pass ? W : strk_read_wd(wd, 1, ws), &b_len, &rowlen);  // (n_hi - est <= W in a stretched window)
+        const int b_len = b->ext.b_len();
+        const int rowlen = b->ext.rowlen(pass ? W : strk_read_wd(wd, 1, ws));  // (n_hi - est <= W in a stretched window)
         plan_reads_kernel<<<(unsigned)((n_slots + threads - 1) / threads), threads, 0, st>>>(
             d_read_ids, n_slots, b->d_seq_off, b->d_lens, b->d_est, b->d_read_locus, b->d_motif_off, b->d_motif_len, wd,
             ws, W, ctx->fams.p, ctx->d_acc + 1, pass == 0 ? b->d_rep : nullptr, d_hint);
@@ -1404,7 +1367,7 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
     CU(cudaSetDevice(ctx->device));
     std::vector<FamDesc> fams((size_t)n_reads);
     uint64_t total = 0;
-    int b_len = 2, rowlen = 2;
+    GenExtent ext = {};
     for (int64_t r = 0; r < n_reads; ++r) {
         const int64_t mi = motif_idx ? motif_idx[r] : r;
         if (mi < 0 || mi >= n_motifs) return set_err(STRK_ERR_ARG, "%s: motif index out of range", who);
@@ -1427,13 +1390,12 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
         if (!ref && f.n_lo == 0 && f.n_fl + f.n_fr == 0)
             return set_err(STRK_ERR_ARG, "%s: family %lld scores an empty candidate (n = 0 without flanks)", who,
                            (long long)r);
-        const int n1 = f.n_fl + f.n_tr + f.n_fr;
         const int64_t cols = (int64_t)std::max(f.n_fl, f.n_fr) + (int64_t)f.m * f.n_hi;
         if (cols > (1 << 26)) return set_err(STRK_ERR_ARG, "%s: candidate too long", who);
-        b_len = std::max(b_len, n1 + 2);
-        if (n1 > 32 * 16) rowlen = std::max(rowlen, (int)cols + 2);
+        ext.add(f.n_fl, f.n_fr, f.n_fl + f.n_tr + f.n_fr, f.m, f.n_hi);  // (rowlen(0): a table has no window margin)
         total = std::max<uint64_t>(total, out_off[r] + (uint64_t)(f.n_hi - f.n_lo + 1));
     }
+    const int b_len = ext.b_len(), rowlen = ext.rowlen(0);
     TmpDev tmp;
     unsigned char *d_arena = nullptr;
     FamDesc *d_fams = nullptr;
@@ -1550,8 +1512,7 @@ static int ref_setup(strk_ctx *ctx, cudaStream_t st, const uint8_t *arena, uint6
     const size_t n = (size_t)n_loci;
     d.h_wd.resize(n);
     for (size_t l = 0; l < n; ++l) {
-        if (start_count[l] < 0 || start_count[l] > (1 << 22) ||
-            (long long)motif_len[l] * (long long)start_count[l] > (1ll << 24) || rc_params[3 * l] < 0 || rc_params[3 * l + 1] < 0 ||
+        if (strk_check_est(start_count[l], motif_len[l]) || rc_params[3 * l] < 0 || rc_params[3 * l + 1] < 0 ||
             rc_params[3 * l + 2] < 0 || rc_params[3 * l + 1] > 1000 || rc_params[3 * l + 2] > 1000)
             return set_err(STRK_ERR_ARG, "strk_ref_counts: bad start count / search parameters for locus %lld", (long long)l);
         d.h_wd[l] = ref_first_wd(rc_params[3 * l + 1], rc_params[3 * l + 2]);
@@ -1655,7 +1616,8 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     const bool packed1 = packed_ok && 2 * stride_w <= PK_WINDOW_MAX;  // a forward and a reverse column per size
 
     // ---- host plan: phase 1's classes, scratch maxima, the tiers in first-appearance order
-    int max_n1 = 0, mb_cols = 0, mb_m = 0, wd2_max = 0;
+    GenExtent ext = {};
+    int wd2_max = 0;
     double cells1 = 0.0;
     ClassLists &lists = d.classes;
     lists.clear();
@@ -1663,13 +1625,9 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     for (int64_t l = 0; l < n_loci; ++l) {
         const int fl = lens[3 * l], tr = lens[3 * l + 1], fr = lens[3 * l + 2], m = motif_len[l];
         const int n1 = fl + tr + fr;
-        max_n1 = std::max(max_n1, n1);
-        if (n1 > 32 * 16) {
-            // boundary row of multi-strip sweeps: the longest candidate prefix of either phase (phase 2 moves at most
-            // both flanks into the tract: (fl + fr) / m + 1 more copies)
-            mb_cols = std::max(mb_cols, std::max(fl, fr) + m * (start_count[l] + (fl + fr) / m + 1));
-            mb_m = std::max(mb_m, m);
-        }
+        // the longest candidate prefix of either phase (phase 2 moves at most both flanks into the tract:
+        // (fl + fr) / m + 1 more copies)
+        ext.add(fl, fr, n1, m, start_count[l] + (fl + fr) / m + 1);
         if (phase1) {  // executed cells of the first pass: two sweeps of db x (flank + motif * n_hi)
             lists.add(packed1 ? strk_pk_class(fl, tr, fr, m) : 0, (int)l, m, fl, fr);
             cells1 += (double)n1 * ((double)fl + fr + 2.0 * m * ((double)start_count[l] + d.h_wd[(size_t)l]));
@@ -1703,8 +1661,7 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
             t.classes.add(packed2 ? strk_pk_class(fl, tr, fr, m) : 0, (int)q, m, fl, fr);
         }
     }
-    auto rowlen_for = [&](int wd) { return max_n1 > 32 * 16 ? mb_cols + mb_m * wd + 2 : 2; };
-    const int b_len = max_n1 + 2, rowlen = rowlen_for(std::max(std::max(wd1, wd2_max), wd1b));
+    const int b_len = ext.b_len(), rowlen = ext.rowlen(std::max(std::max(wd1, wd2_max), wd1b));
 
     // ---- device buffers (context-owned, recycled)
     if (!ctx->ref_batch) ctx->ref_batch = new (std::nothrow) strk_batch();
@@ -1838,7 +1795,7 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
             }
             CU(cudaMemsetAsync(d.cnt.p, 0, 4 * sizeof(unsigned int), st));
             CU(cudaEventRecord(ctx->ev[0], st));
-            rc = ref_widen(ctx, d_ids, (int)n_pending, nullptr, wd, d_again, d.cnt.p, b_len, rowlen_for(wd), vcf_anchor_size);
+            rc = ref_widen(ctx, d_ids, (int)n_pending, nullptr, wd, d_again, d.cnt.p, b_len, ext.rowlen(wd), vcf_anchor_size);
             if (rc) return rc;
             CU(cudaEventRecord(ctx->ev[1], st));
             unsigned int c[4] = {0, 0, 0, 0};

@@ -58,6 +58,7 @@ struct PassCfg {
 #define GEN_WARPS 4
 #endif
 #define GEN_WARPS_MAX 16  // most warps a CTA may be launched with (512 threads x 128 registers = one SM's file)
+#define GEN_STRIP_ROWS (32 * 16)  // rows of one strip (R = 16, strk_pick_rows): a longer family is swept in several
 #define GEN_RING_MAX (GEN_WARPS_MAX + 1)  // ring of boundary rows / progress counters: (warps of the CTA) + 1 slots in use
 #define GEN_FAST_MMAX 256  // longest motif / prefix (flank) whose column tables a sweep keeps in shared memory; longer
 #define GEN_FAST_PMAX 256  // ones take the general loop with a symbol fetch per column

@@ -8,20 +8,66 @@
 #include "dp_packed.cuh"
 #include "strk_common.cuh"
 
+// ---- the rules of a batch: the device planner below, the host planner and the direct entry points (api.cu) call these
+
+enum PlanError {
+    PLAN_ERR_NEG_LEN = 1, PLAN_ERR_EMPTY = 2, PLAN_ERR_TOO_LONG = 3, PLAN_ERR_PAST_ARENA = 4, PLAN_ERR_EST = 5,
+    PLAN_ERR_MOTIF_EMPTY = 6, PLAN_ERR_MOTIF_PAST_ARENA = 7, PLAN_ERR_READ_BEGIN = 8
+};
+
+// A locus whose reads are [r0, r1) of n_reads and whose motif is motif_len bases at motif_off: 0, or its PlanError.
+__host__ __device__ inline int strk_check_locus(long long r0, long long r1, long long n_reads, unsigned long long motif_off,
+                                                int motif_len, unsigned long long arena_bytes) {
+    if (r1 < r0 || r0 < 0 || r1 > n_reads) return PLAN_ERR_READ_BEGIN;
+    if (motif_len <= 0) return PLAN_ERR_MOTIF_EMPTY;
+    if (motif_off > arena_bytes || (unsigned long long)motif_len > arena_bytes - motif_off) return PLAN_ERR_MOTIF_PAST_ARENA;
+    return 0;
+}
+
+// A read of flanks fl / fr around a tract of tr bases at seq_off: 0, or its PlanError.
+__host__ __device__ inline int strk_check_read(int fl, int tr, int fr, unsigned long long seq_off,
+                                               unsigned long long arena_bytes) {
+    if (fl < 0 || tr < 0 || fr < 0) return PLAN_ERR_NEG_LEN;
+    const long long n1 = (long long)fl + tr + fr;
+    if (n1 <= 0) return PLAN_ERR_EMPTY;
+    if (n1 > (1 << 24)) return PLAN_ERR_TOO_LONG;
+    if (seq_off > arena_bytes || (unsigned long long)n1 > arena_bytes - seq_off) return PLAN_ERR_PAST_ARENA;  // (no wrap-around)
+    return 0;
+}
+
+// A start estimate of est copies of an m-base motif: candidate columns are counted in 64 bits, so that a garbage
+// estimate cannot size scratch.
+__host__ __device__ inline int strk_check_est(int est, int m) {
+    return est < 0 || est > (1 << 22) || (long long)m * (long long)est > (1ll << 24) ? PLAN_ERR_EST : 0;
+}
+
+// Scratch of the general kernel (dp_general.cuh) for a set of reads: the backward column of the longest db and, when
+// a read takes more than one strip, the boundary row between strips: the longest candidate prefix, plus wd copies of
+// the largest motif for the sizes a window adds.  No constructor, so that it can live in shared memory and in the
+// zero-filled PlanStats: start from GenExtent{}.
+struct GenExtent {
+    int max_n1;   // longest db
+    int mb_cols;  // reads of more than one strip: max of max(fl, fr) + m * copies
+    int mb_m;     //                               max motif length
+    __host__ __device__ void add(int fl, int fr, int n1, int m, int copies) {
+        if (n1 > max_n1) max_n1 = n1;
+        if (n1 > GEN_STRIP_ROWS) {
+            const int cols = (fl > fr ? fl : fr) + m * copies;
+            if (cols > mb_cols) mb_cols = cols;
+            if (m > mb_m) mb_m = m;
+        }
+    }
+    __host__ __device__ int b_len() const { return max_n1 + 2; }
+    __host__ __device__ int rowlen(int wd) const { return max_n1 > GEN_STRIP_ROWS ? mb_cols + mb_m * wd + 2 : 2; }
+};
+
 struct PlanStats {
     unsigned long long first_error;  // (index << 8 | kind), smallest wins; ~0 = none
     unsigned bin_cnt[STRK_PK_NBIN];  // reads per class: [0] general kernel only, [R] packed kernel with R rows per lane
     unsigned bin_cursor[STRK_PK_NBIN];
     int bin_mmax[STRK_PK_NBIN], bin_flank[STRK_PK_NBIN];
-    int max_n1;
-    int mb_cols_base;  // multi-pass (db > 512) reads: max of max(fl, fr) + m * est
-    int mb_m;          //                              max motif length
-    unsigned n_dup;    // reads that share an earlier read's table (dedupe.cuh)
-};
-
-enum PlanError {
-    PLAN_ERR_NEG_LEN = 1, PLAN_ERR_EMPTY = 2, PLAN_ERR_TOO_LONG = 3, PLAN_ERR_PAST_ARENA = 4, PLAN_ERR_EST = 5,
-    PLAN_ERR_MOTIF_EMPTY = 6, PLAN_ERR_MOTIF_PAST_ARENA = 7, PLAN_ERR_READ_BEGIN = 8
+    GenExtent ext;   // of the valid reads
+    unsigned n_dup;  // reads that share an earlier read's table (dedupe.cuh)
 };
 
 // Rows-per-lane class of the packed kernel for a window of flanks fl / fr around a tract of tr bases and a motif of m
@@ -44,14 +90,11 @@ __global__ void plan_loci_kernel(const long long *__restrict__ read_begin, long 
     const long long l = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (l >= n_loci) return;
     const long long r0 = read_begin[l], r1 = read_begin[l + 1];
-    if (r1 < r0 || r0 < 0 || r1 > n_reads) {
-        plan_report(st, l, PLAN_ERR_READ_BEGIN);
+    const int kind = strk_check_locus(r0, r1, n_reads, motif_off[l], motif_len[l], arena_bytes);
+    if (kind) {
+        plan_report(st, l, kind);
         return;
     }
-    if (motif_len[l] <= 0)
-        plan_report(st, l, PLAN_ERR_MOTIF_EMPTY);
-    else if (motif_off[l] > arena_bytes || (unsigned long long)motif_len[l] > arena_bytes - motif_off[l])
-        plan_report(st, l, PLAN_ERR_MOTIF_PAST_ARENA);
     for (long long r = r0; r < r1; ++r) read_locus[r] = (int)l;
 }
 
@@ -62,37 +105,32 @@ __global__ void plan_reads_scan_kernel(const unsigned long long *__restrict__ se
                                        unsigned long long arena_bytes, int packed_ok, unsigned char *__restrict__ bin,
                                        PlanStats *st) {
     __shared__ unsigned s_cnt[STRK_PK_NBIN];
-    __shared__ int s_mmax[STRK_PK_NBIN], s_flank[STRK_PK_NBIN], s_max_n1, s_mb_cols, s_mb_m;
+    __shared__ int s_mmax[STRK_PK_NBIN], s_flank[STRK_PK_NBIN];
+    __shared__ GenExtent s_ext;
     if (threadIdx.x < STRK_PK_NBIN) s_cnt[threadIdx.x] = 0, s_mmax[threadIdx.x] = 0, s_flank[threadIdx.x] = 0;
-    if (threadIdx.x == 0) s_max_n1 = 0, s_mb_cols = 0, s_mb_m = 0;
+    if (threadIdx.x == 0) s_ext = GenExtent{};
     __syncthreads();
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r < n_reads) {
         const int fl = lens[3 * r], tr = lens[3 * r + 1], fr = lens[3 * r + 2];
-        const long long n1 = (long long)fl + tr + fr;
-        const int est = est_cn[r];
+        const int m = motif_len[read_locus[r]], est = est_cn[r];
+        int kind = strk_check_read(fl, tr, fr, seq_off[r], arena_bytes);
+        if (!kind) kind = strk_check_est(est, m);
         int b = 0;
-        if (fl < 0 || tr < 0 || fr < 0)
-            plan_report(st, r, PLAN_ERR_NEG_LEN);
-        else if (n1 <= 0)
-            plan_report(st, r, PLAN_ERR_EMPTY);
-        else if (n1 > (1 << 24))
-            plan_report(st, r, PLAN_ERR_TOO_LONG);
-        else if (seq_off[r] > arena_bytes || (unsigned long long)n1 > arena_bytes - seq_off[r])  // (no wrap-around)
-            plan_report(st, r, PLAN_ERR_PAST_ARENA);
-        else if (est < 0 || est > (1 << 22) || (long long)motif_len[read_locus[r]] * (long long)est > (1ll << 24))
-            plan_report(st, r, PLAN_ERR_EST);  // candidate columns (64-bit): a garbage estimate must not size scratch
+        if (kind)
+            plan_report(st, r, kind);
         else {
-            const int m = motif_len[read_locus[r]];
             b = packed_ok ? strk_pk_class(fl, tr, fr, m) : 0;
-            atomicMax(&s_max_n1, (int)n1);
             if (b) {
                 atomicMax(&s_mmax[b], m);
                 atomicMax(&s_flank[b], fl > fr ? fl : fr);
             }
-            if (n1 > 32 * 16 && m > 0) {
-                atomicMax(&s_mb_cols, (fl > fr ? fl : fr) + m * est);
-                atomicMax(&s_mb_m, m);
+            GenExtent e = {};
+            e.add(fl, fr, fl + tr + fr, m, est);
+            atomicMax(&s_ext.max_n1, e.max_n1);
+            if (e.mb_m) {
+                atomicMax(&s_ext.mb_cols, e.mb_cols);
+                atomicMax(&s_ext.mb_m, e.mb_m);
             }
         }
         bin[r] = (unsigned char)b;
@@ -105,9 +143,9 @@ __global__ void plan_reads_scan_kernel(const unsigned long long *__restrict__ se
         if (s_flank[threadIdx.x]) atomicMax(&st->bin_flank[threadIdx.x], s_flank[threadIdx.x]);
     }
     if (threadIdx.x == 0) {
-        atomicMax(&st->max_n1, s_max_n1);
-        if (s_mb_cols) atomicMax(&st->mb_cols_base, s_mb_cols);
-        if (s_mb_m) atomicMax(&st->mb_m, s_mb_m);
+        atomicMax(&st->ext.max_n1, s_ext.max_n1);
+        if (s_ext.mb_cols) atomicMax(&st->ext.mb_cols, s_ext.mb_cols);
+        if (s_ext.mb_m) atomicMax(&st->ext.mb_m, s_ext.mb_m);
     }
 }
 
