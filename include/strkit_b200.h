@@ -208,7 +208,8 @@ int strk_get_stats(strk_ctx *ctx, double stats[8]);
  *                  2 = a single distinct copy number (no bootstrap, allele.py:196-214)
  *   ms_out         device time of the kernels (CUDA events), may be NULL
  * The random streams are this library's (counter-based Philox keyed by seed, locus, replicate), not numpy's:
- * results agree with the reference statistically.  n_alleles 1 and 2 are implemented.
+ * results agree with the reference statistically.  n_alleles 1 and 2 are implemented here; per-locus counts up to 8
+ * take the _ploidy entry below.
  */
 int strk_call_alleles(strk_ctx *ctx, const int32_t *cn, const double *weights, const int64_t *read_begin,
                       int64_t n_loci, int n_alleles, int num_bootstrap, int min_reads, int min_allele_reads,
@@ -223,8 +224,43 @@ int strk_gmm_fit_counts(strk_ctx *ctx, const double *x, const int32_t *counts, c
                         int64_t n_problems, int kcap, int n_alleles, int num_bootstrap, int min_allele_reads,
                         int force_gm_filter, double expansion_ratio, int filter_factor, int n_init, double *out);
 
+/*
+ * The same for per-locus allele counts (STRkitLocus.n_alleles, from the ploidy config): n_alleles[l] in 1..8, one
+ * batch for any mix.  Rows have S = the largest count of the batch as their stride:
+ *   out_i[l]       1 + 5 * S ints: modal_n, call[S], call_95_cis[S][2], call_99_cis[S][2]
+ *   out_d[l]       3 * S doubles: means[S], weights[S], stdevs[S]
+ * locus l fills the first n_alleles[l] columns of each group and the rest are 0.
+ *   out_status[l]  0, 1, 2 as above, and 3 = at least min_reads reads and two distinct copy numbers but fewer reads
+ *                  than n_alleles[l]: the reference's GaussianMixture(n_components = n_alleles).fit raises
+ *                  "Expected n_samples >= n_components" there, so no call is made (the row is 0)
+ * Loci with one or two alleles are computed by the same code as in the entry above: with the same seed, and a batch
+ * that fits one chunk of replicate scratch, their rows are identical.  Three or more alleles run fit_gmm's staged
+ * loop (allele.py:56-123: refits with fewer components while the filters find useless ones, the strict filter
+ * 1 / (filter_factor * k) for k > 2) and fill the alleles a replicate has no peak for with components drawn by weight
+ * (:249-293).  An n_alleles outside 1..8 is STRK_ERR_UNSUPPORTED, and the message names the locus.
+ */
+int strk_call_alleles_ploidy(strk_ctx *ctx, const int32_t *cn, const double *weights, const int64_t *read_begin,
+                             int64_t n_loci, const int32_t *n_alleles, int num_bootstrap, int min_reads,
+                             int min_allele_reads, int force_gm_filter, double expansion_ratio, int filter_factor,
+                             int n_init, uint64_t seed, int32_t *out_i, double *out_d, int32_t *out_status,
+                             double *ms_out);
+
+/* The deterministic core of the above for caller-provided replicates with their own allele counts n_alleles[q]
+ * (1..8): problem q = K[q] distinct values x[q * kcap ..] with multiplicities counts[q * kcap ..] (at least
+ * n_alleles[q] points when two or more values are present).  init (NULL = k-means++ from a Philox stream keyed by
+ * seed and q) holds the forced seeds of every fit the staged loop may run: for nc = A, A-1, ..., 2, n_init rows of nc
+ * indices into x; problems follow each other, n_init * (A * (A + 1) / 2 - 1) entries for a problem with A alleles.
+ * out[q] has 3 * S + 1 doubles (S = the largest n_alleles): means[S], weights[S], stdevs[S], n_peaks; the first A of
+ * each group are sorted by mean, the rest are 0; n_peaks is the fitted component count.  When n_peaks < A the other
+ * A - n_peaks entries are copies of fitted components drawn at random by weight, so only the fitted part is
+ * deterministic; a forced problem makes no other random draw. */
+int strk_gmm_fit_counts_ploidy(strk_ctx *ctx, const double *x, const int32_t *counts, const int32_t *K,
+                               const int32_t *n_alleles, const int32_t *init, int64_t n_problems, int kcap,
+                               int num_bootstrap, int min_allele_reads, int force_gm_filter, double expansion_ratio,
+                               int filter_factor, int n_init, uint64_t seed, double *out);
+
 /* The aggregation step alone (allele.py:295-336): replicate arrays [locus][allele][replicate] (+ peaks
- * [locus][replicate]) -> out_i / out_d as in strk_call_alleles. */
+ * [locus][replicate]) -> out_i / out_d as in strk_call_alleles, for n_alleles 1..8. */
 int strk_alleles_aggregate(strk_ctx *ctx, const double *rep_means, const double *rep_weights, const double *rep_stdevs,
                            const uint8_t *rep_peaks, int64_t n_loci, int n_alleles, int num_bootstrap, int32_t *out_i,
                            double *out_d);

@@ -10,8 +10,9 @@ fallback.  Public surface (mirrors strkit.call.repeats / repeat_count_params / a
     BlockSession                                block mode: one device call per block of loci, unchanged bookkeeping
     strkit_rust_ext_shim.get_repeat_count       the 9-argument PyO3 signature (repeats.py:58-68)
     call_alleles, call_alleles_batch            bootstrap + GMM allele calls (strkit.call.allele.call_alleles)
+    call_alleles_ploidy_batch                   the same with an allele count per locus (1..8)
 """
-from .alleles import AlleleCalls, CallData, call_alleles, call_alleles_batch
+from .alleles import AlleleCalls, CallData, call_alleles, call_alleles_batch, call_alleles_ploidy_batch
 from .batcher import ARENA_ASCII, ARENA_NIBBLE, LocusReads, ReadBatch, pack_loci
 from .engine import KERNEL_AUTO, KERNEL_GENERAL, MODE_SG, MODE_SG_QE, DeviceBatch, Engine, default_engine, device_count
 from .install import install, uninstall
@@ -24,5 +25,5 @@ __version__ = "0.1.0"
 __all__ = ["LocusReads", "ReadBatch", "pack_loci", "Engine", "DeviceBatch", "default_engine", "device_count",
            "MODE_SG", "MODE_SG_QE", "KERNEL_AUTO", "KERNEL_GENERAL", "RepeatCountParams", "get_reference_rc_params",
            "get_repeat_count", "get_ref_repeat_count", "install", "uninstall", "count_reads_sharded",
-           "partition_catalog", "call_alleles", "call_alleles_batch", "AlleleCalls", "CallData", "BlockSession",
+           "partition_catalog", "call_alleles", "call_alleles_batch", "call_alleles_ploidy_batch", "AlleleCalls", "CallData", "BlockSession",
            "ARENA_ASCII", "ARENA_NIBBLE"]

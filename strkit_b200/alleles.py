@@ -20,7 +20,8 @@ import numpy as np
 from ._native import check, lib
 from .engine import Engine, default_engine
 
-__all__ = ["AlleleCalls", "CallData", "call_alleles_batch", "call_alleles", "gmm_fit_counts", "aggregate_replicates"]
+__all__ = ["AlleleCalls", "CallData", "call_alleles_batch", "call_alleles_ploidy_batch", "call_alleles", "gmm_fit_counts",
+           "gmm_fit_counts_ploidy", "aggregate_replicates"]
 
 
 def _p(a: np.ndarray) -> int:
@@ -29,8 +30,10 @@ def _p(a: np.ndarray) -> int:
 
 @dataclass
 class AlleleCalls:
-    """Per-locus results of a batch; row l is meaningful where status[l] != 1 (1 = fewer than min_reads reads, the
-    reference returns None; 2 = single distinct copy number, no bootstrap)."""
+    """Per-locus results of a batch; row l is meaningful where status[l] is 0 or 2 (1 = fewer than min_reads reads, the
+    reference returns None; 2 = single distinct copy number, no bootstrap; 3 = fewer reads than alleles, where the
+    reference raises).  With per-locus allele counts the arrays are n_alleles.max() wide and locus l uses the
+    first n_alleles[l] columns (the rest are 0)."""
     call: np.ndarray          # int32  [n_loci, n_alleles]
     call_95_cis: np.ndarray   # int32  [n_loci, n_alleles, 2]
     call_99_cis: np.ndarray   # int32  [n_loci, n_alleles, 2]
@@ -40,6 +43,7 @@ class AlleleCalls:
     modal_n: np.ndarray       # int32  [n_loci]
     status: np.ndarray        # int32  [n_loci]
     kernel_ms: float = 0.0
+    n_alleles: np.ndarray | None = None  # int32 [n_loci]: per-locus allele counts (call_alleles_ploidy_batch)
 
 
 @dataclass
@@ -104,6 +108,36 @@ def call_alleles_batch(cn: np.ndarray, weights: np.ndarray, read_begin: np.ndarr
     return _unpack(out_i, out_d, status, n_alleles, float(ms[0]))
 
 
+def call_alleles_ploidy_batch(cn: np.ndarray, weights: np.ndarray, read_begin: np.ndarray, n_alleles, *,
+                              num_bootstrap: int = 100, min_reads: int = 4, min_allele_reads: int = 2,
+                              force_gm_filter: bool = False, expansion_ratio: float = 5.0, filter_factor: int = 3,
+                              n_init: int = 3, seed: int = 0, engine: Engine | None = None) -> AlleleCalls:
+    """call_alleles_batch with an allele count per locus (1..8; an int applies to every locus), e.g. the
+    `n_alleles` of each STRkitLocus as the ploidy config sets it.  One call serves a catalog of any mix of counts;
+    loci with one or two alleles get the rows call_alleles_batch would give them (same seed, one chunk)."""
+    eng = engine or default_engine()
+    cn = np.ascontiguousarray(cn, dtype=np.int32)
+    weights = np.ascontiguousarray(weights, dtype=np.float64)
+    read_begin = np.ascontiguousarray(read_begin, dtype=np.int64)
+    n_loci = int(read_begin.shape[0]) - 1
+    if n_loci < 0 or cn.shape != weights.shape or cn.ndim != 1:
+        raise ValueError("call_alleles_ploidy_batch: cn and weights must be flat arrays of equal length; "
+                         "read_begin [n_loci + 1]")
+    a_loc = np.ascontiguousarray(np.broadcast_to(np.asarray(n_alleles, dtype=np.int32), (n_loci,)))
+    s = max(1, int(a_loc.max(initial=1)))
+    out_i = np.zeros((n_loci, 1 + 5 * s), dtype=np.int32)
+    out_d = np.zeros((n_loci, 3 * s), dtype=np.float64)
+    status = np.zeros(n_loci, dtype=np.int32)
+    ms = np.zeros(1, dtype=np.float64)
+    check(lib.strk_call_alleles_ploidy(eng._ctx, _p(cn), _p(weights), _p(read_begin), n_loci, _p(a_loc), num_bootstrap,
+                                       min_reads, min_allele_reads, int(force_gm_filter), float(expansion_ratio),
+                                       filter_factor, n_init, int(seed) & 0xFFFFFFFFFFFFFFFF, _p(out_i), _p(out_d),
+                                       _p(status), _p(ms)))
+    res = _unpack(out_i, out_d, status, s, float(ms[0]))
+    res.n_alleles = a_loc
+    return res
+
+
 def call_alleles(repeats_fwd, repeats_rev, read_weights_fwd, read_weights_rev, params, min_reads: int, n_alleles: int,
                  separate_strands: bool, read_bias_corr_min: int, seed: int | None, logger_=None, debug_str: str = "",
                  engine: Engine | None = None) -> CallData | None:
@@ -117,13 +151,16 @@ def call_alleles(repeats_fwd, repeats_rev, read_weights_fwd, read_weights_rev, p
     w = np.concatenate((np.asarray(read_weights_fwd, dtype=np.float64).ravel(),
                         np.asarray(read_weights_rev, dtype=np.float64).ravel()))
     gp = params.gmm_params
-    res = call_alleles_batch(cn, w, np.array([0, cn.shape[0]], dtype=np.int64), n_alleles,
-                             num_bootstrap=params.num_bootstrap, min_reads=min_reads,
-                             min_allele_reads=params.min_allele_reads, force_gm_filter=params.force_gm_filter,
-                             expansion_ratio=gp.expansion_ratio, filter_factor=gp.filter_factor, n_init=gp.n_init,
-                             seed=0 if seed is None else int(seed), engine=engine)
+    batch = call_alleles_batch if n_alleles <= 2 else call_alleles_ploidy_batch
+    res = batch(cn, w, np.array([0, cn.shape[0]], dtype=np.int64), n_alleles, num_bootstrap=params.num_bootstrap,
+                min_reads=min_reads, min_allele_reads=params.min_allele_reads, force_gm_filter=params.force_gm_filter,
+                expansion_ratio=gp.expansion_ratio, filter_factor=gp.filter_factor, n_init=gp.n_init,
+                seed=0 if seed is None else int(seed), engine=engine)
     if res.status[0] == 1:
         return None
+    if res.status[0] == 3:  # scikit-learn's GaussianMixture.fit raises this inside the reference's call_alleles
+        raise ValueError(f"Expected n_samples >= n_components but got n_components = {n_alleles}, "
+                         f"n_samples = {cn.shape[0]}")
     return CallData(call=res.call[0], call_95_cis=res.call_95_cis[0], call_99_cis=res.call_99_cis[0], means=res.means[0],
                     weights=res.weights[0], stdevs=res.stdevs[0], modal_n=int(res.modal_n[0]))
 
@@ -151,6 +188,42 @@ def gmm_fit_counts(values: Sequence[np.ndarray], counts: Sequence[np.ndarray], i
     check(lib.strk_gmm_fit_counts(eng._ctx, _p(x), _p(c), _p(k), _p(init), nq, kcap, n_alleles, num_bootstrap,
                                   min_allele_reads, int(force_gm_filter), float(expansion_ratio), filter_factor, n_init,
                                   _p(out)))
+    return out
+
+
+def gmm_fit_counts_ploidy(values: Sequence[np.ndarray], counts: Sequence[np.ndarray], n_alleles,
+                          init: Sequence[np.ndarray] | None = None, *, n_init: int = 3, num_bootstrap: int = 100,
+                          min_allele_reads: int = 2, force_gm_filter: bool = False, expansion_ratio: float = 5.0,
+                          filter_factor: int = 3, seed: int = 0, engine: Engine | None = None) -> np.ndarray:
+    """gmm_fit_counts for problems with their own allele counts (n_alleles: an int or one per problem, 1..8).
+    init[q] (None: k-means++ draws) holds the forced seeds of every fit fit_gmm's staged loop may run on problem q:
+    for nc = A, A-1, ..., 2, n_init rows of nc indices into values[q], flattened.  Returns [q, 3 * S + 1] with
+    S = max(n_alleles): means[S], weights[S], stdevs[S] (the first A[q] sorted by mean, the rest 0), n_peaks.
+    Entries beyond the fitted n_peaks are random copies of fitted components (the reference's fill)."""
+    eng = engine or default_engine()
+    nq = len(values)
+    a = np.ascontiguousarray(np.broadcast_to(np.asarray(n_alleles, dtype=np.int32), (nq,)))
+    s = max(1, int(a.max(initial=1)))
+    kcap = max(1, max((len(v) for v in values), default=1))
+    x = np.zeros((nq, kcap), dtype=np.float64)
+    c = np.zeros((nq, kcap), dtype=np.int32)
+    k = np.zeros(nq, dtype=np.int32)
+    for q, (v, cc) in enumerate(zip(values, counts)):
+        k[q] = len(v)
+        x[q, :len(v)] = v
+        c[q, :len(v)] = cc
+    if init is not None:
+        init = [np.asarray(i, dtype=np.int32).ravel() for i in init]
+        for q, i in enumerate(init):
+            want = n_init * (int(a[q]) * (int(a[q]) + 1) // 2 - 1) if 1 <= a[q] <= 8 else i.size
+            if i.size != want:
+                raise ValueError(f"gmm_fit_counts_ploidy: problem {q} has {i.size} seed indices, expected {want}")
+        init = np.ascontiguousarray(np.concatenate(init) if init else np.zeros(0, dtype=np.int32), dtype=np.int32)
+    out = np.zeros((nq, 3 * s + 1), dtype=np.float64)
+    check(lib.strk_gmm_fit_counts_ploidy(eng._ctx, _p(x), _p(c), _p(k), _p(a), None if init is None else _p(init), nq,
+                                         kcap, num_bootstrap, min_allele_reads, int(force_gm_filter),
+                                         float(expansion_ratio), filter_factor, n_init, int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                         _p(out)))
     return out
 
 

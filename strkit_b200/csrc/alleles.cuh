@@ -12,6 +12,11 @@
 //   alleles_aggregate_kernel one CTA per locus: per-allele stable sort of the replicate estimates,
 //                            interpolated-inverted-CDF percentiles, median, modal peak count
 //
+// The allele count A belongs to the locus (STRkitLocus.n_alleles, set by the ploidy config), 1..ALL_MAX_ALLELES.
+// A <= 2 runs the two-component code (fit_replicate); A >= 3 runs fit_gmm's staged loop over k components
+// (fit_replicate_k): k-means++ for k centres, EM with k components, refits with fewer components while the
+// filters find useless ones, and the reference's random fill of the alleles a replicate has no peak for.
+//
 // A bootstrap replicate of integer copy numbers is a multiset over the locus' K distinct values, so it is
 // carried as K counts; EM on (value, count) pairs is the same arithmetic as EM on the expanded sample
 // (identical points have identical responsibilities).  Random streams differ from numpy's / sklearn's, so
@@ -23,9 +28,10 @@
 
 #define ALL_MAX_BOOT 4096   // replicates per locus the aggregation kernel sorts in shared memory
 #define ALL_N_INIT_MAX 8
+#define ALL_MAX_ALLELES 8   // components per locus (fit_replicate_k keeps its arrays this wide)
 
 struct AlleleParams {
-    int n_alleles;          // 1 or 2
+    int n_alleles;          // 1 or 2: the batch-wide count of strk_call_alleles (per-locus counts come as an array)
     int num_bootstrap;
     int min_reads;
     int n_init;             // GMMParams.n_init (params.py:166-172: 3)
@@ -36,6 +42,7 @@ struct AlleleParams {
     double allele_filter;   // (min_allele_reads - 0.1) / num_bootstrap  (allele.py:243: concat_samples.shape[0])
     double expansion_ratio; // params.gm_filter_expansion_ratio
     double filter_weight;   // 1 / (filter_factor * 2)
+    int filter_factor;      // the k-component filter's threshold is 1 / (filter_factor * k)
     double small_allele_min;  // allele.py:47
     unsigned long long seed;
 };
@@ -85,9 +92,12 @@ struct Philox {
 
 // ---------------------------------------------------------------------------------------------- prepare
 // status: 0 = bootstrap + GMM, 1 = fewer than min_reads reads (reference returns None, allele.py:192-193),
-//         2 = a single distinct value (no bootstrap, allele.py:196-214)
+//         2 = a single distinct value (no bootstrap, allele.py:196-214),
+//         3 = fewer reads than the locus' allele count A (A_arr; NULL = no per-locus count): every replicate with
+//             two distinct values would reach GaussianMixture(A).fit on fewer than A samples, which raises
 __global__ void alleles_prepare_kernel(const int *__restrict__ cn, const double *__restrict__ w,
-                                       const long long *__restrict__ read_begin, int n_loci, int min_reads, int kcap,
+                                       const long long *__restrict__ read_begin, const int *__restrict__ A_arr,
+                                       int n_loci, int min_reads, int kcap,
                                        int *__restrict__ vals, double *__restrict__ cdf, int *__restrict__ cnt,
                                        int *__restrict__ K_out,
                                        int *__restrict__ n_out, int *__restrict__ status, int *__restrict__ k_max) {
@@ -126,7 +136,7 @@ __global__ void alleles_prepare_kernel(const int *__restrict__ cn, const double 
     }
     for (int j = 0; j < K; ++j) p[j] /= acc;
     K_out[l] = K;
-    status[l] = n < min_reads ? 1 : (K == 1 ? 2 : 0);
+    status[l] = n < min_reads ? 1 : (K == 1 ? 2 : (A_arr && n < A_arr[l] ? 3 : 0));
     atomicMax(k_max, K);
 }
 
@@ -295,11 +305,11 @@ __device__ __forceinline__ int gmm_useless(const Gmm2 &g, const AlleleParams &P)
 // One replicate -> the allele estimates the reference appends per bootstrap iteration (allele.py:249-293):
 // out_m / out_w / out_s [n_alleles] sorted by mean, *n_peaks = g.means_.shape[0].
 template <int KMAX>
-__device__ void fit_replicate(const double *x, const int *c, int K, int n, const AlleleParams &P, Philox &rng,
+__device__ void fit_replicate(const double *x, const int *c, int K, int n, int A, const AlleleParams &P, Philox &rng,
                               const int *forced_init, double *out_m, double *out_w, double *out_s, int *n_peaks) {
     int distinct = 0;
     for (int v = 0; v < K; ++v) distinct += c[v] != 0;
-    bool single = distinct == 1 || P.n_alleles == 1;  // fit_gmm: len(mc) == 1, or n_components == 1
+    bool single = distinct == 1 || A == 1;  // fit_gmm: len(mc) == 1, or n_components == 1
     Gmm2 best;
     if (!single) {
         double best_lb = -INFINITY;
@@ -323,7 +333,7 @@ __device__ void fit_replicate(const double *x, const int *c, int K, int n, const
         double m, var;
         single_gaussian(x, c, K, n, m, var);
         const double s = sqrt(var);
-        for (int a = 0; a < P.n_alleles; ++a) out_m[a] = m, out_w[a] = 1.0, out_s[a] = s;
+        for (int a = 0; a < A; ++a) out_m[a] = m, out_w[a] = 1.0, out_s[a] = s;
         *n_peaks = 1;
     } else {
         const int first = best.mean[1] < best.mean[0] ? 1 : 0;  // stable argsort of two means
@@ -333,12 +343,260 @@ __device__ void fit_replicate(const double *x, const int *c, int K, int n, const
     }
 }
 
-// one thread per (locus, replicate); replicate arrays laid out [locus][allele][replicate]
+// ---------------------------------------------------------------------------------------------- k components
+// fit_gmm for A >= 3 components (allele.py:56-123 over GaussianMixture(n_components = k)); the two-component code
+// above stays the path of A <= 2, so those results do not depend on this one.
+struct GmmK {
+    double mean[ALL_MAX_ALLELES], cov[ALL_MAX_ALLELES], weight[ALL_MAX_ALLELES];
+    int n_comp;
+};
+
+// EM from the seed value indices idx[0..NC): gmm_em with NC components, the same separately rounded products, the
+// same init (one-hot responsibilities on the seed points + 10 eps: two components seeded on one point stay equal),
+// a NC-way log-sum-exp and the same convergence rule.  NC is a template so the component arrays stay in registers.
+template <int NC, int KMAX>
+__device__ double gmm_em_k(const double *x, const int *c, int K, int n, const int *idx, const AlleleParams &P,
+                           GmmK &g) {
+    const double eps10 = 10.0 * 2.220446049250313e-16;
+    double mean[NC], cov[NC], weight[NC], pchol[NC], logw[NC];
+#pragma unroll
+    for (int k = 0; k < NC; ++k) {
+        const double nk = 1.0 + eps10, xv = x[idx[k]];
+        mean[k] = xv / nk;
+        cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(__dmul_rn(xv, xv), nk), __dmul_rn(mean[k], mean[k])), P.reg_covar);
+        weight[k] = nk / (double)n;
+        pchol[k] = 1.0 / sqrt(cov[k]);
+        logw[k] = log(weight[k]);
+    }
+    double lower = -INFINITY;
+    for (int it = 1; it <= P.max_iter; ++it) {
+        const double prev = lower;
+        double nk[NC], sx[NC], sxx[NC], ll = 0.0;
+#pragma unroll
+        for (int k = 0; k < NC; ++k) nk[k] = 0.0, sx[k] = 0.0, sxx[k] = 0.0;
+        for (int v = 0; v < K; ++v) {
+            if (c[v] == 0) continue;
+            double wl[NC];
+#pragma unroll
+            for (int k = 0; k < NC; ++k) {
+                const double prec = __dmul_rn(pchol[k], pchol[k]);
+                const double t1 = __dmul_rn(__dmul_rn(mean[k], mean[k]), prec);
+                const double t2 = __dmul_rn(2.0, __dmul_rn(__dmul_rn(x[v], mean[k]), prec));
+                const double t3 = __dmul_rn(__dmul_rn(x[v], x[v]), prec);
+                const double lp = __dadd_rn(__dsub_rn(t1, t2), t3);
+                wl[k] = __dadd_rn(__dadd_rn(__dmul_rn(-0.5, __dadd_rn(1.8378770664093453, lp)), log(pchol[k])), logw[k]);
+            }
+            double mx = wl[0];
+#pragma unroll
+            for (int k = 1; k < NC; ++k) mx = fmax(mx, wl[k]);
+            double se = 0.0;
+#pragma unroll
+            for (int k = 0; k < NC; ++k) se += exp(wl[k] - mx);
+            const double lse = mx + log(se);
+            const double cv = (double)c[v];
+            ll += cv * lse;
+#pragma unroll
+            for (int k = 0; k < NC; ++k) {
+                const double r = exp(wl[k] - lse) * cv;
+                nk[k] += r;
+                sx[k] += r * x[v];
+                sxx[k] += r * x[v] * x[v];
+            }
+        }
+        lower = ll / (double)n;
+        double wsum = 0.0;
+#pragma unroll
+        for (int k = 0; k < NC; ++k) {
+            nk[k] += eps10;
+            mean[k] = sx[k] / nk[k];
+            cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(sxx[k], nk[k]), __dmul_rn(mean[k], mean[k])), P.reg_covar);
+            weight[k] = nk[k] / (double)n;
+            wsum += weight[k];
+        }
+#pragma unroll
+        for (int k = 0; k < NC; ++k) {
+            weight[k] /= wsum;
+            pchol[k] = 1.0 / sqrt(cov[k] > 0.0 ? cov[k] : P.reg_covar);
+            logw[k] = log(weight[k]);
+        }
+        if (fabs(lower - prev) < P.tol) break;
+    }
+#pragma unroll
+    for (int k = 0; k < NC; ++k) g.mean[k] = mean[k], g.cov[k] = cov[k], g.weight[k] = weight[k];
+    g.n_comp = NC;
+    return lower;
+}
+
+// sklearn _kmeans_plusplus (cluster/_kmeans.py:224-275) for k centres on the (value, count) pairs of a replicate:
+// the first centre uniform over the n points; each further centre the best (first argmin of the potential) of
+// 2 + int(log k) candidates drawn by searchsorted(cumsum(count * closest_dist_sq), u * pot, side="left"), clipped
+// to the last point.  When every point already sits on a centre (pot = 0) every draw lands on point 0, the smallest
+// value, and that centre is duplicated -- as scikit-learn does.
 template <int KMAX>
+__device__ void kmeanspp_k(const double *x, const int *c, int K, int n, int k, Philox &rng, int *idx) {
+    {
+        const double u = rng.uniform();
+        long long pt = (long long)(u * (double)n);
+        if (pt >= n) pt = n - 1;
+        int v = 0;
+        long long acc = 0;
+        for (; v < K; ++v) {
+            acc += c[v];
+            if (pt < acc) break;
+        }
+        idx[0] = v < K ? v : K - 1;
+    }
+    double closest[KMAX];
+    double pot = 0.0;
+    for (int v = 0; v < K; ++v) {
+        const double d = x[v] - x[idx[0]];
+        closest[v] = d * d;
+        pot += (double)c[v] * closest[v];
+    }
+    const int trials = 2 + (int)log((double)k);
+    for (int ci = 1; ci < k; ++ci) {
+        double best_pot = INFINITY;
+        int best = 0;
+#pragma unroll 1
+        for (int t = 0; t < trials; ++t) {
+            const double r = rng.uniform() * pot;
+            int v = 0, last_nonzero = 0;
+            double acc = 0.0;
+            for (; v < K; ++v) {
+                if (c[v]) last_nonzero = v;
+                acc += (double)c[v] * closest[v];
+                if (c[v] && acc >= r) break;
+            }
+            const int cand = v < K ? v : last_nonzero;
+            double cp = 0.0;
+            for (int q = 0; q < K; ++q) {
+                const double d = x[q] - x[cand];
+                cp += (double)c[q] * fmin(closest[q], d * d);
+            }
+            if (cp < best_pot) best_pot = cp, best = cand;
+        }
+        idx[ci] = best;
+        pot = best_pot;
+        for (int q = 0; q < K; ++q) {
+            const double d = x[q] - x[best];
+            closest[q] = fmin(closest[q], d * d);
+        }
+    }
+}
+
+// GaussianMixture(nc).fit: the best of n_init restarts (forced = n_init rows of nc seed indices, or NULL for k-means++)
+template <int KMAX>
+__device__ void gmm_fit_k(const double *x, const int *c, int K, int n, int nc, const AlleleParams &P, Philox &rng,
+                          const int *forced, GmmK &best) {
+    double best_lb = -INFINITY;
+    for (int t = 0; t < P.n_init; ++t) {
+        int idx[ALL_MAX_ALLELES];
+        if (forced) {
+            for (int j = 0; j < nc; ++j) idx[j] = forced[t * nc + j];
+        } else {
+            kmeanspp_k<KMAX>(x, c, K, n, nc, rng, idx);
+        }
+        GmmK g;
+        double lb;
+        switch (nc) {
+        case 2: lb = gmm_em_k<2, KMAX>(x, c, K, n, idx, P, g); break;
+        case 3: lb = gmm_em_k<3, KMAX>(x, c, K, n, idx, P, g); break;
+        case 4: lb = gmm_em_k<4, KMAX>(x, c, K, n, idx, P, g); break;
+        case 5: lb = gmm_em_k<5, KMAX>(x, c, K, n, idx, P, g); break;
+        case 6: lb = gmm_em_k<6, KMAX>(x, c, K, n, idx, P, g); break;
+        case 7: lb = gmm_em_k<7, KMAX>(x, c, K, n, idx, P, g); break;
+        default: lb = gmm_em_k<8, KMAX>(x, c, K, n, idx, P, g); break;
+        }
+        if (lb > best_lb || best_lb == -INFINITY) best_lb = lb, best = g;
+    }
+}
+
+// fit_gmm's peak filters (allele.py:88-121) on a fitted nc-component model: the strict weight threshold
+// 1 / (filter_factor * nc) always applies for nc > 2; for nc = 2 it is gmm_useless
+__device__ __forceinline__ int gmm_useless_k(const GmmK &g, int nc, const AlleleParams &P) {
+    double lo = g.mean[0], hi = g.mean[0];
+    for (int k = 1; k < nc; ++k) lo = fmin(lo, g.mean[k]), hi = fmax(hi, g.mean[k]);
+    const bool strict = nc > 2 || P.force_gm_filter || hi < P.expansion_ratio * fmax(lo, P.small_allele_min);
+    const double thr = strict ? 1.0 / (double)(P.filter_factor * nc) : 1.1920928955078125e-07;
+    int useless = 0;
+    for (int k = 0; k < nc; ++k)
+        if (!(g.weight[k] > P.allele_filter && g.weight[k] > thr)) ++useless;
+    return useless;
+}
+
+// One replicate with A >= 3 alleles (allele.py:56-123,249-293).  fit_gmm's loop: fit with A components, drop the
+// useless count and refit with a fresh restart set, a single Gaussian at 1 component, and at <= 0 components the
+// last fit with all its components.  A replicate with fewer peaks than A gets A - peaks components drawn with
+// probability weight / sum|weight| (Philox stream of the thread), then everything is sorted by mean (stable).
+// *n_peaks = the fitted count, before the fill.  forced_init (NULL = k-means++): for nc = A, A-1, ..., 2, n_init
+// rows of nc seed indices.
+template <int KMAX>
+__device__ void fit_replicate_k(const double *x, const int *c, int K, int n, int A, const AlleleParams &P, Philox &rng,
+                                const int *forced_init, double *out_m, double *out_w, double *out_s, int *n_peaks) {
+    int distinct = 0;
+    for (int v = 0; v < K; ++v) distinct += c[v] != 0;
+    GmmK g;
+    int nc = distinct == 1 ? 1 : A;  // len(mc) == 1: a single Gaussian without a fit
+    while (nc > 1) {
+        const int *forced = forced_init ? forced_init + P.n_init * (A * (A + 1) / 2 - nc * (nc + 1) / 2) : nullptr;
+        gmm_fit_k<KMAX>(x, c, K, n, nc, P, rng, forced, g);
+        const int useless = gmm_useless_k(g, nc, P);
+        if (!useless) break;
+        nc -= useless;
+    }
+    int peaks;
+    if (nc == 1) {
+        double m, var;
+        single_gaussian(x, c, K, n, m, var);
+        out_m[0] = m, out_w[0] = 1.0, out_s[0] = sqrt(var);
+        peaks = 1;
+    } else {
+        peaks = g.n_comp;
+        for (int k = 0; k < peaks; ++k) out_m[k] = g.mean[k], out_w[k] = g.weight[k], out_s[k] = sqrt(g.cov[k]);
+    }
+    *n_peaks = peaks;
+    if (peaks < A) {
+        // Generator.choice(peaks, p = w / sum|w|): cdf normalised by its last entry, searchsorted(side="right")
+        double cdf[ALL_MAX_ALLELES], tot = 0.0, acc = 0.0;
+        for (int k = 0; k < peaks; ++k) tot += fabs(out_w[k]);
+        for (int k = 0; k < peaks; ++k) acc += out_w[k] / tot, cdf[k] = acc;
+        for (int k = 0; k < peaks; ++k) cdf[k] /= acc;
+        for (int a = peaks; a < A; ++a) {
+            int pick = 0;
+            if (peaks > 1) {
+                const double u = rng.uniform();
+                while (pick < peaks - 1 && cdf[pick] <= u) ++pick;
+            }
+            out_m[a] = out_m[pick], out_w[a] = out_w[pick], out_s[a] = out_s[pick];
+        }
+    }
+    for (int i = 1; i < A; ++i) {  // insertion sort by mean: stable, like argsort(kind="stable")
+        const double m = out_m[i], w = out_w[i], s = out_s[i];
+        int j = i;
+        for (; j > 0 && out_m[j - 1] > m; --j) out_m[j] = out_m[j - 1], out_w[j] = out_w[j - 1], out_s[j] = out_s[j - 1];
+        out_m[j] = m, out_w[j] = w, out_s[j] = s;
+    }
+}
+
+// one replicate of a locus with A alleles: the two-component code for A <= 2, the k-component one above
+template <int KMAX, int AMAX>
+__device__ __forceinline__ void fit_replicate_any(const double *x, const int *c, int K, int n, int A,
+                                                  const AlleleParams &P, Philox &rng, const int *forced_init,
+                                                  double *out_m, double *out_w, double *out_s, int *n_peaks) {
+    if (AMAX <= 2 || A <= 2)
+        fit_replicate<KMAX>(x, c, K, n, A, P, rng, forced_init, out_m, out_w, out_s, n_peaks);
+    else
+        fit_replicate_k<KMAX>(x, c, K, n, A, P, rng, forced_init, out_m, out_w, out_s, n_peaks);
+}
+
+// one thread per (locus, replicate); replicate arrays laid out [locus][allele][replicate] with S allele rows per
+// locus; locus l has A_arr[l] alleles (NULL: P.n_alleles).  AMAX = 2 compiles the two-component code only.
+template <int KMAX, int AMAX>
 __global__ void __launch_bounds__(128)
 alleles_fit_kernel(const int *__restrict__ vals, const double *__restrict__ cdf, const int *__restrict__ cnt,
                    const int *__restrict__ K_arr,
-                   const int *__restrict__ n_arr, const int *__restrict__ status, int n_loci, int kcap, AlleleParams P,
+                   const int *__restrict__ n_arr, const int *__restrict__ status, const int *__restrict__ A_arr,
+                   int n_loci, int kcap, int S, AlleleParams P,
                    double *__restrict__ rep_m, double *__restrict__ rep_w, double *__restrict__ rep_s,
                    unsigned char *__restrict__ rep_peaks) {
     const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -347,6 +605,7 @@ alleles_fit_kernel(const int *__restrict__ vals, const double *__restrict__ cdf,
     if (l >= n_loci || status[l] != 0) return;
     const int K = K_arr[l], n = n_arr[l];
     if (K > KMAX) return;  // the host picks KMAX >= the batch maximum
+    const int A = A_arr ? A_arr[l] : P.n_alleles;
     double x[KMAX];
     int c[KMAX];
     const int *v = vals + (size_t)l * kcap;
@@ -366,11 +625,11 @@ alleles_fit_kernel(const int *__restrict__ vals, const double *__restrict__ cdf,
         // num_bootstrap == 1: the replicate is the sample itself (allele.py:163-167)
         for (int j = 0; j < K; ++j) c[j] = cnt[(size_t)l * kcap + j];
     }
-    double m[2], w[2], s[2];
+    double m[AMAX], w[AMAX], s[AMAX];
     int peaks;
-    fit_replicate<KMAX>(x, c, K, n, P, rng, nullptr, m, w, s, &peaks);
-    for (int a = 0; a < P.n_alleles; ++a) {
-        const size_t o = ((size_t)l * P.n_alleles + a) * B + b;
+    fit_replicate_any<KMAX, AMAX>(x, c, K, n, A, P, rng, nullptr, m, w, s, &peaks);
+    for (int a = 0; a < A; ++a) {
+        const size_t o = ((size_t)l * S + a) * B + b;
         rep_m[o] = m[a], rep_w[o] = w[a], rep_s[o] = s[a];
     }
     rep_peaks[(size_t)l * B + b] = (unsigned char)peaks;
@@ -393,9 +652,38 @@ __global__ void gmm_fit_counts_kernel(const double *__restrict__ xs, const int *
     rng.init(P.seed, (uint32_t)q, 0u);
     double m[2] = {0, 0}, w[2] = {0, 0}, s[2] = {0, 0};
     int peaks = 0;
-    fit_replicate<KMAX>(x, c, K, n, P, rng, init + (size_t)q * 2 * P.n_init, m, w, s, &peaks);
+    fit_replicate<KMAX>(x, c, K, n, P.n_alleles, P, rng, init + (size_t)q * 2 * P.n_init, m, w, s, &peaks);
     double *o = out + (size_t)q * 7;
     o[0] = m[0], o[1] = w[0], o[2] = s[0], o[3] = m[1], o[4] = w[1], o[5] = s[1], o[6] = (double)peaks;
+}
+
+// the same for problems with their own allele counts A[q] (1..ALL_MAX_ALLELES): seeds init[init_off[q] ..] in
+// fit_replicate_k's layout (init = NULL: k-means++ from the problem's Philox stream); out[q][3 * S + 1] =
+// means[S], weights[S], stdevs[S] (A[q] of them used, sorted by mean after the fill, the rest 0), n_peaks
+template <int KMAX>
+__global__ void gmm_fit_counts_ploidy_kernel(const double *__restrict__ xs, const int *__restrict__ cs,
+                                             const int *__restrict__ Ks, const int *__restrict__ As,
+                                             const int *__restrict__ init, const long long *__restrict__ init_off,
+                                             int n_problems, int kcap, int S, AlleleParams P, double *__restrict__ out) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_problems) return;
+    const int K = Ks[q], A = As[q];
+    if (K > KMAX) return;
+    double x[KMAX];
+    int c[KMAX], n = 0;
+    for (int j = 0; j < K; ++j) x[j] = xs[(size_t)q * kcap + j], c[j] = cs[(size_t)q * kcap + j], n += c[j];
+    Philox rng;
+    rng.init(P.seed, (uint32_t)q, 0u);
+    double m[ALL_MAX_ALLELES], w[ALL_MAX_ALLELES], s[ALL_MAX_ALLELES];
+    int peaks = 0;
+    fit_replicate_any<KMAX, ALL_MAX_ALLELES>(x, c, K, n, A, P, rng, init ? init + init_off[q] : nullptr, m, w, s, &peaks);
+    double *o = out + (size_t)q * (3 * S + 1);
+    for (int a = 0; a < S; ++a) {
+        o[a] = a < A ? m[a] : 0.0;
+        o[S + a] = a < A ? w[a] : 0.0;
+        o[2 * S + a] = a < A ? s[a] : 0.0;
+    }
+    o[3 * S] = (double)peaks;
 }
 
 // ---------------------------------------------------------------------------------------------- aggregate
@@ -412,12 +700,13 @@ __device__ __forceinline__ double pct_iicdf(const double *a, int n, double q) {
     return g >= 0.5 ? a[hi] - d * (1.0 - g) : a[lo] + d * g;
 }
 
-// out_i [locus][1 + 2*A + 4*A]: modal_n, call[A], ci95[A][2], ci99[A][2]      out_d [locus][3*A]: means, weights, stdevs
+// out_i [locus][1 + 2*S + 4*S]: modal_n, call[S], ci95[S][2], ci99[S][2]      out_d [locus][3*S]: means, weights,
+// stdevs.  Locus l has A = A_arr[l] alleles (NULL: S) in replicate rows [locus][S][B]; its columns A..S-1 are 0.
 __global__ void __launch_bounds__(256)
 alleles_aggregate_kernel(const double *__restrict__ rep_m, const double *__restrict__ rep_w, const double *__restrict__ rep_s,
                          const unsigned char *__restrict__ rep_peaks, const int *__restrict__ status,
-                         const int *__restrict__ vals, int kcap, int n_loci, int A, int B, int *__restrict__ out_i,
-                         double *__restrict__ out_d) {
+                         const int *__restrict__ vals, int kcap, int n_loci, const int *__restrict__ A_arr, int S, int B,
+                         int *__restrict__ out_i, double *__restrict__ out_d) {
     extern __shared__ unsigned char smem_raw_all[];
     const int l = blockIdx.x;
     if (l >= n_loci) return;
@@ -425,8 +714,15 @@ alleles_aggregate_kernel(const double *__restrict__ rep_m, const double *__restr
     while (np2 < B) np2 <<= 1;
     double *key = (double *)smem_raw_all;  // [np2] replicate means of one allele
     int *idx = (int *)(key + np2);         // [np2] replicate index (tie-break = stable order)
-    int *oi = out_i + (size_t)l * (1 + 5 * A);
-    double *od = out_d + (size_t)l * (3 * A);
+    int *oi = out_i + (size_t)l * (1 + 5 * S);
+    double *od = out_d + (size_t)l * (3 * S);
+    const int A = A_arr ? A_arr[l] : S;
+    for (int a = A + threadIdx.x; a < S; a += blockDim.x) {
+        oi[1 + a] = 0;
+        oi[1 + S + 2 * a] = oi[1 + S + 2 * a + 1] = 0;
+        oi[1 + 3 * S + 2 * a] = oi[1 + 3 * S + 2 * a + 1] = 0;
+        od[a] = od[S + a] = od[2 * S + a] = 0.0;
+    }
     const int st = status[l];
     if (st != 0) {
         if (threadIdx.x == 0) {
@@ -434,23 +730,23 @@ alleles_aggregate_kernel(const double *__restrict__ rep_m, const double *__restr
             oi[0] = st == 2 ? 1 : 0;
             for (int a = 0; a < A; ++a) {
                 oi[1 + a] = cnv;
-                oi[1 + A + 2 * a] = oi[1 + A + 2 * a + 1] = cnv;
-                oi[1 + 3 * A + 2 * a] = oi[1 + 3 * A + 2 * a + 1] = cnv;
+                oi[1 + S + 2 * a] = oi[1 + S + 2 * a + 1] = cnv;
+                oi[1 + 3 * S + 2 * a] = oi[1 + 3 * S + 2 * a + 1] = cnv;
                 od[a] = (double)cnv;
-                od[A + a] = st == 2 ? 1.0 / (double)A : 0.0;
-                od[2 * A + a] = 0.0;
+                od[S + a] = st == 2 ? 1.0 / (double)A : 0.0;
+                od[2 * S + a] = 0.0;
             }
         }
         return;
     }
-    __shared__ int s_cnt[3];
-    if (threadIdx.x < 3) s_cnt[threadIdx.x] = 0;
+    __shared__ int s_cnt[256];  // replicates per peak count
+    s_cnt[threadIdx.x] = 0;
     __syncthreads();
-    for (int b = threadIdx.x; b < B; b += blockDim.x) atomicAdd(&s_cnt[rep_peaks[(size_t)l * B + b] == 2 ? 2 : 1], 1);
+    for (int b = threadIdx.x; b < B; b += blockDim.x) atomicAdd(&s_cnt[rep_peaks[(size_t)l * B + b]], 1);
     __syncthreads();
-    double wsel[2] = {0.0, 0.0};
+    double wsel[ALL_MAX_ALLELES];
     for (int a = 0; a < A; ++a) {
-        const double *m = rep_m + ((size_t)l * A + a) * B;
+        const double *m = rep_m + ((size_t)l * S + a) * B;
         for (int b = threadIdx.x; b < np2; b += blockDim.x) {
             key[b] = b < B ? m[b] : INFINITY;
             idx[b] = b;
@@ -473,23 +769,26 @@ alleles_aggregate_kernel(const double *__restrict__ rep_m, const double *__restr
             }
         if (threadIdx.x == 0) {
             const int med = B / 2;
-            const size_t o = ((size_t)l * A + a) * B + idx[med];
+            const size_t o = ((size_t)l * S + a) * B + idx[med];
             od[a] = key[med];
             wsel[a] = rep_w[o];
-            od[2 * A + a] = rep_s[o];
+            od[2 * S + a] = rep_s[o];
             oi[1 + a] = (int)rint(key[med]);
-            oi[1 + A + 2 * a] = (int)rint(pct_iicdf(key, B, 0.025));
-            oi[1 + A + 2 * a + 1] = (int)rint(pct_iicdf(key, B, 0.975));
-            oi[1 + 3 * A + 2 * a] = (int)rint(pct_iicdf(key, B, 0.005));
-            oi[1 + 3 * A + 2 * a + 1] = (int)rint(pct_iicdf(key, B, 0.995));
+            oi[1 + S + 2 * a] = (int)rint(pct_iicdf(key, B, 0.025));
+            oi[1 + S + 2 * a + 1] = (int)rint(pct_iicdf(key, B, 0.975));
+            oi[1 + 3 * S + 2 * a] = (int)rint(pct_iicdf(key, B, 0.005));
+            oi[1 + 3 * S + 2 * a + 1] = (int)rint(pct_iicdf(key, B, 0.995));
         }
         __syncthreads();
     }
     if (threadIdx.x == 0) {
         double ws = 0.0;
         for (int a = 0; a < A; ++a) ws += wsel[a];
-        for (int a = 0; a < A; ++a) od[A + a] = wsel[a] / ws;
+        for (int a = 0; a < A; ++a) od[S + a] = wsel[a] / ws;
         // statistics.mode of the sorted peak counts: the smallest of the most common
-        oi[0] = s_cnt[1] >= s_cnt[2] ? 1 : 2;
+        int modal = 0;
+        for (int k = 1; k < 256; ++k)
+            if (s_cnt[k] > s_cnt[modal]) modal = k;
+        oi[0] = modal;
     }
 }

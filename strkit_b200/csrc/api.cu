@@ -174,7 +174,7 @@ struct strk_ctx {
     // reference path (strk_ref_counts): per-locus state, and the one-read-per-locus batch of phase 2
     RefBufs ref;
     struct strk_batch *ref_batch = nullptr;
-    DevBuf<int> al_i[8];             //                 per-read / per-locus integer arrays (recycled across calls)
+    DevBuf<int> al_i[9];             //                 per-read / per-locus integer arrays (recycled across calls)
     DevBuf<double> al_d[3];
     DevBuf<long long> al_rb;
     unsigned int *d_queue = nullptr;  // [0] work queue, [1] miss counter
@@ -384,7 +384,7 @@ extern "C" int strk_destroy(strk_ctx *ctx) {
     ctx->pk_scratch.release();
     for (int k = 0; k < 3; ++k) ctx->al_rep[k].release();
     ctx->al_peaks.release();
-    for (int k = 0; k < 8; ++k) ctx->al_i[k].release();
+    for (int k = 0; k < 9; ++k) ctx->al_i[k].release();
     for (int k = 0; k < 3; ++k) ctx->al_d[k].release();
     ctx->al_rb.release();
     if (ctx->d_consts) cudaFree(ctx->d_consts);
