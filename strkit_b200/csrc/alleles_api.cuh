@@ -31,25 +31,6 @@ static int alleles_params(AlleleParams *P, int n_alleles, bool per_locus, int nu
     return STRK_OK;
 }
 
-struct AllDev {
-    std::vector<void *> ptrs;
-    ~AllDev() {
-        for (void *p : ptrs) cudaFree(p);
-    }
-    template <typename T>
-    cudaError_t get(T **dst, size_t n) {
-        cudaError_t e = cudaMalloc((void **)dst, (n ? n : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*dst);
-        return e;
-    }
-    template <typename T>
-    cudaError_t up(T **dst, const T *src, size_t n, cudaStream_t st) {
-        cudaError_t e = get(dst, n);
-        if (e == cudaSuccess && n) e = cudaMemcpyAsync(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice, st);
-        return e;
-    }
-};
-
 // the aggregation's dynamic shared memory (sort keys) plus its static array must fit the launch: 4096 replicates
 // take 48 KB of keys, so above 48 KB in all the kernel opts in to the larger carve-out
 static cudaError_t agg_smem_opt_in(size_t dyn) {
@@ -239,13 +220,13 @@ extern "C" int strk_gmm_fit_counts(strk_ctx *ctx, const double *x, const int32_t
     if (n_problems == 0) return STRK_OK;
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    AllDev dev;
+    TmpDev dev{st};
     double *d_x = nullptr, *d_out = nullptr;
     int *d_c = nullptr, *d_K = nullptr, *d_init = nullptr;
-    cudaError_t e = dev.up(&d_x, x, (size_t)n_problems * kcap, st);
-    if (e == cudaSuccess) e = dev.up(&d_c, (const int *)counts, (size_t)n_problems * kcap, st);
-    if (e == cudaSuccess) e = dev.up(&d_K, (const int *)K, (size_t)n_problems, st);
-    if (e == cudaSuccess) e = dev.up(&d_init, (const int *)init, (size_t)n_problems * 2 * n_init, st);
+    cudaError_t e = dev.up(&d_x, x, (size_t)n_problems * kcap);
+    if (e == cudaSuccess) e = dev.up(&d_c, (const int *)counts, (size_t)n_problems * kcap);
+    if (e == cudaSuccess) e = dev.up(&d_K, (const int *)K, (size_t)n_problems);
+    if (e == cudaSuccess) e = dev.up(&d_init, (const int *)init, (size_t)n_problems * 2 * n_init);
     if (e == cudaSuccess) e = dev.get(&d_out, (size_t)n_problems * 7);
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -307,16 +288,16 @@ extern "C" int strk_gmm_fit_counts_ploidy(strk_ctx *ctx, const double *x, const 
                                    init[i], K[q] - 1);
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    AllDev dev;
+    TmpDev dev{st};
     double *d_x = nullptr, *d_out = nullptr;
     int *d_c = nullptr, *d_K = nullptr, *d_A = nullptr, *d_init = nullptr;
     long long *d_off = nullptr;
-    cudaError_t e = dev.up(&d_x, x, (size_t)n_problems * kcap, st);
-    if (e == cudaSuccess) e = dev.up(&d_c, (const int *)counts, (size_t)n_problems * kcap, st);
-    if (e == cudaSuccess) e = dev.up(&d_K, (const int *)K, (size_t)n_problems, st);
-    if (e == cudaSuccess) e = dev.up(&d_A, (const int *)n_alleles, (size_t)n_problems, st);
-    if (e == cudaSuccess && init) e = dev.up(&d_init, (const int *)init, (size_t)off[n_problems], st);
-    if (e == cudaSuccess && init) e = dev.up(&d_off, off.data(), (size_t)n_problems, st);
+    cudaError_t e = dev.up(&d_x, x, (size_t)n_problems * kcap);
+    if (e == cudaSuccess) e = dev.up(&d_c, (const int *)counts, (size_t)n_problems * kcap);
+    if (e == cudaSuccess) e = dev.up(&d_K, (const int *)K, (size_t)n_problems);
+    if (e == cudaSuccess) e = dev.up(&d_A, (const int *)n_alleles, (size_t)n_problems);
+    if (e == cudaSuccess && init) e = dev.up(&d_init, (const int *)init, (size_t)off[n_problems]);
+    if (e == cudaSuccess && init) e = dev.up(&d_off, off.data(), (size_t)n_problems);
     if (e == cudaSuccess) e = dev.get(&d_out, (size_t)n_problems * (3 * S + 1));
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -350,15 +331,15 @@ extern "C" int strk_alleles_aggregate(strk_ctx *ctx, const double *rep_means, co
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const int A = n_alleles, B = num_bootstrap;
-    AllDev dev;
+    TmpDev dev{st};
     double *rm = nullptr, *rw = nullptr, *rs = nullptr, *d_od = nullptr;
     unsigned char *rp = nullptr;
     int *d_status = nullptr, *d_oi = nullptr;
     const size_t nrep = (size_t)n_loci * A * B;
-    cudaError_t e = dev.up(&rm, rep_means, nrep, st);
-    if (e == cudaSuccess) e = dev.up(&rw, rep_weights, nrep, st);
-    if (e == cudaSuccess) e = dev.up(&rs, rep_stdevs, nrep, st);
-    if (e == cudaSuccess) e = dev.up(&rp, (const unsigned char *)rep_peaks, (size_t)n_loci * B, st);
+    cudaError_t e = dev.up(&rm, rep_means, nrep);
+    if (e == cudaSuccess) e = dev.up(&rw, rep_weights, nrep);
+    if (e == cudaSuccess) e = dev.up(&rs, rep_stdevs, nrep);
+    if (e == cudaSuccess) e = dev.up(&rp, (const unsigned char *)rep_peaks, (size_t)n_loci * B);
     if (e == cudaSuccess) e = dev.get(&d_status, (size_t)n_loci);
     if (e == cudaSuccess) e = dev.get(&d_oi, (size_t)n_loci * (1 + 5 * A));
     if (e == cudaSuccess) e = dev.get(&d_od, (size_t)n_loci * 3 * A);

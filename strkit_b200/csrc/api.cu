@@ -77,6 +77,20 @@ struct DevBuf {
     }
 };
 
+// One DP pass (launch_pass): the families, their table, and per rows-per-lane class k the device list of work items
+// (0 = families only the general kernel takes) with the maxima the packed launch of class k sizes its tables by.
+struct DpPass {
+    const FamDesc *fams = nullptr;
+    const unsigned char *arena = nullptr;
+    void *table = nullptr;
+    int ref_mode = 0;  // the families are reference windows and `table` holds the 64-bit boundary keys
+    int b_len = 0, rowlen = 0;
+    long long n_slots = 0;
+    const int *list[STRK_PK_NBIN] = {nullptr};  // list[0] == nullptr: the families 0 .. cnt[0] - 1
+    long long cnt[STRK_PK_NBIN] = {0};
+    int flank[STRK_PK_NBIN] = {0}, mmax[STRK_PK_NBIN] = {0}, w[STRK_PK_NBIN] = {0};  // w: sizes of the widest window
+};
+
 // Work items of a DP pass binned by rows-per-lane class (0 = general kernel only), with the per-class maxima the packed
 // launches size their tables by.
 struct ClassLists {
@@ -93,9 +107,9 @@ struct ClassLists {
         flank[k] = std::max(flank[k], std::max(fl, fr));
         w_max[k] = std::max(w_max[k], w);
     }
-    // Queues the copy of the lists into `buf` on `st` and points seg_list / seg_cnt (launch_pass) at the device
-    // segments.  `flat` is read by the copy until `st` has passed it.
-    int upload(DevBuf<int> &buf, cudaStream_t st, const int **seg_list, long long *seg_cnt) {
+    // Queues the copy of the lists into `buf` on `st` and points the classes of `p` at the device segments, with these
+    // maxima.  `flat` is read by the copy until `st` has passed it.
+    int upload(DevBuf<int> &buf, cudaStream_t st, DpPass &p) {
         size_t at[STRK_PK_NBIN];
         flat.clear();
         for (int k = 0; k < STRK_PK_NBIN; ++k) {
@@ -107,7 +121,10 @@ struct ClassLists {
             return set_err(STRK_ERR_NOMEM, "cannot allocate the class lists of a pass");
         }
         CU(cudaMemcpyAsync(buf.p, flat.data(), flat.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_list[k] = buf.p + at[k], seg_cnt[k] = (long long)items[k].size();
+        for (int k = 0; k < STRK_PK_NBIN; ++k) {
+            p.list[k] = buf.p + at[k], p.cnt[k] = (long long)items[k].size();
+            p.flank[k] = flank[k], p.mmax[k] = mmax[k], p.w[k] = w_max[k];
+        }
         return STRK_OK;
     }
 };
@@ -144,6 +161,18 @@ struct RefBufs {
     }
 };
 
+// The device counter words of a context (strk_ctx::d_queue, addressed through strk_ctx::counter)
+enum CounterSlot : int {
+    Q_GENERAL = 0,   // work queue of the general kernel
+    Q_MISS = 1,      // loci whose search left the window (the replay kernels)
+    Q_FALLBACK = 2,  // reads the packed kernel handed to the general kernel
+    Q_MARGIN = 3,    // loci the wide_short margin saved (the replay kernels count them at Q_MISS + 2)
+    Q_WIDEST = 6,    // the widest stretched window of a widening pass
+    Q_INT_PEAK = 7,  // the output word of strk_measure_int_peak
+    Q_CLASS = 8,     // + k: work queue of packed class k
+};
+static_assert(Q_FALLBACK == Q_MISS + 1 && Q_MARGIN == Q_MISS + 2, "strk_batch_run reads the three words in one copy");
+
 struct strk_ctx {
     int device = 0;
     int n_sm = 0;
@@ -177,7 +206,8 @@ struct strk_ctx {
     DevBuf<int> al_i[9];             //                 per-read / per-locus integer arrays (recycled across calls)
     DevBuf<double> al_d[3];
     DevBuf<long long> al_rb;
-    unsigned int *d_queue = nullptr;  // [0] work queue, [1] miss counter
+    unsigned int *d_queue = nullptr;  // counter words (CounterSlot)
+    unsigned int *counter(int slot) const { return d_queue + slot; }
     double *d_acc = nullptr;          // [0] ref cells, [1] executed cells
     PlanStats *d_plan = nullptr;      // device-side planning counters
     unsigned int *d_bin_off = nullptr;
@@ -340,8 +370,9 @@ extern "C" int strk_init(int device, const int8_t matrix[STRK_NSYM * STRK_NSYM],
         CU(cudaStreamCreateWithPriority(&ctx->fill_stream, cudaStreamNonBlocking, lo));
     }
     CU(cudaMalloc((void **)&ctx->d_consts, sizeof(ScoreConsts)));
-    CU(cudaMemcpy(ctx->d_consts, &ctx->h_consts, sizeof(ScoreConsts), cudaMemcpyHostToDevice));
-    CU(cudaMalloc((void **)&ctx->d_queue, (8 + STRK_PK_NBIN + 1) * sizeof(unsigned int)));  // [8 + k]: work queue of packed class k
+    CU(cudaMemcpyAsync(ctx->d_consts, &ctx->h_consts, sizeof(ScoreConsts), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    CU(cudaMalloc((void **)&ctx->d_queue, (Q_CLASS + STRK_PK_NBIN + 1) * sizeof(unsigned int)));
     CU(cudaMalloc((void **)&ctx->d_acc, 4 * sizeof(double)));
     CU(cudaMalloc((void **)&ctx->d_plan, sizeof(PlanStats)));
     CU(cudaMalloc((void **)&ctx->d_bin_off, STRK_PK_NBIN * sizeof(unsigned int)));
@@ -519,15 +550,14 @@ static int launch_general(strk_ctx *ctx, bool ref, const FamDesc *d_fams, const 
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "cannot allocate %zu bytes of DP scratch", total * sizeof(int));
     }
-    CU(cudaMemsetAsync(ctx->d_queue, 0, sizeof(unsigned int), st));
+    unsigned int *queue = ctx->counter(Q_GENERAL);
+    CU(cudaMemsetAsync(queue, 0, sizeof(unsigned int), st));
     if (ref)
         dp_general_kernel<true><<<grid, GEN_THREADS, 0, st>>>(d_fams, d_order, (int)n_fams, d_arena, ctx->d_consts,
-                                                              d_table, ctx->scratch.p, rowlen, b_len, ctx->d_queue,
-                                                              d_count);
+                                                              d_table, ctx->scratch.p, rowlen, b_len, queue, d_count);
     else
         dp_general_kernel<false><<<grid, GEN_THREADS, 0, st>>>(d_fams, d_order, (int)n_fams, d_arena, ctx->d_consts,
-                                                               d_table, ctx->scratch.p, rowlen, b_len, ctx->d_queue,
-                                                               d_count);
+                                                               d_table, ctx->scratch.p, rowlen, b_len, queue, d_count);
     CU(cudaGetLastError());
     ctx->stats[2] += 1;
     return STRK_OK;
@@ -576,11 +606,12 @@ static int launch_packed_r(strk_ctx *ctx, const FamDesc *fams, const int *list, 
     // per launch of the R = 10 class, no change in kernel time (the kernel is integer-issue bound, the write-backs use
     // ~10 % of HBM bandwidth), -2 % on the streamed path where two contexts' windows compete for the set-aside: it is
     // not pinned (DESIGN.md 5.1).
-    unsigned int *work_counter = ctx->d_queue + 8 + (L == 16 ? R / 2 : R);  // one queue per rows-per-lane class
+    unsigned int *work_counter = ctx->counter(Q_CLASS + (L == 16 ? R / 2 : R));  // one queue per rows-per-lane class
     CU(cudaMemsetAsync(work_counter, 0, sizeof(unsigned int), st));
     dp_packed_kernel<R, L><<<(unsigned)grid, pk_warps(L) * 32, smem, st>>>(fams, list, n, arena, ctx->d_consts, table, dims,
                                                                         ctx->pk_scratch.p + (scratch_off > 0 ? scratch_off : 0),
-                                                                        ctx->fallback.p, ctx->d_queue + 2, ref_mode, work_counter);
+                                                                        ctx->fallback.p, ctx->counter(Q_FALLBACK), ref_mode,
+                                                                        work_counter);
     CU(cudaGetLastError());
     ctx->stats[2] += 1;
     return STRK_OK;
@@ -635,128 +666,129 @@ static int launch_packed(strk_ctx *ctx, int R, const FamDesc *fams, const int *l
     }
 }
 
-// One launch per rows-per-lane class k >= 1 of a pass (list[k], cnt[k]; tables sized by flank[k], mmax[k], w_max[k]);
-// a class whose tables do not fit shared memory goes to the general kernel.  Large passes: back to back on the
-// run's stream (spreading the classes over several streams was measured slower there, -2.8 %: concurrent grids with
-// different footprints fragment the SMs).  Small passes, where a class is less than a wave of CTAs and each launch
-// lasts one read's sweep whatever its grid: every class on its own side stream with its own slice of the capture
-// scratch, so the launches overlap (blocks of a few hundred loci, per-locus calls, second passes, the reference path).
-static int launch_packed_classes(strk_ctx *ctx, const int *const *list, const long long *cnt, const int *flank,
-                                 const int *mmax, const int *w_max, long long n_slots, const FamDesc *fams,
-                                 const unsigned char *arena, void *table, int b_len, int rowlen, cudaStream_t st,
-                                 int ref_mode, long long *n_packed) {
+// Whether the packed kernel takes a pass of windows of W sizes (a reference window, a forward and a reverse column per
+// size, counts twice), and a family's class in such a pass.  The planners gate on the matrix only: a batch's windows are
+// decided per pass.
+static bool pk_window_ok(const strk_ctx *ctx, int kernel, int ref_mode, int W) {
+    return kernel != STRK_KERNEL_GENERAL && ctx->h_consts.packed_ok && (ref_mode ? 2 * W : W) <= PK_WINDOW_MAX;
+}
+static int pk_class(const strk_ctx *ctx, int kernel, int ref_mode, int W, int fl, int tr, int fr, int m) {
+    return pk_window_ok(ctx, kernel, ref_mode, W) ? strk_pk_class(fl, tr, fr, m) : 0;
+}
+
+// Table width (PackedDims::w_max) of a packed class whose widest window holds W sizes
+static int pk_table_w(int ref_mode, int W) { return ref_mode ? 2 * W - 1 : (W + 3) / 4 * 4; }
+
+// One DP pass: list[0] through the general kernel, list[k >= 1] through the packed kernel (or, when the class' tables do
+// not fit shared memory, the general kernel), then the packed kernel's fallbacks (a device-side list, Q_FALLBACK long)
+// through the general kernel; *n_packed = the items the packed launches took.  A pass without packed items is one
+// general launch.  The general launch of list[0] is a handful of families (reads / reference windows of 512+ bases,
+// IUPAC reads) whose duration is the LATENCY of one family's chain (0.3 - 0.6 ms) whatever the grid: it starts first, on
+// its own side stream, under the packed launches (it used to be 3 % of a 32 768-locus read step).  Large passes run the
+// classes back to back on `st` (several streams were measured slower there, -2.8 %: concurrent grids with different
+// footprints fragment the SMs); small passes, where each launch lasts one read's sweep whatever its grid, run every
+// class on its own side stream with its own slice of the capture scratch, so the launches overlap.
+// strk_ref_counts queues several passes before it synchronises, so no reservation here may reallocate a buffer that a
+// queued pass still reads: it reserves the fallback list (and its class lists) for the whole call up front.
+static int launch_pass(strk_ctx *ctx, const DpPass &p, cudaStream_t st, long long *n_packed) {
     static const long long fan_max = [] {
         const char *e = getenv("STRK_PK_FANOUT_MAX");  // reads per pass up to which the classes overlap
         return e ? atoll(e) : 131072LL;
     }();
+    const bool ref = p.ref_mode != 0;
+    *n_packed = 0;
+    long long packed_total = 0;
+    for (int k = 1; k < STRK_PK_NBIN; ++k) packed_total += p.cnt[k];
+    if (!packed_total) return launch_general(ctx, ref, p.fams, p.list[0], p.cnt[0], p.arena, p.table, p.b_len, p.rowlen, st);
+
+    PackedDims dims[STRK_PK_NBIN];
+    bool fits[STRK_PK_NBIN] = {false};
+    bool overlap = p.cnt[0] > 0;  // (not when a class runs on the general kernel itself)
+    long long fams_max = std::max(p.cnt[0], std::min(packed_total, (long long)ctx->n_sm * 4));
+    for (int k = 1; k < STRK_PK_NBIN; ++k) {
+        if (!p.cnt[k]) continue;
+        dims[k] = pk_dims_for_class(k, p.flank[k], p.mmax[k], pk_table_w(p.ref_mode, p.w[k]));
+        fits[k] = pk_smem_for_class(k, dims[k]) <= 200 * 1024;
+        overlap = overlap && fits[k];
+        fams_max = std::max(fams_max, p.cnt[k]);
+    }
+    // scratch of the largest general launch of this pass, reserved before anything is in flight
+    const size_t total = general_scratch_max(ctx, fams_max, p.b_len, p.rowlen);
+    if (ctx->scratch.reserve(total) != cudaSuccess) {
+        cudaGetLastError();
+        return set_err(STRK_ERR_NOMEM, "cannot allocate %zu bytes of DP scratch", total * sizeof(int));
+    }
+    if (ctx->fallback.reserve((size_t)packed_total) != cudaSuccess) {
+        cudaGetLastError();
+        return set_err(STRK_ERR_NOMEM, "cannot allocate the fallback list");
+    }
+    CU(cudaMemsetAsync(ctx->counter(Q_FALLBACK), 0, sizeof(unsigned int), st));
+    if (!ctx->fork_ev) CU(cudaEventCreateWithFlags(&ctx->fork_ev, cudaEventDisableTiming));
     int rc = STRK_OK;
+    if (overlap) {
+        if (!ctx->side[0]) CU(cudaStreamCreateWithPriority(&ctx->side[0], cudaStreamNonBlocking, ctx->prio_hi));
+        if (!ctx->side_ev[0]) CU(cudaEventCreateWithFlags(&ctx->side_ev[0], cudaEventDisableTiming));
+        CU(cudaEventRecord(ctx->fork_ev, st));
+        CU(cudaStreamWaitEvent(ctx->side[0], ctx->fork_ev, 0));
+        rc = launch_general(ctx, ref, p.fams, p.list[0], p.cnt[0], p.arena, p.table, p.b_len, p.rowlen, ctx->side[0]);
+        if (rc) return rc;
+        CU(cudaEventRecord(ctx->side_ev[0], ctx->side[0]));
+    }
     long long fan_off[STRK_PK_NBIN];
     bool fan_out = false;
-    if (n_slots <= fan_max) {
-        size_t total = 0;
+    if (p.n_slots <= fan_max) {
+        size_t scratch = 0;
         int n_classes = 0;
         for (int k = STRK_PK_RMAX; k >= 1; --k) {
-            fan_off[k] = -1;
-            if (!cnt[k]) continue;
-            const PackedDims dims = pk_dims_for_class(k, flank[k], mmax[k], w_max[k]);
-            if (pk_smem_for_class(k, dims) > 200 * 1024) continue;
+            if (!p.cnt[k] || !fits[k]) continue;
             size_t need = 0;
-            rc = launch_packed(ctx, k, fams, list[k], (int)cnt[k], arena, (int *)table, dims, st, ref_mode, &need);
+            rc = launch_packed(ctx, k, p.fams, p.list[k], (int)p.cnt[k], p.arena, (int *)p.table, dims[k], st, p.ref_mode,
+                               &need);
             if (rc) return rc;
-            fan_off[k] = (long long)total;
-            total += need;
+            fan_off[k] = (long long)scratch;
+            scratch += need;
             ++n_classes;
         }
         if (n_classes >= 2) {
-            if (ctx->pk_scratch.reserve(total) != cudaSuccess) {
+            if (ctx->pk_scratch.reserve(scratch) != cudaSuccess) {
                 cudaGetLastError();
-                return set_err(STRK_ERR_NOMEM, "cannot allocate %zu bytes of capture scratch", total * sizeof(uint4));
+                return set_err(STRK_ERR_NOMEM, "cannot allocate %zu bytes of capture scratch", scratch * sizeof(uint4));
             }
-            if (!ctx->fork_ev) CU(cudaEventCreateWithFlags(&ctx->fork_ev, cudaEventDisableTiming));
             CU(cudaEventRecord(ctx->fork_ev, st));
             fan_out = true;
         }
     }
     for (int k = STRK_PK_RMAX; k >= 1; --k) {
-        if (!cnt[k]) continue;
-        const PackedDims dims = pk_dims_for_class(k, flank[k], mmax[k], w_max[k]);
-        if (fan_out && fan_off[k] >= 0) {
+        if (!p.cnt[k]) continue;
+        if (!fits[k]) {
+            rc = launch_general(ctx, ref, p.fams, p.list[k], p.cnt[k], p.arena, p.table, p.b_len, p.rowlen, st);
+            if (rc) return rc;
+            continue;
+        }
+        if (fan_out) {
             if (!ctx->side[k]) CU(cudaStreamCreateWithPriority(&ctx->side[k], cudaStreamNonBlocking, ctx->prio_hi));
             if (!ctx->side_ev[k]) CU(cudaEventCreateWithFlags(&ctx->side_ev[k], cudaEventDisableTiming));
             CU(cudaStreamWaitEvent(ctx->side[k], ctx->fork_ev, 0));
-            rc = launch_packed(ctx, k, fams, list[k], (int)cnt[k], arena, (int *)table, dims, ctx->side[k], ref_mode, nullptr,
-                               fan_off[k]);
+            rc = launch_packed(ctx, k, p.fams, p.list[k], (int)p.cnt[k], p.arena, (int *)p.table, dims[k], ctx->side[k],
+                               p.ref_mode, nullptr, fan_off[k]);
             if (rc) return rc;
             CU(cudaEventRecord(ctx->side_ev[k], ctx->side[k]));
             CU(cudaStreamWaitEvent(st, ctx->side_ev[k], 0));
-            *n_packed += cnt[k];
-            continue;
-        }
-        if (pk_smem_for_class(k, dims) > 200 * 1024) {
-            // shared memory would not fit: hand the whole segment to the general kernel
-            rc = launch_general(ctx, ref_mode != 0, fams, list[k], cnt[k], arena, table, b_len, rowlen, st);
+        } else {
+            rc = launch_packed(ctx, k, p.fams, p.list[k], (int)p.cnt[k], p.arena, (int *)p.table, dims[k], st, p.ref_mode);
             if (rc) return rc;
-            continue;
         }
-        rc = launch_packed(ctx, k, fams, list[k], (int)cnt[k], arena, (int *)table, dims, st, ref_mode);
-        if (rc) return rc;
-        *n_packed += cnt[k];
+        *n_packed += p.cnt[k];
     }
-    return STRK_OK;
-}
-
-// One DP pass over a work plan: list[0] = families only the general kernel takes, list[k >= 1] = the packed classes,
-// then the packed kernel's fallbacks (a device-side list) through the general kernel.  The general launch of list[0]
-// is a handful of families (reads / reference windows of 512+ bases, IUPAC reads) whose duration is the LATENCY of one
-// family's dependency chain (0.3 - 0.6 ms) whatever the grid: it starts first, on its own side stream, and runs under
-// the packed launches instead of after them (it used to be 3 % of a 32 768-locus read step and a quarter of the
-// reference path of the same block).
-static int launch_pass(strk_ctx *ctx, const int *const *list, const long long *cnt, const int *flank, const int *mmax,
-                       const int *w_max, long long n_slots, const FamDesc *fams, const unsigned char *arena, void *table,
-                       int b_len, int rowlen, cudaStream_t st, int ref_mode, long long *n_packed) {
-    bool overlap = cnt[0] > 0;
-    long long packed_total = 0;
-    for (int k = 1; k < STRK_PK_NBIN; ++k) {
-        if (!cnt[k]) continue;
-        packed_total += cnt[k];
-        const PackedDims dims = pk_dims_for_class(k, flank[k], mmax[k], w_max[k]);
-        if (pk_smem_for_class(k, dims) > 200 * 1024) overlap = false;  // that class runs on the general kernel itself
-    }
-    {
-        // scratch of the largest general launch of this pass, reserved before anything is in flight
-        long long fams_max = std::max(cnt[0], std::min(packed_total, (long long)ctx->n_sm * 4));
-        for (int k = 1; k < STRK_PK_NBIN; ++k) fams_max = std::max(fams_max, cnt[k]);
-        const size_t total = general_scratch_max(ctx, fams_max, b_len, rowlen);
-        if (ctx->scratch.reserve(total) != cudaSuccess) {
-            cudaGetLastError();
-            return set_err(STRK_ERR_NOMEM, "cannot allocate %zu bytes of DP scratch", total * sizeof(int));
-        }
-    }
-    int rc = STRK_OK;
-    if (overlap) {
-        if (!ctx->side[0]) CU(cudaStreamCreateWithPriority(&ctx->side[0], cudaStreamNonBlocking, ctx->prio_hi));
-        if (!ctx->side_ev[0]) CU(cudaEventCreateWithFlags(&ctx->side_ev[0], cudaEventDisableTiming));
-        if (!ctx->fork_ev) CU(cudaEventCreateWithFlags(&ctx->fork_ev, cudaEventDisableTiming));
-        CU(cudaEventRecord(ctx->fork_ev, st));
-        CU(cudaStreamWaitEvent(ctx->side[0], ctx->fork_ev, 0));
-        rc = launch_general(ctx, ref_mode != 0, fams, list[0], cnt[0], arena, table, b_len, rowlen, ctx->side[0]);
-        if (rc) return rc;
-        CU(cudaEventRecord(ctx->side_ev[0], ctx->side[0]));
-    }
-    rc = launch_packed_classes(ctx, list, cnt, flank, mmax, w_max, n_slots, fams, arena, table, b_len, rowlen, st, ref_mode,
-                               n_packed);
-    if (rc) return rc;
     if (overlap) {
         CU(cudaStreamWaitEvent(st, ctx->side_ev[0], 0));
     } else {
-        rc = launch_general(ctx, ref_mode != 0, fams, list[0], cnt[0], arena, table, b_len, rowlen, st);
+        rc = launch_general(ctx, ref, p.fams, p.list[0], p.cnt[0], p.arena, p.table, p.b_len, p.rowlen, st);
         if (rc) return rc;
     }
-    if (*n_packed) {
-        rc = launch_general(ctx, ref_mode != 0, fams, ctx->fallback.p, *n_packed, arena, table, b_len, rowlen, st,
-                            ctx->d_queue + 2);
-        if (rc) return rc;
-    }
+    if (*n_packed)
+        return launch_general(ctx, ref, p.fams, ctx->fallback.p, *n_packed, p.arena, p.table, p.b_len, p.rowlen, st,
+                              ctx->counter(Q_FALLBACK));
     return STRK_OK;
 }
 
@@ -1041,14 +1073,86 @@ static int launch_replay(strk_ctx *ctx, const strk_batch *b, int W, int wd, int 
     if (W <= REPLAY_WMAX)
         replay_reads_small_kernel<<<(unsigned)((n_list + REPLAY_THREADS - 1) / REPLAY_THREADS), REPLAY_THREADS, 0, st>>>(
             ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
-            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->d_queue + 1, ctx->d_acc,
+            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->counter(Q_MISS), ctx->d_acc,
             d_rep, d_hint);
     else
         replay_reads_kernel<<<(unsigned)((n_list + 127) / 128), 128, 0, st>>>(
             ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
-            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->d_queue + 1, ctx->d_acc,
+            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->counter(Q_MISS), ctx->d_acc,
             d_rep, d_hint);
     CU(cudaGetLastError());
+    return STRK_OK;
+}
+
+// The classes of a widening pass over the reads of h_read_ids (slot sl = read h_read_ids[sl]): each read in the class
+// planned for it at upload time (h_bin, read back once per run), with the batch's class maxima.
+static int widening_pass(strk_ctx *ctx, const strk_batch *b, const std::vector<int> &h_read_ids,
+                         std::vector<unsigned char> &h_bin, int W, cudaStream_t st, DpPass &p) {
+    if (h_bin.empty()) {
+        h_bin.resize((size_t)b->n_reads);
+        CU(cudaMemcpyAsync(h_bin.data(), b->bin.p, (size_t)b->n_reads, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    ClassLists lists;
+    for (int k = 0; k < STRK_PK_NBIN; ++k) lists.flank[k] = b->bin_flank[k], lists.mmax[k] = b->bin_mmax[k], lists.w_max[k] = W;
+    // A small pass is launch-latency bound (one read's sweep is ~100 us whatever the grid): its reads run in the largest
+    // class of their lane group (pad rows cost nothing there), two launches instead of 15.
+    int merged[STRK_PK_NBIN];
+    for (int k = 0; k < STRK_PK_NBIN; ++k) merged[k] = k;
+    if (h_read_ids.size() <= 8192) {
+        bool used[STRK_PK_NBIN] = {false};
+        for (int r : h_read_ids) used[h_bin[(size_t)r]] = true;
+        for (int L = 16; L <= 32; L += 16) {
+            int top = 0;
+            for (int k = 1; k < STRK_PK_NBIN; ++k)
+                if (used[k] && pk_lanes_for_class(k) == L) top = k;
+            for (int k = 1; k < top; ++k)
+                if (used[k] && pk_lanes_for_class(k) == L) {
+                    merged[k] = top;
+                    lists.flank[top] = std::max(lists.flank[top], lists.flank[k]);
+                    lists.mmax[top] = std::max(lists.mmax[top], lists.mmax[k]);
+                }
+        }
+    }
+    for (size_t sl = 0; sl < h_read_ids.size(); ++sl) lists.add(merged[h_bin[(size_t)h_read_ids[sl]]], (int)sl);
+    const int rc = lists.upload(ctx->list_d, st, p);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(st));  // `lists` is read by the copy
+    return STRK_OK;
+}
+
+// The loci of the next widening pass: those of the last pass (pass 0: every locus) whose search left its window
+// (status 1; status 2 is an error), their reads as the slots of the pass and each locus' first slot, uploaded to
+// ctx->list_a (reads), list_b (loci) and list_c (first slots).
+static int next_loci(strk_ctx *ctx, const strk_batch *b, bool from_pass0, int max_iters, std::vector<int> &h_locus_ids,
+                     std::vector<int> &h_read_ids, std::vector<long long> &h_slot_begin, cudaStream_t st) {
+    std::vector<unsigned char> h_status((size_t)b->n_loci);
+    CU(cudaMemcpy(h_status.data(), b->d_status, (size_t)b->n_loci, cudaMemcpyDeviceToHost));
+    std::vector<int> loci;
+    h_read_ids.clear();
+    h_slot_begin.clear();
+    const long long n_last = from_pass0 ? b->n_loci : (long long)h_locus_ids.size();
+    for (long long i = 0; i < n_last; ++i) {
+        const int l = from_pass0 ? (int)i : h_locus_ids[(size_t)i];
+        if (!h_status[(size_t)l]) continue;
+        if (h_status[(size_t)l] == 2)
+            return set_err(STRK_ERR_SEARCH, "locus %d: the search scored no size (max_iters = %d)", l, max_iters);
+        loci.push_back(l);
+        h_slot_begin.push_back((long long)h_read_ids.size());
+        for (long long r = b->h_read_begin[(size_t)l]; r < b->h_read_begin[(size_t)l + 1]; ++r)
+            h_read_ids.push_back((int)r);
+    }
+    h_locus_ids.swap(loci);
+    if (ctx->list_a.reserve(h_read_ids.size()) != cudaSuccess || ctx->list_b.reserve(h_locus_ids.size()) != cudaSuccess ||
+        ctx->list_c.reserve(h_slot_begin.size()) != cudaSuccess) {
+        cudaGetLastError();
+        return set_err(STRK_ERR_NOMEM, "cannot allocate widening lists");
+    }
+    CU(cudaMemcpyAsync(ctx->list_a.p, h_read_ids.data(), h_read_ids.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(ctx->list_b.p, h_locus_ids.data(), h_locus_ids.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(ctx->list_c.p, h_slot_begin.data(), h_slot_begin.size() * sizeof(long long), cudaMemcpyHostToDevice,
+                       st));
+    CU(cudaStreamSynchronize(st));
     return STRK_OK;
 }
 
@@ -1077,13 +1181,9 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
     int ws = b->wide_short;
     if (const char *env = getenv("STRK_WIDE_SHORT")) ws = atoi(env) != 0;  // tuning only
     const int wd_cap = (STRK_MAX_WINDOW - 1) / 2 - 2;
-    long long n_slots = b->n_reads;
-    long long n_list = b->n_loci;
-    const int *d_read_ids = nullptr, *d_locus_ids = nullptr;
-    const long long *d_slot_begin = nullptr;
-    std::vector<int> h_read_ids, h_locus_ids;
+    std::vector<int> h_read_ids, h_locus_ids;  // widening passes: the reads of the slots, the loci being redone
     std::vector<long long> h_slot_begin;
-    std::vector<unsigned char> h_status, h_bin;
+    std::vector<unsigned char> h_bin;
     float ms_dp = 0.f, ms_replay = 0.f;
     double acc[2] = {0, 0};  // [0] reference-equivalent cells, [1] executed cells
 
@@ -1097,17 +1197,22 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
     for (int pass = 0;; ++pass) {
         if (wd > wd_cap) wd = wd_cap;
         const int threads = 256;
+        // pass 0: every read of every locus; a widening pass: the reads of the loci being redone (next_loci)
+        const long long n_slots = pass ? (long long)h_read_ids.size() : b->n_reads;
+        const long long n_list = pass ? (long long)h_locus_ids.size() : b->n_loci;
+        const int *d_read_ids = pass ? ctx->list_a.p : nullptr, *d_locus_ids = pass ? ctx->list_b.p : nullptr;
+        const long long *d_slot_begin = pass ? ctx->list_c.p : nullptr;
         const double *d_hint = pass ? b->hint.p : nullptr;
         int W = 2 * strk_read_wd(wd, 1, ws) + 1;  // table stride: the widest per-read window
         if (pass) {
             // windows of a widening pass are stretched towards the starts the locus' offset has produced: measure the widest
-            CU(cudaMemsetAsync(ctx->d_queue + 6, 0, sizeof(unsigned int), st));
+            CU(cudaMemsetAsync(ctx->counter(Q_WIDEST), 0, sizeof(unsigned int), st));
             plan_reads_kernel<<<(unsigned)((n_slots + threads - 1) / threads), threads, 0, st>>>(
                 d_read_ids, n_slots, b->d_seq_off, b->d_lens, b->d_est, b->d_read_locus, b->d_motif_off, b->d_motif_len, wd, ws,
-                W, ctx->fams.p, ctx->d_acc + 1, nullptr, d_hint, ctx->d_queue + 6);
+                W, ctx->fams.p, ctx->d_acc + 1, nullptr, d_hint, ctx->counter(Q_WIDEST));
             CU(cudaGetLastError());
             unsigned int w_needed = 0;
-            CU(cudaMemcpyAsync(&w_needed, ctx->d_queue + 6, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(&w_needed, ctx->counter(Q_WIDEST), sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
             CU(cudaStreamSynchronize(st));
             if ((int)w_needed > W) W = (int)w_needed;
             if (W > STRK_MAX_WINDOW)
@@ -1126,71 +1231,30 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
         ctx->stats[2] += 1;
         CU(cudaEventRecord(ctx->ev[0], st));
         int rc = STRK_OK;
-        // packed kernel: every pass whose window it can hold (the first widening pass included: 8x the first window)
-        const bool use_packed = kernel != STRK_KERNEL_GENERAL && ctx->h_consts.packed_ok && W <= PK_WINDOW_MAX;
-        long long n_packed = 0;
+        // packed kernel per rows-per-lane class, for every pass whose window it can hold (the first widening pass
+        // included: 8x the first window); what it cannot take goes to the general kernel
+        const bool use_packed = pk_window_ok(ctx, kernel, 0, W);
+        DpPass dp{ctx->fams.p, b->d_arena, ctx->table.p, 0, b_len, rowlen, n_slots};
         if (!use_packed) {
             // (first pass: the work order lists the representatives only when identical reads share tables)
-            rc = launch_general(ctx, false, ctx->fams.p, pass ? nullptr : b->d_order, n_slots - (pass == 0 ? b->n_dup : 0),
-                                b->d_arena, ctx->table.p, b_len, rowlen, st);
-            if (rc) return rc;
+            dp.list[0] = pass ? nullptr : b->d_order;
+            dp.cnt[0] = n_slots - (pass == 0 ? b->n_dup : 0);
+        } else if (pass == 0) {  // the batch's work plan: the general kernel's reads, then one segment per class
+            for (int k = 0; k < STRK_PK_NBIN; ++k) {
+                dp.list[k] = b->d_order + b->bin_off[k], dp.cnt[k] = b->bin_cnt[k];
+                dp.flank[k] = b->bin_flank[k], dp.mmax[k] = b->bin_mmax[k], dp.w[k] = W;
+            }
+            dp.list[0] = b->d_order, dp.cnt[0] = b->n_general;
         } else {
-            // Packed kernel per rows-per-lane class; what it cannot take goes to the general kernel.
-            // Pass 0: slot == read, the class segments of the batch's work order.  Widening passes: the slots of
-            // the loci being redone, binned on the host by the class planned for their reads at upload time.
-            if (ctx->fallback.reserve((size_t)b->n_reads) != cudaSuccess) {
-                cudaGetLastError();
-                return set_err(STRK_ERR_NOMEM, "cannot allocate the fallback list");
-            }
-            const int *seg_list[STRK_PK_NBIN];
-            long long seg_cnt[STRK_PK_NBIN];
-            int seg_flank[STRK_PK_NBIN], seg_mmax[STRK_PK_NBIN];
-            for (int k = 0; k < STRK_PK_NBIN; ++k) seg_flank[k] = b->bin_flank[k], seg_mmax[k] = b->bin_mmax[k];
-            if (pass == 0) {
-                for (int k = 0; k < STRK_PK_NBIN; ++k) seg_list[k] = b->d_order + b->bin_off[k], seg_cnt[k] = b->bin_cnt[k];
-                seg_cnt[0] = b->n_general;
-                seg_list[0] = b->d_order;
-            } else {
-                if (h_bin.empty()) {
-                    h_bin.resize((size_t)b->n_reads);
-                    CU(cudaMemcpyAsync(h_bin.data(), b->bin.p, (size_t)b->n_reads, cudaMemcpyDeviceToHost, st));
-                    CU(cudaStreamSynchronize(st));
-                }
-                // A small pass is launch-latency bound (one read's sweep is ~100 us whatever the grid): its reads run
-                // in the largest class of their lane group (pad rows cost nothing there), two launches instead of 15.
-                int merged[STRK_PK_NBIN];
-                for (int k = 0; k < STRK_PK_NBIN; ++k) merged[k] = k;
-                if (h_read_ids.size() <= 8192) {
-                    bool used[STRK_PK_NBIN] = {false};
-                    for (int r : h_read_ids) used[h_bin[(size_t)r]] = true;
-                    for (int L = 16; L <= 32; L += 16) {
-                        int top = 0;
-                        for (int k = 1; k < STRK_PK_NBIN; ++k)
-                            if (used[k] && pk_lanes_for_class(k) == L) top = k;
-                        for (int k = 1; k < top; ++k)
-                            if (used[k] && pk_lanes_for_class(k) == L) {
-                                merged[k] = top;
-                                seg_flank[top] = seg_flank[top] > seg_flank[k] ? seg_flank[top] : seg_flank[k];
-                                seg_mmax[top] = seg_mmax[top] > seg_mmax[k] ? seg_mmax[top] : seg_mmax[k];
-                            }
-                    }
-                }
-                ClassLists lists;
-                for (size_t sl = 0; sl < h_read_ids.size(); ++sl) lists.add(merged[h_bin[(size_t)h_read_ids[sl]]], (int)sl);
-                rc = lists.upload(ctx->list_d, st, seg_list, seg_cnt);
-                if (rc) return rc;
-                CU(cudaStreamSynchronize(st));  // `lists` is read by the copy
-            }
-            CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
-            int seg_w[STRK_PK_NBIN];
-            for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w[k] = (W + 3) / 4 * 4;
-            rc = launch_pass(ctx, seg_list, seg_cnt, seg_flank, seg_mmax, seg_w, n_slots, ctx->fams.p, b->d_arena, ctx->table.p,
-                             b_len, rowlen, st, 0, &n_packed);
+            rc = widening_pass(ctx, b, h_read_ids, h_bin, W, st, dp);
             if (rc) return rc;
         }
+        long long n_packed = 0;
+        rc = launch_pass(ctx, dp, st, &n_packed);
+        if (rc) return rc;
         CU(cudaEventRecord(ctx->ev[1], st));
-        CU(cudaMemsetAsync(ctx->d_queue + 1, 0, sizeof(unsigned int), st));
-        CU(cudaMemsetAsync(ctx->d_queue + 3, 0, sizeof(unsigned int), st));
+        CU(cudaMemsetAsync(ctx->counter(Q_MISS), 0, sizeof(unsigned int), st));
+        CU(cudaMemsetAsync(ctx->counter(Q_MARGIN), 0, sizeof(unsigned int), st));
         rc = launch_replay(ctx, b, W, wd, ws, d_locus_ids, d_slot_begin, n_list, max_iters, local_search_range, step_size,
                            pass == 0 ? b->d_rep : nullptr, b->hint.p, st);
         if (rc) return rc;
@@ -1198,14 +1262,13 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
         CU(cudaEventRecord(ctx->ev[2], st));
         // [0] loci whose search left the window, [1] packed-kernel fallbacks, [2] loci saved by the wide_short margin
         unsigned int miss_fb[3] = {0, 0, 0};
-        CU(cudaMemcpyAsync(miss_fb, ctx->d_queue + 1, 3 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(miss_fb, ctx->counter(Q_MISS), 3 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
         CU(cudaMemcpyAsync(acc, ctx->d_acc, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));  // cumulative over passes
         CU(cudaStreamSynchronize(st));
-        const unsigned int miss = miss_fb[0];
-        if (use_packed) {
-            ctx->stats[6] += (double)(n_packed - (long long)miss_fb[1]);
-            ctx->stats[7] -= (double)(n_packed - (long long)miss_fb[1]);
-        }
+        // (launch_pass zeroes the fallback counter of a pass with packed items only)
+        const unsigned int miss = miss_fb[0], fallbacks = n_packed ? miss_fb[1] : 0;
+        ctx->stats[6] += (double)(n_packed - (long long)fallbacks);
+        ctx->stats[7] -= (double)(n_packed - (long long)fallbacks);
         float t0 = 0.f, t1 = 0.f;
         CU(cudaEventElapsedTime(&t0, ctx->ev[0], ctx->ev[1]));
         CU(cudaEventElapsedTime(&t1, ctx->ev[1], ctx->ev[2]));
@@ -1215,52 +1278,19 @@ extern "C" int strk_batch_run(strk_ctx *ctx, strk_batch *b, int max_iters, int l
         if (trace)
             fprintf(stderr, "[strk_batch_run %p] pass %d: wd %d (wide_short %d, %d sizes), %lld reads of %lld loci, %s kernel, "
                     "dp %.3f ms, replay %.3f ms, %u loci left the window, %u used the margin, %u fallbacks\n", (void *)ctx, pass, wd, ws, W,
-                    n_slots, n_list, use_packed ? "packed" : "general", t0, t1, miss, miss_fb[2], miss_fb[1]);
+                    n_slots, n_list, use_packed ? "packed" : "general", t0, t1, miss, miss_fb[2], fallbacks);
         if (pass == 0 && b->n_loci >= 256) {  // policy for the next block filled into this batch object
             if (!ws && (long long)miss * 40 > b->n_loci) b->wide_short = 1;
             if (ws && (long long)(miss + miss_fb[2]) * 100 < b->n_loci) b->wide_short = 0;
         }
         if (miss == 0) break;
 
-        // widening pass: redo the loci whose search left the window (status 1); status 2 is an error
+        // widening pass: redo the loci whose search left the window
         ctx->stats[5] += 1;
         if (wd >= wd_cap)
             return set_err(STRK_ERR_SEARCH, "search left the widest supported window (%d sizes)", STRK_MAX_WINDOW);
-        h_status.resize((size_t)b->n_loci);
-        CU(cudaMemcpy(h_status.data(), b->d_status, (size_t)b->n_loci, cudaMemcpyDeviceToHost));
-        std::vector<int> loci;
-        if (pass == 0) {
-            for (long long l = 0; l < b->n_loci; ++l)
-                if (h_status[(size_t)l]) loci.push_back((int)l);
-        } else {
-            for (int l : h_locus_ids)
-                if (h_status[(size_t)l]) loci.push_back(l);
-        }
-        h_locus_ids.swap(loci);
-        h_read_ids.clear();
-        h_slot_begin.clear();
-        for (int l : h_locus_ids) {
-            if (h_status[(size_t)l] == 2)
-                return set_err(STRK_ERR_SEARCH, "locus %d: the search scored no size (max_iters = %d)", l, max_iters);
-            h_slot_begin.push_back((long long)h_read_ids.size());
-            for (long long r = b->h_read_begin[(size_t)l]; r < b->h_read_begin[(size_t)l + 1]; ++r)
-                h_read_ids.push_back((int)r);
-        }
-        n_slots = (long long)h_read_ids.size();
-        n_list = (long long)h_locus_ids.size();
-        if (ctx->list_a.reserve(h_read_ids.size()) != cudaSuccess || ctx->list_b.reserve(h_locus_ids.size()) != cudaSuccess ||
-            ctx->list_c.reserve(h_slot_begin.size()) != cudaSuccess) {
-            cudaGetLastError();
-            return set_err(STRK_ERR_NOMEM, "cannot allocate widening lists");
-        }
-        CU(cudaMemcpyAsync(ctx->list_a.p, h_read_ids.data(), h_read_ids.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(ctx->list_b.p, h_locus_ids.data(), h_locus_ids.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(ctx->list_c.p, h_slot_begin.data(), h_slot_begin.size() * sizeof(long long),
-                           cudaMemcpyHostToDevice, st));
-        CU(cudaStreamSynchronize(st));
-        d_read_ids = ctx->list_a.p;
-        d_locus_ids = ctx->list_b.p;
-        d_slot_begin = ctx->list_c.p;
+        rc = next_loci(ctx, b, pass == 0, max_iters, h_locus_ids, h_read_ids, h_slot_begin, st);
+        if (rc) return rc;
         // The next pass looks where the misses happened (hints) with twice the margin; once that has not been enough twice
         // it widens 8x per pass like the blind scheme did (a search that goes nowhere near its start or its estimate).
         int widen = pass < 2 ? 2 : 8;
@@ -1337,17 +1367,26 @@ extern "C" int strk_get_repeat_count(strk_ctx *ctx, int start_count, const char 
 // ------------------------------------------------------------------------------------------------
 // raw tables (parity checks of the DP itself) and the reference-boundary path
 // ------------------------------------------------------------------------------------------------
+// Device buffers of one call (the entry points below and alleles_api.cuh / realign_api.cuh).  Uploads are queued on
+// `st`, the stream the call's kernels run on; on every way out, the destructor waits for `st` before it frees the
+// buffers, so neither they nor the caller's host arrays are released under a queued copy or kernel.
 struct TmpDev {
+    cudaStream_t st;
     std::vector<void *> ptrs;
     ~TmpDev() {
+        if (!ptrs.empty()) cudaStreamSynchronize(st);
         for (void *p : ptrs) cudaFree(p);
     }
     template <typename T>
-    cudaError_t up(T **dst, const T *src, size_t n) {
+    cudaError_t get(T **dst, size_t n) {
         cudaError_t e = cudaMalloc((void **)dst, (n ? n : 1) * sizeof(T));
-        if (e != cudaSuccess) return e;
-        ptrs.push_back(*dst);
-        if (n && src) e = cudaMemcpy(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) ptrs.push_back(*dst);
+        return e;
+    }
+    template <typename T>
+    cudaError_t up(T **dst, const T *src, size_t n) {
+        cudaError_t e = get(dst, n);
+        if (e == cudaSuccess && n) e = cudaMemcpyAsync(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice, st);
         return e;
     }
 };
@@ -1396,58 +1435,39 @@ static int tables_common(strk_ctx *ctx, bool ref, const uint8_t *arena, uint64_t
         total = std::max<uint64_t>(total, out_off[r] + (uint64_t)(f.n_hi - f.n_lo + 1));
     }
     const int b_len = ext.b_len(), rowlen = ext.rowlen(0);
-    TmpDev tmp;
-    unsigned char *d_arena = nullptr;
+    // same routing as the batch paths: packed kernel per class, the rest (and its fallbacks) to the general kernel
+    ClassLists lists;
+    for (int64_t r = 0; r < n_reads; ++r) {
+        const FamDesc &f = fams[(size_t)r];
+        const int w = f.n_hi - f.n_lo + 1;
+        lists.add(pk_class(ctx, kernel, ref, w, f.n_fl, f.n_tr, f.n_fr, f.m), (int)r, f.m, f.n_fl, f.n_fr, w);
+    }
+    TmpDev tmp{ctx->stream};
+    unsigned char *d_arena = nullptr, *d_table = nullptr;
     FamDesc *d_fams = nullptr;
     cudaError_t e = tmp.up(&d_arena, arena, (size_t)arena_bytes);
     if (e == cudaSuccess) e = tmp.up(&d_fams, fams.data(), fams.size());
-    void *d_table = nullptr;
-    const size_t elem = ref ? 2 * sizeof(long long) : sizeof(int);
-    if (e == cudaSuccess) {
-        e = cudaMalloc(&d_table, (size_t)total * elem);
-        if (e == cudaSuccess) tmp.ptrs.push_back(d_table);
-    }
+    if (e == cudaSuccess) e = tmp.get(&d_table, (size_t)total * (ref ? 2 * sizeof(long long) : sizeof(int)));
     if (e != cudaSuccess) {
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "%s: %s", who, cudaGetErrorString(e));
     }
     for (int k = 0; k < 8; ++k) ctx->stats[k] = 0;
-    if (kernel == STRK_KERNEL_GENERAL || !ctx->h_consts.packed_ok) {
-        rc = launch_general(ctx, ref, d_fams, nullptr, n_reads, d_arena, d_table, b_len, rowlen, ctx->stream);
-        if (rc) return rc;
+    DpPass p{d_fams, d_arena, d_table, ref ? 1 : 0, b_len, rowlen, n_reads};
+    if (lists.items[0].size() == (size_t)n_reads) {
+        p.cnt[0] = n_reads;  // every family on the general kernel, in order
     } else {
-        // same routing as the batch paths (strk_batch_run, the first pass of strk_ref_counts): packed kernel per R,
-        // the rest (and its fallbacks) to the general kernel.  A reference window holds a forward and a reverse
-        // column per size, so it counts twice against PK_WINDOW_MAX.
-        ClassLists lists;
-        for (int64_t r = 0; r < n_reads; ++r) {
-            const FamDesc &f = fams[(size_t)r];
-            const int w = f.n_hi - f.n_lo + 1;
-            const int cls = (ref ? 2 * w : w) > PK_WINDOW_MAX ? 0 : strk_pk_class(f.n_fl, f.n_tr, f.n_fr, f.m);
-            lists.add(cls, (int)r, f.m, f.n_fl, f.n_fr, w);
-        }
-        if (ctx->fallback.reserve((size_t)n_reads) != cudaSuccess) {
-            cudaGetLastError();
-            return set_err(STRK_ERR_NOMEM, "%s: cannot allocate the fallback list", who);
-        }
-        const int *seg_list[STRK_PK_NBIN];
-        long long seg_cnt[STRK_PK_NBIN];
-        int seg_w[STRK_PK_NBIN];
-        for (int k = 0; k < STRK_PK_NBIN; ++k)  // reference mode: forward + reverse columns of every size
-            seg_w[k] = ref ? 2 * lists.w_max[k] - 1 : (lists.w_max[k] + 3) / 4 * 4;
-        rc = lists.upload(ctx->list_d, ctx->stream, seg_list, seg_cnt);
+        rc = lists.upload(ctx->list_d, ctx->stream, p);
         if (rc) return rc;
-        CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), ctx->stream));
-        long long n_packed = 0;
-        rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w, n_reads, d_fams, d_arena, d_table, b_len,
-                         rowlen, ctx->stream, ref ? 1 : 0, &n_packed);
-        if (rc) return rc;
-        if (n_packed) {
-            unsigned int fb = 0;
-            CU(cudaMemcpyAsync(&fb, ctx->d_queue + 2, sizeof(unsigned int), cudaMemcpyDeviceToHost, ctx->stream));
-            CU(cudaStreamSynchronize(ctx->stream));
-            ctx->stats[6] = (double)(n_packed - (long long)fb);
-        }
+    }
+    long long n_packed = 0;
+    rc = launch_pass(ctx, p, ctx->stream, &n_packed);
+    if (rc) return rc;
+    if (n_packed) {
+        unsigned int fb = 0;
+        CU(cudaMemcpyAsync(&fb, ctx->counter(Q_FALLBACK), sizeof(unsigned int), cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        ctx->stats[6] = (double)(n_packed - (long long)fb);
     }
     ctx->stats[7] = (double)n_reads - ctx->stats[6];
     CU(cudaStreamSynchronize(ctx->stream));
@@ -1608,12 +1628,10 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     RefBufs &d = ctx->ref;
     const size_t n = (size_t)n_loci;
     const bool phase1 = !respect_coords;
-    const bool packed_ok = ctx->h_consts.packed_ok;
     const int CAP2 = 4096, WD_MAX = (STRK_MAX_WINDOW - 1) / 2, T = 128;
     // phase 1's table stride: the widest first window; the second look's: 4x that
     const int wd1 = *std::max_element(d.h_wd.begin(), d.h_wd.end()), stride_w = 2 * wd1 + 1;
     const int wd1b = std::min(WD_MAX, 4 * wd1), stride_w2 = 2 * wd1b + 1;
-    const bool packed1 = packed_ok && 2 * stride_w <= PK_WINDOW_MAX;  // a forward and a reverse column per size
 
     // ---- host plan: phase 1's classes, scratch maxima, the tiers in first-appearance order
     GenExtent ext = {};
@@ -1629,7 +1647,7 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
         // (fl + fr) / m + 1 more copies)
         ext.add(fl, fr, n1, m, start_count[l] + (fl + fr) / m + 1);
         if (phase1) {  // executed cells of the first pass: two sweeps of db x (flank + motif * n_hi)
-            lists.add(packed1 ? strk_pk_class(fl, tr, fr, m) : 0, (int)l, m, fl, fr);
+            lists.add(pk_class(ctx, STRK_KERNEL_AUTO, 1, stride_w, fl, tr, fr, m), (int)l, m, fl, fr, stride_w);
             cells1 += (double)n1 * ((double)fl + fr + 2.0 * m * ((double)start_count[l] + d.h_wd[(size_t)l]));
         }
         const int32_t *p = rc_params + 3 * l;
@@ -1650,15 +1668,15 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     d.tiers.resize(n_tiers);  // (the vectors of the tiers kept keep their capacity for the next call)
     // one tier classed like phase 1: phase 2 takes phase 1's lists (moving bases between flank and tract does not change
     // a window's class), slot q = locus q
-    const bool reuse = phase1 && d.tiers.size() == 1 && packed1 == (packed_ok && d.tiers[0].W2 <= PK_WINDOW_MAX);
+    const bool reuse = phase1 && d.tiers.size() == 1 &&
+                       pk_window_ok(ctx, STRK_KERNEL_AUTO, 1, stride_w) == pk_window_ok(ctx, STRK_KERNEL_AUTO, 0, d.tiers[0].W2);
     size_t table2 = 0;
     for (RefTier &t : d.tiers) {
         table2 = std::max(table2, t.ids.size() * (size_t)t.W2);
-        const bool packed2 = packed_ok && t.W2 <= PK_WINDOW_MAX;
         for (size_t q = 0; q < t.ids.size() && !reuse; ++q) {
             const int l = t.ids[q];
             const int fl = lens[3 * l], tr = lens[3 * l + 1], fr = lens[3 * l + 2], m = motif_len[l];
-            t.classes.add(packed2 ? strk_pk_class(fl, tr, fr, m) : 0, (int)q, m, fl, fr);
+            t.classes.add(pk_class(ctx, STRK_KERNEL_AUTO, 0, t.W2, fl, tr, fr, m), (int)q, m, fl, fr, t.W2);
         }
     }
     const int b_len = ext.b_len(), rowlen = ext.rowlen(std::max(std::max(wd1, wd2_max), wd1b));
@@ -1671,21 +1689,19 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     if (e == cudaSuccess) e = ctx->fams.reserve(std::max(n, (size_t)CAP2));
     if (e == cudaSuccess) e = ctx->table64.reserve(std::max(n * (size_t)stride_w * 2, (size_t)CAP2 * (size_t)stride_w2 * 2));
     if (e == cudaSuccess) e = ctx->table.reserve(table2);
-    if (e == cudaSuccess) e = ctx->fallback.reserve(n);
+    if (e == cudaSuccess) e = ctx->fallback.reserve(n);  // (for every pass of the call: see launch_pass)
     if (e != cudaSuccess) {
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "strk_ref_counts: %s", cudaGetErrorString(e));
     }
     b->d_arena = d.arena.p;
-    const int *seg_list[STRK_PK_NBIN];
-    long long seg_cnt[STRK_PK_NBIN];
+    DpPass p1{ctx->fams.p, d.arena.p, ctx->table64.p, 1, b_len, rowlen, n_loci};
     if (phase1) {
-        rc = lists.upload(d.lists, st, seg_list, seg_cnt);
+        rc = lists.upload(d.lists, st, p1);
         if (rc) return rc;
     }
     CU(cudaMemsetAsync(d.cnt.p, 0, 8 * sizeof(unsigned int), st));
     CU(cudaMemsetAsync(ctx->d_acc, 0, 4 * sizeof(double), st));
-    CU(cudaMemsetAsync(ctx->d_queue + 1, 0, 3 * sizeof(unsigned int), st));
 
     // ---- phase 1, then the second look: the loci whose search left the first window (a percent of a block at +-6
     // sizes), listed and counted on the device (ids_a, cnt[0]), up to CAP2 of them 4x wider; the rest keep their flag
@@ -1694,11 +1710,8 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
                                                                    d.motif_off.p, d.motif_len.p, stride_w, ctx->fams.p);
         CU(cudaGetLastError());
         CU(cudaEventRecord(ctx->ev[0], st));
-        int seg_w1[STRK_PK_NBIN];
-        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w1[k] = 2 * stride_w - 1;  // forward + reverse columns of every size
         long long n_packed = 0;
-        rc = launch_pass(ctx, seg_list, seg_cnt, lists.flank, lists.mmax, seg_w1, n_loci, ctx->fams.p, d.arena.p,
-                         ctx->table64.p, b_len, rowlen, st, 1, &n_packed);
+        rc = launch_pass(ctx, p1, st, &n_packed);
         if (rc) return rc;
         CU(cudaEventRecord(ctx->ev[1], st));
         ref_replay1_kernel<<<(unsigned)((n + T - 1) / T), T, 0, st>>>(nullptr, (int)n, ctx->table64.p, ctx->fams.p, d.start.p,
@@ -1716,12 +1729,15 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
     for (size_t t = 0; t < d.tiers.size(); ++t) {
         RefTier &tier = d.tiers[t];
         const int nt = (int)tier.ids.size();
-        const ClassLists &cl = reuse ? lists : tier.classes;
+        DpPass p2{ctx->fams.p, d.arena.p, ctx->table.p, 0, b_len, rowlen, nt};
         int *ids = nullptr;
-        if (!reuse) {
+        if (reuse) {  // phase 1's classes at phase 2's window
+            p2 = p1, p2.table = ctx->table.p, p2.ref_mode = 0;
+            std::fill_n(p2.w, STRK_PK_NBIN, tier.W2);
+        } else {
             ids = d.tier_ids.p + at;
             CU(cudaMemcpyAsync(ids, tier.ids.data(), nt * sizeof(int), cudaMemcpyHostToDevice, st));
-            rc = tier.classes.upload(d.lists, st, seg_list, seg_cnt);
+            rc = tier.classes.upload(d.lists, st, p2);
             if (rc) return rc;
         }
         at += (size_t)nt;
@@ -1736,12 +1752,8 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
                                                                        ctx->d_acc + 1, nullptr);
         CU(cudaGetLastError());
         if (t == 0) CU(cudaEventRecord(ctx->ev[2], st));
-        CU(cudaMemsetAsync(ctx->d_queue + 2, 0, sizeof(unsigned int), st));
-        int seg_w2[STRK_PK_NBIN];
-        for (int k = 0; k < STRK_PK_NBIN; ++k) seg_w2[k] = (tier.W2 + 3) / 4 * 4;
         long long n_packed = 0;
-        rc = launch_pass(ctx, seg_list, seg_cnt, cl.flank, cl.mmax, seg_w2, nt, ctx->fams.p, d.arena.p, ctx->table.p, b_len,
-                         rowlen, st, 0, &n_packed);
+        rc = launch_pass(ctx, p2, st, &n_packed);
         if (rc) return rc;
         if (t + 1 == d.tiers.size()) CU(cudaEventRecord(ctx->ev[3], st));
         rc = launch_replay(ctx, b, tier.W2, tier.wd2, 0, nullptr, nullptr, nt, tier.rc[0], tier.rc[1], tier.rc[2], nullptr,
@@ -1863,7 +1875,7 @@ extern "C" int strk_ref_counts(strk_ctx *ctx, const uint8_t *arena, uint64_t are
 extern "C" int strk_measure_int_peak(strk_ctx *ctx, double out_tiops[3]) {
     if (!ctx || !out_tiops) return set_err(STRK_ERR_ARG, "strk_measure_int_peak: null argument");
     CU(cudaSetDevice(ctx->device));
-    int *d_out = (int *)(ctx->d_queue + 7);  // context-owned scratch word and events: nothing to release on an error path
+    int *d_out = (int *)ctx->counter(Q_INT_PEAK);  // context-owned scratch word and events: nothing to release on an error path
     const int grid = ctx->n_sm * 8, threads = 256, iters = 4096;
     const double instr = (double)grid * threads * (double)iters * 64.0;  // lane-level integer instructions
     cudaEvent_t e0 = ctx->ev[0], e1 = ctx->ev[1];

@@ -36,7 +36,7 @@ extern "C" int strk_realign(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_
     // groups of alignments whose traces fit the budget (1 byte per cell; STRK_REALIGN_TRACE_MB, default 2048)
     size_t budget = 2048ull << 20;
     if (const char *e = getenv("STRK_REALIGN_TRACE_MB")) budget = (size_t)std::max(1, atoi(e)) << 20;
-    TmpDev tmp;
+    TmpDev tmp{st};
     unsigned char *d_arena = nullptr;
     cudaError_t e = tmp.up(&d_arena, arena, (size_t)arena_bytes);
     const uint64_t cigar_total = cigar_off[n];
@@ -44,16 +44,16 @@ extern "C" int strk_realign(strk_ctx *ctx, const uint8_t *arena, uint64_t arena_
     int *d_score = nullptr, *d_end = nullptr, *d_len = nullptr;
     RealignDesc *d_descs = nullptr;
     unsigned int *d_q = nullptr;
-    if (e == cudaSuccess) e = tmp.up(&d_cigar, (const unsigned int *)nullptr, (size_t)cigar_total);
-    if (e == cudaSuccess) e = tmp.up(&d_score, (const int *)nullptr, (size_t)n);
-    if (e == cudaSuccess) e = tmp.up(&d_end, (const int *)nullptr, (size_t)n);
-    if (e == cudaSuccess) e = tmp.up(&d_len, (const int *)nullptr, (size_t)n);
-    if (e == cudaSuccess) e = tmp.up(&d_descs, (const RealignDesc *)nullptr, (size_t)n);
-    if (e == cudaSuccess) e = tmp.up(&d_q, (const unsigned int *)nullptr, 1);
+    if (e == cudaSuccess) e = tmp.get(&d_cigar, (size_t)cigar_total);
+    if (e == cudaSuccess) e = tmp.get(&d_score, (size_t)n);
+    if (e == cudaSuccess) e = tmp.get(&d_end, (size_t)n);
+    if (e == cudaSuccess) e = tmp.get(&d_len, (size_t)n);
+    if (e == cudaSuccess) e = tmp.get(&d_descs, (size_t)n);
+    if (e == cudaSuccess) e = tmp.get(&d_q, 1);
     const int grid_max = ctx->n_sm * 4;
     const int bound_stride = 4 * (max_n2 + 1);
     int *d_bound = nullptr;
-    if (e == cudaSuccess) e = tmp.up(&d_bound, (const int *)nullptr, (size_t)grid_max * RA_WARPS * (size_t)bound_stride);
+    if (e == cudaSuccess) e = tmp.get(&d_bound, (size_t)grid_max * RA_WARPS * (size_t)bound_stride);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "strk_realign: %s", cudaGetErrorString(e));
