@@ -1070,16 +1070,11 @@ extern "C" int strk_batch_upload(strk_ctx *ctx, const uint8_t *arena, uint64_t a
 static int launch_replay(strk_ctx *ctx, const strk_batch *b, int W, int wd, int ws, const int *d_locus_ids,
                          const long long *d_slot_begin, long long n_list, int max_iters, int range, int step,
                          const int *d_rep, double *d_hint, cudaStream_t st) {
-    if (W <= REPLAY_WMAX)
-        replay_reads_small_kernel<<<(unsigned)((n_list + REPLAY_THREADS - 1) / REPLAY_THREADS), REPLAY_THREADS, 0, st>>>(
-            ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
-            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->counter(Q_MISS), ctx->d_acc,
-            d_rep, d_hint);
-    else
-        replay_reads_kernel<<<(unsigned)((n_list + 127) / 128), 128, 0, st>>>(
-            ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
-            b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->counter(Q_MISS), ctx->d_acc,
-            d_rep, d_hint);
+    const auto kernel = W <= REPLAY_WMAX ? replay_reads_small_kernel : replay_reads_kernel;
+    kernel<<<(unsigned)((n_list + REPLAY_THREADS - 1) / REPLAY_THREADS), REPLAY_THREADS, 0, st>>>(
+        ctx->table.p, W, wd, ws, d_locus_ids, d_slot_begin, (int)n_list, b->d_read_begin, b->d_est, b->d_lens,
+        b->d_motif_len, max_iters, range, step, ctx->tie_flags, b->d_out, b->d_status, ctx->counter(Q_MISS), ctx->d_acc,
+        d_rep, d_hint);
     CU(cudaGetLastError());
     return STRK_OK;
 }

@@ -3,13 +3,16 @@
 // The DP kernels score a whole window of candidate sizes in parallel; the reference instead walks
 // sizes serially (strkit_rust_ext.get_repeat_count, called at repeats.py:58-68; the in-tree
 // statement of the same search is repeats.py:100-156) and its answer depends on the start size,
-// the visitation order, the iteration budget and the tie-breaks -- it is NOT an arg-max.  These
-// routines run that search verbatim with every "score this size" replaced by a table look-up, so
-// the parallel sweep returns bit-identical (n, score, n_explored).  A look-up outside the table
-// window is reported as a miss; the host widens the window and runs the locus again.
+// the visitation order, the iteration budget and the tie-breaks -- it is NOT an arg-max.  climb()
+// runs that search verbatim with every "score this size" replaced by a table look-up, so the parallel
+// sweep returns bit-identical (n, score, n_explored).  A look-up outside the table window is reported
+// as a miss; the host widens the window and runs the locus again.  What a window of the search scores
+// is a visitor: climb_single (read path, one score per size) and climb_ref (the boundary search of
+// get_ref_repeat_count, a forward and a reverse score per size).
 //
-// Also replayed here: the per-locus read loop of call_locus.py:1079,1129-1161 (start guess with the
-// carried offset fraction; float64, round-half-even like CPython's round()).
+// Also replayed here, once for both replay kernels: the per-locus read loop of call_locus.py:1079,1129-1161
+// (start guess with the carried offset fraction; float64, round-half-even like CPython's round()).  The
+// kernels differ only in where a read's table row comes from.
 #pragma once
 #include "strk_common.cuh"
 
@@ -55,67 +58,35 @@ struct SeenSmall {
     __host__ __device__ void add(int n) { w |= 1u << (n - lo); }
 };
 
-// Single-score search (read path).  table[n - n_lo] for n in [n_lo, n_hi].
-template <typename Seen>
-__host__ __device__ inline ClimbResult climb_single(const int *table, int n_lo, int n_hi, int start_count,
-                                                    int max_iters, int range, int step, int tie_flags,
-                                                    Seen &seen) {
-    ClimbResult res;
-    res.best_n = 0;
-    res.best_score = 0;
-    res.n_explored = 0;
-    res.status = 0;
-    res.sum_n = 0.0;
-    res.lo_touched = 0x7fffffff;
-    res.hi_touched = -1;
+// The stack walk of the search (repeats.py:100-151) over a table of the sizes [n_lo, n_hi].  window(lo, hi) scores the
+// sizes lo..hi in order: it adds those not yet in `seen` to it, counts them in n_scored (the count max_iters limits)
+// and returns the size the climb moves to.  Returns the status: 0 ok, 1 a window left the table, 2 nothing scored.
+// narrow = the search-policy switches (tie_flags bits 2-3, STRK_SEARCH_* in the header): the Rust body of this search
+// is not in the reference tree and repeat_count_params.py:13 says the range "can be narrowed within the
+// get_repeat_count fn".  0 = the in-tree statement (range fixed); the two narrowing hypotheses only ever shrink the
+// windows, so the score table of a pass always covers them.
+template <typename Seen, typename Window>
+__host__ __device__ __forceinline__ int climb(int n_lo, int n_hi, int start_count, int max_iters, int range, int step,
+                                              int narrow, Seen &seen, const int &n_scored, Window window) {
     seen.reset(n_lo, n_hi);
     int st_size[4], st_dir[4];
     int top = 0;
     st_size[top] = start_count - step, st_dir[top++] = -1;
     st_size[top] = start_count + step, st_dir[top++] = 1;
     st_size[top] = start_count, st_dir[top++] = 0;
-    bool have_best = false;
-    // Search-policy switches (tie_flags bits 2-3, STRK_SEARCH_* in the header): the Rust body of this search is not in
-    // the reference tree and repeat_count_params.py:13 says the range "can be narrowed within the get_repeat_count
-    // fn".  0 = the in-tree statement (range fixed, repeats.py:100-151); the two narrowing hypotheses only ever shrink
-    // the windows, so the score table of a pass always covers them.
-    while (top > 0 && res.n_explored < max_iters) {
+    while (top > 0 && n_scored < max_iters) {
         --top;
         const int size = st_size[top], dir = st_dir[top];
         if (size < 0) continue;
         const bool wide = step > range;
-        int start_size = size - ((dir < 1 || wide) ? range : 0);
-        if (start_size < 0) start_size = 0;
-        const int end_size = size + ((dir > -1 || wide) ? range : 0);
-        if ((tie_flags & 4) && range > 1) range = 1;              // STRK_SEARCH_NARROW_FIRST: after the first window
-        if ((tie_flags & 8) && range > 1) range = range / 2;      // STRK_SEARCH_NARROW_HALVE: after every window
-        res.lo_touched = start_size < res.lo_touched ? start_size : res.lo_touched;
-        res.hi_touched = end_size > res.hi_touched ? end_size : res.hi_touched;
-        bool have = false;
-        int mv_size = 0, mv_score = 0;
-        for (int i = start_size; i <= end_size; ++i) {
-            if (!seen.inside(i)) {
-                res.status = 1;
-                return res;
-            }
-            const int sc = table[i - n_lo];
-            if (!seen.has(i)) {
-                seen.add(i);
-                ++res.n_explored;
-                res.sum_n += (double)i;
-                // final pick = first-inserted maximum (repeats.py:154) unless STRK_TIE_FINAL_LAST
-                if (!have_best || sc > res.best_score || ((tie_flags & 2) && sc == res.best_score)) {
-                    have_best = true;
-                    res.best_n = i;
-                    res.best_score = sc;
-                }
-            }
-            if (!have || sc > mv_score || ((tie_flags & 1) && sc == mv_score)) {
-                have = true;
-                mv_size = i;
-                mv_score = sc;
-            }
-        }
+        int lo = size - ((dir < 1 || wide) ? range : 0);
+        if (lo < 0) lo = 0;
+        const int hi = size + ((dir > -1 || wide) ? range : 0);
+        // the window and the table are both contiguous: a window with a size outside the table has an end outside it
+        if (!seen.inside(lo) || !seen.inside(hi)) return 1;
+        if ((narrow & 4) && range > 1) range = 1;          // STRK_SEARCH_NARROW_FIRST: after the first window
+        if ((narrow & 8) && range > 1) range = range / 2;  // STRK_SEARCH_NARROW_HALVE: after every window
+        const int mv_size = window(lo, hi);
         // at most one of the two pushes can fire, so the stack never exceeds 3 entries
         if (mv_size > size) {
             const int new_rc = mv_size + step;
@@ -126,7 +97,42 @@ __host__ __device__ inline ClimbResult climb_single(const int *table, int n_lo, 
             if (!seen.has(new_rc) && new_rc >= 0) st_size[top] = new_rc, st_dir[top++] = -1;
         }
     }
-    if (!have_best) res.status = 2;
+    return n_scored ? 0 : 2;
+}
+
+// Single-score search (read path).  table[n - n_lo] for n in [n_lo, n_hi].
+template <typename Seen>
+__host__ __device__ inline ClimbResult climb_single(const int *table, int n_lo, int n_hi, int start_count,
+                                                    int max_iters, int range, int step, int tie_flags,
+                                                    Seen &seen) {
+    ClimbResult res = {0, 0, 0, 0, 0.0, 0x7fffffff, -1};
+    res.status = climb(n_lo, n_hi, start_count, max_iters, range, step, tie_flags & 12, seen, res.n_explored,
+                       [&](int lo, int hi) {
+        res.lo_touched = lo < res.lo_touched ? lo : res.lo_touched;
+        res.hi_touched = hi > res.hi_touched ? hi : res.hi_touched;
+        bool have = false;
+        int mv_size = 0, mv_score = 0;
+        for (int i = lo; i <= hi; ++i) {
+            const int sc = table[i - n_lo];
+            if (!seen.has(i)) {
+                seen.add(i);
+                // final pick = first-inserted maximum (repeats.py:154) unless STRK_TIE_FINAL_LAST
+                if (!res.n_explored || sc > res.best_score || ((tie_flags & 2) && sc == res.best_score)) {
+                    res.best_n = i;
+                    res.best_score = sc;
+                }
+                ++res.n_explored;
+                res.sum_n += (double)i;
+            }
+            // the move = first maximum of the window unless STRK_TIE_WINDOW_LAST
+            if (!have || sc > mv_score || ((tie_flags & 1) && sc == mv_score)) {
+                have = true;
+                mv_size = i;
+                mv_score = sc;
+            }
+        }
+        return mv_size;
+    });
     return res;
 }
 
@@ -146,35 +152,16 @@ __host__ __device__ inline void ref_unpack(long long key, int &score, int &end_q
 __host__ __device__ inline RefClimbResult climb_ref(const long long *tab, int n_lo, int n_hi, int start_count,
                                                    int max_iters, int range, int step, int n_fl, int n_fr,
                                                    int ref_size, int vcf_anchor_size, SeenSet &seen) {
-    RefClimbResult res;
-    res.l_offset = res.r_offset = res.n_offset_scores = 0;
-    res.status = 0;
+    RefClimbResult res = {0, 0, 0, 0};
     const int W = n_hi - n_lo + 1;
-    seen.reset(n_lo, n_hi);
-    int st_size[4], st_dir[4];
-    int top = 0;
-    st_size[top] = start_count - step, st_dir[top++] = -1;
-    st_size[top] = start_count + step, st_dir[top++] = 1;
-    st_size[top] = start_count, st_dir[top++] = 0;
-    bool have_best = false;
     int bf_score = 0, bf_adj = 0, br_score = 0, br_adj = 0;
-    const bool wide = step > range;
-    while (top > 0 && res.n_offset_scores < max_iters) {
-        --top;
-        const int size = st_size[top], dir = st_dir[top];
-        if (size < 0) continue;
-        int start_size = size - ((dir < 1 || wide) ? range : 0);
-        if (start_size < 0) start_size = 0;
-        const int end_size = size + ((dir > -1 || wide) ? range : 0);
+    res.status = climb(n_lo, n_hi, start_count, max_iters, range, step, 0, seen, res.n_offset_scores,
+                       [&](int lo, int hi) {
         bool have = false;
         int mv_size = 0, mv_s = 0, mv_a = 0;
         // max((*fwd_scores, *rev_scores), key=(score, adj)): first maximal, fwd entries first (:135)
         for (int pass = 0; pass < 2; ++pass) {
-            for (int i = start_size; i <= end_size; ++i) {
-                if (!seen.inside(i)) {
-                    res.status = 1;
-                    return res;
-                }
+            for (int i = lo; i <= hi; ++i) {
                 int fs, fe, rs, re;
                 ref_unpack(tab[i - n_lo], fs, fe);
                 ref_unpack(tab[W + i - n_lo], rs, re);
@@ -182,10 +169,9 @@ __host__ __device__ inline RefClimbResult climb_ref(const long long *tab, int n_
                 const int l_adj = re + 1 - n_fr - ref_size;  // :41
                 if (!seen.has(i)) {
                     seen.add(i);
-                    ++res.n_offset_scores;
-                    if (!have_best || fs > bf_score) bf_score = fs, bf_adj = r_adj;  // :154
-                    if (!have_best || rs > br_score) br_score = rs, br_adj = l_adj;  // :156
-                    have_best = true;
+                    const bool first = res.n_offset_scores++ == 0;
+                    if (first || fs > bf_score) bf_score = fs, bf_adj = r_adj;  // :154
+                    if (first || rs > br_score) br_score = rs, br_adj = l_adj;  // :156
                 }
                 const int s = pass == 0 ? fs : rs, a = pass == 0 ? r_adj : l_adj;
                 if (!have || s > mv_s || (s == mv_s && a > mv_a)) {
@@ -196,19 +182,9 @@ __host__ __device__ inline RefClimbResult climb_ref(const long long *tab, int n_
                 }
             }
         }
-        if (mv_size > size) {
-            const int new_rc = mv_size + step;
-            if (!seen.has(new_rc) && new_rc >= 0) st_size[top] = new_rc, st_dir[top++] = 1;
-        }
-        if (mv_size < size) {
-            const int new_rc = mv_size - step;
-            if (!seen.has(new_rc) && new_rc >= 0) st_size[top] = new_rc, st_dir[top++] = -1;
-        }
-    }
-    if (!have_best) {
-        res.status = 2;
-        return res;
-    }
+        return mv_size;
+    });
+    if (res.status) return res;
     res.l_offset = br_adj;  // :161
     res.r_offset = bf_adj;  // :162
     if (res.l_offset >= n_fl - vcf_anchor_size) res.l_offset = 0;  // :164-167
@@ -216,12 +192,118 @@ __host__ __device__ inline RefClimbResult climb_ref(const long long *tab, int n_
     return res;
 }
 
-// One thread per locus: the read loop of call_locus.py:1129-1161 over the score tables.
-//   table row of slot s = table + s * W ; window of the slot = [max(0, est - wdr), est + wdr], wdr = strk_read_wd()
+// What the read loop needs of read r: its table row, estimate and lengths.
+struct ReadRow {
+    const int *row;
+    int est, n_fl, n_tr, n_fr;
+};
+
+// Row source of replay_reads_kernel: the row of the read's slot (table + slot * W), or, when rep != nullptr (first
+// pass only, slot == read), the row of read rep[r], whose table identical reads share.
+struct GlobalRows {
+    const int *table;
+    int W;
+    const int *rep, *est_cn, *lens;
+    __device__ __forceinline__ ReadRow load(long long r, long long slot) const {
+        return {table + (size_t)(rep ? (long long)rep[r] : slot) * (size_t)W, est_cn[r], lens[3 * r], lens[3 * r + 1],
+                lens[3 * r + 2]};
+    }
+    __device__ __forceinline__ void begin(long long, long long, long long) {}
+    __device__ __forceinline__ ReadRow next(long long r, long long, long long slot) { return load(r, slot); }
+};
+
+// Row source of replay_reads_small_kernel (W <= REPLAY_WMAX: every first pass).  The search reads a dozen table entries
+// per read one after the other, each a trip to L2 (~4 us per read, 0.11 ms for a 30-read locus whatever the batch
+// size): here read r is searched on a copy of its row in the thread's stripe of shared memory (stride REPLAY_WMAX + 1
+// words: conflict-free) while the row, estimate and lengths of read r + 1 are fetched as independent loads.
+#define REPLAY_WMAX 20
+#define REPLAY_THREADS 128
+struct StagedRows {
+    GlobalRows src;
+    int *stripe;
+    int nrow[REPLAY_WMAX];
+    ReadRow nxt;
+    __device__ __forceinline__ void fetch(long long r, long long slot) {
+        nxt = src.load(r, slot);
+#pragma unroll
+        for (int k = 0; k < REPLAY_WMAX; ++k) nrow[k] = k < src.W ? nxt.row[k] : 0;
+    }
+    __device__ __forceinline__ void begin(long long r0, long long r1, long long slot) {
+        if (r0 < r1) fetch(r0, slot);
+    }
+    __device__ __forceinline__ ReadRow next(long long r, long long r1, long long slot) {
+#pragma unroll
+        for (int k = 0; k < REPLAY_WMAX; ++k) stripe[k] = nrow[k];
+        ReadRow cur = nxt;
+        cur.row = stripe;
+        if (r + 1 < r1) fetch(r + 1, slot + 1);  // before the search of read r, which it overlaps
+        return cur;
+    }
+};
+
+// Locus q of a replay pass, one thread per locus: the read loop of call_locus.py:1129-1161 over the score tables.
+//   window of a read = strk_slot_window, the table planner's; hint != nullptr: per locus {smallest, largest} offset
+//   fraction seen at a miss, and a locus that misses adds the fraction it missed at
 //   miss_count[0] += loci whose search left the window; miss_count[2] += loci that stayed inside it but went
 //   beyond est +- wd, i.e. that only the wide_short margin saved from a second pass
 //   locus_ids == nullptr: locus q is q and its slots are read_begin[q]..; otherwise the widening
 //   pass lists the loci to redo and slot_begin[q] is the first slot of locus_ids[q].
+template <typename Seen, typename Rows>
+__device__ __forceinline__ void replay_locus(int q, Rows &rows, int wd, int wide_short, const int *locus_ids,
+                                             const long long *slot_begin, const long long *read_begin,
+                                             const int *motif_len, int max_iters, int range, int step, int tie_flags,
+                                             int *out, unsigned char *locus_status, unsigned int *miss_count,
+                                             double *ref_cells, double *hint) {
+    const int locus = locus_ids ? locus_ids[q] : q;
+    const long long r0 = read_begin[locus], r1 = read_begin[locus + 1];
+    long long slot = locus_ids ? slot_begin[q] : r0;
+    // a locus' hint changes only at its miss, which ends its loop
+    double *h = hint ? hint + 2 * (size_t)locus : nullptr;
+    double hl[2] = {0.0, 0.0};
+    if (h) hl[0] = h[0], hl[1] = h[1];
+    Seen seen;
+    double frac = 0.0;  // read_offset_frac_from_starting_guess (:1079)
+    double cells = 0.0;
+    const int m = motif_len[locus];
+    int status = 0;
+    bool margin_used = false;
+    rows.begin(r0, r1, slot);
+    for (long long r = r0; r < r1; ++r, ++slot) {
+        const ReadRow rd = rows.next(r, r1, slot);
+        const int est = rd.est;
+        int read_sc = est;
+        const int off = (int)rint(frac * (double)read_sc);  // round(), :1130
+        if (off < -read_sc)
+            frac = 0.0;  // :1133
+        else
+            read_sc += off;  // :1136
+        int n_lo, n_hi;
+        strk_slot_window(est, m, wd, wide_short, h ? hl : nullptr, n_lo, n_hi);
+        const ClimbResult cr = climb_single(rd.row, n_lo, n_hi, read_sc, max_iters, range, step, tie_flags, seen);
+        if (cr.status) {
+            status = cr.status;
+            if (h && cr.status == 1) {  // where the next pass has to look: the fraction this read started from
+                const double fr_used = read_sc == est ? 0.0 : frac;
+                h[0] = fr_used < hl[0] ? fr_used : hl[0];
+                h[1] = fr_used > hl[1] ? fr_used : hl[1];
+            }
+            break;
+        }
+        margin_used |= cr.lo_touched < est - wd || cr.hi_touched > est + wd;
+        *(int4 *)(out + 4 * r) = make_int4(cr.best_n, cr.best_score, cr.n_explored, read_sc);
+        frac += (double)(cr.best_n - read_sc) / (double)(cr.best_n > 1 ? cr.best_n : 1);  // :1161
+        const double n1 = (double)(rd.n_fl + rd.n_tr + rd.n_fr);
+        cells += n1 * ((double)cr.n_explored * (double)(rd.n_fl + rd.n_fr) + (double)m * cr.sum_n);
+    }
+    locus_status[locus] = (unsigned char)status;
+    if (status) {
+        atomicAdd(miss_count, 1u);
+    } else {
+        atomicAdd(ref_cells, cells);
+        if (margin_used) atomicAdd(miss_count + 2, 1u);
+    }
+}
+
 __global__ void replay_reads_kernel(const int *__restrict__ table, int W, int wd, int wide_short,
                                     const int *__restrict__ locus_ids,
                                     const long long *__restrict__ slot_begin, int n_list,
@@ -230,67 +312,13 @@ __global__ void replay_reads_kernel(const int *__restrict__ table, int W, int wd
                                     int range, int step, int tie_flags, int *__restrict__ out,
                                     unsigned char *__restrict__ locus_status, unsigned int *miss_count,
                                     double *ref_cells, const int *__restrict__ rep, double *__restrict__ hint = nullptr) {
-    // rep != nullptr (first pass only, slot == read): read r looks its scores up in the row of read rep[r]
-    // hint != nullptr (widening passes): per locus {smallest, largest} offset fraction seen at a miss (strk_slot_window);
-    // a locus that misses again adds the fraction it missed at
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n_list) return;
-    const int locus = locus_ids ? locus_ids[q] : q;
-    const long long r0 = read_begin[locus], r1 = read_begin[locus + 1];
-    long long slot = locus_ids ? slot_begin[q] : r0;
-    SeenSet seen;
-    double frac = 0.0;  // read_offset_frac_from_starting_guess (:1079)
-    double cells = 0.0;
-    const int m = motif_len[locus];
-    const int wdr = strk_read_wd(wd, m, wide_short);
-    int status = 0;
-    bool margin_used = false;
-    for (long long r = r0; r < r1; ++r, ++slot) {
-        const int est = est_cn[r];
-        int read_sc = est;
-        const int off = (int)rint(frac * (double)read_sc);  // round(), :1130
-        if (off < -read_sc)
-            frac = 0.0;  // :1133
-        else
-            read_sc += off;  // :1136
-        int n_lo, n_hi;
-        strk_slot_window(est, m, wd, wide_short, hint ? hint + 2 * (size_t)locus : nullptr, n_lo, n_hi);
-        ClimbResult cr = climb_single(table + (size_t)(rep ? (long long)rep[r] : slot) * (size_t)W, n_lo, n_hi, read_sc,
-                                      max_iters, range, step, tie_flags, seen);
-        if (cr.status) {
-            status = cr.status;
-            if (hint && cr.status == 1) {  // where the next pass has to look: the fraction this read started from
-                double *h = hint + 2 * (size_t)locus;
-                const double fr_used = read_sc == est ? 0.0 : frac;
-                h[0] = fr_used < h[0] ? fr_used : h[0];
-                h[1] = fr_used > h[1] ? fr_used : h[1];
-            }
-            break;
-        }
-        margin_used |= cr.lo_touched < est - wd || cr.hi_touched > est + wd;
-        out[4 * r + 0] = cr.best_n;
-        out[4 * r + 1] = cr.best_score;
-        out[4 * r + 2] = cr.n_explored;
-        out[4 * r + 3] = read_sc;
-        frac += (double)(cr.best_n - read_sc) / (double)(cr.best_n > 1 ? cr.best_n : 1);  // :1161
-        const double n1 = (double)(lens[3 * r] + lens[3 * r + 1] + lens[3 * r + 2]);
-        cells += n1 * ((double)cr.n_explored * (double)(lens[3 * r] + lens[3 * r + 2]) + (double)m * cr.sum_n);
-    }
-    locus_status[locus] = (unsigned char)status;
-    if (status) {
-        atomicAdd(miss_count, 1u);
-    } else {
-        atomicAdd(ref_cells, cells);
-        if (margin_used) atomicAdd(miss_count + 2, 1u);
-    }
+    GlobalRows rows = {table, W, rep, est_cn, lens};
+    replay_locus<SeenSet>(q, rows, wd, wide_short, locus_ids, slot_begin, read_begin, motif_len, max_iters, range, step,
+                          tie_flags, out, locus_status, miss_count, ref_cells, hint);
 }
 
-// The same loop for narrow windows (W <= REPLAY_WMAX: every first pass).  The search reads a dozen table entries per
-// read one after the other, each a trip to L2 (~4 us per read, 0.11 ms for a 30-read locus whatever the batch size):
-// here the row, estimate and lengths of read r + 1 are fetched as independent loads while read r is searched on a
-// copy of its row in shared memory (stride REPLAY_WMAX + 1 words per thread: conflict-free).
-#define REPLAY_WMAX 20
-#define REPLAY_THREADS 128
 __global__ void __launch_bounds__(REPLAY_THREADS)
     replay_reads_small_kernel(const int *__restrict__ table, int W, int wd, int wide_short,
                               const int *__restrict__ locus_ids, const long long *__restrict__ slot_begin, int n_list,
@@ -299,67 +327,14 @@ __global__ void __launch_bounds__(REPLAY_THREADS)
                               int step, int tie_flags, int *__restrict__ out, unsigned char *__restrict__ locus_status,
                               unsigned int *miss_count, double *ref_cells, const int *__restrict__ rep,
                               double *__restrict__ hint = nullptr) {
-    // hint != nullptr: a locus that misses records the offset fraction it missed at (first pass: windows are est +- wdr)
-    __shared__ int rows[REPLAY_THREADS * (REPLAY_WMAX + 1)];
+    __shared__ int stripes[REPLAY_THREADS * (REPLAY_WMAX + 1)];
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n_list) return;
-    int *row = rows + threadIdx.x * (REPLAY_WMAX + 1);
-    const int locus = locus_ids ? locus_ids[q] : q;
-    const long long r0 = read_begin[locus], r1 = read_begin[locus + 1];
-    long long slot = locus_ids ? slot_begin[q] : r0;
-    SeenSmall seen;
-    double frac = 0.0;
-    double cells = 0.0;
-    const int m = motif_len[locus];
-    const int wdr = strk_read_wd(wd, m, wide_short);
-    int status = 0;
-    bool margin_used = false;
-    int nrow[REPLAY_WMAX], nest = 0, nl0 = 0, nl1 = 0, nl2 = 0;
-    auto fetch = [&](long long r, long long sl) {
-        const int *src = table + (size_t)(rep ? (long long)rep[r] : sl) * (size_t)W;
-#pragma unroll
-        for (int k = 0; k < REPLAY_WMAX; ++k) nrow[k] = k < W ? src[k] : 0;
-        nest = est_cn[r];
-        nl0 = lens[3 * r], nl1 = lens[3 * r + 1], nl2 = lens[3 * r + 2];
-    };
-    if (r0 < r1) fetch(r0, slot);
-    for (long long r = r0; r < r1; ++r, ++slot) {
-#pragma unroll
-        for (int k = 0; k < REPLAY_WMAX; ++k) row[k] = nrow[k];
-        const int est = nest;
-        const double n1 = (double)(nl0 + nl1 + nl2), fl_fr = (double)(nl0 + nl2);
-        if (r + 1 < r1) fetch(r + 1, slot + 1);
-        int read_sc = est;
-        const int off = (int)rint(frac * (double)read_sc);  // round(), :1130
-        if (off < -read_sc)
-            frac = 0.0;  // :1133
-        else
-            read_sc += off;  // :1136
-        const int n_lo = est - wdr > 0 ? est - wdr : 0;
-        const int n_hi = est + wdr;
-        ClimbResult cr = climb_single(row, n_lo, n_hi, read_sc, max_iters, range, step, tie_flags, seen);
-        if (cr.status) {
-            status = cr.status;
-            if (hint && cr.status == 1) {
-                double *h = hint + 2 * (size_t)locus;
-                const double fr_used = read_sc == est ? 0.0 : frac;
-                h[0] = fr_used < h[0] ? fr_used : h[0];
-                h[1] = fr_used > h[1] ? fr_used : h[1];
-            }
-            break;
-        }
-        margin_used |= cr.lo_touched < est - wd || cr.hi_touched > est + wd;
-        *(int4 *)(out + 4 * r) = make_int4(cr.best_n, cr.best_score, cr.n_explored, read_sc);
-        frac += (double)(cr.best_n - read_sc) / (double)(cr.best_n > 1 ? cr.best_n : 1);  // :1161
-        cells += n1 * ((double)cr.n_explored * fl_fr + (double)m * cr.sum_n);
-    }
-    locus_status[locus] = (unsigned char)status;
-    if (status) {
-        atomicAdd(miss_count, 1u);
-    } else {
-        atomicAdd(ref_cells, cells);
-        if (margin_used) atomicAdd(miss_count + 2, 1u);
-    }
+    StagedRows rows;
+    rows.src = {table, W, rep, est_cn, lens};
+    rows.stripe = stripes + threadIdx.x * (REPLAY_WMAX + 1);
+    replay_locus<SeenSmall>(q, rows, wd, wide_short, locus_ids, slot_begin, read_begin, motif_len, max_iters, range,
+                            step, tie_flags, out, locus_status, miss_count, ref_cells, hint);
 }
 
 // Builds the family descriptors of a pass on the device (no descriptor H2D traffic).

@@ -293,16 +293,19 @@ def test_batch_search_parameters(sb, oracle, params):
     assert np.array_equal(got, want)
 
 
-@pytest.mark.parametrize("tie", [1, 2, 3, 4, 8, 7])
-def test_tie_break_switches(sb, oracle, tie):
+# (50, 3, 1): first windows of 13 sizes, replayed by replay_reads_small_kernel; (50, 8, 3): 27 sizes, replay_reads_kernel
+@pytest.mark.parametrize("tie,search", [pytest.param(t, s, id=f"{t}{sfx}") for s, sfx in [((50, 3, 1), ""), ((50, 8, 3), "-w27")]
+                                        for t in [1, 2, 3, 4, 8, 7]])
+def test_tie_break_switches(sb, oracle, tie, search):
     rng = np.random.default_rng(9)
     # homopolymer-ish tracts with wildcards produce many equal scores
     fams = [("A", "A" * int(rng.integers(3, 20)) + "X" * int(rng.integers(0, 4)), "", "ACGTT") for _ in range(40)]
     batch = families_to_batch(fams, est=[int(rng.integers(0, 25)) for _ in fams])
     eng = sb.Engine(tie_flags=tie)
-    got = eng.count_reads(batch, sb.RepeatCountParams("repalign", 50, 3, 1))
+    got = eng.count_reads(batch, sb.RepeatCountParams("repalign", *search))
     want, _ = oracle.count_loci(batch.arena, batch.seq_off, batch.lens, batch.est_cn, batch.read_begin,
-                                batch.motif_off, batch.motif_len, tie_flags=tie)
+                                batch.motif_off, batch.motif_len, max_iters=search[0], local_search_range=search[1],
+                                step_size=search[2], tie_flags=tie)
     assert np.array_equal(got, want)
 
 
