@@ -210,6 +210,12 @@ int strk_get_stats(strk_ctx *ctx, double stats[8]);
  * The random streams are this library's (counter-based Philox keyed by seed, locus, replicate), not numpy's:
  * results agree with the reference statistically.  n_alleles 1 and 2 are implemented here; per-locus counts up to 8
  * take the _ploidy entry below.
+ * Read depth: a locus of at most 256 reads is shallow (one thread per replicate, arrays strided by the batch's
+ * largest shallow locus); a locus of more reads is deep: it is resampled and fitted one warp per replicate (see
+ * strk_gmm_fit_counts_deep) from ragged per-locus storage, on random streams of its own keyed by seed, locus and
+ * replicate, so its rows depend neither on the chunking nor on the other loci, and shallow rows do not depend on it.
+ * The rule follows from the read count alone.  A deep locus may have up to 4096 distinct copy numbers; one with more
+ * is STRK_ERR_UNSUPPORTED, and the message names the locus.
  */
 int strk_call_alleles(strk_ctx *ctx, const int32_t *cn, const double *weights, const int64_t *read_begin,
                       int64_t n_loci, int n_alleles, int num_bootstrap, int min_reads, int min_allele_reads,
@@ -258,6 +264,15 @@ int strk_gmm_fit_counts_ploidy(strk_ctx *ctx, const double *x, const int32_t *co
                                const int32_t *n_alleles, const int32_t *init, int64_t n_problems, int kcap,
                                int num_bootstrap, int min_allele_reads, int force_gm_filter, double expansion_ratio,
                                int filter_factor, int n_init, uint64_t seed, double *out);
+
+/* strk_gmm_fit_counts_ploidy through the warp-cooperative fit of deep loci, for K[q] up to kcap <= 4096 and any
+ * number of points: one warp per problem, k-means++ and EM over its nonzero (value, count) pairs with warp reductions
+ * (the same arithmetic per pair, sums in another order), fit_gmm's staged loop and the fill as above.  Same arguments
+ * and output; the k-means++ stream (init NULL) is keyed by seed and q but differs from the per-thread entry's. */
+int strk_gmm_fit_counts_deep(strk_ctx *ctx, const double *x, const int32_t *counts, const int32_t *K,
+                             const int32_t *n_alleles, const int32_t *init, int64_t n_problems, int kcap,
+                             int num_bootstrap, int min_allele_reads, int force_gm_filter, double expansion_ratio,
+                             int filter_factor, int n_init, uint64_t seed, double *out);
 
 /* The aggregation step alone (allele.py:295-336): replicate arrays [locus][allele][replicate] (+ peaks
  * [locus][replicate]) -> out_i / out_d as in strk_call_alleles, for n_alleles 1..8. */

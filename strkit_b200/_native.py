@@ -67,6 +67,8 @@ def _load() -> C.CDLL:
                                                C.c_double, C.c_int, C.c_int, _u64, _vp, _vp, _vp, _vp]),
         "strk_gmm_fit_counts_ploidy": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, C.c_int, C.c_int, C.c_int, C.c_int,
                                                  C.c_double, C.c_int, C.c_int, _u64, _vp]),
+        "strk_gmm_fit_counts_deep": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_double, C.c_int, C.c_int, _u64, _vp]),
         "strk_alleles_aggregate": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, C.c_int, C.c_int, _vp, _vp]),
         "strk_realign": (C.c_int, [_vp, _vp, _u64, _vp, _vp, _vp, _vp, _i64, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _vp,
                                    _vp]),
@@ -84,7 +86,7 @@ lib = _load()
 EXPORTED = ("strk_last_error", "strk_version", "strk_device_count", "strk_init", "strk_destroy", "strk_sync", "strk_host_register",
             "strk_host_unregister", "strk_batch_upload", "strk_batch_create", "strk_batch_fill", "strk_batch_fill_fmt", "strk_count_reads_fmt", "strk_batch_run", "strk_batch_download", "strk_batch_free",
             "strk_count_reads", "strk_get_repeat_count", "strk_score_tables", "strk_ref_boundary_tables", "strk_ref_counts", "strk_call_alleles", "strk_gmm_fit_counts",
-            "strk_call_alleles_ploidy", "strk_gmm_fit_counts_ploidy", "strk_alleles_aggregate", "strk_realign", "strk_get_stats", "strk_measure_int_peak")
+            "strk_call_alleles_ploidy", "strk_gmm_fit_counts_ploidy", "strk_gmm_fit_counts_deep", "strk_alleles_aggregate", "strk_realign", "strk_get_stats", "strk_measure_int_peak")
 
 
 def check(rc: int) -> None:

@@ -3,8 +3,9 @@
 Mirrors the reference's `call_alleles` (strkit/call/allele.py:176-336) and, batched over many loci,
 the loop `call_locus` runs around it (call_alleles_with_gmm, call_locus.py:177-219).  The arithmetic is in
 the native library (csrc/alleles.cuh): one CUDA thread per (locus, bootstrap replicate) resamples, seeds
-with k-means++, runs sklearn's EM in float64 and applies the reference's peak filters; one CTA per locus
-sorts the replicate estimates and takes medians / confidence intervals.
+with k-means++, runs sklearn's EM in float64 and applies the reference's peak filters (one warp per replicate
+for loci of more than 256 reads); one CTA per locus sorts the replicate estimates and takes medians /
+confidence intervals.
 
 The random streams are the library's own (counter-based, keyed by seed / locus / replicate), so calls and
 intervals agree with the reference statistically (tests/test_alleles_*.py state the tolerance), while
@@ -21,7 +22,7 @@ from ._native import check, lib
 from .engine import Engine, default_engine
 
 __all__ = ["AlleleCalls", "CallData", "call_alleles_batch", "call_alleles_ploidy_batch", "call_alleles", "gmm_fit_counts",
-           "gmm_fit_counts_ploidy", "aggregate_replicates"]
+           "gmm_fit_counts_ploidy", "gmm_fit_counts_deep", "aggregate_replicates"]
 
 
 def _p(a: np.ndarray) -> int:
@@ -200,6 +201,24 @@ def gmm_fit_counts_ploidy(values: Sequence[np.ndarray], counts: Sequence[np.ndar
     for nc = A, A-1, ..., 2, n_init rows of nc indices into values[q], flattened.  Returns [q, 3 * S + 1] with
     S = max(n_alleles): means[S], weights[S], stdevs[S] (the first A[q] sorted by mean, the rest 0), n_peaks.
     Entries beyond the fitted n_peaks are random copies of fitted components (the reference's fill)."""
+    return _fit_counts(lib.strk_gmm_fit_counts_ploidy, values, counts, n_alleles, init, n_init, num_bootstrap,
+                       min_allele_reads, force_gm_filter, expansion_ratio, filter_factor, seed, engine)
+
+
+def gmm_fit_counts_deep(values: Sequence[np.ndarray], counts: Sequence[np.ndarray], n_alleles,
+                        init: Sequence[np.ndarray] | None = None, *, n_init: int = 3, num_bootstrap: int = 100,
+                        min_allele_reads: int = 2, force_gm_filter: bool = False, expansion_ratio: float = 5.0,
+                        filter_factor: int = 3, seed: int = 0, engine: Engine | None = None) -> np.ndarray:
+    """gmm_fit_counts_ploidy through the warp-cooperative fit that deep loci (more than 256 reads) use: the same
+    arguments and output, for up to 4096 distinct values per problem and any number of points.  Without forced
+    seeds its k-means++ draws come from another stream than gmm_fit_counts_ploidy's."""
+    return _fit_counts(lib.strk_gmm_fit_counts_deep, values, counts, n_alleles, init, n_init, num_bootstrap,
+                       min_allele_reads, force_gm_filter, expansion_ratio, filter_factor, seed, engine)
+
+
+def _fit_counts(fn, values, counts, n_alleles, init, n_init, num_bootstrap, min_allele_reads, force_gm_filter,
+                expansion_ratio, filter_factor, seed, engine):
+    name = fn.__name__[len("strk_"):]
     eng = engine or default_engine()
     nq = len(values)
     a = np.ascontiguousarray(np.broadcast_to(np.asarray(n_alleles, dtype=np.int32), (nq,)))
@@ -217,13 +236,12 @@ def gmm_fit_counts_ploidy(values: Sequence[np.ndarray], counts: Sequence[np.ndar
         for q, i in enumerate(init):
             want = n_init * (int(a[q]) * (int(a[q]) + 1) // 2 - 1) if 1 <= a[q] <= 8 else i.size
             if i.size != want:
-                raise ValueError(f"gmm_fit_counts_ploidy: problem {q} has {i.size} seed indices, expected {want}")
+                raise ValueError(f"{name}: problem {q} has {i.size} seed indices, expected {want}")
         init = np.ascontiguousarray(np.concatenate(init) if init else np.zeros(0, dtype=np.int32), dtype=np.int32)
     out = np.zeros((nq, 3 * s + 1), dtype=np.float64)
-    check(lib.strk_gmm_fit_counts_ploidy(eng._ctx, _p(x), _p(c), _p(k), _p(a), None if init is None else _p(init), nq,
-                                         kcap, num_bootstrap, min_allele_reads, int(force_gm_filter),
-                                         float(expansion_ratio), filter_factor, n_init, int(seed) & 0xFFFFFFFFFFFFFFFF,
-                                         _p(out)))
+    check(fn(eng._ctx, _p(x), _p(c), _p(k), _p(a), None if init is None else _p(init), nq, kcap, num_bootstrap,
+             min_allele_reads, int(force_gm_filter), float(expansion_ratio), filter_factor, n_init,
+             int(seed) & 0xFFFFFFFFFFFFFFFF, _p(out)))
     return out
 
 

@@ -29,6 +29,10 @@
 #define ALL_MAX_BOOT 4096   // replicates per locus the aggregation kernel sorts in shared memory
 #define ALL_N_INIT_MAX 8
 #define ALL_MAX_ALLELES 8   // components per locus (fit_replicate_k keeps its arrays this wide)
+#define ALL_SHALLOW_READS 256  // loci with more reads are deep: alleles_deep_prepare_kernel / alleles_deep_fit_kernel
+#define ALL_DEEP_MAX_K 4096    // distinct copy numbers of a deep locus (bounds the deep fit's shared memory)
+#define ALL_DEEP_WARPS 4       // warps per CTA of the deep fit, one (locus, replicate) each
+#define ALL_DEEP_STREAM 0x80000000u  // replicate-word bit of deep streams: shallow replicates are < ALL_MAX_BOOT
 
 struct AlleleParams {
     int n_alleles;          // 1 or 2: the batch-wide count of strk_call_alleles (per-locus counts come as an array)
@@ -59,6 +63,12 @@ struct Philox {
         c1 = 0;
         c2 = a;
         c3 = b;
+        have = 0;
+    }
+    // jump to counter (lo, hi): the next two uniforms are the pair of that counter
+    __device__ __forceinline__ void seek(uint32_t lo, uint32_t hi) {
+        c0 = lo;
+        c1 = hi;
         have = 0;
     }
     __device__ __forceinline__ void round(uint32_t &x0, uint32_t &x1, uint32_t &x2, uint32_t &x3, uint32_t k0,
@@ -106,6 +116,7 @@ __global__ void alleles_prepare_kernel(const int *__restrict__ cn, const double 
     const long long r0 = read_begin[l], r1 = read_begin[l + 1];
     const int n = (int)(r1 - r0);
     n_out[l] = n;
+    if (n > ALL_SHALLOW_READS) return;  // deep: alleles_deep_prepare_kernel
     int *v = vals + (size_t)l * kcap;
     double *p = cdf + (size_t)l * kcap;
     int *q = cnt + (size_t)l * kcap;
@@ -146,20 +157,22 @@ struct Gmm2 {
     int n_comp;
 };
 
-// sklearn _estimate_log_gaussian_prob (spherical, one feature) + log weights, for one x
+// sklearn _estimate_log_gaussian_prob (spherical, one feature) + log weight of one component, for one x
+__device__ __forceinline__ double gmm_wlp1(double x, double mean, double pchol, double logw) {
+    // separately rounded products and sums, in sklearn's order: the three terms cancel almost completely for
+    // a point near the mean (precision up to 1e6), so a fused multiply-add here would change the low bits
+    const double prec = __dmul_rn(pchol, pchol);
+    const double t1 = __dmul_rn(__dmul_rn(mean, mean), prec);
+    const double t2 = __dmul_rn(2.0, __dmul_rn(__dmul_rn(x, mean), prec));
+    const double t3 = __dmul_rn(__dmul_rn(x, x), prec);
+    const double lp = __dadd_rn(__dsub_rn(t1, t2), t3);
+    return __dadd_rn(__dadd_rn(__dmul_rn(-0.5, __dadd_rn(1.8378770664093453, lp)), log(pchol)), logw);
+}
+
 __device__ __forceinline__ void gmm_wlp(double x, const double mean[2], const double pchol[2], const double logw[2],
                                         double out[2]) {
 #pragma unroll
-    for (int k = 0; k < 2; ++k) {
-        // separately rounded products and sums, in sklearn's order: the three terms cancel almost completely for
-        // a point near the mean (precision up to 1e6), so a fused multiply-add here would change the low bits
-        const double prec = __dmul_rn(pchol[k], pchol[k]);
-        const double t1 = __dmul_rn(__dmul_rn(mean[k], mean[k]), prec);
-        const double t2 = __dmul_rn(2.0, __dmul_rn(__dmul_rn(x, mean[k]), prec));
-        const double t3 = __dmul_rn(__dmul_rn(x, x), prec);
-        const double lp = __dadd_rn(__dsub_rn(t1, t2), t3);
-        out[k] = __dadd_rn(__dadd_rn(__dmul_rn(-0.5, __dadd_rn(1.8378770664093453, lp)), log(pchol[k])), logw[k]);
-    }
+    for (int k = 0; k < 2; ++k) out[k] = gmm_wlp1(x, mean[k], pchol[k], logw[k]);
 }
 
 // EM from the k-means++ seeds (value indices i0, i1): GaussianMixture._initialize with one-hot responsibilities on
@@ -378,14 +391,7 @@ __device__ double gmm_em_k(const double *x, const int *c, int K, int n, const in
             if (c[v] == 0) continue;
             double wl[NC];
 #pragma unroll
-            for (int k = 0; k < NC; ++k) {
-                const double prec = __dmul_rn(pchol[k], pchol[k]);
-                const double t1 = __dmul_rn(__dmul_rn(mean[k], mean[k]), prec);
-                const double t2 = __dmul_rn(2.0, __dmul_rn(__dmul_rn(x[v], mean[k]), prec));
-                const double t3 = __dmul_rn(__dmul_rn(x[v], x[v]), prec);
-                const double lp = __dadd_rn(__dsub_rn(t1, t2), t3);
-                wl[k] = __dadd_rn(__dadd_rn(__dmul_rn(-0.5, __dadd_rn(1.8378770664093453, lp)), log(pchol[k])), logw[k]);
-            }
+            for (int k = 0; k < NC; ++k) wl[k] = gmm_wlp1(x[v], mean[k], pchol[k], logw[k]);
             double mx = wl[0];
 #pragma unroll
             for (int k = 1; k < NC; ++k) mx = fmax(mx, wl[k]);
@@ -529,17 +535,17 @@ __device__ __forceinline__ int gmm_useless_k(const GmmK &g, int nc, const Allele
 // last fit with all its components.  A replicate with fewer peaks than A gets A - peaks components drawn with
 // probability weight / sum|weight| (Philox stream of the thread), then everything is sorted by mean (stable).
 // *n_peaks = the fitted count, before the fill.  forced_init (NULL = k-means++): for nc = A, A-1, ..., 2, n_init
-// rows of nc seed indices.
-template <int KMAX>
-__device__ void fit_replicate_k(const double *x, const int *c, int K, int n, int A, const AlleleParams &P, Philox &rng,
-                                const int *forced_init, double *out_m, double *out_w, double *out_s, int *n_peaks) {
-    int distinct = 0;
-    for (int v = 0; v < K; ++v) distinct += c[v] != 0;
+// rows of nc seed indices.  The loop and the bookkeeping are shared with the warp-cooperative fit of deep loci:
+// fit(nc, forced, g) is GaussianMixture(nc).fit, single(m, var) make_single_gaussian.
+template <class Fit, class Single>
+__device__ __forceinline__ void fit_staged(int distinct, int A, const AlleleParams &P, Philox &rng,
+                                           const int *forced_init, Fit fit, Single single, double *out_m, double *out_w,
+                                           double *out_s, int *n_peaks) {
     GmmK g;
     int nc = distinct == 1 ? 1 : A;  // len(mc) == 1: a single Gaussian without a fit
     while (nc > 1) {
         const int *forced = forced_init ? forced_init + P.n_init * (A * (A + 1) / 2 - nc * (nc + 1) / 2) : nullptr;
-        gmm_fit_k<KMAX>(x, c, K, n, nc, P, rng, forced, g);
+        fit(nc, forced, g);
         const int useless = gmm_useless_k(g, nc, P);
         if (!useless) break;
         nc -= useless;
@@ -547,7 +553,7 @@ __device__ void fit_replicate_k(const double *x, const int *c, int K, int n, int
     int peaks;
     if (nc == 1) {
         double m, var;
-        single_gaussian(x, c, K, n, m, var);
+        single(m, var);
         out_m[0] = m, out_w[0] = 1.0, out_s[0] = sqrt(var);
         peaks = 1;
     } else {
@@ -578,6 +584,17 @@ __device__ void fit_replicate_k(const double *x, const int *c, int K, int n, int
     }
 }
 
+template <int KMAX>
+__device__ void fit_replicate_k(const double *x, const int *c, int K, int n, int A, const AlleleParams &P, Philox &rng,
+                                const int *forced_init, double *out_m, double *out_w, double *out_s, int *n_peaks) {
+    int distinct = 0;
+    for (int v = 0; v < K; ++v) distinct += c[v] != 0;
+    fit_staged(
+        distinct, A, P, rng, forced_init,
+        [&](int nc, const int *forced, GmmK &g) { gmm_fit_k<KMAX>(x, c, K, n, nc, P, rng, forced, g); },
+        [&](double &m, double &var) { single_gaussian(x, c, K, n, m, var); }, out_m, out_w, out_s, n_peaks);
+}
+
 // one replicate of a locus with A alleles: the two-component code for A <= 2, the k-component one above
 template <int KMAX, int AMAX>
 __device__ __forceinline__ void fit_replicate_any(const double *x, const int *c, int K, int n, int A,
@@ -602,7 +619,7 @@ alleles_fit_kernel(const int *__restrict__ vals, const double *__restrict__ cdf,
     const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int B = P.num_bootstrap;
     const int l = (int)(tid / B), b = (int)(tid % B);
-    if (l >= n_loci || status[l] != 0) return;
+    if (l >= n_loci || status[l] != 0 || n_arr[l] > ALL_SHALLOW_READS) return;  // deep loci: alleles_deep_fit_kernel
     const int K = K_arr[l], n = n_arr[l];
     if (K > KMAX) return;  // the host picks KMAX >= the batch maximum
     const int A = A_arr ? A_arr[l] : P.n_alleles;
@@ -684,6 +701,426 @@ __global__ void gmm_fit_counts_ploidy_kernel(const double *__restrict__ xs, cons
         o[2 * S + a] = a < A ? s[a] : 0.0;
     }
     o[3 * S] = (double)peaks;
+}
+
+// ---------------------------------------------------------------------------------------------- deep loci
+// Loci with more than ALL_SHALLOW_READS reads.  K can be as large as the read count, so the per-thread arrays above
+// do not scale to them: one CTA per deep locus builds its distinct values and CDF in ragged storage, and one warp
+// per (locus, replicate) resamples and fits.  A replicate is held as its D nonzero (value, count) pairs in shared
+// memory; every sum over them is a lane-strided partial sum followed by a butterfly (xor) reduction, which leaves
+// the bitwise same total in every lane, so all lanes carry the same model, the same random state and take the same
+// branches.  Given the seeds, the arithmetic per pair is gmm_em_k's; only the order of the sums differs.
+
+__device__ __forceinline__ double warp_sum(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// searchsorted over the cumulative sum of term(0..D): the first j whose inclusive prefix sum is >= r (> r with
+// `strict`), D - 1 if none.  32 terms at a time: a shuffle-up scan plus the carry of the chunks before.
+template <class T, class Term>
+__device__ __forceinline__ int warp_search(int D, T r, bool strict, Term term) {
+    const int lane = threadIdx.x & 31;
+    T carry = 0;
+    for (int j0 = 0; j0 < D; j0 += 32) {
+        const int j = j0 + lane;
+        T s = j < D ? term(j) : (T)0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const T t = __shfl_up_sync(0xffffffffu, s, o);
+            if (lane >= o) s += t;
+        }
+        s += carry;
+        const unsigned hit = __ballot_sync(0xffffffffu, j < D && (strict ? s > r : s >= r));
+        if (hit) return j0 + __ffs(hit) - 1;
+        carry = __shfl_sync(0xffffffffu, s, 31);
+    }
+    return D - 1;
+}
+
+// the nonzero counts cnt(0..K) with their values val(j), in ascending j, to cv[0..D) / xv[0..D); returns D.
+// cv may be the array cnt reads (every lane reads its entry of a chunk before any lane writes, and writes land at
+// or below the chunk).
+template <class Cnt, class Val>
+__device__ __forceinline__ int warp_compact(int K, Cnt cnt, Val val, double *xv, int *cv) {
+    const int lane = threadIdx.x & 31;
+    int D = 0;
+    for (int j0 = 0; j0 < K; j0 += 32) {
+        const int j = j0 + lane;
+        const int c = j < K ? cnt(j) : 0;
+        const unsigned nz = __ballot_sync(0xffffffffu, c != 0);
+        __syncwarp();
+        if (c) {
+            const int q = D + __popc(nz & ((1u << lane) - 1u));
+            cv[q] = c;
+            xv[q] = val(j);
+        }
+        D += __popc(nz);
+    }
+    __syncwarp();
+    return D;
+}
+
+// closest squared distance of x to the first nce centres (kmeanspp_k's running fmin, recomputed)
+__device__ __forceinline__ double closest_sq(double x, const double *cen, int nce) {
+    double d = x - cen[0], cl = d * d;
+#pragma unroll
+    for (int i = 1; i < ALL_MAX_ALLELES; ++i)
+        if (i < nce) d = x - cen[i], cl = fmin(cl, d * d);
+    return cl;
+}
+
+// kmeanspp_k on D nonzero pairs, warp-cooperative: the centres' values to cen[0..k)
+__device__ void kmeanspp_warp(const double *xv, const int *cv, int D, int n, int k, Philox &rng, double *cen) {
+    const int lane = threadIdx.x & 31;
+    {
+        const double u = rng.uniform();
+        long long pt = (long long)(u * (double)n);
+        if (pt >= n) pt = n - 1;
+        cen[0] = xv[warp_search<long long>(D, pt, true, [&](int j) { return (long long)cv[j]; })];
+    }
+    double pot = 0.0;
+    for (int j = lane; j < D; j += 32) pot += (double)cv[j] * closest_sq(xv[j], cen, 1);
+    pot = warp_sum(pot);
+    const int trials = 2 + (int)log((double)k);
+    for (int ci = 1; ci < k; ++ci) {
+        double best_pot = INFINITY;
+        int best = 0;
+#pragma unroll 1
+        for (int t = 0; t < trials; ++t) {
+            const double r = rng.uniform() * pot;
+            const int cand = warp_search<double>(D, r, false,
+                                                 [&](int j) { return (double)cv[j] * closest_sq(xv[j], cen, ci); });
+            double cp = 0.0;
+            for (int j = lane; j < D; j += 32) {
+                const double d = xv[j] - xv[cand];
+                cp += (double)cv[j] * fmin(closest_sq(xv[j], cen, ci), d * d);
+            }
+            cp = warp_sum(cp);
+            if (cp < best_pot) best_pot = cp, best = cand;
+        }
+        cen[ci] = xv[best];
+        pot = best_pot;
+    }
+}
+
+// gmm_em_k from the seed values cen[0..NC) on D nonzero pairs, warp-cooperative
+template <int NC>
+__device__ double gmm_em_warp(const double *xv, const int *cv, int D, int n, const double *cen, const AlleleParams &P,
+                              GmmK &g) {
+    const int lane = threadIdx.x & 31;
+    const double eps10 = 10.0 * 2.220446049250313e-16;
+    double mean[NC], cov[NC], weight[NC], pchol[NC], logw[NC];
+#pragma unroll
+    for (int k = 0; k < NC; ++k) {
+        const double nk = 1.0 + eps10, xk = cen[k];
+        mean[k] = xk / nk;
+        cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(__dmul_rn(xk, xk), nk), __dmul_rn(mean[k], mean[k])), P.reg_covar);
+        weight[k] = nk / (double)n;
+        pchol[k] = 1.0 / sqrt(cov[k]);
+        logw[k] = log(weight[k]);
+    }
+    double lower = -INFINITY;
+    for (int it = 1; it <= P.max_iter; ++it) {
+        const double prev = lower;
+        double nk[NC], sx[NC], sxx[NC], ll = 0.0;
+#pragma unroll
+        for (int k = 0; k < NC; ++k) nk[k] = 0.0, sx[k] = 0.0, sxx[k] = 0.0;
+        for (int j = lane; j < D; j += 32) {
+            const double x = xv[j];
+            double wl[NC];
+#pragma unroll
+            for (int k = 0; k < NC; ++k) wl[k] = gmm_wlp1(x, mean[k], pchol[k], logw[k]);
+            double mx = wl[0];
+#pragma unroll
+            for (int k = 1; k < NC; ++k) mx = fmax(mx, wl[k]);
+            double se = 0.0;
+#pragma unroll
+            for (int k = 0; k < NC; ++k) se += exp(wl[k] - mx);
+            const double lse = mx + log(se);
+            const double c = (double)cv[j];
+            ll += c * lse;
+#pragma unroll
+            for (int k = 0; k < NC; ++k) {
+                const double r = exp(wl[k] - lse) * c;
+                nk[k] += r;
+                sx[k] += r * x;
+                sxx[k] += r * x * x;
+            }
+        }
+        ll = warp_sum(ll);
+#pragma unroll
+        for (int k = 0; k < NC; ++k) nk[k] = warp_sum(nk[k]), sx[k] = warp_sum(sx[k]), sxx[k] = warp_sum(sxx[k]);
+        lower = ll / (double)n;
+        double wsum = 0.0;
+#pragma unroll
+        for (int k = 0; k < NC; ++k) {
+            nk[k] += eps10;
+            mean[k] = sx[k] / nk[k];
+            cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(sxx[k], nk[k]), __dmul_rn(mean[k], mean[k])), P.reg_covar);
+            weight[k] = nk[k] / (double)n;
+            wsum += weight[k];
+        }
+#pragma unroll
+        for (int k = 0; k < NC; ++k) {
+            weight[k] /= wsum;
+            pchol[k] = 1.0 / sqrt(cov[k] > 0.0 ? cov[k] : P.reg_covar);
+            logw[k] = log(weight[k]);
+        }
+        if (fabs(lower - prev) < P.tol) break;
+    }
+#pragma unroll
+    for (int k = 0; k < NC; ++k) g.mean[k] = mean[k], g.cov[k] = cov[k], g.weight[k] = weight[k];
+    g.n_comp = NC;
+    return lower;
+}
+
+// gmm_fit_k, warp-cooperative: forced seed indices point into x_forced (the caller's value list)
+__device__ void gmm_fit_warp(const double *xv, const int *cv, int D, int n, int nc, const AlleleParams &P, Philox &rng,
+                             const int *forced, const double *x_forced, GmmK &best) {
+    double best_lb = -INFINITY;
+    for (int t = 0; t < P.n_init; ++t) {
+        double cen[ALL_MAX_ALLELES];
+        if (forced) {
+            for (int j = 0; j < nc; ++j) cen[j] = x_forced[forced[t * nc + j]];
+        } else {
+            kmeanspp_warp(xv, cv, D, n, nc, rng, cen);
+        }
+        GmmK g;
+        double lb;
+        switch (nc) {
+        case 2: lb = gmm_em_warp<2>(xv, cv, D, n, cen, P, g); break;
+        case 3: lb = gmm_em_warp<3>(xv, cv, D, n, cen, P, g); break;
+        case 4: lb = gmm_em_warp<4>(xv, cv, D, n, cen, P, g); break;
+        case 5: lb = gmm_em_warp<5>(xv, cv, D, n, cen, P, g); break;
+        case 6: lb = gmm_em_warp<6>(xv, cv, D, n, cen, P, g); break;
+        case 7: lb = gmm_em_warp<7>(xv, cv, D, n, cen, P, g); break;
+        default: lb = gmm_em_warp<8>(xv, cv, D, n, cen, P, g); break;
+        }
+        if (lb > best_lb || best_lb == -INFINITY) best_lb = lb, best = g;
+    }
+}
+
+// One replicate of a deep locus (any A, 1..8): fit_gmm's staged loop and bookkeeping (fit_staged) over the warp
+// fits.  For A <= 2 this is the two-component code's result too: the staged loop at 2 components is fit_replicate
+// (the same k-means++ draws, EM and filter).
+__device__ void fit_replicate_warp(const double *xv, const int *cv, int D, int n, int A, const AlleleParams &P,
+                                   Philox &rng, const int *forced_init, const double *x_forced, double *out_m,
+                                   double *out_w, double *out_s, int *n_peaks) {
+    const int lane = threadIdx.x & 31;
+    fit_staged(
+        D, A, P, rng, forced_init,
+        [&](int nc, const int *forced, GmmK &g) { gmm_fit_warp(xv, cv, D, n, nc, P, rng, forced, x_forced, g); },
+        [&](double &m, double &var) {
+            double s = 0.0;
+            for (int j = lane; j < D; j += 32) s += (double)cv[j] * xv[j];
+            m = warp_sum(s) / (double)n;
+            double q = 0.0;
+            for (int j = lane; j < D; j += 32) {
+                const double d = xv[j] - m;
+                q += (double)cv[j] * d * d;
+            }
+            var = warp_sum(q) / (double)n;
+        },
+        out_m, out_w, out_s, n_peaks);
+}
+
+// one CTA per deep locus deep_l[d]: its sorted distinct values and resampling CDF at deep_off[d] (ragged, up to
+// ALL_DEEP_MAX_K entries), K, status (1: fewer than min_reads reads, 2: one distinct value, else 0; fewer reads
+// than A cannot occur above ALL_SHALLOW_READS reads), and its first value at vals[l * kcap], where the aggregation
+// reads the value of a status-2 locus.  More than ALL_DEEP_MAX_K distinct values: deep_K[d] > ALL_DEEP_MAX_K and
+// nothing else is written (the host reports the locus).
+// The per-value weight sums are fixed-point integers (each weight scaled to 2^63 / (n * max weight) and rounded):
+// integer atomics make them independent of the order the threads add in, and the CDF of exact integer sums is
+// cdf[j] = sum[0..j] / sum[0..K), normalised by the total as Generator.choice does (cdf /= cdf[-1]).
+#define ALL_DEEP_TABLE (2 * ALL_DEEP_MAX_K)  // open-addressing hash set of the distinct values (load <= 0.53)
+__global__ void __launch_bounds__(256)
+alleles_deep_prepare_kernel(const int *__restrict__ cn, const double *__restrict__ w,
+                            const long long *__restrict__ read_begin, const int *__restrict__ deep_l,
+                            const long long *__restrict__ deep_off, int min_reads, int kcap, int *__restrict__ dvals,
+                            double *__restrict__ dcdf, int *__restrict__ K_out, int *__restrict__ deep_K,
+                            int *__restrict__ status, int *__restrict__ vals) {
+    extern __shared__ unsigned long long smem_deep_prep[];
+    unsigned long long *table = smem_deep_prep;                  // [ALL_DEEP_TABLE]; then wsum[ALL_DEEP_MAX_K]
+    int *sv = (int *)(smem_deep_prep + ALL_DEEP_TABLE);          // [ALL_DEEP_MAX_K] sorted distinct values
+    __shared__ int s_K, s_slot;
+    __shared__ double s_wmax;
+    const unsigned long long EMPTY = ~0ull;
+    const int d = blockIdx.x, l = deep_l[d];
+    const long long r0 = read_begin[l], r1 = read_begin[l + 1];
+    const int n = (int)(r1 - r0);
+    for (int i = threadIdx.x; i < ALL_DEEP_TABLE; i += blockDim.x) table[i] = EMPTY;
+    if (threadIdx.x == 0) s_K = 0, s_slot = 0, s_wmax = 0.0;
+    __syncthreads();
+    // distinct values; a thread stops once the set is over the cap, so at most cap + blockDim entries are inserted
+    double wmax = 0.0;
+    for (long long r = r0 + threadIdx.x; r < r1; r += blockDim.x) {
+        wmax = fmax(wmax, w[r]);
+        if (*(volatile int *)&s_K > ALL_DEEP_MAX_K) continue;
+        const unsigned long long key = (unsigned)cn[r];
+        unsigned h = ((unsigned)cn[r] * 2654435761u) & (ALL_DEEP_TABLE - 1);
+        for (;;) {
+            const unsigned long long old = atomicCAS(&table[h], EMPTY, key);
+            if (old == EMPTY) {
+                atomicAdd(&s_K, 1);
+                break;
+            }
+            if (old == key) break;
+            h = (h + 1) & (ALL_DEEP_TABLE - 1);
+        }
+    }
+    // weights are >= 0: their doubles order like their bit patterns
+    atomicMax((unsigned long long *)&s_wmax, (unsigned long long)__double_as_longlong(wmax));
+    __syncthreads();
+    const int K = s_K;
+    if (K > ALL_DEEP_MAX_K) {
+        if (threadIdx.x == 0) deep_K[d] = K;
+        return;
+    }
+    int np2 = 1;
+    while (np2 < K) np2 <<= 1;
+    for (int i = threadIdx.x; i < ALL_DEEP_TABLE; i += blockDim.x)
+        if (table[i] != EMPTY) sv[atomicAdd(&s_slot, 1)] = (int)(unsigned)table[i];
+    for (int i = K + threadIdx.x; i < np2; i += blockDim.x) sv[i] = 0x7fffffff;
+    __syncthreads();
+    for (int k = 2; k <= np2; k <<= 1)  // bitonic sort of the distinct values (slot order above is arbitrary)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int t = threadIdx.x; t < np2; t += blockDim.x) {
+                const int u = t ^ j;
+                if (u > t) {
+                    const int a = sv[t], b = sv[u];
+                    if ((a > b) == ((t & k) == 0)) sv[t] = b, sv[u] = a;
+                }
+            }
+            __syncthreads();
+        }
+    unsigned long long *wsum = table;
+    for (int j = threadIdx.x; j < K; j += blockDim.x) wsum[j] = 0;
+    __syncthreads();
+    const double scale = s_wmax > 0.0 ? 9223372036854775808.0 / ((double)n * s_wmax) : 0.0;
+    for (long long r = r0 + threadIdx.x; r < r1; r += blockDim.x) {
+        const int x = cn[r];
+        int lo = 0, hi = K - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (sv[mid] < x) lo = mid + 1;
+            else hi = mid;
+        }
+        const double wr = w[r];
+        atomicAdd(&wsum[lo], (unsigned long long)rint((wr > 0.0 ? wr : 0.0) * scale));
+    }
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int j = 1; j < K; ++j) wsum[j] += wsum[j - 1];
+    __syncthreads();
+    const double tot = (double)wsum[K - 1];
+    int *v = dvals + deep_off[d];
+    double *p = dcdf + deep_off[d];
+    for (int j = threadIdx.x; j < K; j += blockDim.x) v[j] = sv[j], p[j] = (double)wsum[j] / tot;
+    if (threadIdx.x == 0) {
+        deep_K[d] = K_out[l] = K;
+        status[l] = n < min_reads ? 1 : (K == 1 ? 2 : 0);
+        vals[(size_t)l * kcap] = sv[0];
+    }
+}
+
+// one warp per (deep locus, replicate): CTA (d, y) takes replicates y * ALL_DEEP_WARPS + warp of deep locus deep_l[d].
+// Shared memory: the locus' CDF [K], then per warp the replicate's counts [K] (int) and its compacted values [K].
+// Resampling: draw i of replicate b is uniform i of the Philox stream (seed, l, b | ALL_DEEP_STREAM) from counter
+// (0, 0), two per counter, and searchsorted(cdf, u, side="right") by binary search; the lanes take alternate
+// counters and add to the warp's counts with integer atomics.  The fit draws from the same key from counter (0, 1).
+// Keys are the batch's seed and locus index, not the chunk's, so a deep row depends on neither the chunking nor the
+// launch shape.  Rows go to the chunk's replicate scratch at locus l - l0.
+__global__ void __launch_bounds__(32 * ALL_DEEP_WARPS)
+alleles_deep_fit_kernel(const int *__restrict__ deep_l, const long long *__restrict__ deep_off,
+                        const int *__restrict__ dvals, const double *__restrict__ dcdf, const int *__restrict__ K_arr,
+                        const int *__restrict__ n_arr, const int *__restrict__ status, const int *__restrict__ A_arr,
+                        int l0, int S, AlleleParams P, double *__restrict__ rep_m, double *__restrict__ rep_w,
+                        double *__restrict__ rep_s, unsigned char *__restrict__ rep_peaks) {
+    extern __shared__ double smem_deep_fit[];
+    const int d = blockIdx.x, l = deep_l[d];
+    if (status[l] != 0) return;
+    const int K = K_arr[l], n = n_arr[l], B = P.num_bootstrap;
+    const int A = A_arr ? A_arr[l] : P.n_alleles;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    double *cdf = smem_deep_fit;
+    double *xv = cdf + (size_t)K * (1 + warp);
+    int *cv = (int *)(cdf + (size_t)K * (1 + ALL_DEEP_WARPS)) + (size_t)K * warp;
+    const int *v = dvals + deep_off[d];
+    const double *p = dcdf + deep_off[d];
+    for (int j = threadIdx.x; j < K; j += blockDim.x) cdf[j] = p[j];
+    for (int j = lane; j < K; j += 32) cv[j] = 0;
+    __syncthreads();
+    const int b = blockIdx.y * ALL_DEEP_WARPS + warp;
+    if (b >= B) return;
+    Philox rng;
+    rng.init(P.seed, (uint32_t)l, (uint32_t)b | ALL_DEEP_STREAM);
+    for (unsigned pr = lane; pr < ((unsigned)n + 1u) / 2u; pr += 32) {
+        rng.seek(pr, 0u);
+        for (int h = 0; h < 2 && 2 * (long long)pr + h < n; ++h) {
+            const double u = rng.uniform();
+            int lo = 0, hi = K - 1;
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (cdf[mid] <= u) lo = mid + 1;
+                else hi = mid;
+            }
+            atomicAdd(&cv[lo], 1);
+        }
+    }
+    __syncwarp();
+    const int D = warp_compact(K, [&](int j) { return cv[j]; }, [&](int j) { return (double)v[j]; }, xv, cv);
+    rng.seek(0u, 1u);
+    double m[ALL_MAX_ALLELES], w[ALL_MAX_ALLELES], s[ALL_MAX_ALLELES];
+    int peaks;
+    fit_replicate_warp(xv, cv, D, n, A, P, rng, nullptr, nullptr, m, w, s, &peaks);
+    if (lane == 0) {
+        const size_t ll = (size_t)(l - l0);
+        for (int a = 0; a < A; ++a) {
+            const size_t o = (ll * S + a) * B + b;
+            rep_m[o] = m[a], rep_w[o] = w[a], rep_s[o] = s[a];
+        }
+        rep_peaks[ll * B + b] = (unsigned char)peaks;
+    }
+}
+
+// gmm_fit_counts_ploidy_kernel through the warp fit, for any K up to kcap <= ALL_DEEP_MAX_K: one warp per problem,
+// its nonzero (value, count) pairs in shared memory ([warp][kcap] values, then [warp][kcap] counts); the stream of
+// problem q is (seed, q, ALL_DEEP_STREAM) from counter (0, 1), as a deep replicate's fit
+__global__ void __launch_bounds__(32 * ALL_DEEP_WARPS)
+gmm_fit_counts_deep_kernel(const double *__restrict__ xs, const int *__restrict__ cs, const int *__restrict__ Ks,
+                           const int *__restrict__ As, const int *__restrict__ init,
+                           const long long *__restrict__ init_off, int n_problems, int kcap, int S, AlleleParams P,
+                           double *__restrict__ out) {
+    extern __shared__ double smem_deep_fit[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int q = blockIdx.x * ALL_DEEP_WARPS + warp;
+    if (q >= n_problems) return;
+    double *xv = smem_deep_fit + (size_t)kcap * warp;
+    int *cv = (int *)(smem_deep_fit + (size_t)kcap * ALL_DEEP_WARPS) + (size_t)kcap * warp;
+    const double *x = xs + (size_t)q * kcap;
+    const int *c = cs + (size_t)q * kcap;
+    const int D = warp_compact(Ks[q], [&](int j) { return c[j]; }, [&](int j) { return x[j]; }, xv, cv);
+    int n = 0;
+    for (int j = lane; j < D; j += 32) n += cv[j];
+    n = __reduce_add_sync(0xffffffffu, n);
+    Philox rng;
+    rng.init(P.seed, (uint32_t)q, ALL_DEEP_STREAM);
+    rng.seek(0u, 1u);
+    double m[ALL_MAX_ALLELES], w[ALL_MAX_ALLELES], s[ALL_MAX_ALLELES];
+    int peaks = 0;
+    const int A = As[q];
+    fit_replicate_warp(xv, cv, D, n, A, P, rng, init ? init + init_off[q] : nullptr, x, m, w, s, &peaks);
+    if (lane == 0) {
+        double *o = out + (size_t)q * (3 * S + 1);
+        for (int a = 0; a < S; ++a) {
+            o[a] = a < A ? m[a] : 0.0;
+            o[S + a] = a < A ? w[a] : 0.0;
+            o[2 * S + a] = a < A ? s[a] : 0.0;
+        }
+        o[3 * S] = (double)peaks;
+    }
 }
 
 // ---------------------------------------------------------------------------------------------- aggregate

@@ -31,13 +31,14 @@ static int alleles_params(AlleleParams *P, int n_alleles, bool per_locus, int nu
     return STRK_OK;
 }
 
-// the aggregation's dynamic shared memory (sort keys) plus its static array must fit the launch: 4096 replicates
-// take 48 KB of keys, so above 48 KB in all the kernel opts in to the larger carve-out
-static cudaError_t agg_smem_opt_in(size_t dyn) {
+// a kernel's dynamic shared memory plus its static arrays must fit the launch: above 48 KB in all the kernel opts in
+// to the larger carve-out (the aggregation's sort keys take 48 KB at 4096 replicates; the deep kernels' tables)
+template <class Kernel>
+static cudaError_t smem_opt_in(Kernel kernel, size_t dyn) {
     cudaFuncAttributes fa;
-    cudaError_t e = cudaFuncGetAttributes(&fa, alleles_aggregate_kernel);
+    cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
     if (e == cudaSuccess && dyn + fa.sharedSizeBytes > 48 * 1024)
-        e = cudaFuncSetAttribute(alleles_aggregate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     return e;
 }
 
@@ -88,15 +89,23 @@ static int call_alleles_impl(const char *fn, strk_ctx *ctx, const int32_t *cn, c
     const int64_t n_reads = read_begin[n_loci];
     if (read_begin[0] != 0 || n_reads < 0 || (n_reads && (!cn || !weights)))
         return set_err(STRK_ERR_ARG, "%s: read_begin must run from 0 to the number of reads", fn);
+    // shallow loci (<= ALL_SHALLOW_READS reads) set the stride of the per-locus arrays; deep ones are listed with
+    // ragged offsets of min(reads, ALL_DEEP_MAX_K) entries
     int max_n = 1;
+    std::vector<int> deep;
+    std::vector<long long> doff(1, 0);
     for (int64_t l = 0; l < n_loci; ++l) {
         const int64_t d = read_begin[l + 1] - read_begin[l];
         if (d < 0) return set_err(STRK_ERR_ARG, "%s: locus %lld has a non-monotone read_begin", fn, (long long)l);
-        if (d > 256)
-            return set_err(STRK_ERR_UNSUPPORTED, "%s: locus %lld has %lld reads (limit 256; the reference "
-                                                 "caps at max_reads = 250)", fn, (long long)l, (long long)d);
-        if (d > max_n) max_n = (int)d;
+        if (d > 0x7fffffffLL) return set_err(STRK_ERR_UNSUPPORTED, "%s: locus %lld has %lld reads", fn, (long long)l, (long long)d);
+        if (d > ALL_SHALLOW_READS) {
+            deep.push_back((int)l);
+            doff.push_back(doff.back() + std::min<int64_t>(d, ALL_DEEP_MAX_K));
+        } else if (d > max_n) {
+            max_n = (int)d;
+        }
     }
+    const int n_deep = (int)deep.size();
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const int kcap = max_n, B = num_bootstrap;
@@ -116,13 +125,20 @@ static int call_alleles_impl(const char *fn, strk_ctx *ctx, const int32_t *cn, c
     int *d_A = A_loc ? take_i(8, (size_t)n_loci) : nullptr;
     double *d_w = take_d(0, (size_t)n_reads), *d_cdf = take_d(1, (size_t)n_loci * kcap);
     double *d_od = take_d(2, (size_t)n_loci * 3 * S);
+    int *d_deep = take_i(9, (size_t)n_deep), *d_dvals = take_i(10, (size_t)doff.back()), *d_dK = take_i(11, (size_t)n_deep);
+    double *d_dcdf = take_d(3, (size_t)doff.back());
     if (e == cudaSuccess) e = ctx->al_rb.reserve((size_t)n_loci + 1);
-    long long *d_rb = ctx->al_rb.p;
+    if (e == cudaSuccess) e = ctx->al_doff.reserve((size_t)n_deep + 1);
+    long long *d_rb = ctx->al_rb.p, *d_doff = ctx->al_doff.p;
     if (e == cudaSuccess && n_reads) e = cudaMemcpyAsync(d_cn, cn, (size_t)n_reads * sizeof(int), cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess && n_reads) e = cudaMemcpyAsync(d_w, weights, (size_t)n_reads * sizeof(double), cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(d_rb, read_begin, ((size_t)n_loci + 1) * sizeof(long long), cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess && d_A) e = cudaMemcpyAsync(d_A, A_loc, (size_t)n_loci * sizeof(int), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n_deep)
+        e = cudaMemcpyAsync(d_deep, deep.data(), (size_t)n_deep * sizeof(int), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n_deep)
+        e = cudaMemcpyAsync(d_doff, doff.data(), ((size_t)n_deep + 1) * sizeof(long long), cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "%s: %s", fn, cudaGetErrorString(e));
@@ -135,9 +151,23 @@ static int call_alleles_impl(const char *fn, strk_ctx *ctx, const int32_t *cn, c
                                                                              kcap, d_vals, d_cdf, d_cnt, d_K, d_n,
                                                                              d_status, d_kmax);
     CU(cudaGetLastError());
+    std::vector<int> deep_K((size_t)n_deep);
+    if (n_deep) {
+        const size_t prep_smem = ALL_DEEP_TABLE * sizeof(unsigned long long) + ALL_DEEP_MAX_K * sizeof(int);
+        CU(smem_opt_in(alleles_deep_prepare_kernel, prep_smem));
+        alleles_deep_prepare_kernel<<<(unsigned)n_deep, 256, prep_smem, st>>>(d_cn, d_w, d_rb, d_deep, d_doff, min_reads,
+                                                                             kcap, d_dvals, d_dcdf, d_K, d_dK, d_status,
+                                                                             d_vals);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(deep_K.data(), d_dK, (size_t)n_deep * sizeof(int), cudaMemcpyDeviceToHost, st));
+    }
     int kmax = 0;
     CU(cudaMemcpyAsync(&kmax, d_kmax, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
+    for (int d = 0; d < n_deep; ++d)
+        if (deep_K[d] > ALL_DEEP_MAX_K)
+            return set_err(STRK_ERR_UNSUPPORTED, "%s: locus %d has more than %d distinct copy numbers", fn, deep[d],
+                           ALL_DEEP_MAX_K);
     // replicate estimates, in chunks of loci that keep the scratch near 256 MB (context-owned, recycled across calls)
     const size_t per_locus = (size_t)S * B * 3 * sizeof(double) + (size_t)B;
     int64_t chunk = (int64_t)((size_t)1 << 28) / (int64_t)per_locus;
@@ -154,7 +184,7 @@ static int call_alleles_impl(const char *fn, strk_ctx *ctx, const int32_t *cn, c
     int np2 = 1;
     while (np2 < B) np2 <<= 1;
     const size_t agg_smem = (size_t)np2 * (sizeof(double) + sizeof(int));
-    CU(agg_smem_opt_in(agg_smem));
+    CU(smem_opt_in(alleles_aggregate_kernel, agg_smem));
     for (int64_t l0 = 0; l0 < n_loci; l0 += chunk) {
         const int nl = (int)std::min<int64_t>(chunk, n_loci - l0);
         const int *v = d_vals + (size_t)l0 * kcap, *c = d_cnt + (size_t)l0 * kcap;
@@ -168,6 +198,19 @@ static int call_alleles_impl(const char *fn, strk_ctx *ctx, const int32_t *cn, c
             launch_fit_k<ALL_MAX_ALLELES>(kmax, v, p, c, d_K + l0, d_n + l0, d_status + l0, a, nl, kcap, S, Pc, rm, rw,
                                           rs, rp, st);
         CU(cudaGetLastError());
+        const int d0 = (int)(std::lower_bound(deep.begin(), deep.end(), (int)l0) - deep.begin());
+        const int d1 = (int)(std::lower_bound(deep.begin(), deep.end(), (int)(l0 + nl)) - deep.begin());
+        if (d1 > d0) {
+            // every (deep locus, replicate) a warp; shared memory sized by the chunk's largest deep K
+            const int kd = *std::max_element(deep_K.begin() + d0, deep_K.begin() + d1);
+            const size_t fit_smem = (size_t)kd * (sizeof(double) * (1 + ALL_DEEP_WARPS) + sizeof(int) * ALL_DEEP_WARPS);
+            CU(smem_opt_in(alleles_deep_fit_kernel, fit_smem));
+            const dim3 grid((unsigned)(d1 - d0), (unsigned)((B + ALL_DEEP_WARPS - 1) / ALL_DEEP_WARPS));
+            alleles_deep_fit_kernel<<<grid, 32 * ALL_DEEP_WARPS, fit_smem, st>>>(d_deep + d0, d_doff + d0, d_dvals, d_dcdf,
+                                                                               d_K, d_n, d_status, d_A, (int)l0, S, P,
+                                                                               rm, rw, rs, rp);
+            CU(cudaGetLastError());
+        }
         alleles_aggregate_kernel<<<(unsigned)nl, 256, agg_smem, st>>>(rm, rw, rs, rp, d_status + l0, v, kcap, nl, a, S, B,
                                                                       d_oi + (size_t)l0 * (1 + 5 * S),
                                                                       d_od + (size_t)l0 * 3 * S);
@@ -247,14 +290,15 @@ extern "C" int strk_gmm_fit_counts(strk_ctx *ctx, const double *x, const int32_t
     return STRK_OK;
 }
 
-extern "C" int strk_gmm_fit_counts_ploidy(strk_ctx *ctx, const double *x, const int32_t *counts, const int32_t *K,
-                                          const int32_t *n_alleles, const int32_t *init, int64_t n_problems, int kcap,
-                                          int num_bootstrap, int min_allele_reads, int force_gm_filter,
-                                          double expansion_ratio, int filter_factor, int n_init, uint64_t seed,
-                                          double *out) {
-    const char *fn = "strk_gmm_fit_counts_ploidy";
+// strk_gmm_fit_counts_ploidy (per-thread fit, kcap <= 256) and strk_gmm_fit_counts_deep (warp fit of deep loci,
+// kcap <= ALL_DEEP_MAX_K): the same arguments, checks and output
+static int gmm_fit_counts_impl(const char *fn, bool deep, strk_ctx *ctx, const double *x, const int32_t *counts,
+                               const int32_t *K, const int32_t *n_alleles, const int32_t *init, int64_t n_problems,
+                               int kcap, int num_bootstrap, int min_allele_reads, int force_gm_filter,
+                               double expansion_ratio, int filter_factor, int n_init, uint64_t seed, double *out) {
     if (!ctx || !x || !counts || !K || !n_alleles || !out) return set_err(STRK_ERR_ARG, "%s: null argument", fn);
-    if (n_problems < 0 || n_problems > 0x7fffffff || kcap < 1 || kcap > 256) return set_err(STRK_ERR_ARG, "%s: bad sizes", fn);
+    if (n_problems < 0 || n_problems > 0x7fffffff || kcap < 1 || kcap > (deep ? ALL_DEEP_MAX_K : 256))
+        return set_err(STRK_ERR_ARG, "%s: bad sizes", fn);
     AlleleParams P;
     int rc = alleles_params(&P, 0, true, num_bootstrap, 0, min_allele_reads, force_gm_filter, expansion_ratio,
                             filter_factor, n_init, seed);
@@ -303,20 +347,47 @@ extern "C" int strk_gmm_fit_counts_ploidy(strk_ctx *ctx, const double *x, const 
         cudaGetLastError();
         return set_err(STRK_ERR_NOMEM, "%s: %s", fn, cudaGetErrorString(e));
     }
-    const unsigned grid = (unsigned)((n_problems + 127) / 128);
-    if (kcap <= 8)
-        gmm_fit_counts_ploidy_kernel<8><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap, S,
-                                                              P, d_out);
-    else if (kcap <= 32)
-        gmm_fit_counts_ploidy_kernel<32><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap, S,
-                                                               P, d_out);
-    else
-        gmm_fit_counts_ploidy_kernel<256><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap,
-                                                                S, P, d_out);
+    if (deep) {
+        const size_t smem = (size_t)kcap * (sizeof(double) + sizeof(int)) * ALL_DEEP_WARPS;
+        CU(smem_opt_in(gmm_fit_counts_deep_kernel, smem));
+        gmm_fit_counts_deep_kernel<<<(unsigned)((n_problems + ALL_DEEP_WARPS - 1) / ALL_DEEP_WARPS), 32 * ALL_DEEP_WARPS,
+                                     smem, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap, S, P, d_out);
+    } else {
+        const unsigned grid = (unsigned)((n_problems + 127) / 128);
+        if (kcap <= 8)
+            gmm_fit_counts_ploidy_kernel<8><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap,
+                                                                  S, P, d_out);
+        else if (kcap <= 32)
+            gmm_fit_counts_ploidy_kernel<32><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap,
+                                                                   S, P, d_out);
+        else
+            gmm_fit_counts_ploidy_kernel<256><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems,
+                                                                    kcap, S, P, d_out);
+    }
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, d_out, (size_t)n_problems * (3 * S + 1) * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return STRK_OK;
+}
+
+extern "C" int strk_gmm_fit_counts_ploidy(strk_ctx *ctx, const double *x, const int32_t *counts, const int32_t *K,
+                                          const int32_t *n_alleles, const int32_t *init, int64_t n_problems, int kcap,
+                                          int num_bootstrap, int min_allele_reads, int force_gm_filter,
+                                          double expansion_ratio, int filter_factor, int n_init, uint64_t seed,
+                                          double *out) {
+    return gmm_fit_counts_impl("strk_gmm_fit_counts_ploidy", false, ctx, x, counts, K, n_alleles, init, n_problems, kcap,
+                               num_bootstrap, min_allele_reads, force_gm_filter, expansion_ratio, filter_factor, n_init,
+                               seed, out);
+}
+
+extern "C" int strk_gmm_fit_counts_deep(strk_ctx *ctx, const double *x, const int32_t *counts, const int32_t *K,
+                                        const int32_t *n_alleles, const int32_t *init, int64_t n_problems, int kcap,
+                                        int num_bootstrap, int min_allele_reads, int force_gm_filter,
+                                        double expansion_ratio, int filter_factor, int n_init, uint64_t seed,
+                                        double *out) {
+    return gmm_fit_counts_impl("strk_gmm_fit_counts_deep", true, ctx, x, counts, K, n_alleles, init, n_problems, kcap,
+                               num_bootstrap, min_allele_reads, force_gm_filter, expansion_ratio, filter_factor, n_init,
+                               seed, out);
 }
 
 extern "C" int strk_alleles_aggregate(strk_ctx *ctx, const double *rep_means, const double *rep_weights,
@@ -351,7 +422,7 @@ extern "C" int strk_alleles_aggregate(strk_ctx *ctx, const double *rep_means, co
     int np2 = 1;
     while (np2 < B) np2 <<= 1;
     const size_t agg_smem = (size_t)np2 * (sizeof(double) + sizeof(int));
-    CU(agg_smem_opt_in(agg_smem));
+    CU(smem_opt_in(alleles_aggregate_kernel, agg_smem));
     alleles_aggregate_kernel<<<(unsigned)n_loci, 256, agg_smem, st>>>(rm, rw, rs, rp, d_status, nullptr, 1, (int)n_loci,
                                                                       nullptr, A, B, d_oi, d_od);
     CU(cudaGetLastError());

@@ -203,9 +203,10 @@ struct strk_ctx {
     // reference path (strk_ref_counts): per-locus state, and the one-read-per-locus batch of phase 2
     RefBufs ref;
     struct strk_batch *ref_batch = nullptr;
-    DevBuf<int> al_i[9];             //                 per-read / per-locus integer arrays (recycled across calls)
-    DevBuf<double> al_d[3];
+    DevBuf<int> al_i[12];            //                 per-read / per-locus integer arrays (recycled across calls)
+    DevBuf<double> al_d[4];
     DevBuf<long long> al_rb;
+    DevBuf<long long> al_doff;       //                 offsets of the deep loci's ragged values / CDF
     unsigned int *d_queue = nullptr;  // counter words (CounterSlot)
     unsigned int *counter(int slot) const { return d_queue + slot; }
     double *d_acc = nullptr;          // [0] ref cells, [1] executed cells
@@ -415,9 +416,10 @@ extern "C" int strk_destroy(strk_ctx *ctx) {
     ctx->pk_scratch.release();
     for (int k = 0; k < 3; ++k) ctx->al_rep[k].release();
     ctx->al_peaks.release();
-    for (int k = 0; k < 9; ++k) ctx->al_i[k].release();
-    for (int k = 0; k < 3; ++k) ctx->al_d[k].release();
+    for (int k = 0; k < 12; ++k) ctx->al_i[k].release();
+    for (int k = 0; k < 4; ++k) ctx->al_d[k].release();
     ctx->al_rb.release();
+    ctx->al_doff.release();
     if (ctx->d_consts) cudaFree(ctx->d_consts);
     if (ctx->d_queue) cudaFree(ctx->d_queue);
     if (ctx->d_acc) cudaFree(ctx->d_acc);
