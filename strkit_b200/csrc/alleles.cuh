@@ -358,25 +358,172 @@ __device__ void fit_replicate(const double *x, const int *c, int K, int n, int A
 
 // ---------------------------------------------------------------------------------------------- k components
 // fit_gmm for A >= 3 components (allele.py:56-123 over GaussianMixture(n_components = k)); the two-component code
-// above stays the path of A <= 2, so those results do not depend on this one.
+// above stays the path of A <= 2 on shallow loci, so those results do not depend on this one.
+//
+// The fit runs on the D nonzero (value, count) pairs of a replicate, by a team of W threads: W = 1 is one thread
+// (shallow loci, the pairs in its own arrays), W = 32 one warp (deep loci, the pairs in shared memory).  Lane i of a
+// team visits pairs i, i + W, ...; every sum over them is a lane partial sum followed by a butterfly (xor) reduction,
+// which leaves the bitwise same total in every lane, so all lanes carry the same model, the same random state and
+// take the same branches.  At W = 1 every sum runs in pair order.
 struct GmmK {
     double mean[ALL_MAX_ALLELES], cov[ALL_MAX_ALLELES], weight[ALL_MAX_ALLELES];
     int n_comp;
 };
 
-// EM from the seed value indices idx[0..NC): gmm_em with NC components, the same separately rounded products, the
-// same init (one-hot responsibilities on the seed points + 10 eps: two components seeded on one point stay equal),
-// a NC-way log-sum-exp and the same convergence rule.  NC is a template so the component arrays stay in registers.
-template <int NC, int KMAX>
-__device__ double gmm_em_k(const double *x, const int *c, int K, int n, const int *idx, const AlleleParams &P,
+template <int W>
+__device__ __forceinline__ int team_lane() {
+    static_assert(W == 1 || W == 32, "a team is one thread or one warp");
+    return W == 1 ? 0 : (int)(threadIdx.x & 31);
+}
+
+template <int W>
+__device__ __forceinline__ double team_sum(double v) {
+#pragma unroll
+    for (int o = W / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// searchsorted over the cumulative sum of term(0..D): the first j whose inclusive prefix sum is >= r (> r with
+// `strict`), D - 1 if none.  A warp takes 32 terms at a time: a shuffle-up scan plus the carry of the chunks before.
+template <int W, class T, class Term>
+__device__ __forceinline__ int team_search(int D, T r, bool strict, Term term) {
+    if constexpr (W == 1) {
+        T s = 0;
+        for (int j = 0; j < D; ++j) {
+            s += term(j);
+            if (strict ? s > r : s >= r) return j;
+        }
+    } else {
+        const int lane = team_lane<W>();
+        T carry = 0;
+        for (int j0 = 0; j0 < D; j0 += 32) {
+            const int j = j0 + lane;
+            T s = j < D ? term(j) : (T)0;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const T t = __shfl_up_sync(0xffffffffu, s, o);
+                if (lane >= o) s += t;
+            }
+            s += carry;
+            const unsigned hit = __ballot_sync(0xffffffffu, j < D && (strict ? s > r : s >= r));
+            if (hit) return j0 + __ffs(hit) - 1;
+            carry = __shfl_sync(0xffffffffu, s, 31);
+        }
+    }
+    return D - 1;
+}
+
+// the nonzero counts cnt(0..K) with their values val(j), in ascending j, to cv[0..D) / xv[0..D); returns D.
+// cv may be the array cnt reads (a warp reads every entry of a chunk before any lane writes, and writes land at or
+// below the chunk); one thread may also compact val's array in place.
+template <int W, class Cnt, class Val>
+__device__ __forceinline__ int team_compact(int K, Cnt cnt, Val val, double *xv, int *cv) {
+    int D = 0;
+    if constexpr (W == 1) {
+        for (int j = 0; j < K; ++j) {
+            const int c = cnt(j);
+            if (c) cv[D] = c, xv[D] = val(j), ++D;
+        }
+    } else {
+        const int lane = team_lane<W>();
+        for (int j0 = 0; j0 < K; j0 += 32) {
+            const int j = j0 + lane;
+            const int c = j < K ? cnt(j) : 0;
+            const unsigned nz = __ballot_sync(0xffffffffu, c != 0);
+            __syncwarp();
+            if (c) {
+                const int q = D + __popc(nz & ((1u << lane) - 1u));
+                cv[q] = c;
+                xv[q] = val(j);
+            }
+            D += __popc(nz);
+        }
+        __syncwarp();
+    }
+    return D;
+}
+
+// closest squared distance of x to the first nce centres (fmin is exact, so the order of the centres does not matter)
+__device__ __forceinline__ double closest_sq(double x, const double *cen, int nce) {
+    double d = x - cen[0], cl = d * d;
+#pragma unroll
+    for (int i = 1; i < ALL_MAX_ALLELES; ++i)
+        if (i < nce) d = x - cen[i], cl = fmin(cl, d * d);
+    return cl;
+}
+
+// sklearn _kmeans_plusplus (cluster/_kmeans.py:224-275) for k centres on the D nonzero pairs: the first centre uniform
+// over the n points; each further centre the best (first argmin of the potential) of 2 + int(log k) candidates drawn
+// by searchsorted(cumsum(count * closest_dist_sq), u * pot, side="left"), clipped to the last pair.  When every point
+// already sits on a centre (pot = 0) every draw lands on pair 0, the smallest value, and that centre is duplicated --
+// as scikit-learn does.  The centres' values go to cen[0..k).  closest_dist_sq: one thread keeps it per pair in cl,
+// updated once per centre (a thread has at most KMAX <= 256 pairs); a warp, whose pairs can be 4096, recomputes it
+// from the centres.  Both give the same value.
+template <int W>
+__device__ void kmeanspp(const double *xv, const int *cv, int D, int n, int k, Philox &rng, double *cen) {
+    const int lane = team_lane<W>();
+    double cl_pair[W == 1 ? 256 : 1], *cl = cl_pair;  // read through a pointer: nvcc takes the lambda's read for one
+                                                      // before any write
+    const auto closest = [&](int j, int nce) {
+        if constexpr (W == 1)
+            return cl[j];
+        else
+            return closest_sq(xv[j], cen, nce);
+    };
+    {
+        const double u = rng.uniform();
+        long long pt = (long long)(u * (double)n);
+        if (pt >= n) pt = n - 1;
+        cen[0] = xv[team_search<W, long long>(D, pt, true, [&](int j) { return (long long)cv[j]; })];
+    }
+    double pot = 0.0;
+    for (int j = lane; j < D; j += W) {
+        const double d = xv[j] - cen[0];
+        if constexpr (W == 1) cl[j] = d * d;
+        pot += (double)cv[j] * closest(j, 1);
+    }
+    pot = team_sum<W>(pot);
+    const int trials = 2 + (int)log((double)k);
+    for (int ci = 1; ci < k; ++ci) {
+        double best_pot = INFINITY;
+        int best = 0;
+#pragma unroll 1
+        for (int t = 0; t < trials; ++t) {
+            const double r = rng.uniform() * pot;
+            const int cand = team_search<W, double>(D, r, false, [&](int j) { return (double)cv[j] * closest(j, ci); });
+            double cp = 0.0;
+            for (int j = lane; j < D; j += W) {
+                const double d = xv[j] - xv[cand];
+                cp += (double)cv[j] * fmin(closest(j, ci), d * d);
+            }
+            cp = team_sum<W>(cp);
+            if (cp < best_pot) best_pot = cp, best = cand;
+        }
+        cen[ci] = xv[best];
+        pot = best_pot;
+        if constexpr (W == 1)
+            for (int j = 0; j < D; ++j) {
+                const double d = xv[j] - cen[ci];
+                cl[j] = fmin(cl[j], d * d);
+            }
+    }
+}
+
+// EM from the seed values cen[0..NC) on the D nonzero pairs: gmm_em with NC components, the same separately rounded
+// products, the same init (one-hot responsibilities on the seed points + 10 eps: two components seeded on one point
+// stay equal), a NC-way log-sum-exp and the same convergence rule.  NC is a template so the component arrays stay in
+// registers.
+template <int NC, int W>
+__device__ double gmm_em_k(const double *xv, const int *cv, int D, int n, const double *cen, const AlleleParams &P,
                            GmmK &g) {
+    const int lane = team_lane<W>();
     const double eps10 = 10.0 * 2.220446049250313e-16;
     double mean[NC], cov[NC], weight[NC], pchol[NC], logw[NC];
 #pragma unroll
     for (int k = 0; k < NC; ++k) {
-        const double nk = 1.0 + eps10, xv = x[idx[k]];
-        mean[k] = xv / nk;
-        cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(__dmul_rn(xv, xv), nk), __dmul_rn(mean[k], mean[k])), P.reg_covar);
+        const double nk = 1.0 + eps10, xk = cen[k];
+        mean[k] = xk / nk;
+        cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(__dmul_rn(xk, xk), nk), __dmul_rn(mean[k], mean[k])), P.reg_covar);
         weight[k] = nk / (double)n;
         pchol[k] = 1.0 / sqrt(cov[k]);
         logw[k] = log(weight[k]);
@@ -387,11 +534,11 @@ __device__ double gmm_em_k(const double *x, const int *c, int K, int n, const in
         double nk[NC], sx[NC], sxx[NC], ll = 0.0;
 #pragma unroll
         for (int k = 0; k < NC; ++k) nk[k] = 0.0, sx[k] = 0.0, sxx[k] = 0.0;
-        for (int v = 0; v < K; ++v) {
-            if (c[v] == 0) continue;
+        for (int j = lane; j < D; j += W) {
+            const double x = xv[j];
             double wl[NC];
 #pragma unroll
-            for (int k = 0; k < NC; ++k) wl[k] = gmm_wlp1(x[v], mean[k], pchol[k], logw[k]);
+            for (int k = 0; k < NC; ++k) wl[k] = gmm_wlp1(x, mean[k], pchol[k], logw[k]);
             double mx = wl[0];
 #pragma unroll
             for (int k = 1; k < NC; ++k) mx = fmax(mx, wl[k]);
@@ -399,16 +546,20 @@ __device__ double gmm_em_k(const double *x, const int *c, int K, int n, const in
 #pragma unroll
             for (int k = 0; k < NC; ++k) se += exp(wl[k] - mx);
             const double lse = mx + log(se);
-            const double cv = (double)c[v];
-            ll += cv * lse;
+            const double c = (double)cv[j];
+            ll += c * lse;
 #pragma unroll
             for (int k = 0; k < NC; ++k) {
-                const double r = exp(wl[k] - lse) * cv;
+                const double r = exp(wl[k] - lse) * c;
                 nk[k] += r;
-                sx[k] += r * x[v];
-                sxx[k] += r * x[v] * x[v];
+                sx[k] += r * x;
+                sxx[k] += r * x * x;
             }
         }
+        ll = team_sum<W>(ll);
+#pragma unroll
+        for (int k = 0; k < NC; ++k)
+            nk[k] = team_sum<W>(nk[k]), sx[k] = team_sum<W>(sx[k]), sxx[k] = team_sum<W>(sxx[k]);
         lower = ll / (double)n;
         double wsum = 0.0;
 #pragma unroll
@@ -433,85 +584,29 @@ __device__ double gmm_em_k(const double *x, const int *c, int K, int n, const in
     return lower;
 }
 
-// sklearn _kmeans_plusplus (cluster/_kmeans.py:224-275) for k centres on the (value, count) pairs of a replicate:
-// the first centre uniform over the n points; each further centre the best (first argmin of the potential) of
-// 2 + int(log k) candidates drawn by searchsorted(cumsum(count * closest_dist_sq), u * pot, side="left"), clipped
-// to the last point.  When every point already sits on a centre (pot = 0) every draw lands on point 0, the smallest
-// value, and that centre is duplicated -- as scikit-learn does.
-template <int KMAX>
-__device__ void kmeanspp_k(const double *x, const int *c, int K, int n, int k, Philox &rng, int *idx) {
-    {
-        const double u = rng.uniform();
-        long long pt = (long long)(u * (double)n);
-        if (pt >= n) pt = n - 1;
-        int v = 0;
-        long long acc = 0;
-        for (; v < K; ++v) {
-            acc += c[v];
-            if (pt < acc) break;
-        }
-        idx[0] = v < K ? v : K - 1;
-    }
-    double closest[KMAX];
-    double pot = 0.0;
-    for (int v = 0; v < K; ++v) {
-        const double d = x[v] - x[idx[0]];
-        closest[v] = d * d;
-        pot += (double)c[v] * closest[v];
-    }
-    const int trials = 2 + (int)log((double)k);
-    for (int ci = 1; ci < k; ++ci) {
-        double best_pot = INFINITY;
-        int best = 0;
-#pragma unroll 1
-        for (int t = 0; t < trials; ++t) {
-            const double r = rng.uniform() * pot;
-            int v = 0, last_nonzero = 0;
-            double acc = 0.0;
-            for (; v < K; ++v) {
-                if (c[v]) last_nonzero = v;
-                acc += (double)c[v] * closest[v];
-                if (c[v] && acc >= r) break;
-            }
-            const int cand = v < K ? v : last_nonzero;
-            double cp = 0.0;
-            for (int q = 0; q < K; ++q) {
-                const double d = x[q] - x[cand];
-                cp += (double)c[q] * fmin(closest[q], d * d);
-            }
-            if (cp < best_pot) best_pot = cp, best = cand;
-        }
-        idx[ci] = best;
-        pot = best_pot;
-        for (int q = 0; q < K; ++q) {
-            const double d = x[q] - x[best];
-            closest[q] = fmin(closest[q], d * d);
-        }
-    }
-}
-
-// GaussianMixture(nc).fit: the best of n_init restarts (forced = n_init rows of nc seed indices, or NULL for k-means++)
-template <int KMAX>
-__device__ void gmm_fit_k(const double *x, const int *c, int K, int n, int nc, const AlleleParams &P, Philox &rng,
-                          const int *forced, GmmK &best) {
+// GaussianMixture(nc).fit: the best of n_init restarts (forced = n_init rows of nc seed indices into x_forced, the
+// caller's value list, or NULL for k-means++)
+template <int W>
+__device__ void gmm_fit_k(const double *xv, const int *cv, int D, int n, int nc, const AlleleParams &P, Philox &rng,
+                          const int *forced, const double *x_forced, GmmK &best) {
     double best_lb = -INFINITY;
     for (int t = 0; t < P.n_init; ++t) {
-        int idx[ALL_MAX_ALLELES];
+        double cen[ALL_MAX_ALLELES];
         if (forced) {
-            for (int j = 0; j < nc; ++j) idx[j] = forced[t * nc + j];
+            for (int j = 0; j < nc; ++j) cen[j] = x_forced[forced[t * nc + j]];
         } else {
-            kmeanspp_k<KMAX>(x, c, K, n, nc, rng, idx);
+            kmeanspp<W>(xv, cv, D, n, nc, rng, cen);
         }
         GmmK g;
         double lb;
         switch (nc) {
-        case 2: lb = gmm_em_k<2, KMAX>(x, c, K, n, idx, P, g); break;
-        case 3: lb = gmm_em_k<3, KMAX>(x, c, K, n, idx, P, g); break;
-        case 4: lb = gmm_em_k<4, KMAX>(x, c, K, n, idx, P, g); break;
-        case 5: lb = gmm_em_k<5, KMAX>(x, c, K, n, idx, P, g); break;
-        case 6: lb = gmm_em_k<6, KMAX>(x, c, K, n, idx, P, g); break;
-        case 7: lb = gmm_em_k<7, KMAX>(x, c, K, n, idx, P, g); break;
-        default: lb = gmm_em_k<8, KMAX>(x, c, K, n, idx, P, g); break;
+        case 2: lb = gmm_em_k<2, W>(xv, cv, D, n, cen, P, g); break;
+        case 3: lb = gmm_em_k<3, W>(xv, cv, D, n, cen, P, g); break;
+        case 4: lb = gmm_em_k<4, W>(xv, cv, D, n, cen, P, g); break;
+        case 5: lb = gmm_em_k<5, W>(xv, cv, D, n, cen, P, g); break;
+        case 6: lb = gmm_em_k<6, W>(xv, cv, D, n, cen, P, g); break;
+        case 7: lb = gmm_em_k<7, W>(xv, cv, D, n, cen, P, g); break;
+        default: lb = gmm_em_k<8, W>(xv, cv, D, n, cen, P, g); break;
         }
         if (lb > best_lb || best_lb == -INFINITY) best_lb = lb, best = g;
     }
@@ -530,12 +625,11 @@ __device__ __forceinline__ int gmm_useless_k(const GmmK &g, int nc, const Allele
     return useless;
 }
 
-// One replicate with A >= 3 alleles (allele.py:56-123,249-293).  fit_gmm's loop: fit with A components, drop the
-// useless count and refit with a fresh restart set, a single Gaussian at 1 component, and at <= 0 components the
-// last fit with all its components.  A replicate with fewer peaks than A gets A - peaks components drawn with
-// probability weight / sum|weight| (Philox stream of the thread), then everything is sorted by mean (stable).
-// *n_peaks = the fitted count, before the fill.  forced_init (NULL = k-means++): for nc = A, A-1, ..., 2, n_init
-// rows of nc seed indices.  The loop and the bookkeeping are shared with the warp-cooperative fit of deep loci:
+// One replicate with A alleles (allele.py:56-123,249-293).  fit_gmm's loop: fit with A components, drop the useless
+// count and refit with a fresh restart set, a single Gaussian at 1 component, and at <= 0 components the last fit with
+// all its components.  A replicate with fewer peaks than A gets A - peaks components drawn with probability
+// weight / sum|weight| (the team's Philox stream), then everything is sorted by mean (stable).  *n_peaks = the fitted
+// count, before the fill.  forced_init (NULL = k-means++): for nc = A, A-1, ..., 2, n_init rows of nc seed indices.
 // fit(nc, forced, g) is GaussianMixture(nc).fit, single(m, var) make_single_gaussian.
 template <class Fit, class Single>
 __device__ __forceinline__ void fit_staged(int distinct, int A, const AlleleParams &P, Philox &rng,
@@ -584,26 +678,47 @@ __device__ __forceinline__ void fit_staged(int distinct, int A, const AllelePara
     }
 }
 
-template <int KMAX>
-__device__ void fit_replicate_k(const double *x, const int *c, int K, int n, int A, const AlleleParams &P, Philox &rng,
-                                const int *forced_init, double *out_m, double *out_w, double *out_s, int *n_peaks) {
-    int distinct = 0;
-    for (int v = 0; v < K; ++v) distinct += c[v] != 0;
+// fit_staged over the D nonzero pairs (xv, cv), forced seed indices into x_forced.  On deep loci this runs for every
+// A, 1..8: for A <= 2 it is the two-component code's result too, since the staged loop at 2 components is
+// fit_replicate (the same k-means++ draws, EM and filter).
+template <int W>
+__device__ void fit_replicate_k(const double *xv, const int *cv, int D, int n, int A, const AlleleParams &P, Philox &rng,
+                                const int *forced_init, const double *x_forced, double *out_m, double *out_w,
+                                double *out_s, int *n_peaks) {
+    const int lane = team_lane<W>();
     fit_staged(
-        distinct, A, P, rng, forced_init,
-        [&](int nc, const int *forced, GmmK &g) { gmm_fit_k<KMAX>(x, c, K, n, nc, P, rng, forced, g); },
-        [&](double &m, double &var) { single_gaussian(x, c, K, n, m, var); }, out_m, out_w, out_s, n_peaks);
+        D, A, P, rng, forced_init,
+        [&](int nc, const int *forced, GmmK &g) { gmm_fit_k<W>(xv, cv, D, n, nc, P, rng, forced, x_forced, g); },
+        [&](double &m, double &var) {  // make_single_gaussian (gmm.py:72-80): mean and population variance
+            double s = 0.0;
+            for (int j = lane; j < D; j += W) s += (double)cv[j] * xv[j];
+            m = team_sum<W>(s) / (double)n;
+            double q = 0.0;
+            for (int j = lane; j < D; j += W) {
+                const double d = xv[j] - m;
+                q += (double)cv[j] * d * d;
+            }
+            var = team_sum<W>(q) / (double)n;
+        },
+        out_m, out_w, out_s, n_peaks);
 }
 
-// one replicate of a locus with A alleles: the two-component code for A <= 2, the k-component one above
+// one replicate of a shallow locus with A alleles: the two-component code for A <= 2; else the thread compacts its
+// K values and counts in place to the nonzero pairs and runs the k-component fit, forced seed indices pointing into
+// x_forced (the uncompacted values)
 template <int KMAX, int AMAX>
-__device__ __forceinline__ void fit_replicate_any(const double *x, const int *c, int K, int n, int A,
-                                                  const AlleleParams &P, Philox &rng, const int *forced_init,
+__device__ __forceinline__ void fit_replicate_any(double *x, int *c, int K, int n, int A, const AlleleParams &P,
+                                                  Philox &rng, const int *forced_init, const double *x_forced,
                                                   double *out_m, double *out_w, double *out_s, int *n_peaks) {
-    if (AMAX <= 2 || A <= 2)
+    if (AMAX <= 2 || A <= 2) {
         fit_replicate<KMAX>(x, c, K, n, A, P, rng, forced_init, out_m, out_w, out_s, n_peaks);
-    else
-        fit_replicate_k<KMAX>(x, c, K, n, A, P, rng, forced_init, out_m, out_w, out_s, n_peaks);
+    } else {
+        // named: CUDA 12.9's front end stops with an internal error when these lambdas are written in the call
+        auto cnt = [&](int j) { return c[j]; };
+        auto val = [&](int j) { return x[j]; };
+        const int D = team_compact<1>(K, cnt, val, x, c);
+        fit_replicate_k<1>(x, c, D, n, A, P, rng, forced_init, x_forced, out_m, out_w, out_s, n_peaks);
+    }
 }
 
 // one thread per (locus, replicate); replicate arrays laid out [locus][allele][replicate] with S allele rows per
@@ -644,7 +759,7 @@ alleles_fit_kernel(const int *__restrict__ vals, const double *__restrict__ cdf,
     }
     double m[AMAX], w[AMAX], s[AMAX];
     int peaks;
-    fit_replicate_any<KMAX, AMAX>(x, c, K, n, A, P, rng, nullptr, m, w, s, &peaks);
+    fit_replicate_any<KMAX, AMAX>(x, c, K, n, A, P, rng, nullptr, nullptr, m, w, s, &peaks);
     for (int a = 0; a < A; ++a) {
         const size_t o = ((size_t)l * S + a) * B + b;
         rep_m[o] = m[a], rep_w[o] = w[a], rep_s[o] = s[a];
@@ -693,7 +808,8 @@ __global__ void gmm_fit_counts_ploidy_kernel(const double *__restrict__ xs, cons
     rng.init(P.seed, (uint32_t)q, 0u);
     double m[ALL_MAX_ALLELES], w[ALL_MAX_ALLELES], s[ALL_MAX_ALLELES];
     int peaks = 0;
-    fit_replicate_any<KMAX, ALL_MAX_ALLELES>(x, c, K, n, A, P, rng, init ? init + init_off[q] : nullptr, m, w, s, &peaks);
+    fit_replicate_any<KMAX, ALL_MAX_ALLELES>(x, c, K, n, A, P, rng, init ? init + init_off[q] : nullptr,
+                                             xs + (size_t)q * kcap, m, w, s, &peaks);
     double *o = out + (size_t)q * (3 * S + 1);
     for (int a = 0; a < S; ++a) {
         o[a] = a < A ? m[a] : 0.0;
@@ -706,225 +822,8 @@ __global__ void gmm_fit_counts_ploidy_kernel(const double *__restrict__ xs, cons
 // ---------------------------------------------------------------------------------------------- deep loci
 // Loci with more than ALL_SHALLOW_READS reads.  K can be as large as the read count, so the per-thread arrays above
 // do not scale to them: one CTA per deep locus builds its distinct values and CDF in ragged storage, and one warp
-// per (locus, replicate) resamples and fits.  A replicate is held as its D nonzero (value, count) pairs in shared
-// memory; every sum over them is a lane-strided partial sum followed by a butterfly (xor) reduction, which leaves
-// the bitwise same total in every lane, so all lanes carry the same model, the same random state and take the same
-// branches.  Given the seeds, the arithmetic per pair is gmm_em_k's; only the order of the sums differs.
-
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
-// searchsorted over the cumulative sum of term(0..D): the first j whose inclusive prefix sum is >= r (> r with
-// `strict`), D - 1 if none.  32 terms at a time: a shuffle-up scan plus the carry of the chunks before.
-template <class T, class Term>
-__device__ __forceinline__ int warp_search(int D, T r, bool strict, Term term) {
-    const int lane = threadIdx.x & 31;
-    T carry = 0;
-    for (int j0 = 0; j0 < D; j0 += 32) {
-        const int j = j0 + lane;
-        T s = j < D ? term(j) : (T)0;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const T t = __shfl_up_sync(0xffffffffu, s, o);
-            if (lane >= o) s += t;
-        }
-        s += carry;
-        const unsigned hit = __ballot_sync(0xffffffffu, j < D && (strict ? s > r : s >= r));
-        if (hit) return j0 + __ffs(hit) - 1;
-        carry = __shfl_sync(0xffffffffu, s, 31);
-    }
-    return D - 1;
-}
-
-// the nonzero counts cnt(0..K) with their values val(j), in ascending j, to cv[0..D) / xv[0..D); returns D.
-// cv may be the array cnt reads (every lane reads its entry of a chunk before any lane writes, and writes land at
-// or below the chunk).
-template <class Cnt, class Val>
-__device__ __forceinline__ int warp_compact(int K, Cnt cnt, Val val, double *xv, int *cv) {
-    const int lane = threadIdx.x & 31;
-    int D = 0;
-    for (int j0 = 0; j0 < K; j0 += 32) {
-        const int j = j0 + lane;
-        const int c = j < K ? cnt(j) : 0;
-        const unsigned nz = __ballot_sync(0xffffffffu, c != 0);
-        __syncwarp();
-        if (c) {
-            const int q = D + __popc(nz & ((1u << lane) - 1u));
-            cv[q] = c;
-            xv[q] = val(j);
-        }
-        D += __popc(nz);
-    }
-    __syncwarp();
-    return D;
-}
-
-// closest squared distance of x to the first nce centres (kmeanspp_k's running fmin, recomputed)
-__device__ __forceinline__ double closest_sq(double x, const double *cen, int nce) {
-    double d = x - cen[0], cl = d * d;
-#pragma unroll
-    for (int i = 1; i < ALL_MAX_ALLELES; ++i)
-        if (i < nce) d = x - cen[i], cl = fmin(cl, d * d);
-    return cl;
-}
-
-// kmeanspp_k on D nonzero pairs, warp-cooperative: the centres' values to cen[0..k)
-__device__ void kmeanspp_warp(const double *xv, const int *cv, int D, int n, int k, Philox &rng, double *cen) {
-    const int lane = threadIdx.x & 31;
-    {
-        const double u = rng.uniform();
-        long long pt = (long long)(u * (double)n);
-        if (pt >= n) pt = n - 1;
-        cen[0] = xv[warp_search<long long>(D, pt, true, [&](int j) { return (long long)cv[j]; })];
-    }
-    double pot = 0.0;
-    for (int j = lane; j < D; j += 32) pot += (double)cv[j] * closest_sq(xv[j], cen, 1);
-    pot = warp_sum(pot);
-    const int trials = 2 + (int)log((double)k);
-    for (int ci = 1; ci < k; ++ci) {
-        double best_pot = INFINITY;
-        int best = 0;
-#pragma unroll 1
-        for (int t = 0; t < trials; ++t) {
-            const double r = rng.uniform() * pot;
-            const int cand = warp_search<double>(D, r, false,
-                                                 [&](int j) { return (double)cv[j] * closest_sq(xv[j], cen, ci); });
-            double cp = 0.0;
-            for (int j = lane; j < D; j += 32) {
-                const double d = xv[j] - xv[cand];
-                cp += (double)cv[j] * fmin(closest_sq(xv[j], cen, ci), d * d);
-            }
-            cp = warp_sum(cp);
-            if (cp < best_pot) best_pot = cp, best = cand;
-        }
-        cen[ci] = xv[best];
-        pot = best_pot;
-    }
-}
-
-// gmm_em_k from the seed values cen[0..NC) on D nonzero pairs, warp-cooperative
-template <int NC>
-__device__ double gmm_em_warp(const double *xv, const int *cv, int D, int n, const double *cen, const AlleleParams &P,
-                              GmmK &g) {
-    const int lane = threadIdx.x & 31;
-    const double eps10 = 10.0 * 2.220446049250313e-16;
-    double mean[NC], cov[NC], weight[NC], pchol[NC], logw[NC];
-#pragma unroll
-    for (int k = 0; k < NC; ++k) {
-        const double nk = 1.0 + eps10, xk = cen[k];
-        mean[k] = xk / nk;
-        cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(__dmul_rn(xk, xk), nk), __dmul_rn(mean[k], mean[k])), P.reg_covar);
-        weight[k] = nk / (double)n;
-        pchol[k] = 1.0 / sqrt(cov[k]);
-        logw[k] = log(weight[k]);
-    }
-    double lower = -INFINITY;
-    for (int it = 1; it <= P.max_iter; ++it) {
-        const double prev = lower;
-        double nk[NC], sx[NC], sxx[NC], ll = 0.0;
-#pragma unroll
-        for (int k = 0; k < NC; ++k) nk[k] = 0.0, sx[k] = 0.0, sxx[k] = 0.0;
-        for (int j = lane; j < D; j += 32) {
-            const double x = xv[j];
-            double wl[NC];
-#pragma unroll
-            for (int k = 0; k < NC; ++k) wl[k] = gmm_wlp1(x, mean[k], pchol[k], logw[k]);
-            double mx = wl[0];
-#pragma unroll
-            for (int k = 1; k < NC; ++k) mx = fmax(mx, wl[k]);
-            double se = 0.0;
-#pragma unroll
-            for (int k = 0; k < NC; ++k) se += exp(wl[k] - mx);
-            const double lse = mx + log(se);
-            const double c = (double)cv[j];
-            ll += c * lse;
-#pragma unroll
-            for (int k = 0; k < NC; ++k) {
-                const double r = exp(wl[k] - lse) * c;
-                nk[k] += r;
-                sx[k] += r * x;
-                sxx[k] += r * x * x;
-            }
-        }
-        ll = warp_sum(ll);
-#pragma unroll
-        for (int k = 0; k < NC; ++k) nk[k] = warp_sum(nk[k]), sx[k] = warp_sum(sx[k]), sxx[k] = warp_sum(sxx[k]);
-        lower = ll / (double)n;
-        double wsum = 0.0;
-#pragma unroll
-        for (int k = 0; k < NC; ++k) {
-            nk[k] += eps10;
-            mean[k] = sx[k] / nk[k];
-            cov[k] = __dadd_rn(__dsub_rn(__ddiv_rn(sxx[k], nk[k]), __dmul_rn(mean[k], mean[k])), P.reg_covar);
-            weight[k] = nk[k] / (double)n;
-            wsum += weight[k];
-        }
-#pragma unroll
-        for (int k = 0; k < NC; ++k) {
-            weight[k] /= wsum;
-            pchol[k] = 1.0 / sqrt(cov[k] > 0.0 ? cov[k] : P.reg_covar);
-            logw[k] = log(weight[k]);
-        }
-        if (fabs(lower - prev) < P.tol) break;
-    }
-#pragma unroll
-    for (int k = 0; k < NC; ++k) g.mean[k] = mean[k], g.cov[k] = cov[k], g.weight[k] = weight[k];
-    g.n_comp = NC;
-    return lower;
-}
-
-// gmm_fit_k, warp-cooperative: forced seed indices point into x_forced (the caller's value list)
-__device__ void gmm_fit_warp(const double *xv, const int *cv, int D, int n, int nc, const AlleleParams &P, Philox &rng,
-                             const int *forced, const double *x_forced, GmmK &best) {
-    double best_lb = -INFINITY;
-    for (int t = 0; t < P.n_init; ++t) {
-        double cen[ALL_MAX_ALLELES];
-        if (forced) {
-            for (int j = 0; j < nc; ++j) cen[j] = x_forced[forced[t * nc + j]];
-        } else {
-            kmeanspp_warp(xv, cv, D, n, nc, rng, cen);
-        }
-        GmmK g;
-        double lb;
-        switch (nc) {
-        case 2: lb = gmm_em_warp<2>(xv, cv, D, n, cen, P, g); break;
-        case 3: lb = gmm_em_warp<3>(xv, cv, D, n, cen, P, g); break;
-        case 4: lb = gmm_em_warp<4>(xv, cv, D, n, cen, P, g); break;
-        case 5: lb = gmm_em_warp<5>(xv, cv, D, n, cen, P, g); break;
-        case 6: lb = gmm_em_warp<6>(xv, cv, D, n, cen, P, g); break;
-        case 7: lb = gmm_em_warp<7>(xv, cv, D, n, cen, P, g); break;
-        default: lb = gmm_em_warp<8>(xv, cv, D, n, cen, P, g); break;
-        }
-        if (lb > best_lb || best_lb == -INFINITY) best_lb = lb, best = g;
-    }
-}
-
-// One replicate of a deep locus (any A, 1..8): fit_gmm's staged loop and bookkeeping (fit_staged) over the warp
-// fits.  For A <= 2 this is the two-component code's result too: the staged loop at 2 components is fit_replicate
-// (the same k-means++ draws, EM and filter).
-__device__ void fit_replicate_warp(const double *xv, const int *cv, int D, int n, int A, const AlleleParams &P,
-                                   Philox &rng, const int *forced_init, const double *x_forced, double *out_m,
-                                   double *out_w, double *out_s, int *n_peaks) {
-    const int lane = threadIdx.x & 31;
-    fit_staged(
-        D, A, P, rng, forced_init,
-        [&](int nc, const int *forced, GmmK &g) { gmm_fit_warp(xv, cv, D, n, nc, P, rng, forced, x_forced, g); },
-        [&](double &m, double &var) {
-            double s = 0.0;
-            for (int j = lane; j < D; j += 32) s += (double)cv[j] * xv[j];
-            m = warp_sum(s) / (double)n;
-            double q = 0.0;
-            for (int j = lane; j < D; j += 32) {
-                const double d = xv[j] - m;
-                q += (double)cv[j] * d * d;
-            }
-            var = warp_sum(q) / (double)n;
-        },
-        out_m, out_w, out_s, n_peaks);
-}
+// per (locus, replicate) resamples and runs the k-component fit with W = 32 on the replicate's nonzero pairs in
+// shared memory.  Given the seeds, the arithmetic per pair is a shallow locus'; only the order of the sums differs.
 
 // one CTA per deep locus deep_l[d]: its sorted distinct values and resampling CDF at deep_off[d] (ragged, up to
 // ALL_DEEP_MAX_K entries), K, status (1: fewer than min_reads reads, 2: one distinct value, else 0; fewer reads
@@ -1070,11 +969,11 @@ alleles_deep_fit_kernel(const int *__restrict__ deep_l, const long long *__restr
         }
     }
     __syncwarp();
-    const int D = warp_compact(K, [&](int j) { return cv[j]; }, [&](int j) { return (double)v[j]; }, xv, cv);
+    const int D = team_compact<32>(K, [&](int j) { return cv[j]; }, [&](int j) { return (double)v[j]; }, xv, cv);
     rng.seek(0u, 1u);
     double m[ALL_MAX_ALLELES], w[ALL_MAX_ALLELES], s[ALL_MAX_ALLELES];
     int peaks;
-    fit_replicate_warp(xv, cv, D, n, A, P, rng, nullptr, nullptr, m, w, s, &peaks);
+    fit_replicate_k<32>(xv, cv, D, n, A, P, rng, nullptr, nullptr, m, w, s, &peaks);
     if (lane == 0) {
         const size_t ll = (size_t)(l - l0);
         for (int a = 0; a < A; ++a) {
@@ -1101,7 +1000,7 @@ gmm_fit_counts_deep_kernel(const double *__restrict__ xs, const int *__restrict_
     int *cv = (int *)(smem_deep_fit + (size_t)kcap * ALL_DEEP_WARPS) + (size_t)kcap * warp;
     const double *x = xs + (size_t)q * kcap;
     const int *c = cs + (size_t)q * kcap;
-    const int D = warp_compact(Ks[q], [&](int j) { return c[j]; }, [&](int j) { return x[j]; }, xv, cv);
+    const int D = team_compact<32>(Ks[q], [&](int j) { return c[j]; }, [&](int j) { return x[j]; }, xv, cv);
     int n = 0;
     for (int j = lane; j < D; j += 32) n += cv[j];
     n = __reduce_add_sync(0xffffffffu, n);
@@ -1111,7 +1010,7 @@ gmm_fit_counts_deep_kernel(const double *__restrict__ xs, const int *__restrict_
     double m[ALL_MAX_ALLELES], w[ALL_MAX_ALLELES], s[ALL_MAX_ALLELES];
     int peaks = 0;
     const int A = As[q];
-    fit_replicate_warp(xv, cv, D, n, A, P, rng, init ? init + init_off[q] : nullptr, x, m, w, s, &peaks);
+    fit_replicate_k<32>(xv, cv, D, n, A, P, rng, init ? init + init_off[q] : nullptr, x, m, w, s, &peaks);
     if (lane == 0) {
         double *o = out + (size_t)q * (3 * S + 1);
         for (int a = 0; a < S; ++a) {

@@ -1,6 +1,8 @@
 // alleles_api.cuh -- C entry points of the bootstrap / GMM allele caller (included at the end of api.cu, which
 // defines strk_ctx, set_err and CU).  Declarations and the reference lines they replace: include/strkit_b200.h.
 #pragma once
+#include <type_traits>
+
 #include "alleles.cuh"
 
 // per_locus: the allele counts come per locus (validated by the caller) and n_alleles is 0; else n_alleles is the
@@ -42,25 +44,27 @@ static cudaError_t smem_opt_in(Kernel kernel, size_t dyn) {
     return e;
 }
 
-template <int KMAX, int AMAX>
-static void launch_fit(const int *vals, const double *cdf, const int *cnt, const int *K, const int *n, const int *status,
-                       const int *A, int n_loci, int kcap, int S, const AlleleParams &P, double *rm, double *rw,
-                       double *rs, unsigned char *rp, cudaStream_t st) {
-    const long long threads = (long long)n_loci * P.num_bootstrap;
-    alleles_fit_kernel<KMAX, AMAX><<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(vals, cdf, cnt, K, n, status, A,
-                                                                                      n_loci, kcap, S, P, rm, rw, rs, rp);
+// the per-thread kernels keep a replicate's values in arrays of KMAX = 8, 32 or 256 entries, the smallest that holds
+// the largest K: launch(std::integral_constant<int, KMAX>)
+template <class Launch>
+static void with_kmax(int k, Launch launch) {
+    if (k <= 8)
+        launch(std::integral_constant<int, 8>());
+    else if (k <= 32)
+        launch(std::integral_constant<int, 32>());
+    else
+        launch(std::integral_constant<int, 256>());
 }
 
 template <int AMAX>
-static void launch_fit_k(int kmax, const int *vals, const double *cdf, const int *cnt, const int *K, const int *n,
-                         const int *status, const int *A, int n_loci, int kcap, int S, const AlleleParams &P, double *rm,
-                         double *rw, double *rs, unsigned char *rp, cudaStream_t st) {
-    if (kmax <= 8)
-        launch_fit<8, AMAX>(vals, cdf, cnt, K, n, status, A, n_loci, kcap, S, P, rm, rw, rs, rp, st);
-    else if (kmax <= 32)
-        launch_fit<32, AMAX>(vals, cdf, cnt, K, n, status, A, n_loci, kcap, S, P, rm, rw, rs, rp, st);
-    else
-        launch_fit<256, AMAX>(vals, cdf, cnt, K, n, status, A, n_loci, kcap, S, P, rm, rw, rs, rp, st);
+static void launch_fit(int kmax, const int *vals, const double *cdf, const int *cnt, const int *K, const int *n,
+                       const int *status, const int *A, int n_loci, int kcap, int S, const AlleleParams &P, double *rm,
+                       double *rw, double *rs, unsigned char *rp, cudaStream_t st) {
+    const unsigned grid = (unsigned)(((long long)n_loci * P.num_bootstrap + 127) / 128);
+    with_kmax(kmax, [&](auto km) {
+        alleles_fit_kernel<decltype(km)::value, AMAX><<<grid, 128, 0, st>>>(vals, cdf, cnt, K, n, status, A, n_loci, kcap,
+                                                                             S, P, rm, rw, rs, rp);
+    });
 }
 
 // strk_call_alleles (n_alleles = the batch-wide count, A_loc = NULL) and strk_call_alleles_ploidy (A_loc = per-locus
@@ -193,10 +197,10 @@ static int call_alleles_impl(const char *fn, strk_ctx *ctx, const int32_t *cn, c
         Pc.seed = seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(l0 / chunk);  // distinct streams per chunk
         const int *a = d_A ? d_A + l0 : nullptr;
         if (S <= 2)  // the two-component code only
-            launch_fit_k<2>(kmax, v, p, c, d_K + l0, d_n + l0, d_status + l0, a, nl, kcap, S, Pc, rm, rw, rs, rp, st);
+            launch_fit<2>(kmax, v, p, c, d_K + l0, d_n + l0, d_status + l0, a, nl, kcap, S, Pc, rm, rw, rs, rp, st);
         else
-            launch_fit_k<ALL_MAX_ALLELES>(kmax, v, p, c, d_K + l0, d_n + l0, d_status + l0, a, nl, kcap, S, Pc, rm, rw,
-                                          rs, rp, st);
+            launch_fit<ALL_MAX_ALLELES>(kmax, v, p, c, d_K + l0, d_n + l0, d_status + l0, a, nl, kcap, S, Pc, rm, rw, rs,
+                                        rp, st);
         CU(cudaGetLastError());
         const int d0 = (int)(std::lower_bound(deep.begin(), deep.end(), (int)l0) - deep.begin());
         const int d1 = (int)(std::lower_bound(deep.begin(), deep.end(), (int)(l0 + nl)) - deep.begin());
@@ -278,12 +282,10 @@ extern "C" int strk_gmm_fit_counts(strk_ctx *ctx, const double *x, const int32_t
     for (int64_t q = 0; q < n_problems; ++q)
         if (K[q] < 1 || K[q] > kcap) return set_err(STRK_ERR_ARG, "strk_gmm_fit_counts: problem %lld has K = %d", (long long)q, K[q]);
     const unsigned grid = (unsigned)((n_problems + 127) / 128);
-    if (kcap <= 8)
-        gmm_fit_counts_kernel<8><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_init, (int)n_problems, kcap, P, d_out);
-    else if (kcap <= 32)
-        gmm_fit_counts_kernel<32><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_init, (int)n_problems, kcap, P, d_out);
-    else
-        gmm_fit_counts_kernel<256><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_init, (int)n_problems, kcap, P, d_out);
+    with_kmax(kcap, [&](auto km) {
+        gmm_fit_counts_kernel<decltype(km)::value><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_init, (int)n_problems, kcap, P,
+                                                                         d_out);
+    });
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, d_out, (size_t)n_problems * 7 * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -354,15 +356,10 @@ static int gmm_fit_counts_impl(const char *fn, bool deep, strk_ctx *ctx, const d
                                      smem, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap, S, P, d_out);
     } else {
         const unsigned grid = (unsigned)((n_problems + 127) / 128);
-        if (kcap <= 8)
-            gmm_fit_counts_ploidy_kernel<8><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap,
-                                                                  S, P, d_out);
-        else if (kcap <= 32)
-            gmm_fit_counts_ploidy_kernel<32><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems, kcap,
-                                                                   S, P, d_out);
-        else
-            gmm_fit_counts_ploidy_kernel<256><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off, (int)n_problems,
-                                                                    kcap, S, P, d_out);
+        with_kmax(kcap, [&](auto km) {
+            gmm_fit_counts_ploidy_kernel<decltype(km)::value><<<grid, 128, 0, st>>>(d_x, d_c, d_K, d_A, d_init, d_off,
+                                                                                    (int)n_problems, kcap, S, P, d_out);
+        });
     }
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, d_out, (size_t)n_problems * (3 * S + 1) * sizeof(double), cudaMemcpyDeviceToHost, st));
